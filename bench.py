@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SpMV GFLOPS and HBM GB/s for CSR and HLL on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--quick]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--quick] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 N = 1  workload "lap2d_4096_csr" (BASELINE.json configs[1]): fp64 CSR product of the 2-D 5-point
@@ -218,6 +218,23 @@ def ramp_vector(n, device):
     return 1.0 + (torch.arange(n, device=device, dtype=torch.int64) % 7).to(torch.float64) / 8.0
 
 
+DUMP_ROWS = 1 << 21   # 16 MiB of values + 16 MiB of row indices: the whole headline y (134 MB) exceeds a dump's 64 MB
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out_dir, y):
+    """What the caller of the timed product receives, y, at a fixed seeded sample of rows, so that two builds can be
+    compared output for output: DIR/y_sample.npy (float64) and DIR/y_sample_rows.npy (its row indices, float64)."""
+    import torch
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(y.numel(), size=min(DUMP_ROWS, y.numel()), replace=False))
+    values = y[torch.from_numpy(rows).to(y.device)].cpu().numpy()
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "y_sample.npy", values.astype(np.float64))
+    np.save(out / "y_sample_rows.npy", rows.astype(np.float64))
+    log(f"[bench] wrote {len(rows)} sampled rows of y to {out}")
+
+
 # ---------------------------------------------------------------------------------------------------
 # CPU baseline (the reference's own CPU path on the host cores)
 # ---------------------------------------------------------------------------------------------------
@@ -412,6 +429,8 @@ def bench_single_gpu(args):
     head = spmv_stats(nnz, bytes_alg, ms, peak)
     log(f"[bench] {workload}: {head['gflops']:.1f} GFLOP/s, {head['gbs']:.0f} GB/s, {ms*1e3:.1f} us/product "
         f"(min {min(per)*1e3:.1f}, median {statistics.median(per)*1e3:.1f})")
+    if args.dump_outputs:   # before the legs below reuse y
+        dump_outputs(args.dump_outputs, y)
 
     # ---- end to end through the C-ABI host call: pinned host x -> H2D, product, D2H -> pinned host y ----
     xh = torch.empty(M, dtype=torch.float64).pin_memory()
@@ -1034,12 +1053,18 @@ def main():
     ap.add_argument("--no-t1", action="store_true", help="multi-GPU: skip the single-GPU leg of the same workload")
     ap.add_argument("--no-parity", action="store_true", help="multi-GPU: skip the parity check of every exchange mode against the single-GPU iteration")
     ap.add_argument("--modes", default="", help="multi-GPU: comma-separated subset of the exchange modes (fused_mailbox always runs)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="single GPU: after the timed steps, write a fixed seeded sample of the headline product's y as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1 or args.gpus > 1):
+        ap.error("--dump-outputs is implemented for the single-GPU run of this implementation (--gpus 1)")
     capture_stdout()
     if args.impl == "reference":
         return run_reference(args)
-    world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1 or args.gpus > 1:
         if world == 1:
             log("bench.py --gpus N>1 must be launched with torch.distributed.run (one rank per GPU)")

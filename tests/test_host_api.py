@@ -100,17 +100,17 @@ def test_long_rows_with_and_without_duplicates(checker):
         assert np.array_equal(JA, h.JA) and np.array_equal(bits(AS), bits(h.AS)), case
 
 
-def test_sort_row_is_the_reference_quicksort(reference):
+def test_sort_row_is_the_reference_quicksort(checker):
+    """The checker's CSR builder keeps file order inside a row and then runs the reference's quicksort on it, so a
+    one-row matrix yields exactly what sort_row leaves (duplicates make the unstable order observable)."""
+    from oracle import oracle as O
     rng = np.random.default_rng(5)
     for n in (2, 3, 17, 200):
         c = rng.integers(0, 6, n).astype(np.int32)  # many duplicates
         v = rng.standard_normal(n)
         c1, v1 = c.copy(), v.copy()
         host.sort_row(c1, v1, 0, n - 1)
-        c2, v2 = c.copy(), v.copy()
-        reference.lib.sort_row.argtypes = [host.N.c_int_p, host.N.c_dbl_p, host.C.c_size_t, host.C.c_size_t]
-        reference.lib.sort_row.restype = None
-        reference.lib.sort_row(c2.ctypes.data_as(host.N.c_int_p), v2.ctypes.data_as(host.N.c_dbl_p), 0, n - 1)
+        _, c2, v2 = checker.coo_to_csr(O.Coo(1, 6, n, np.zeros(n, np.int32), c.copy(), v.copy()))
         assert np.array_equal(c1, c2) and np.array_equal(bits(v1), bits(v2))
 
 
@@ -202,9 +202,9 @@ def test_parallel_parser_equals_serial_on_fixtures(name, monkeypatch):
 
 @pytest.mark.parametrize("kind,field", [("general", "real"), ("symmetric", "real"), ("general", "pattern"),
                                         ("symmetric", "pattern"), ("general", "integer"), ("skew-symmetric", "real")])
-def test_parallel_parser_on_a_large_file(tmp_path, reference, kind, field):
+def test_parallel_parser_on_a_large_file(tmp_path, checker, kind, field):
     """A 300k-entry file (3-9 MB; the parallel pass is forced, and the default path is checked too) with ragged white space, entries spanning lines and
-    exponents: default (parallel) parse == forced-serial parse == the reference's fscanf parser."""
+    exponents: default (parallel) parse == forced-serial parse == the checker's fscanf parser."""
     rng = np.random.default_rng(len(kind) * 31 + len(field))
     M, N, nz = 5000, 4000 if kind == "general" else 5000, 300_000
     I = rng.integers(1, M + 1, nz)
@@ -234,7 +234,7 @@ def test_parallel_parser_on_a_large_file(tmp_path, reference, kind, field):
         del os.environ["SPMV_B200_PARSER_PARALLEL_MIN_BYTES"]
     assert _same_pre(default, slow)
     assert _same_pre(fast, slow)
-    ref = reference.read_matrix_market(path)
+    ref = checker.read_matrix_market(path)
     assert (ref.M, ref.N, ref.nz) == (fast.M, fast.N, fast.nz)
     assert np.array_equal(ref.I, fast.I) and np.array_equal(ref.J, fast.J)
     assert np.array_equal(np.asarray(ref.val).view(np.uint64), fast.val.view(np.uint64))
@@ -271,15 +271,15 @@ def test_parallel_parser_falls_back_on_irregular_bodies(tmp_path, monkeypatch, c
 
 
 @pytest.mark.parametrize("dup", [False, True])
-def test_large_inputs_take_the_parallel_scatter(reference, dup, monkeypatch):
+def test_large_inputs_take_the_parallel_scatter(checker, dup, monkeypatch):
     """Above 2^20 entries convert_in_csr / convert_to_hll spread the counting scatter over the OpenMP threads (every
-    thread owns a range of rows and scans the whole COO list): same arrays as the reference, bit for bit, for any
+    thread owns a range of rows and scans the whole COO list): same arrays as the checker, bit for bit, for any
     thread count, duplicates included."""
     rng = np.random.default_rng(99 + dup)
     M, N, nz = 70_001, 50_000, 1_300_000
     coo = random_coo(rng, M, N, nz, dup=dup)
-    rp, ci, va = reference.coo_to_csr(coo)
-    h = reference.coo_to_hll(coo)
+    rp, ci, va = checker.coo_to_csr(coo)
+    h = checker.coo_to_hll(coo)
     import ctypes
     gomp = ctypes.CDLL("libgomp.so.1")            # the OpenMP runtime the library is linked against
     before = gomp.omp_get_max_threads()
@@ -296,8 +296,8 @@ def test_large_inputs_take_the_parallel_scatter(reference, dup, monkeypatch):
     gomp.omp_set_num_threads(before)
 
 
-def test_parser_speed_report(tmp_path, reference, capsys):
-    """Not a pass/fail bar (shared CPUs are noisy): prints the time of the reference's fscanf parser and of this repo's
+def test_parser_speed_report(tmp_path, checker, capsys):
+    """Not a pass/fail bar (shared CPUs are noisy): prints the time of the checker's fscanf parser and of this repo's
     read_matrix_market on the same 400k-entry file, and checks they return the same COO.  Larger runs: tools/bench_parser.py."""
     import time
     rng = np.random.default_rng(3)
@@ -311,9 +311,9 @@ def test_parser_speed_report(tmp_path, reference, capsys):
     t0 = time.perf_counter()
     ours = host.read_matrix_market(path)
     t1 = time.perf_counter()
-    ref = reference.read_matrix_market(path)
+    ref = checker.read_matrix_market(path)
     t2 = time.perf_counter()
     assert np.array_equal(ref.I, ours.I) and np.array_equal(ref.J, ours.J)
     assert np.array_equal(np.asarray(ref.val).view(np.uint64), ours.val.view(np.uint64))
     with capsys.disabled():
-        print(f"\n[parser] {nz} entries, {path.stat().st_size / 1e6:.0f} MB: this repo {t1 - t0:.3f} s, reference fscanf loop {t2 - t1:.3f} s")
+        print(f"\n[parser] {nz} entries, {path.stat().st_size / 1e6:.0f} MB: this repo {t1 - t0:.3f} s, {checker.kind} fscanf loop {t2 - t1:.3f} s")

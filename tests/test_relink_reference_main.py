@@ -21,7 +21,11 @@ PKG = ROOT / "sparsematrixvectormultiplication_b200"
 
 @pytest.fixture(scope="module")
 def relinked(tmp_path_factory):
-    if not (REF / "main.c").exists():
+    try:
+        present = (REF / "main.c").is_file()
+    except OSError:                      # a tree this user may not enter counts as absent
+        present = False
+    if not present:
         pytest.skip("reference tree not present")
     N.lib()
     build = tmp_path_factory.mktemp("relink") / "build"
