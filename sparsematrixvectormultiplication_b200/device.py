@@ -33,11 +33,26 @@ def _stream(stream=None):
     return C.c_void_p(s.cuda_stream)
 
 
-def _check_vec(t, n, what):
+def _check_vec(t, n, what, dtype="float64"):
+    """A device vector the kernels may read or write n elements of: a contiguous CUDA tensor of `dtype`."""
     import torch
-    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and t.is_contiguous()
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == getattr(torch, dtype) and t.is_contiguous()
             and t.numel() >= n):
-        raise ValueError(f"{what} must be a contiguous float64 CUDA tensor with at least {n} elements")
+        raise ValueError(f"{what} must be a contiguous {dtype} CUDA tensor with at least {n} elements")
+
+
+def _host_vectors(x, y, n, m, dtype):
+    """x and y of a host round trip: x is converted to `dtype` and must hold n elements; a caller's y is written in place,
+    so it must already be a contiguous numpy array of `dtype` with m elements."""
+    x = np.ascontiguousarray(x, dtype)
+    if x.ndim != 1 or x.size != n:
+        raise ValueError(f"x must be a vector of {n} elements (got shape {x.shape})")
+    if y is None:
+        return x, np.zeros(m, dtype)
+    if not (isinstance(y, np.ndarray) and y.dtype == dtype and y.ndim == 1 and y.size == m and y.flags.c_contiguous
+            and y.flags.writeable):
+        raise ValueError(f"y must be a writable contiguous {np.dtype(dtype).name} numpy vector of {m} elements")
+    return x, y
 
 
 FORMAT_CSR, FORMAT_HLL = 0, 1
@@ -224,15 +239,16 @@ class DeviceCSR:
         return lo.value, hi.value
 
     def spmv_rows(self, row_begin, row_end, x, y, stream=None):
+        i = self.info()
+        _check_vec(x, i.N, "x")
+        _check_vec(y, i.M, "y")
         N.check(N.lib().spmv_b200_csr_spmv_rows(self._h, int(row_begin), int(row_end), _ptr(x), _ptr(y), _stream(stream)))
         return y
 
     def spmv_host(self, x, y=None, accumulate=False, algo=ALGO_AUTO):
         """Host numpy x -> H2D, product, D2H -> host numpy y (synchronous): the end-to-end call."""
         i = self.info()
-        x = np.ascontiguousarray(x, np.float64)
-        if y is None:
-            y = np.zeros(i.M, np.float64)
+        x, y = _host_vectors(x, y, i.N, i.M, np.float64)
         N.check(N.lib().spmv_b200_csr_spmv_host(self._h, _ptr(x), _ptr(y), int(bool(accumulate)), algo))
         return y
 
@@ -251,14 +267,15 @@ class DeviceCSR:
 
     def spmv_f32(self, x, y, accumulate=False, algo=ALGO_AUTO, stream=None):
         """y = A x on float32 CUDA tensors (float values, x, y; products and sums in double)."""
+        i = self.info()
+        _check_vec(x, i.N, "x", "float32")
+        _check_vec(y, i.M, "y", "float32")
         N.check(N.lib().spmv_b200_csr_spmv_f32(self._h, _ptr(x), _ptr(y), int(bool(accumulate)), algo, _stream(stream)))
         return y
 
     def spmv_host_f32(self, x, y=None):
         i = self.info()
-        x = np.ascontiguousarray(x, np.float32)
-        if y is None:
-            y = np.zeros(i.M, np.float32)
+        x, y = _host_vectors(x, y, i.N, i.M, np.float32)
         N.check(N.lib().spmv_b200_csr_spmv_host_f32(self._h, _ptr(x), _ptr(y)))
         return y
 
@@ -343,14 +360,15 @@ class DeviceHLL:
         return row_form_name(FORMAT_HLL, N.lib().spmv_b200_hll_row_form(self._h), "double")
 
     def spmv_f32(self, x, y, stream=None):
+        i = self.info()
+        _check_vec(x, i.N, "x", "float32")
+        _check_vec(y, i.M, "y", "float32")
         N.check(N.lib().spmv_b200_hll_spmv_f32(self._h, _ptr(x), _ptr(y), _stream(stream)))
         return y
 
     def spmv_host_f32(self, x, y=None):
         i = self.info()
-        x = np.ascontiguousarray(x, np.float32)
-        if y is None:
-            y = np.zeros(i.M, np.float32)
+        x, y = _host_vectors(x, y, i.N, i.M, np.float32)
         N.check(N.lib().spmv_b200_hll_spmv_host_f32(self._h, _ptr(x), _ptr(y)))
         return y
 
@@ -387,14 +405,15 @@ class DeviceHLL:
                                                       C.byref(peers) if peers is not None else None, _stream(stream)))
 
     def spmv_hacks(self, hack_begin, hack_end, x, y, stream=None):
+        i = self.info()
+        _check_vec(x, i.N, "x")
+        _check_vec(y, i.M, "y")
         N.check(N.lib().spmv_b200_hll_spmv_hacks(self._h, int(hack_begin), int(hack_end), _ptr(x), _ptr(y), _stream(stream)))
         return y
 
     def spmv_host(self, x, y=None):
         i = self.info()
-        x = np.ascontiguousarray(x, np.float64)
-        if y is None:
-            y = np.zeros(i.M, np.float64)
+        x, y = _host_vectors(x, y, i.N, i.M, np.float64)
         N.check(N.lib().spmv_b200_hll_spmv_host(self._h, _ptr(x), _ptr(y)))
         return y
 
