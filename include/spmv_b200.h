@@ -304,6 +304,28 @@ int spmv_b200_hll_spmv_fused_flat(const spmv_b200_hll *H, const double *d_x, dou
                                   double *d_partials, const spmv_b200_peers_t *peers, void *stream);
 void spmv_b200_hll_free(spmv_b200_hll *H);
 
+/* ---- multi-vector products Y = A X (SpMM), fp64, device arrays (spmv_b200_version() >= 101) ----------------------------
+ * X is N x k and Y is M x k, both row-major with leading dimensions ldx >= k and ldy >= k counted in elements: element
+ * (i, c) is at i*ld + c (64-bit offsets).  One call streams the matrix once for all k columns.  Only rows < M and columns
+ * < k of Y are written; the elements between k and ldy are never touched.  X and Y must not overlap.
+ *   CSR, rows of at most info.long_threshold nonzeros: column c of Y is bit for bit the serial loop csr_matrix_vector_mult
+ *     on column c of X (one lane per (row, column), index order, mul and add rounded separately), i.e. the bits of
+ *     spmv_b200_csr_spmv(..., SPMV_B200_ALGO_ROW) on that column; accumulate != 0 starts each sum from Y's value.
+ *   CSR, longer rows (the plan's long rows, in fragments of 8192 nonzeros): each fragment is summed as 32 fixed
+ *     index-ordered sub-ranges and a fixed tree, the fragments are added in order; no atomics.  Within
+ *     (len + 2) 2^-53 sum_j |a_ij x_jc| of the exact sum, identical bits from call to call, and the bits of a column do not
+ *     depend on k, ldx, ldy or the column's position in X.
+ *   HLL: column c is bit for bit spmv_hll_serial on column c, padding slots (x 0.0) included -- the bits of
+ *     spmv_b200_hll_spmv_rows.  No accumulate flag (as spmv_b200_hll_spmv).
+ * k = 0 and M = 0 are no-ops; with nnz = 0, Y becomes zero (or is left as it is with accumulate).  A negative k, ldx < k,
+ * ldy < k, or a NULL handle or array with k > 0 returns SPMV_B200_ERR_INVALID and launches nothing.  The CSR product
+ * on a matrix with long rows keeps num_fragments x 32 partial sums on the handle (allocated by the first such call, freed
+ * with the plan): as with spmv_b200_csr_spmv, products on one handle must be stream-ordered. */
+int spmv_b200_csr_spmm(const spmv_b200_csr *A, int k, const double *d_X, long long ldx, double *d_Y, long long ldy,
+                       int accumulate, void *stream);
+int spmv_b200_hll_spmm(const spmv_b200_hll *H, int k, const double *d_X, long long ldx, double *d_Y, long long ldy,
+                       void *stream);
+
 /* ---- fp32 storage with fp64 arithmetic (BASELINE.json: y within 1e-5 relative of the serial fp64 product).  The value
  * stream, x and y are float (algorithmic bytes 8 nnz + 4 (M+1) + 4 M + 4 N instead of 12 nnz + ...); every product is
  * formed and summed in double and rounded once on the store.  enable_f32 adds a float copy of the values to the

@@ -167,6 +167,8 @@ SIGNATURES = {
     "spmv_b200_hll_time": (_I, [_V, _V, _V, _I, _I, _I, c_dbl_p, c_dbl_p]),
     "spmv_b200_hll_spmv_hacks": (_I, [_V, _I, _I, _V, _V, _V]),
     "spmv_b200_hll_free": (None, [_V]),
+    "spmv_b200_csr_spmm": (_I, [_V, _I, _V, _LL, _V, _LL, _I, _V]),
+    "spmv_b200_hll_spmm": (_I, [_V, _I, _V, _LL, _V, _LL, _V]),
     "spmv_b200_hll_partials_count": (_I, [_V]),
     "spmv_b200_hll_spmv_fused": (_I, [_V, _V, _V, _V, _V, C.POINTER(Peers), _V]),
     "spmv_b200_hll_spmv_fused_mail": (_I, [_V, _V, _V, _V, C.POINTER(Peers), C.POINTER(Mail), _V]),

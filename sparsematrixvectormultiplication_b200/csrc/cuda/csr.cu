@@ -946,10 +946,12 @@ static void free_plan(spmv_b200_csr *A) {
     cudaFree(A->long_rows);
     cudaFree(A->frag_first);
     cudaFree(A->frag_partial);
+    cudaFree(A->spmm_partial);
     A->tiles = nullptr;
     A->long_rows = nullptr;
     A->frag_first = nullptr;
     A->frag_partial = nullptr;
+    A->spmm_partial = nullptr;
     A->num_tiles = A->num_long = A->num_frag = 0;
 }
 

@@ -219,6 +219,10 @@ struct spmv_b200_csr {
     int *frag_first = nullptr;
     int num_frag = 0;
     double *frag_partial = nullptr;
+    // spmv_b200_csr_spmm: num_frag x 32 partial sums of the long rows for one column tile, allocated by the first product
+    // that needs it and freed with the plan (replan changes num_frag); like frag_partial it makes products on one handle
+    // stream-ordered
+    mutable double *spmm_partial = nullptr;
     spmv::BinPlan bins;
     int max_row = 0;     // longest row (plan time)
     int row_batch = 4;   // csr_row_kernel: column/value/gather batch per thread (tuned at plan time on large matrices)

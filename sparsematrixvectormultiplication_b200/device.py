@@ -55,6 +55,51 @@ def _host_vectors(x, y, n, m, dtype):
     return x, y
 
 
+def _check_dense(t, rows, what):
+    """A row-major block of a multi-vector product: a 2-D float64 CUDA tensor of `rows` rows whose columns are
+    adjacent (column stride 1) and whose row stride, the leading dimension, is at least the column count.  Strides
+    of dimensions of size 1 do not matter, as in torch.  Returns (columns, leading dimension)."""
+    import torch
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and t.dim() == 2):
+        raise ValueError(f"{what} must be a 2-D float64 CUDA tensor")
+    n, k = t.shape
+    if n != rows:
+        raise ValueError(f"{what} must have {rows} rows (got shape {tuple(t.shape)})")
+    if k > 1 and t.stride(1) != 1:
+        raise ValueError(f"{what} must have column stride 1 (got strides {t.stride()})")
+    ld = t.stride(0) if n > 1 else k
+    if ld < k:
+        raise ValueError(f"{what} must have a row stride of at least {k} elements (got {ld})")
+    return k, ld
+
+
+def _dense_overlap(a, lda, b, ldb, k):
+    """Do the row-major k-column blocks a (leading dimension lda) and b (ldb) share an element?  Exact when the
+    leading dimensions are equal (interleaved column slices of one buffer do not overlap), conservative otherwise:
+    then any intersection of the two address ranges counts."""
+    if k == 0 or a.numel() == 0 or b.numel() == 0:
+        return False
+    pa, pb = a.data_ptr(), b.data_ptr()
+    ea = pa + 8 * ((a.shape[0] - 1) * lda + k)
+    eb = pb + 8 * ((b.shape[0] - 1) * ldb + k)
+    if ea <= pb or eb <= pa:
+        return False
+    if lda != ldb or (pb - pa) % 8:
+        return True
+    s = ((pb - pa) // 8) % lda  # b's columns sit at residues [s, s + k) modulo ld, a's at [0, k)
+    return s < k or s + k > lda
+
+
+def _spmm_operands(X, Y, M, N_):
+    k, ldx = _check_dense(X, N_, "X")
+    ky, ldy = _check_dense(Y, M, "Y")
+    if ky != k:
+        raise ValueError(f"X and Y must have the same number of columns (got {k} and {ky})")
+    if _dense_overlap(X, ldx, Y, ldy, k):
+        raise ValueError("Y must not overlap X")
+    return k, ldx, ldy
+
+
 FORMAT_CSR, FORMAT_HLL = 0, 1
 
 
@@ -184,6 +229,17 @@ class DeviceCSR:
         _check_vec(y, i.M, "y")
         N.check(N.lib().spmv_b200_csr_spmv(self._h, _ptr(x), _ptr(y), int(bool(accumulate)), algo, _stream(stream)))
         return y
+
+    def spmm(self, X, Y, accumulate=False, stream=None):
+        """Y = A X (or Y += A X) for X of shape (N, k) and Y of shape (M, k): float64 CUDA tensors, row-major with column
+        stride 1 and row stride >= k, so column slices such as Xbig[:, a:a+k] work.  One pass over the matrix for all
+        k columns (spmv_b200_csr_spmm): each column bit for bit the serial loop on rows up to the long-row threshold.
+        Asynchronous on ``stream``; raises ValueError before any launch on a bad or overlapping operand."""
+        i = self.info()
+        k, ldx, ldy = _spmm_operands(X, Y, i.M, i.N)
+        if k and i.M:
+            N.check(N.lib().spmv_b200_csr_spmm(self._h, k, _ptr(X), ldx, _ptr(Y), ldy, int(bool(accumulate)), _stream(stream)))
+        return Y
 
     def partials_count(self) -> int:
         return N.lib().spmv_b200_csr_partials_count(self._h)
@@ -347,6 +403,15 @@ class DeviceHLL:
               False: N.lib().spmv_b200_hll_spmv_stream, "rows": N.lib().spmv_b200_hll_spmv_rows}[slice_kernel]
         N.check(fn(self._h, _ptr(x), _ptr(y), _stream(stream)))
         return y
+
+    def spmm(self, X, Y, stream=None):
+        """Y = A X for X of shape (N, k) and Y of shape (M, k), as DeviceCSR.spmm (spmv_b200_hll_spmm): each column bit
+        for bit spmv_hll_serial, i.e. spmv(slice_kernel="rows") on that column.  No accumulate flag."""
+        i = self.info()
+        k, ldx, ldy = _spmm_operands(X, Y, i.M, i.N)
+        if k and i.M:
+            N.check(N.lib().spmv_b200_hll_spmm(self._h, k, _ptr(X), ldx, _ptr(Y), ldy, _stream(stream)))
+        return Y
 
     def enable_f32(self, stream=None):
         N.check(N.lib().spmv_b200_hll_enable_f32(self._h, _stream(stream)))
