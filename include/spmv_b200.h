@@ -42,13 +42,15 @@ extern "C" {
 #define SPMV_B200_ERR_NOMEM (-4)
 
 /* CSR kernel selection for spmv_b200_csr_spmv */
-#define SPMV_B200_ALGO_AUTO 0     /* ROW (or STREAM: timed at plan time, same bits) when no row exceeds 12 nonzeros; STREAM for
-                                     <= 12 nnz/row on average; else VECTOR (even rows) or BINNED (skewed rows) */
+#define SPMV_B200_ALGO_AUTO 0     /* ROW, STREAM or ROW_IMAGE (timed at plan time, same bits) when no row exceeds 12 nonzeros;
+                                     STREAM for <= 12 nnz/row on average; else VECTOR (even rows) or BINNED (skewed rows) */
 #define SPMV_B200_ALGO_VECTOR 1   /* plain vector-per-row kernel with shuffle reduction      */
 #define SPMV_B200_ALGO_TILE 2     /* retired (round 2): accepted for compatibility, runs STREAM */
 #define SPMV_B200_ALGO_STREAM 3   /* persistent row-binned kernel, TMA bulk-copy pipeline    */
 #define SPMV_B200_ALGO_BINNED 4   /* rows binned by length: 1..32 lanes per row, longest rows split */
 #define SPMV_B200_ALGO_ROW 5      /* one thread per row, serial order (bit-identical to the reference loop) */
+#define SPMV_B200_ALGO_ROW_IMAGE 6 /* one lane per row on the handle's private column-major image (spmv_b200_csr_set_image);
+                                      the same bits as ROW.  SPMV_B200_ERR_INVALID when the handle holds no image */
 
 /* synthetic CSR generators (BASELINE.json configs 2, 3, 5) */
 #define SPMV_B200_SYNTH_LAP2D 1   /* p0 = n   : 5-point Laplacian on an n x n grid           */
@@ -73,6 +75,8 @@ typedef struct {
     int row_batch;       /* batch of the thread-per-row kernel (tuned at plan time)          */
     int fused_batch;     /* fused iterated product: 0 = fused stream kernel, else batch of the fused row kernel */
     int flat_batch, flat_chunks; /* the FLAT fused row kernel of the two-launch iterated product (plan-time choice) */
+    long long image_bytes; /* device bytes of the private image (12 per slot; 0: none, see spmv_b200_csr_set_image) */
+    int image_form;      /* its kernel: 64 + B hll_rowu_kernel<B,double,true>, B hll_row_kernel<B,double,true>, 0 none */
 } spmv_b200_csr_info_t;
 
 typedef struct {
@@ -137,6 +141,8 @@ int spmv_b200_csr_from_coo_device(int M, int N, long long nz, const int *d_I, co
 int spmv_b200_csr_replan(spmv_b200_csr *A, int tile_items, int long_threshold, int threads_per_row,
                          void *stream);
 int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info);
+/* The arrays of the handle, READ-ONLY: a handle that owns its arrays may hold a private image of them (below), which a
+ * write through these pointers would leave stale. */
 int spmv_b200_csr_device_arrays(const spmv_b200_csr *A, const int **d_row_ptr, const int **d_col_idx,
                                 const double **d_values);
 int spmv_b200_csr_download(const spmv_b200_csr *A, int *row_ptr, int *col_idx, double *values);
@@ -246,12 +252,24 @@ int spmv_b200_csr_spmv_rows(const spmv_b200_csr *A, int row_begin, int row_end, 
  * rank-major layout, part p's entries at [p*stride, p*stride + rows_p), and the column indices of the resident matrix
  * are rewritten once: c in [starts[p], starts[p+1]) -> p*stride + (c - starts[p]) (monotonic, rows stay sorted).  The
  * matrix must own its arrays (upload / synth / from_coo); N becomes nparts*stride (the kernel plan does not depend on
- * column ids and stays). */
+ * column ids and stays; a private image is dropped). */
 int spmv_b200_csr_remap_columns(spmv_b200_csr *A, int nparts, const long long *starts, long long stride, void *stream);
 /* largest contiguous row range around the middle row whose columns all lie in [col_lo, col_hi): the rows a rank can
  * multiply BEFORE the refresh of x has landed (their columns are its own slice), overlapping the collective */
 int spmv_b200_csr_interior_rows(const spmv_b200_csr *A, long long col_lo, long long col_hi, int *row_lo, int *row_hi,
                                 void *stream);
+/* Private image.  A handle that owns its arrays (upload, synth, from_coo[_device]; never wrap_device), whose rows hold at
+ * most 12 nonzeros and that is large enough for plan-time timing, may keep a second copy of the matrix in HLL layout
+ * (hacks of 32 rows, column-major, 12 bytes per slot; padding slots marked in bit 31 of the column and skipped, so the
+ * products are bit for bit SPMV_B200_ALGO_ROW for every x, accumulate included).  Its kernels need no row_ptr load and
+ * find a hack's first slot by arithmetic, which makes them faster on stencils (lap2d 4096^2: DESIGN.md section 3).  The
+ * plan keeps it only when it times faster than every other candidate and its padding adds at most a quarter to nnz;
+ * then AUTO uses it.  Cost: about 12 bytes per nonzero on top of the CSR arrays (+1.007 GB on lap2d 4096^2).
+ * mode 0 drops the image (AUTO falls back to the plan's choice among ROW / STREAM); mode 1 builds it whenever the
+ * matrix is eligible in structure (owned arrays, no row above 12 nonzeros, no long rows), whatever its size or timing,
+ * and returns SPMV_B200_ERR_INVALID otherwise.  replan decides again; remap_columns drops it.  The fp32, SpMM, fused,
+ * row-range and host-buffer products do not use it. */
+int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream);
 void spmv_b200_csr_free(spmv_b200_csr *A);
 
 /* plan-free launch on raw device arrays: drop-in for

@@ -61,7 +61,7 @@ class CsrInfo(C.Structure):  # include/spmv_b200.h spmv_b200_csr_info_t
                 ("num_long_rows", C.c_int), ("num_fragments", C.c_int), ("threads_per_row", C.c_int),
                 ("tile_items", C.c_int), ("long_threshold", C.c_int), ("algorithmic_bytes", C.c_longlong),
                 ("max_row_nnz", C.c_int), ("auto_algo", C.c_int), ("row_batch", C.c_int), ("fused_batch", C.c_int),
-                ("flat_batch", C.c_int), ("flat_chunks", C.c_int)]
+                ("flat_batch", C.c_int), ("flat_chunks", C.c_int), ("image_bytes", C.c_longlong), ("image_form", C.c_int)]
 
 
 class HllInfo(C.Structure):  # include/spmv_b200.h spmv_b200_hll_info_t
@@ -121,6 +121,7 @@ SIGNATURES = {
     "spmv_b200_csr_from_coo": (_I, [_I, _I, _LL, _V, _V, _V, C.POINTER(_V)]),
     "spmv_b200_csr_from_coo_device": (_I, [_I, _I, _LL, _V, _V, _V, _V, C.POINTER(_V)]),
     "spmv_b200_csr_spmv_rows": (_I, [_V, _I, _I, _V, _V, _V]),
+    "spmv_b200_csr_set_image": (_I, [_V, _I, _V]),
     "spmv_b200_csr_partials_count": (_I, [_V]),
     "spmv_b200_csr_remap_columns": (_I, [_V, _I, c_ll_p, _LL, _V]),
     "spmv_b200_csr_interior_rows": (_I, [_V, _LL, _LL, c_int_p, c_int_p, _V]),

@@ -953,6 +953,9 @@ static void free_plan(spmv_b200_csr *A) {
     A->frag_partial = nullptr;
     A->spmm_partial = nullptr;
     A->num_tiles = A->num_long = A->num_frag = 0;
+    spmv_b200_hll_free(A->image);
+    A->image = nullptr;
+    A->image_form = 0;
 }
 
 template <typename V>
@@ -1067,13 +1070,46 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
     if (forced_batch >= 1 && forced_batch <= 8) {
         A->row_batch = forced_batch;
     } else if (A->max_row <= kRowKernelMaxLen && A->nnz >= kAutotuneMinNnz && env_int("SPMV_B200_AUTOTUNE", 1)) {
-        // candidates: row kernel with batch 2..7 and (0) the TMA stream kernel; all give the same bits on such rows
-        const int best = tune_batch(M, A->N, A->row_batch, stream, [&](int batch, double *x, double *y) {
-            if (batch == 0) return stream_launch_csr(A, x, y, 0, nullptr, stream);
-            return launch_rows(0, M, A->row_ptr, A->col_idx, A->values, x, y, batch, 0, stream);
-        }, 0);
-        if (best == 0) A->short_rows_stream = true;
-        else A->row_batch = best;
+        // candidates: (0) the TMA stream kernel, the row kernel with batch 2..7 and, on a matrix that owns its arrays, the
+        // private image (csr_image_build) in each of its forms: 64 + B hll_rowu_kernel, 32 + B hll_row_kernel.  All give
+        // the same bits on such rows.  The image qualifies when its padding adds at most a quarter to nnz and it fits in a
+        // quarter of the free memory; it is freed again unless it wins.
+        if (A->owns && A->num_long == 0) {
+            size_t free_bytes = 0, total_bytes = 0;
+            if (cudaMemGetInfo(&free_bytes, &total_bytes) == cudaSuccess) {
+                const long long fit = ((long long)(free_bytes / 4) - 8LL * ((long long)M / 32 + 2)) / 12;
+                const long long max_slots = std::min(A->nnz + A->nnz / 4, fit);
+                if (max_slots >= 0 && csr_image_build(A, max_slots, stream, &A->image) != SPMV_B200_OK) A->image = nullptr;
+            }
+            cudaGetLastError();
+        }
+        int ids[16], n = 0, fallback = 0;
+        ids[n++] = 0;
+        for (int batch = 2; batch <= 7; ++batch) {
+            if (batch == A->row_batch) fallback = n;
+            ids[n++] = batch;
+        }
+        const int plain = n;
+        for (int batch = 2; A->image && batch <= 7; ++batch)
+            if (A->image->segments.count == 0) ids[n++] = 32 + batch;
+            else if (batch >= 4) ids[n++] = 64 + batch;
+        float ms[16];
+        const int pick = tune_candidates(M, A->N, n, fallback, stream, [&](int i, double *x, double *y) {
+            if (ids[i] == 0) return stream_launch_csr(A, x, y, 0, nullptr, stream);
+            if (ids[i] < 16) return launch_rows(0, M, A->row_ptr, A->col_idx, A->values, x, y, ids[i], 0, stream);
+            return csr_image_launch(A->image, ids[i] >= 64 ? ids[i] : ids[i] - 32, 0, A->image->num_hacks, x, y, 0, stream);
+        }, ms);
+        int best = fallback;  // the plain choice stays for ALGO_ROW and the other entry points even when the image wins
+        for (int i = 0; i < plain; ++i)
+            if (ms[i] >= 0.0f && (ms[best] < 0.0f || ms[i] < ms[best])) best = i;
+        if (ids[best] == 0) A->short_rows_stream = true;
+        else A->row_batch = ids[best];
+        if (pick >= plain) {
+            A->image_form = ids[pick] >= 64 ? ids[pick] : ids[pick] - 32;
+        } else {
+            spmv_b200_hll_free(A->image);
+            A->image = nullptr;
+        }
         // the fused iterated product (scale + |w|^2 partials in the tail): fused stream kernel (0) or fused row kernel
         if (A->num_long == 0) {
             double *partials = nullptr;
@@ -1355,9 +1391,11 @@ CsrPath csr_resolve(const spmv_b200_csr *A, int algo) {
         case SPMV_B200_ALGO_VECTOR: return kPathVector;
         case SPMV_B200_ALGO_BINNED: return kPathBinned;
         case SPMV_B200_ALGO_ROW: return kPathRow;
+        case SPMV_B200_ALGO_ROW_IMAGE: return kPathImage;
         default:
-            // every row short: one thread per row (serial order, so forced_tpr == 1 is honoured as well)
-            if (A->max_row <= kRowKernelMaxLen) return A->short_rows_stream ? kPathStream : kPathRow;
+            // every row short: one thread per row (serial order, so forced_tpr == 1 is honoured as well) -- on the
+            // private image when the handle holds one
+            if (A->max_row <= kRowKernelMaxLen) return A->image ? kPathImage : A->short_rows_stream ? kPathStream : kPathRow;
             if (A->forced_tpr == 1 || A->nnz <= (long long)kAutoStreamMaxAvg * A->M) return kPathStream;
             {   // longer rows: one lane count for all rows (vector kernel) only while the lengths are even; a longest row
                 // far above the mean (or above the long-row threshold) means skew -> lanes per row by length class
@@ -1373,6 +1411,8 @@ int csr_launch_window(const spmv_b200_csr *A, CsrPath path, int unit_begin, int 
     if (path == kPathBinned) return launch_binned<double>(A, A->values, x, y, accumulate, stream);  // whole matrix: rows are permuted
     if (path == kPathRow)
         return launch_rows(unit_begin, unit_end, A->row_ptr, A->col_idx, A->values, x, y, A->row_batch, accumulate, stream);
+    if (path == kPathImage)  // rows, in whole hacks: unit_begin must be a multiple of 32
+        return csr_image_launch(A->image, A->image_form, unit_begin / 32, (unit_end + 31) / 32, x, y, accumulate, stream);
     if (path == kPathVector)
         return launch_vector(unit_begin, unit_end, A->row_ptr, A->col_idx, A->values, x, y, pick_vector_width(A->nnz, A->M),
                              accumulate, stream, (size_t)A->N * sizeof(double), safe_vector_nnz(A));
@@ -1579,8 +1619,12 @@ int spmv_b200_csr_upload(int M, int N, long long nnz, const int *row_ptr, const 
     return SPMV_B200_OK;
 }
 
-int spmv_b200_csr_wrap_device(int M, int N, long long nnz, const int *d_row_ptr, const int *d_col_idx,
-                              const double *d_values, void *stream, spmv_b200_csr **out) {
+}  // extern "C"
+
+// a handle over device arrays; owns: freed with the handle, and eligible for the private image (the caller of
+// wrap_device may rewrite its arrays, which would leave an image stale)
+static int csr_from_device(int M, int N, long long nnz, const int *d_row_ptr, const int *d_col_idx, const double *d_values,
+                           bool owns, void *stream, spmv_b200_csr **out) {
     if (!out) return fail(SPMV_B200_ERR_INVALID, "csr_wrap_device: out is NULL");
     *out = nullptr;
     if (M < 0 || N < 0 || nnz < 0 || nnz > 0x7fffffffLL || !d_row_ptr || (nnz > 0 && (!d_col_idx || !d_values)))
@@ -1598,9 +1642,10 @@ int spmv_b200_csr_wrap_device(int M, int N, long long nnz, const int *d_row_ptr,
     A->row_ptr = const_cast<int *>(d_row_ptr);
     A->col_idx = const_cast<int *>(d_col_idx);
     A->values = const_cast<double *>(d_values);
-    A->owns = false;
+    A->owns = owns;
     int rc = build_plan(A, as_stream(stream));
     if (rc != SPMV_B200_OK) {
+        A->owns = false;  // on failure the arrays stay the caller's
         spmv_b200_csr_free(A);
         return rc;
     }
@@ -1608,12 +1653,17 @@ int spmv_b200_csr_wrap_device(int M, int N, long long nnz, const int *d_row_ptr,
     return SPMV_B200_OK;
 }
 
-// used by synth.cu: adopt freshly generated device arrays
+extern "C" {
+
+int spmv_b200_csr_wrap_device(int M, int N, long long nnz, const int *d_row_ptr, const int *d_col_idx,
+                              const double *d_values, void *stream, spmv_b200_csr **out) {
+    return csr_from_device(M, N, nnz, d_row_ptr, d_col_idx, d_values, false, stream, out);
+}
+
+// used by synth.cu and convert.cu: adopt freshly generated device arrays
 int spmv_b200_csr_adopt_device_(int M, int N, long long nnz, int *d_row_ptr, int *d_col_idx, double *d_values,
                                 void *stream, spmv_b200_csr **out) {
-    int rc = spmv_b200_csr_wrap_device(M, N, nnz, d_row_ptr, d_col_idx, d_values, stream, out);
-    if (rc == SPMV_B200_OK) (*out)->owns = true;
-    return rc;
+    return csr_from_device(M, N, nnz, d_row_ptr, d_col_idx, d_values, true, stream, out);
 }
 
 int spmv_b200_csr_replan(spmv_b200_csr *A, int tile_items, int long_threshold, int threads_per_row, void *stream) {
@@ -1642,6 +1692,7 @@ int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info) {
     info->max_row_nnz = A->max_row;
     switch (csr_resolve(A, SPMV_B200_ALGO_AUTO)) {
         case kPathRow: info->auto_algo = SPMV_B200_ALGO_ROW; break;
+        case kPathImage: info->auto_algo = SPMV_B200_ALGO_ROW_IMAGE; break;
         case kPathStream: info->auto_algo = SPMV_B200_ALGO_STREAM; break;
         case kPathVector: info->auto_algo = SPMV_B200_ALGO_VECTOR; break;
         case kPathBinned: info->auto_algo = SPMV_B200_ALGO_BINNED; break;
@@ -1651,6 +1702,8 @@ int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info) {
     info->fused_batch = A->fused_batch;
     info->flat_batch = A->flat_batch;
     info->flat_chunks = A->flat_chunks;
+    info->image_bytes = A->image ? 12 * A->image->slots : 0;
+    info->image_form = A->image ? A->image_form : 0;
     return SPMV_B200_OK;
 }
 
@@ -1674,9 +1727,10 @@ int spmv_b200_csr_download(const spmv_b200_csr *A, int *row_ptr, int *col_idx, d
 int spmv_b200_csr_spmv(const spmv_b200_csr *A, const double *d_x, double *d_y, int accumulate, int algo, void *stream) {
     if (!A || !d_y || (A->N > 0 && !d_x)) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: NULL argument");
     if (A->M == 0) return SPMV_B200_OK;
-    if (algo < SPMV_B200_ALGO_AUTO || algo > SPMV_B200_ALGO_ROW) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: unknown algo %d", algo);
+    if (algo < SPMV_B200_ALGO_AUTO || algo > SPMV_B200_ALGO_ROW_IMAGE) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: unknown algo %d", algo);
+    if (algo == SPMV_B200_ALGO_ROW_IMAGE && !A->image) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: the matrix holds no image (spmv_b200_csr_set_image)");
     const CsrPath path = csr_resolve(A, algo);
-    const bool by_rows = path == kPathVector || path == kPathRow;
+    const bool by_rows = path == kPathVector || path == kPathRow || path == kPathImage;
     return csr_launch_window(A, path, 0, by_rows ? A->M : A->num_tiles, d_x, d_y, accumulate, as_stream(stream));
 }
 
@@ -1805,8 +1859,30 @@ int spmv_b200_csr_remap_columns(spmv_b200_csr *A, int nparts, const long long *s
         remap_columns_kernel<<<blocks_for(A->nnz, 256), 256, 0, as_stream(stream)>>>(A->nnz, A->col_idx, t);
         SPMV_TRY_CUDA(cudaGetLastError());
     }
-    A->N = (int)(nparts * stride);  // plans, tiles and the fp32 copy of the values do not depend on the column ids
+    A->N = (int)(nparts * stride);  // plans, tiles and the fp32 copy of the values do not depend on the column ids;
+    spmv_b200_hll_free(A->image);   // the private image does
+    A->image = nullptr;
+    A->image_form = 0;
     SPMV_TRY_CUDA(cudaStreamSynchronize(as_stream(stream)));
+    return SPMV_B200_OK;
+}
+
+int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream) {
+    if (!A) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: NULL matrix");
+    if (mode != 0 && mode != 1) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: unknown mode %d", mode);
+    if (mode == 0) {
+        spmv_b200_hll_free(A->image);
+        A->image = nullptr;
+        A->image_form = 0;
+        return SPMV_B200_OK;
+    }
+    if (!A->owns) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: the matrix wraps arrays it does not own");
+    if (A->max_row > kRowKernelMaxLen || A->num_long > 0)
+        return fail(SPMV_B200_ERR_INVALID, "csr_set_image: rows of up to %d nonzeros and no long rows only (longest row: %d)",
+                    kRowKernelMaxLen, A->max_row);
+    if (A->image) return SPMV_B200_OK;
+    SPMV_TRY(csr_image_build(A, -1, as_stream(stream), &A->image));
+    A->image_form = csr_image_default_form(A->image);
     return SPMV_B200_OK;
 }
 

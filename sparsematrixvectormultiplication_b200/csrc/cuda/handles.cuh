@@ -156,8 +156,10 @@ struct HllTile {      // tiles[t] = first hack of tile t and its first slot; til
 
 
 // Times launch(i) for candidates i = 0 .. n-1 on scratch vectors and returns the fastest index (plan time, large matrices)
+// fastest_out (n entries, optional): each candidate's best time in ms, < 0 where it could not be timed
 template <class Launch>
-int tune_candidates(long long M, long long N, int n, int fallback, cudaStream_t stream, Launch launch) {
+int tune_candidates(long long M, long long N, int n, int fallback, cudaStream_t stream, Launch launch,
+                    float *fastest_out = nullptr) {
     // ROUNDS passes over all candidates, REPS launches each, the MINIMUM per candidate decides: a transient slowdown of the
     // GPU (power capping under sustained load shifts timings by 10 % for seconds) then cannot favour whichever candidate
     // happened to run in a quiet moment -- round 2 saw a one-pass tuner pick a 25 % slower kernel at the end of bench.py.
@@ -165,6 +167,7 @@ int tune_candidates(long long M, long long N, int n, int fallback, cudaStream_t 
     double *x = nullptr, *y = nullptr;
     cudaEvent_t a = nullptr, b = nullptr;
     int best = fallback;
+    for (int i = 0; fastest_out && i < n; ++i) fastest_out[i] = -1.0f;
     if (n > 0 && cudaMalloc(&x, (size_t)(N > 0 ? N : 1) * sizeof(double)) == cudaSuccess &&
         cudaMalloc(&y, (size_t)(M > 0 ? M : 1) * sizeof(double)) == cudaSuccess &&
         cudaMemsetAsync(x, 0, (size_t)(N > 0 ? N : 1) * sizeof(double), stream) == cudaSuccess &&
@@ -182,6 +185,7 @@ int tune_candidates(long long M, long long N, int n, int fallback, cudaStream_t 
                 if (ok && (fastest[i] < 0.0f || ms < fastest[i])) fastest[i] = ms;
             }
         }
+        for (int i = 0; fastest_out && ok && i < n; ++i) fastest_out[i] = fastest[i];
         if (ok) {
             float best_ms = -1.0f;
             for (int i = 0; i < n; ++i)
@@ -234,6 +238,11 @@ struct spmv_b200_csr {
     int stages = spmv::kDefaultStages;
     int consumers = 12;
     int stream_grid = 0;
+    // private column-major image of the matrix (csr_image_build, spmv_b200_csr_set_image): HLL layout with the padding
+    // slots marked, multiplied by the masked hll_rowu / hll_row kernels -- bit for bit csr_row_kernel.  Held only when
+    // plan-time timing found it faster (or set_image asked for it); owned arrays only, dropped by remap_columns.
+    spmv_b200_hll *image = nullptr;
+    int image_form = 0;  // 64 + B: hll_rowu_kernel<B, double, true>; B: hll_row_kernel<B, double, true>
     // staging vectors of the *_host entry points
     double *stage_x = nullptr;
     double *stage_y = nullptr;
@@ -291,7 +300,7 @@ int stream_plan_hll(spmv_b200_hll *H, cudaStream_t stream);
 int stream_launch_hll(const spmv_b200_hll *H, const double *x, double *y, cudaStream_t stream, int tile_begin = 0,
                       int tile_count = -1);
 // csr.cu / hll.cu: which kernel the automatic choice resolves to, and launches restricted to a window
-enum CsrPath { kPathStream, kPathTile, kPathVector, kPathBinned, kPathRow };
+enum CsrPath { kPathStream, kPathTile, kPathVector, kPathBinned, kPathRow, kPathImage };
 constexpr int kRowKernelMaxLen = 12;  // AUTO: one thread per row when no row is longer than this (= kSerialRowMax: the
                                       // stream kernel then gives the same bits, so plan-time timing may pick either)
 CsrPath csr_resolve(const spmv_b200_csr *A, int algo);
@@ -302,6 +311,12 @@ HllPath hll_resolve(const spmv_b200_hll *H);
 int hll_launch_window(const spmv_b200_hll *H, HllPath path, int unit_begin, int unit_end, const double *x, double *y,
                       cudaStream_t stream);  // units: tiles (stream kernel) or hacks (slice and row kernels)
 int env_int(const char *name, int fallback);
+// hll.cu: the private image of a CSR handle.  csr_image_build leaves *out NULL when the image would exceed max_slots
+// slots (max_slots < 0: no limit); forms as in spmv_b200_csr::image_form.
+int csr_image_build(const spmv_b200_csr *A, long long max_slots, cudaStream_t stream, spmv_b200_hll **out);
+int csr_image_default_form(const spmv_b200_hll *H);
+int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
+                     int accumulate, cudaStream_t stream);
 int hll_row_forms();                                             // hll.cu: forms of hll_rowm_kernel (spmv_b200_row_forms)
 int hll_row_form(int index, int *hacks, int *batch, int *ctas);  // 0 = ok
 int fused_ctas_per_sm();  // csr.cu: CTAs per SM in the grid of the fused row kernels (CSR and HLL use the same value)

@@ -32,6 +32,7 @@ namespace spmv {
 constexpr int kHack = HACK_SIZE;
 constexpr int kHllThreads = 256;
 constexpr int kHllWarps = kHllThreads / 32;
+constexpr int kPadMark = (int)0x80000000u;  // bit 31 of JA: a padding slot of a CSR handle's private image (masked kernels)
 
 __device__ __forceinline__ void ldg_stream_f64x4(const float *p, double (&v)[4]) {  // fp32 storage: one 128-bit load
     float4 f;
@@ -92,31 +93,39 @@ hll_slice_kernel(int hack_begin, int hack_end, const long long *__restrict__ hac
 // warp one contiguous 128 B (JA) / 256 B (AS) segment -- no shared memory, no reliance on L1 for the stream.  BATCH
 // slots are requested before the first gather.  One lane per row, sequential in j, mul and add rounded separately:
 // bit-identical to the reference's spmv_hll_serial (src/hll_matrix.c:294-306), padding slots (x 0.0) included.
-template <int BATCH, typename V>
+// MASKED: the private image of a CSR handle (csr_image_build), whose padding slots carry bit 31 of the column.  Such a slot
+// gathers x[c & 0x7fffffff] like any other and skips the add; ACCUM: the sum starts from y[row].  Bit-identical to
+// csr_row_kernel for every x.  (Adding the padding's 0 * x[c] would give NaN for an infinite x[c], and +0 turns an
+// untouched -0.0 positive.)  The loads are never predicated on the loaded column.  ACCUM is a template flag, not an
+// argument: a y[row] load hoisted ahead of the step holds two of the 32 registers and pushed two of the 15 loads of
+// hll_rowu_kernel<5> behind the first multiply (cuobjdump, tools/rowm_survey.py).
+template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false>
 __global__ void __launch_bounds__(256, 8)
 hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_off, const int *__restrict__ JA,
                const V *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M) {
     const int hack = hack_begin + blockIdx.x * 8 + (threadIdx.x >> 5);
     if (hack >= hack_end) return;  // warp-uniform
     const int lane = threadIdx.x & 31;
+    const long long row = (long long)hack * kHack + lane;
     const long long off = __ldg(hack_off + hack);
     const int width = (int)((__ldg(hack_off + hack + 1) - off) >> 5);
     const long long base = off + lane;
-    double acc = 0.0;
+    double acc = ACCUM && row < M ? (double)y[row] : 0.0;
     for (int j = 0; j < width; j += BATCH) {
         int c[BATCH];
         double v[BATCH], xv[BATCH];
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) c[u] = j + u < width ? ldg_stream_s32(JA + base + (long long)(j + u) * kHack) : -1;
+        for (int u = 0; u < BATCH; ++u)
+            c[u] = j + u < width ? ldg_stream_s32(JA + base + (long long)(j + u) * kHack) : (MASKED ? kPadMark : -1);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_f64(AS + base + (long long)(j + u) * kHack) : 0.0;
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) xv[u] = c[u] >= 0 ? ldg_x(x, c[u]) : 0.0;
+        for (int u = 0; u < BATCH; ++u)
+            xv[u] = MASKED ? ldg_x(x, c[u] & ~kPadMark) : (c[u] >= 0 ? ldg_x(x, c[u]) : 0.0);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
             if (c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
     }
-    const long long row = (long long)hack * kHack + lane;
     if (row < M) y[row] = (V)acc;
 }
 
@@ -186,7 +195,8 @@ hll_rowm_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack
 // other ways to shorten that trip on images that are NOT regular, tried and removed: the hack_off line of the CTA N CTAs
 // further on prefetched into L2 by one thread per CTA (141-142 us at every N from 148 to 9472: the same 3 %), and the
 // offset array held in the persisting L2 carve-out (194.6 us: the carve-out costs the gathers more than the trip saves).
-template <int BATCH, typename V>
+// MASKED / ACCUM: as in hll_row_kernel -- the private image of a CSR handle, bit for bit csr_row_kernel.
+template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false>
 __global__ void __launch_bounds__(256, 8)
 hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegments seg, const int *__restrict__ JA,
                 const V *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M) {
@@ -203,7 +213,8 @@ hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegment
             base = seg.base[s];
         }
     const long long off = base + (long long)(hack - first) * kHack * width + lane;
-    double acc = 0.0;
+    const long long row = (long long)hack * kHack + lane;
+    double acc = ACCUM && row < M ? (double)y[row] : 0.0;
     if (width == BATCH) {
         // the run's width IS the batch (the form the tuner ends up with on a stencil): straight-line code, no predicates.
         // ncu on the predicated loop alone (profiles/r02e_ncu_f32_summary.md): issue slots 70 % busy, SM throughput 84 %
@@ -215,9 +226,10 @@ hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegment
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) v[u] = ldg_stream_f64(AS + off + (long long)u * kHack);
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, c[u]);
+        for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, MASKED ? c[u] & ~kPadMark : c[u]);
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
+        for (int u = 0; u < BATCH; ++u)
+            if (!MASKED || c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
     } else
     for (int j = 0; j < width; j += BATCH) {
         int c[BATCH];
@@ -227,12 +239,11 @@ hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegment
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_f64(AS + off + (long long)(j + u) * kHack) : 0.0;
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, c[u]);
+        for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, MASKED ? c[u] & ~kPadMark : c[u]);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
-            if (j + u < width) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
+            if (j + u < width && (!MASKED || c[u] >= 0)) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
     }
-    const long long row = (long long)hack * kHack + lane;
     if (row < M) y[row] = (V)acc;
 }
 
@@ -380,7 +391,7 @@ __global__ void hll_width_kernel(int M, int num_hacks, const int *__restrict__ r
 
 __global__ void hll_fill_kernel(int M, int num_hacks, const int *__restrict__ row_ptr, const int *__restrict__ col_idx,
                                 const double *__restrict__ values, const long long *__restrict__ hack_off,
-                                int *__restrict__ JA, double *__restrict__ AS) {
+                                int *__restrict__ JA, double *__restrict__ AS, int mark) {
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= (long long)num_hacks * kHack) return;
     const int hack = (int)(r / kHack), lr = (int)(r % kHack);
@@ -391,7 +402,7 @@ __global__ void hll_fill_kernel(int M, int num_hacks, const int *__restrict__ ro
         begin = row_ptr[r];
         len = row_ptr[r + 1] - begin;
     }
-    int pad_col = 0;  // reference: padding repeats the last real column, 0 for an empty row
+    int pad_col = 0;  // reference: padding repeats the last real column, 0 for an empty row (| kPadMark: masked image)
     for (int j = 0; j < width; ++j) {
         const long long slot = off + (long long)j * kHack + lr;
         if (j < len) {
@@ -399,7 +410,7 @@ __global__ void hll_fill_kernel(int M, int num_hacks, const int *__restrict__ ro
             JA[slot] = pad_col;
             AS[slot] = values[begin + j];
         } else {
-            JA[slot] = pad_col;
+            JA[slot] = pad_col | mark;
             AS[slot] = 0.0;
         }
     }
@@ -651,6 +662,119 @@ static void hll_pick_row_batch(spmv_b200_hll *H, cudaStream_t stream) {
 }
 }  // namespace spmv
 
+// CSR -> column-major image on the device: widths, scan, fill (spmv_b200_hll_from_csr and the private image of a CSR
+// handle).  mark: OR'ed into the column of every padding slot.  max_slots >= 0: an image of more slots is not filled
+// (H->JA stays NULL, H->slots tells its size).
+static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, int mark, long long max_slots, spmv_b200_hll *H) {
+    spmv_b200_csr_info_t ci;
+    const int *row_ptr, *col_idx;
+    const double *values;
+    SPMV_TRY(spmv_b200_csr_info(A, &ci));
+    SPMV_TRY(spmv_b200_csr_device_arrays(A, &row_ptr, &col_idx, &values));
+    H->M = ci.M;
+    H->N = ci.N;
+    const int nb = H->num_hacks = (ci.M + kHack - 1) / kHack;
+    long long *slots = nullptr;
+    int *widths = nullptr, *d_max = nullptr;
+    void *temp = nullptr;
+    auto body = [&]() -> int {
+        SPMV_TRY_CUDA(cudaMalloc(&H->hack_off, ((size_t)nb + 1) * sizeof(long long)));
+        SPMV_TRY_CUDA(cudaMalloc(&slots, ((size_t)nb + 1) * sizeof(long long)));
+        SPMV_TRY_CUDA(cudaMalloc(&widths, (size_t)std::max(nb, 1) * sizeof(int)));
+        SPMV_TRY_CUDA(cudaMalloc(&d_max, sizeof(int)));
+        SPMV_TRY_CUDA(cudaMemsetAsync(d_max, 0, sizeof(int), stream));
+        hll_width_kernel<<<blocks_for(nb + 1, 8), 256, 0, stream>>>(ci.M, nb, row_ptr, slots, widths);
+        SPMV_TRY_CUDA(cudaGetLastError());
+        size_t temp_bytes = 0;
+        SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, slots, H->hack_off, nb + 1, stream));
+        SPMV_TRY_CUDA(cudaMalloc(&temp, temp_bytes ? temp_bytes : 1));
+        SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, slots, H->hack_off, nb + 1, stream));
+        if (nb > 0) {
+            max_int_kernel<<<std::min(blocks_for(nb, 256), 1024u), 256, 0, stream>>>(widths, nb, d_max);
+            SPMV_TRY_CUDA(cudaGetLastError());
+        }
+        H->host_off.resize((size_t)nb + 1);
+        SPMV_TRY_CUDA(cudaMemcpyAsync(H->host_off.data(), H->hack_off, ((size_t)nb + 1) * sizeof(long long),
+                                      cudaMemcpyDeviceToHost, stream));
+        SPMV_TRY_CUDA(cudaMemcpyAsync(&H->max_width, d_max, sizeof(int), cudaMemcpyDeviceToHost, stream));
+        SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
+        H->slots = H->host_off[nb];
+        // reference layout keeps the last block short: its padded rows do not exist there
+        const int last_rows = nb > 0 ? ci.M - (nb - 1) * kHack : 0;
+        H->ref_slots = H->slots;
+        if (nb > 0) H->ref_slots -= ((H->host_off[nb] - H->host_off[nb - 1]) / kHack) * (kHack - last_rows);
+        if (max_slots >= 0 && H->slots > max_slots) return SPMV_B200_OK;
+        SPMV_TRY(hll_alloc_arena(H));
+        if (nb > 0) {
+            hll_fill_kernel<<<blocks_for((long long)nb * kHack, 256), 256, 0, stream>>>(ci.M, nb, row_ptr, col_idx, values,
+                                                                                       H->hack_off, H->JA, H->AS, mark);
+            SPMV_TRY_CUDA(cudaGetLastError());
+        }
+        SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
+        return SPMV_B200_OK;
+    };
+    const int rc = body();
+    cudaFree(slots);
+    cudaFree(widths);
+    cudaFree(d_max);
+    cudaFree(temp);
+    return rc;
+}
+
+namespace spmv {
+int csr_image_build(const spmv_b200_csr *A, long long max_slots, cudaStream_t stream, spmv_b200_hll **out) {
+    *out = nullptr;
+    spmv_b200_hll *H = new (std::nothrow) spmv_b200_hll();
+    if (!H) return fail(SPMV_B200_ERR_NOMEM, "csr image: out of host memory");
+    const int rc = hll_convert(A, stream, kPadMark, max_slots, H);
+    if (rc != SPMV_B200_OK || !H->JA) {
+        spmv_b200_hll_free(H);
+        return rc;
+    }
+    hll_find_segments(H);
+    const long long mean = H->num_hacks > 0 ? (H->slots / 32 + H->num_hacks - 1) / H->num_hacks : 4;
+    H->row_batch = (int)std::max<long long>(2, std::min<long long>(7, mean));
+    *out = H;
+    return SPMV_B200_OK;
+}
+
+int csr_image_default_form(const spmv_b200_hll *H) {
+    return H->segments.count > 0 ? 64 + std::max(3, std::min(7, H->max_width)) : H->row_batch;
+}
+
+template <bool ACCUM>
+static int csr_image_launch_t(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
+                              cudaStream_t stream) {
+    const XPolicy keep = matrix_policy(H->JA, (size_t)H->slots * sizeof(int));
+    const unsigned int g = blocks_for(hack_end - hack_begin, 8);
+    if (form >= 64) {
+        if (H->segments.count <= 0) return fail(SPMV_B200_ERR_INVALID, "csr image: not regular enough for the offset-free form");
+#define IROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, double, true, ACCUM>, g, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, H->AS, x, y, H->M)); break;
+        switch (form - 64) {
+            IROWU_CASE(3) IROWU_CASE(4) IROWU_CASE(6) IROWU_CASE(7)
+            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, double, true, ACCUM>, g, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, H->AS, x, y, H->M)); break;
+        }
+#undef IROWU_CASE
+    } else {
+#define IROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, double, true, ACCUM>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, H->AS, x, y, H->M)); break;
+        switch (form) {
+            IROW_CASE(2) IROW_CASE(3) IROW_CASE(5) IROW_CASE(6) IROW_CASE(7)
+            default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, double, true, ACCUM>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, H->AS, x, y, H->M)); break;
+        }
+#undef IROW_CASE
+    }
+    SPMV_TRY_CUDA(cudaGetLastError());
+    return SPMV_B200_OK;
+}
+
+int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
+                     int accumulate, cudaStream_t stream) {
+    if (hack_end <= hack_begin) return SPMV_B200_OK;
+    return accumulate ? csr_image_launch_t<true>(H, form, hack_begin, hack_end, x, y, stream)
+                      : csr_image_launch_t<false>(H, form, hack_begin, hack_end, x, y, stream);
+}
+}  // namespace spmv
+
 extern "C" {
 
 int spmv_b200_hll_upload(const HLLMatrix *hll, int M, int N, spmv_b200_hll **out) {
@@ -730,65 +854,15 @@ int spmv_b200_hll_from_csr(const spmv_b200_csr *A, void *stream_, spmv_b200_hll 
     *out = nullptr;
     if (!A) return fail(SPMV_B200_ERR_INVALID, "hll_from_csr: NULL matrix");
     cudaStream_t stream = as_stream(stream_);
-    spmv_b200_csr_info_t ci;
-    const int *row_ptr, *col_idx;
-    const double *values;
-    SPMV_TRY(spmv_b200_csr_info(A, &ci));
-    SPMV_TRY(spmv_b200_csr_device_arrays(A, &row_ptr, &col_idx, &values));
     spmv_b200_hll *H = new (std::nothrow) spmv_b200_hll();
     if (!H) return fail(SPMV_B200_ERR_NOMEM, "hll_from_csr: out of host memory");
-    H->M = ci.M;
-    H->N = ci.N;
-    const int nb = H->num_hacks = (ci.M + kHack - 1) / kHack;
-    long long *slots = nullptr;
-    int *widths = nullptr, *d_max = nullptr;
-    void *temp = nullptr;
-    auto body = [&]() -> int {
-        SPMV_TRY_CUDA(cudaMalloc(&H->hack_off, ((size_t)nb + 1) * sizeof(long long)));
-        SPMV_TRY_CUDA(cudaMalloc(&slots, ((size_t)nb + 1) * sizeof(long long)));
-        SPMV_TRY_CUDA(cudaMalloc(&widths, (size_t)std::max(nb, 1) * sizeof(int)));
-        SPMV_TRY_CUDA(cudaMalloc(&d_max, sizeof(int)));
-        SPMV_TRY_CUDA(cudaMemsetAsync(d_max, 0, sizeof(int), stream));
-        hll_width_kernel<<<blocks_for(nb + 1, 8), 256, 0, stream>>>(ci.M, nb, row_ptr, slots, widths);
-        SPMV_TRY_CUDA(cudaGetLastError());
-        size_t temp_bytes = 0;
-        SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, slots, H->hack_off, nb + 1, stream));
-        SPMV_TRY_CUDA(cudaMalloc(&temp, temp_bytes ? temp_bytes : 1));
-        SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, slots, H->hack_off, nb + 1, stream));
-        if (nb > 0) {
-            max_int_kernel<<<std::min(blocks_for(nb, 256), 1024u), 256, 0, stream>>>(widths, nb, d_max);
-            SPMV_TRY_CUDA(cudaGetLastError());
-        }
-        H->host_off.resize((size_t)nb + 1);
-        SPMV_TRY_CUDA(cudaMemcpyAsync(H->host_off.data(), H->hack_off, ((size_t)nb + 1) * sizeof(long long),
-                                      cudaMemcpyDeviceToHost, stream));
-        SPMV_TRY_CUDA(cudaMemcpyAsync(&H->max_width, d_max, sizeof(int), cudaMemcpyDeviceToHost, stream));
-        SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
-        H->slots = H->host_off[nb];
-        // reference layout keeps the last block short: its padded rows do not exist there
-        const int last_rows = nb > 0 ? ci.M - (nb - 1) * kHack : 0;
-        H->ref_slots = H->slots;
-        if (nb > 0) H->ref_slots -= ((H->host_off[nb] - H->host_off[nb - 1]) / kHack) * (kHack - last_rows);
-        SPMV_TRY(hll_alloc_arena(H));
-        if (nb > 0) {
-            hll_fill_kernel<<<blocks_for((long long)nb * kHack, 256), 256, 0, stream>>>(ci.M, nb, row_ptr, col_idx, values,
-                                                                                       H->hack_off, H->JA, H->AS);
-            SPMV_TRY_CUDA(cudaGetLastError());
-        }
-        SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
-        SPMV_TRY(stream_plan_hll(H, stream));
-        hll_pick_row_batch(H, stream);
-        return SPMV_B200_OK;
-    };
-    int rc = body();
-    cudaFree(slots);
-    cudaFree(widths);
-    cudaFree(d_max);
-    cudaFree(temp);
+    int rc = hll_convert(A, stream, 0, -1, H);
+    if (rc == SPMV_B200_OK) rc = stream_plan_hll(H, stream);
     if (rc != SPMV_B200_OK) {
         spmv_b200_hll_free(H);
         return rc;
     }
+    hll_pick_row_batch(H, stream);
     *out = H;
     return SPMV_B200_OK;
 }

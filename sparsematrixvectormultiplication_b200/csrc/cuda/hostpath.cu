@@ -348,12 +348,14 @@ extern "C" {
 
 int spmv_b200_csr_spmv_host(spmv_b200_csr *A, const double *x, double *y, int accumulate, int algo) {
     if (!A || (A->M > 0 && !y) || (A->N > 0 && A->nnz > 0 && !x)) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_host: NULL argument");
-    if (algo < SPMV_B200_ALGO_AUTO || algo > SPMV_B200_ALGO_ROW) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_host: unknown algo %d", algo);
+    if (algo < SPMV_B200_ALGO_AUTO || algo > SPMV_B200_ALGO_ROW_IMAGE) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_host: unknown algo %d", algo);
+    if (algo == SPMV_B200_ALGO_ROW_IMAGE && !A->image) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_host: the matrix holds no image");
     if (A->M == 0) return SPMV_B200_OK;
     if (!A->stage_x) SPMV_TRY_CUDA(cudaMalloc(&A->stage_x, std::max<size_t>(A->N, 1) * sizeof(double)));
     if (!A->stage_y) SPMV_TRY_CUDA(cudaMalloc(&A->stage_y, std::max<size_t>(A->M, 1) * sizeof(double)));
     if (!A->pipe) SPMV_TRY(pipe_create(&A->pipe));
-    const CsrPath path = csr_resolve(A, algo);
+    CsrPath path = csr_resolve(A, algo);
+    if (path == kPathImage) path = kPathRow;  // row windows need not fall on hacks; the row kernel gives the same bits
     if (A->pipe->path != (int)path) SPMV_TRY(csr_plan_windows(A, path));
     HostPipe *p = A->pipe;
     // the binned kernel's long rows are combined by a second kernel that may read y (accumulate); tiles with long rows too

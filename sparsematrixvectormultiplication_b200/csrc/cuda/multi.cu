@@ -469,6 +469,11 @@ int spmv_b200_multi_iterate(spmv_b200_multi *ctx, int iters, int exchange, doubl
     if (exchange == SPMV_B200_EXCHANGE_MAILBOX) {
         for (const Part &p : ctx->parts)
             if (!p.fusable) return fail(SPMV_B200_ERR_INVALID, "multi_iterate: rows above the long-row threshold on GPU %d; use SPMV_B200_EXCHANGE_ALLGATHER", p.dev);
+        for (Part &p : ctx->parts)  // the fused products never read a CSR part's private image
+            if (p.A) {
+                SPMV_TRY(multi_set(p));
+                SPMV_TRY(spmv_b200_csr_set_image(p.A, 0, p.stream));
+            }
     } else if (n > 1 && exchange == SPMV_B200_EXCHANGE_ALLGATHER) {
         SPMV_TRY(multi_nccl(ctx, &api));
     }

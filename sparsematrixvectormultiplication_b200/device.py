@@ -12,8 +12,9 @@ import numpy as np
 
 from . import _native as N
 
-ALGO_AUTO, ALGO_VECTOR, ALGO_TILE, ALGO_STREAM, ALGO_BINNED, ALGO_ROW = 0, 1, 2, 3, 4, 5
-ALGO_NAMES = {0: "auto", 1: "csr_vector_kernel", 2: "csr_stream_kernel (ALGO_TILE is retired)", 3: "csr_stream_kernel", 4: "csr_binned_kernel", 5: "csr_row_kernel"}
+ALGO_AUTO, ALGO_VECTOR, ALGO_TILE, ALGO_STREAM, ALGO_BINNED, ALGO_ROW, ALGO_ROW_IMAGE = 0, 1, 2, 3, 4, 5, 6
+ALGO_NAMES = {0: "auto", 1: "csr_vector_kernel", 2: "csr_stream_kernel (ALGO_TILE is retired)", 3: "csr_stream_kernel", 4: "csr_binned_kernel", 5: "csr_row_kernel",
+              6: "hll_rowu_kernel / hll_row_kernel on the handle's private image (masked padding)"}
 HLL_KERNEL_NAMES = {0: "hll_slice_kernel", 1: "hll_stream_kernel", 2: "hll_row_kernel"}
 SYNTH_LAP2D, SYNTH_LAP3D, SYNTH_UNIFORM = 1, 2, 3
 
@@ -293,6 +294,19 @@ class DeviceCSR:
         lo, hi = C.c_int(), C.c_int()
         N.check(N.lib().spmv_b200_csr_interior_rows(self._h, int(col_lo), int(col_hi), C.byref(lo), C.byref(hi), _stream(stream)))
         return lo.value, hi.value
+
+    def set_image(self, mode, stream=None):
+        """mode 0: drop the private column-major image; mode 1: build it on any matrix eligible in structure (owned arrays,
+        rows of at most 12 nonzeros), whatever its size or timing (spmv_b200_csr_set_image).  Raises SpmvError otherwise."""
+        N.check(N.lib().spmv_b200_csr_set_image(self._h, int(mode), _stream(stream)))
+        return self
+
+    def image_form(self) -> str:
+        """Name of the kernel that multiplies the private image ("none" without one)."""
+        form = self.info().image_form
+        if form >= 64:
+            return f"hll_rowu_kernel<{form - 64},double,true>"
+        return f"hll_row_kernel<{form},double,true>" if form > 0 else "none"
 
     def spmv_rows(self, row_begin, row_end, x, y, stream=None):
         i = self.info()

@@ -212,6 +212,7 @@ class FusedPowerIteration(PowerIteration):
                          hack_aligned=hack_aligned)
         from . import _native as N
         d = self.dev
+        self.A.set_image(0)   # the fused products never read the private image
         if self.A.info().num_long_rows:
             raise ValueError("FusedPowerIteration needs a matrix without long rows")
         self.fmt = fmt
@@ -387,6 +388,7 @@ class AsyncPowerIteration(PowerIteration):
         super().__init__(kind, p0, p1, p2, seed=seed, exchange="halo", group=group, parts=parts, single=single)
         from . import _native as N
         d = self.dev
+        self.A.set_image(0)   # the fused products never read the private image
         cu = self.x.device
         del self.x, self.y
         nbytes = 8 * self.N
@@ -607,7 +609,8 @@ class PeerAllgatherPowerIteration(PowerIteration):
         self.blocks = []
         for b_lo, b_hi in ((lo, hi), (0, lo), (hi, self.rows)):
             if b_hi > b_lo:
-                self.blocks.append((b_lo, d.DeviceCSR.synth(kind, p0, p1, p2, seed=seed, row_begin=rb + b_lo, row_end=rb + b_hi)))
+                self.blocks.append((b_lo, d.DeviceCSR.synth(kind, p0, p1, p2, seed=seed, row_begin=rb + b_lo, row_end=rb + b_hi)
+                                    .set_image(0)))   # only the fused products run on these blocks
         self.has_interior = hi > lo
         counts = [A.flat_partials_count() for _, A in self.blocks]
         self.partials = torch.zeros(max(sum(counts), 1), dtype=torch.float64, device=cu)
