@@ -75,8 +75,12 @@ typedef struct {
     int row_batch;       /* batch of the thread-per-row kernel (tuned at plan time)          */
     int fused_batch;     /* fused iterated product: 0 = fused stream kernel, else batch of the fused row kernel */
     int flat_batch, flat_chunks; /* the FLAT fused row kernel of the two-launch iterated product (plan-time choice) */
-    long long image_bytes; /* device bytes of the private image (12 per slot; 0: none, see spmv_b200_csr_set_image) */
+    long long image_bytes; /* size of the private image at 12 bytes per slot, as defined in version 102, whatever the
+                              width of its column field (0: none, see spmv_b200_csr_set_image); image_device_bytes
+                              is what it occupies */
     int image_form;      /* its kernel: 64 + B hll_rowu_kernel<B,double,true>, B hll_row_kernel<B,double,true>, 0 none */
+    int image_index_bytes; /* bytes of its column field: 2 (col - row; every column within 2^14 of its row), 4, 0 none */
+    long long image_device_bytes; /* device bytes of its columns and values: (8 + image_index_bytes) per slot */
 } spmv_b200_csr_info_t;
 
 typedef struct {
@@ -260,15 +264,19 @@ int spmv_b200_csr_interior_rows(const spmv_b200_csr *A, long long col_lo, long l
                                 void *stream);
 /* Private image.  A handle that owns its arrays (upload, synth, from_coo[_device]; never wrap_device), whose rows hold at
  * most 12 nonzeros and that is large enough for plan-time timing, may keep a second copy of the matrix in HLL layout
- * (hacks of 32 rows, column-major, 12 bytes per slot; padding slots marked in bit 31 of the column and skipped, so the
- * products are bit for bit SPMV_B200_ALGO_ROW for every x, accumulate included).  Its kernels need no row_ptr load and
- * find a hack's first slot by arithmetic, which makes them faster on stencils (lap2d 4096^2: DESIGN.md section 3).  The
- * plan keeps it only when it times faster than every other candidate and its padding adds at most a quarter to nnz;
- * then AUTO uses it.  Cost: about 12 bytes per nonzero on top of the CSR arrays (+1.007 GB on lap2d 4096^2).
+ * (hacks of 32 rows, column-major; padding slots marked and skipped, so the products are bit for bit
+ * SPMV_B200_ALGO_ROW for every x, accumulate included).  When every slot's column lies within 2^14 of its row
+ * (col - row in [-16384, 16383]: banded matrices, 2-D stencils up to a 16383-wide grid) the column field is 2 bytes,
+ * col - row with bit 15 marking padding, and the image takes 10 bytes per slot; otherwise it is the column itself with
+ * bit 31 marking padding, 12 bytes per slot.  The width follows from the matrix (image_index_bytes).  Its kernels need
+ * no row_ptr load and find a hack's first slot by arithmetic, which makes them faster on stencils (lap2d 4096^2:
+ * DESIGN.md section 3).  The plan keeps it only when it times faster than every other candidate and its padding adds at
+ * most a quarter to nnz; then AUTO uses it.  Cost: about 10 or 12 bytes per nonzero on top of the CSR arrays (+839 MB
+ * on lap2d 4096^2, narrow).
  * mode 0 drops the image (AUTO falls back to the plan's choice among ROW / STREAM); mode 1 builds it whenever the
  * matrix is eligible in structure (owned arrays, no row above 12 nonzeros, no long rows), whatever its size or timing,
- * and returns SPMV_B200_ERR_INVALID otherwise.  replan decides again; remap_columns drops it.  The fp32, SpMM, fused,
- * row-range and host-buffer products do not use it. */
+ * narrow when the matrix qualifies, and returns SPMV_B200_ERR_INVALID otherwise.  replan decides again; remap_columns
+ * drops it.  The fp32, SpMM, fused, row-range and host-buffer products do not use it. */
 int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream);
 void spmv_b200_csr_free(spmv_b200_csr *A);
 

@@ -1073,13 +1073,13 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
         // candidates: (0) the TMA stream kernel, the row kernel with batch 2..7 and, on a matrix that owns its arrays, the
         // private image (csr_image_build) in each of its forms: 64 + B hll_rowu_kernel, 32 + B hll_row_kernel.  All give
         // the same bits on such rows.  The image qualifies when its padding adds at most a quarter to nnz and it fits in a
-        // quarter of the free memory; it is freed again unless it wins.
+        // quarter of the free memory (10 or 12 bytes per slot: narrow or wide column field); it is freed again unless it wins.
         if (A->owns && A->num_long == 0) {
             size_t free_bytes = 0, total_bytes = 0;
             if (cudaMemGetInfo(&free_bytes, &total_bytes) == cudaSuccess) {
-                const long long fit = ((long long)(free_bytes / 4) - 8LL * ((long long)M / 32 + 2)) / 12;
-                const long long max_slots = std::min(A->nnz + A->nnz / 4, fit);
-                if (max_slots >= 0 && csr_image_build(A, max_slots, stream, &A->image) != SPMV_B200_OK) A->image = nullptr;
+                const long long fit_bytes = (long long)(free_bytes / 4) - 8LL * ((long long)M / 32 + 2);
+                if (fit_bytes >= 0 && csr_image_build(A, A->nnz + A->nnz / 4, fit_bytes, stream, &A->image) != SPMV_B200_OK)
+                    A->image = nullptr;
             }
             cudaGetLastError();
         }
@@ -1704,6 +1704,8 @@ int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info) {
     info->flat_chunks = A->flat_chunks;
     info->image_bytes = A->image ? 12 * A->image->slots : 0;
     info->image_form = A->image ? A->image_form : 0;
+    info->image_index_bytes = !A->image ? 0 : A->image->JA16 ? 2 : 4;
+    info->image_device_bytes = A->image ? csr_image_bytes(A->image) : 0;
     return SPMV_B200_OK;
 }
 
@@ -1881,7 +1883,7 @@ int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream) {
         return fail(SPMV_B200_ERR_INVALID, "csr_set_image: rows of up to %d nonzeros and no long rows only (longest row: %d)",
                     kRowKernelMaxLen, A->max_row);
     if (A->image) return SPMV_B200_OK;
-    SPMV_TRY(csr_image_build(A, -1, as_stream(stream), &A->image));
+    SPMV_TRY(csr_image_build(A, -1, -1, as_stream(stream), &A->image));
     A->image_form = csr_image_default_form(A->image);
     return SPMV_B200_OK;
 }

@@ -239,10 +239,11 @@ struct spmv_b200_csr {
     int consumers = 12;
     int stream_grid = 0;
     // private column-major image of the matrix (csr_image_build, spmv_b200_csr_set_image): HLL layout with the padding
-    // slots marked, multiplied by the masked hll_rowu / hll_row kernels -- bit for bit csr_row_kernel.  Held only when
-    // plan-time timing found it faster (or set_image asked for it); owned arrays only, dropped by remap_columns.
+    // slots marked, multiplied by the masked hll_rowu / hll_row kernels -- bit for bit csr_row_kernel.  Narrow (JA16, 10
+    // bytes per slot) when every slot's column lies within 2^14 of its row, else wide (JA, 12 bytes per slot).  Held only
+    // when plan-time timing found it faster (or set_image asked for it); owned arrays only, dropped by remap_columns.
     spmv_b200_hll *image = nullptr;
-    int image_form = 0;  // 64 + B: hll_rowu_kernel<B, double, true>; B: hll_row_kernel<B, double, true>
+    int image_form = 0;  // 64 + B: hll_rowu_kernel<B, double, true>; B: hll_row_kernel<B, double, true> (index type: JA16 / JA)
     // staging vectors of the *_host entry points
     double *stage_x = nullptr;
     double *stage_y = nullptr;
@@ -268,6 +269,8 @@ struct spmv_b200_hll {
     long long slots = 0, ref_slots = 0;
     long long *hack_off = nullptr;  // device [num_hacks+1]
     int *JA = nullptr;              // device [slots]
+    uint16_t *JA16 = nullptr;       // device [slots]: the narrow column field of a CSR handle's private image (JA is then
+                                    // NULL): bits 0-14 hold col - row as a 15-bit two's complement, bit 15 marks padding
     double *AS = nullptr;           // device [slots]
     float *AS32 = nullptr;          // fp32 copy of AS (spmv_b200_hll_enable_f32)
     std::vector<long long> host_off;
@@ -312,8 +315,10 @@ int hll_launch_window(const spmv_b200_hll *H, HllPath path, int unit_begin, int 
                       cudaStream_t stream);  // units: tiles (stream kernel) or hacks (slice and row kernels)
 int env_int(const char *name, int fallback);
 // hll.cu: the private image of a CSR handle.  csr_image_build leaves *out NULL when the image would exceed max_slots
-// slots (max_slots < 0: no limit); forms as in spmv_b200_csr::image_form.
-int csr_image_build(const spmv_b200_csr *A, long long max_slots, cudaStream_t stream, spmv_b200_hll **out);
+// slots or its column and value arrays max_bytes bytes (< 0: no limit); forms as in spmv_b200_csr::image_form.
+int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_bytes, cudaStream_t stream,
+                    spmv_b200_hll **out);
+long long csr_image_bytes(const spmv_b200_hll *H);  // device bytes of JA / JA16 and AS: 10 or 12 per slot
 int csr_image_default_form(const spmv_b200_hll *H);
 int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
                      int accumulate, cudaStream_t stream);

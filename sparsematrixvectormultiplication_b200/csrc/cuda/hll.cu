@@ -33,6 +33,33 @@ constexpr int kHack = HACK_SIZE;
 constexpr int kHllThreads = 256;
 constexpr int kHllWarps = kHllThreads / 32;
 constexpr int kPadMark = (int)0x80000000u;  // bit 31 of JA: a padding slot of a CSR handle's private image (masked kernels)
+constexpr int kPadMark16 = 0x8000;          // bit 15 of JA16: the same in the narrow image
+constexpr int kDeltaMin = -16384, kDeltaMax = 16383;  // col - row of every slot of a narrow image (15-bit two's complement)
+
+// The column field of a slot of a CSR handle's private image: the column a slot gathers, whether it adds, and the field of
+// a slot past the width of its hack (gathers an in-range column, never adds).  int: the column, kPadMark on padding.
+// uint16_t (JA16): bits 0-14 hold col - row, kPadMark16 on padding; a padding slot carries the delta of an in-range column
+// too, so no gather is predicated on the loaded field.  first: the field of the first slot of the same batch.
+__device__ __forceinline__ int ldg_stream_index(const int *p) { return ldg_stream_s32(p); }
+__device__ __forceinline__ int ldg_stream_index(const uint16_t *p) { return ldg_stream_u16(p); }
+
+template <typename I>
+__device__ __forceinline__ int image_column(int c, unsigned row) {
+    if constexpr (sizeof(I) == 2) return (int)(row + (unsigned)((int)((unsigned)c << 17) >> 17));  // modulo 2^32: exact
+    else return c & ~kPadMark;
+}
+
+template <typename I>
+__device__ __forceinline__ bool image_adds(int c) {
+    if constexpr (sizeof(I) == 2) return (c & kPadMark16) == 0;
+    else return c >= 0;
+}
+
+template <typename I>
+__device__ __forceinline__ int image_past_width(int first) {
+    if constexpr (sizeof(I) == 2) return first | kPadMark16;
+    else return kPadMark;
+}
 
 __device__ __forceinline__ void ldg_stream_f64x4(const float *p, double (&v)[4]) {  // fp32 storage: one 128-bit load
     float4 f;
@@ -93,16 +120,18 @@ hll_slice_kernel(int hack_begin, int hack_end, const long long *__restrict__ hac
 // warp one contiguous 128 B (JA) / 256 B (AS) segment -- no shared memory, no reliance on L1 for the stream.  BATCH
 // slots are requested before the first gather.  One lane per row, sequential in j, mul and add rounded separately:
 // bit-identical to the reference's spmv_hll_serial (src/hll_matrix.c:294-306), padding slots (x 0.0) included.
-// MASKED: the private image of a CSR handle (csr_image_build), whose padding slots carry bit 31 of the column.  Such a slot
-// gathers x[c & 0x7fffffff] like any other and skips the add; ACCUM: the sum starts from y[row].  Bit-identical to
-// csr_row_kernel for every x.  (Adding the padding's 0 * x[c] would give NaN for an infinite x[c], and +0 turns an
-// untouched -0.0 positive.)  The loads are never predicated on the loaded column.  ACCUM is a template flag, not an
-// argument: a y[row] load hoisted ahead of the step holds two of the 32 registers and pushed two of the 15 loads of
-// hll_rowu_kernel<5> behind the first multiply (cuobjdump, tools/rowm_survey.py).
-template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false>
+// MASKED: the private image of a CSR handle (csr_image_build), whose padding slots carry bit 31 of the column (I = int) or
+// bit 15 of a row-relative 16-bit field (I = uint16_t, image_column).  Such a slot gathers its column like any other and
+// skips the add; ACCUM: the sum starts from y[row].  Bit-identical to csr_row_kernel for every x.  (Adding the padding's
+// 0 * x[c] would give NaN for an infinite x[c], and +0 turns an untouched -0.0 positive.)  The loads are never predicated
+// on the loaded column.  ACCUM is a template flag, not an argument: a y[row] load hoisted ahead of the step holds two of
+// the 32 registers and pushed two of the 15 loads of hll_rowu_kernel<5> behind the first multiply (cuobjdump,
+// tools/rowm_survey.py).
+template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false, typename I = int>
 __global__ void __launch_bounds__(256, 8)
-hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_off, const int *__restrict__ JA,
+hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_off, const I *__restrict__ JA,
                const V *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M) {
+    static_assert(sizeof(I) == 4 || (MASKED && sizeof(V) == 8), "the narrow index exists in the fp64 private image only");
     const int hack = hack_begin + blockIdx.x * 8 + (threadIdx.x >> 5);
     if (hack >= hack_end) return;  // warp-uniform
     const int lane = threadIdx.x & 31;
@@ -115,16 +144,16 @@ hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_
         int c[BATCH];
         double v[BATCH], xv[BATCH];
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u)
-            c[u] = j + u < width ? ldg_stream_s32(JA + base + (long long)(j + u) * kHack) : (MASKED ? kPadMark : -1);
+        for (int u = 0; u < BATCH; ++u)  // u = 0 is always within the width
+            c[u] = j + u < width ? ldg_stream_index(JA + base + (long long)(j + u) * kHack) : (MASKED ? image_past_width<I>(u ? c[0] : 0) : -1);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_f64(AS + base + (long long)(j + u) * kHack) : 0.0;
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
-            xv[u] = MASKED ? ldg_x(x, c[u] & ~kPadMark) : (c[u] >= 0 ? ldg_x(x, c[u]) : 0.0);
+            xv[u] = MASKED ? ldg_x(x, image_column<I>(c[u], (unsigned)row)) : (c[u] >= 0 ? ldg_x(x, c[u]) : 0.0);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
-            if (c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
+            if (MASKED ? image_adds<I>(c[u]) : c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
     }
     if (row < M) y[row] = (V)acc;
 }
@@ -195,11 +224,12 @@ hll_rowm_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack
 // other ways to shorten that trip on images that are NOT regular, tried and removed: the hack_off line of the CTA N CTAs
 // further on prefetched into L2 by one thread per CTA (141-142 us at every N from 148 to 9472: the same 3 %), and the
 // offset array held in the persisting L2 carve-out (194.6 us: the carve-out costs the gathers more than the trip saves).
-// MASKED / ACCUM: as in hll_row_kernel -- the private image of a CSR handle, bit for bit csr_row_kernel.
-template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false>
+// MASKED / ACCUM / I: as in hll_row_kernel -- the private image of a CSR handle, bit for bit csr_row_kernel.
+template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false, typename I = int>
 __global__ void __launch_bounds__(256, 8)
-hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegments seg, const int *__restrict__ JA,
+hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegments seg, const I *__restrict__ JA,
                 const V *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M) {
+    static_assert(sizeof(I) == 4 || (MASKED && sizeof(V) == 8), "the narrow index exists in the fp64 private image only");
     const int hack = hack_begin + blockIdx.x * 8 + (threadIdx.x >> 5);
     if (hack >= hack_end) return;  // warp-uniform
     const int lane = threadIdx.x & 31;
@@ -214,7 +244,7 @@ hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegment
         }
     const long long off = base + (long long)(hack - first) * kHack * width + lane;
     const long long row = (long long)hack * kHack + lane;
-    double acc = ACCUM && row < M ? (double)y[row] : 0.0;
+    double acc = ACCUM && row < M && width != BATCH ? (double)y[row] : 0.0;
     if (width == BATCH) {
         // the run's width IS the batch (the form the tuner ends up with on a stencil): straight-line code, no predicates.
         // ncu on the predicated loop alone (profiles/r02e_ncu_f32_summary.md): issue slots 70 % busy, SM throughput 84 %
@@ -222,27 +252,29 @@ hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegment
         int c[BATCH];
         double v[BATCH], xv[BATCH];
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) c[u] = ldg_stream_s32(JA + off + (long long)u * kHack);
+        for (int u = 0; u < BATCH; ++u) c[u] = ldg_stream_index(JA + off + (long long)u * kHack);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) v[u] = ldg_stream_f64(AS + off + (long long)u * kHack);
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, MASKED ? c[u] & ~kPadMark : c[u]);
+        for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, MASKED ? image_column<I>(c[u], (unsigned)row) : c[u]);
+        if (ACCUM && row < M) acc = y[row];  // after the step's loads: held from the start, it pushed the narrow form to spill
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
-            if (!MASKED || c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
+            if (!MASKED || image_adds<I>(c[u])) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
     } else
     for (int j = 0; j < width; j += BATCH) {
         int c[BATCH];
         double v[BATCH], xv[BATCH];
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) c[u] = j + u < width ? ldg_stream_s32(JA + off + (long long)(j + u) * kHack) : 0;
+        for (int u = 0; u < BATCH; ++u)  // u = 0 is always within the width
+            c[u] = j + u < width ? ldg_stream_index(JA + off + (long long)(j + u) * kHack) : (MASKED ? image_past_width<I>(u ? c[0] : 0) : 0);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_f64(AS + off + (long long)(j + u) * kHack) : 0.0;
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, MASKED ? c[u] & ~kPadMark : c[u]);
+        for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, MASKED ? image_column<I>(c[u], (unsigned)row) : c[u]);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
-            if (j + u < width && (!MASKED || c[u] >= 0)) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
+            if (j + u < width && (!MASKED || image_adds<I>(c[u]))) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
     }
     if (row < M) y[row] = (V)acc;
 }
@@ -389,9 +421,18 @@ __global__ void hll_width_kernel(int M, int num_hacks, const int *__restrict__ r
     }
 }
 
-__global__ void hll_fill_kernel(int M, int num_hacks, const int *__restrict__ row_ptr, const int *__restrict__ col_idx,
+// the column field of a slot (mark: OR'ed into a padding slot's column of the wide image; the narrow one is always masked)
+__device__ __forceinline__ void put_index(int *JA, long long slot, int col, long long, bool pad, int mark) {
+    JA[slot] = pad ? col | mark : col;
+}
+__device__ __forceinline__ void put_index(uint16_t *JA, long long slot, int col, long long row, bool pad, int) {
+    JA[slot] = (uint16_t)(((unsigned long long)(col - row) & 0x7fffu) | (pad ? kPadMark16 : 0));
+}
+
+template <typename I>
+__global__ void hll_fill_kernel(int M, int N, int num_hacks, const int *__restrict__ row_ptr, const int *__restrict__ col_idx,
                                 const double *__restrict__ values, const long long *__restrict__ hack_off,
-                                int *__restrict__ JA, double *__restrict__ AS, int mark) {
+                                I *__restrict__ JA, double *__restrict__ AS, int mark) {
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= (long long)num_hacks * kHack) return;
     const int hack = (int)(r / kHack), lr = (int)(r % kHack);
@@ -402,18 +443,41 @@ __global__ void hll_fill_kernel(int M, int num_hacks, const int *__restrict__ ro
         begin = row_ptr[r];
         len = row_ptr[r + 1] - begin;
     }
-    int pad_col = 0;  // reference: padding repeats the last real column, 0 for an empty row (| kPadMark: masked image)
+    // reference: padding repeats the last real column, 0 for an empty row.  The narrow image stores col - row, so an
+    // empty row (or a row past M) gathers the in-range column nearest to it instead (hll_narrow_check_kernel)
+    int pad_col = sizeof(I) == 2 ? (int)min(r, (long long)N - 1) : 0;
     for (int j = 0; j < width; ++j) {
         const long long slot = off + (long long)j * kHack + lr;
         if (j < len) {
             pad_col = col_idx[begin + j];
-            JA[slot] = pad_col;
+            put_index(JA, slot, pad_col, r, false, mark);
             AS[slot] = values[begin + j];
         } else {
-            JA[slot] = pad_col | mark;
+            put_index(JA, slot, pad_col, r, true, mark);
             AS[slot] = 0.0;
         }
     }
+}
+
+// Does every slot of the image fit the narrow field (col - row in [kDeltaMin, kDeltaMax])?  One thread per row of the
+// padded image, after hll_width_kernel: a real slot holds col - row, a padding slot repeats the delta of its row's last
+// real column or, in a row without one that still has slots, gathers min(row, N - 1) (hll_fill_kernel).  Clears *fits.
+__global__ void hll_narrow_check_kernel(int M, int N, int num_hacks, const int *__restrict__ row_ptr,
+                                        const int *__restrict__ col_idx, const int *__restrict__ widths, int *__restrict__ fits) {
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= (long long)num_hacks * kHack) return;
+    int begin = 0, end = 0;
+    if (r < M) {
+        begin = row_ptr[r];
+        end = row_ptr[r + 1];
+    }
+    bool ok = true;
+    for (int k = begin; k < end; ++k) {
+        const long long d = col_idx[k] - r;
+        ok = ok && d >= kDeltaMin && d <= kDeltaMax;
+    }
+    if (begin == end && widths[r / kHack] > 0) ok = r - (N - 1) <= -kDeltaMin;
+    if (!ok) *fits = 0;
 }
 
 __global__ void max_int_kernel(const int *__restrict__ v, int n, int *__restrict__ out) {
@@ -548,9 +612,10 @@ static int hll_launch(const spmv_b200_hll *H, int hack_begin, int hack_end, cons
     return SPMV_B200_OK;
 }
 
-static int hll_alloc_arena(spmv_b200_hll *H) {
+static int hll_alloc_arena(spmv_b200_hll *H, bool narrow = false) {
     const size_t n = (size_t)std::max<long long>(H->slots, 32);
-    SPMV_TRY_CUDA(cudaMalloc(&H->JA, n * sizeof(int)));
+    if (narrow) SPMV_TRY_CUDA(cudaMalloc(&H->JA16, n * sizeof(uint16_t)));
+    else SPMV_TRY_CUDA(cudaMalloc(&H->JA, n * sizeof(int)));
     SPMV_TRY_CUDA(cudaMalloc(&H->AS, n * sizeof(double)));
     return SPMV_B200_OK;
 }
@@ -663,9 +728,11 @@ static void hll_pick_row_batch(spmv_b200_hll *H, cudaStream_t stream) {
 }  // namespace spmv
 
 // CSR -> column-major image on the device: widths, scan, fill (spmv_b200_hll_from_csr and the private image of a CSR
-// handle).  mark: OR'ed into the column of every padding slot.  max_slots >= 0: an image of more slots is not filled
-// (H->JA stays NULL, H->slots tells its size).
-static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, int mark, long long max_slots, spmv_b200_hll *H) {
+// handle).  image: the private image -- padding slots marked, and narrow (JA16) when every slot fits it.  max_slots /
+// max_bytes >= 0: an image of more slots or more bytes of JA and AS is not filled (H->JA and H->JA16 stay NULL, H->slots
+// tells its size).
+static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, bool image, long long max_slots, long long max_bytes,
+                       spmv_b200_hll *H) {
     spmv_b200_csr_info_t ci;
     const int *row_ptr, *col_idx;
     const double *values;
@@ -675,16 +742,23 @@ static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, int mark, lo
     H->N = ci.N;
     const int nb = H->num_hacks = (ci.M + kHack - 1) / kHack;
     long long *slots = nullptr;
-    int *widths = nullptr, *d_max = nullptr;
+    int *widths = nullptr, *d_max = nullptr;  // d_max[0]: widest hack; d_max[1]: every slot fits the narrow field
     void *temp = nullptr;
+    int fits = 0;
     auto body = [&]() -> int {
         SPMV_TRY_CUDA(cudaMalloc(&H->hack_off, ((size_t)nb + 1) * sizeof(long long)));
         SPMV_TRY_CUDA(cudaMalloc(&slots, ((size_t)nb + 1) * sizeof(long long)));
         SPMV_TRY_CUDA(cudaMalloc(&widths, (size_t)std::max(nb, 1) * sizeof(int)));
-        SPMV_TRY_CUDA(cudaMalloc(&d_max, sizeof(int)));
-        SPMV_TRY_CUDA(cudaMemsetAsync(d_max, 0, sizeof(int), stream));
+        SPMV_TRY_CUDA(cudaMalloc(&d_max, 2 * sizeof(int)));
+        const int init[2] = {0, image ? 1 : 0};
+        SPMV_TRY_CUDA(cudaMemcpyAsync(d_max, init, sizeof init, cudaMemcpyHostToDevice, stream));
         hll_width_kernel<<<blocks_for(nb + 1, 8), 256, 0, stream>>>(ci.M, nb, row_ptr, slots, widths);
         SPMV_TRY_CUDA(cudaGetLastError());
+        if (image && nb > 0) {
+            hll_narrow_check_kernel<<<blocks_for((long long)nb * kHack, 256), 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx,
+                                                                                            widths, d_max + 1);
+            SPMV_TRY_CUDA(cudaGetLastError());
+        }
         size_t temp_bytes = 0;
         SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, slots, H->hack_off, nb + 1, stream));
         SPMV_TRY_CUDA(cudaMalloc(&temp, temp_bytes ? temp_bytes : 1));
@@ -697,6 +771,7 @@ static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, int mark, lo
         SPMV_TRY_CUDA(cudaMemcpyAsync(H->host_off.data(), H->hack_off, ((size_t)nb + 1) * sizeof(long long),
                                       cudaMemcpyDeviceToHost, stream));
         SPMV_TRY_CUDA(cudaMemcpyAsync(&H->max_width, d_max, sizeof(int), cudaMemcpyDeviceToHost, stream));
+        SPMV_TRY_CUDA(cudaMemcpyAsync(&fits, d_max + 1, sizeof(int), cudaMemcpyDeviceToHost, stream));
         SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
         H->slots = H->host_off[nb];
         // reference layout keeps the last block short: its padded rows do not exist there
@@ -704,10 +779,15 @@ static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, int mark, lo
         H->ref_slots = H->slots;
         if (nb > 0) H->ref_slots -= ((H->host_off[nb] - H->host_off[nb - 1]) / kHack) * (kHack - last_rows);
         if (max_slots >= 0 && H->slots > max_slots) return SPMV_B200_OK;
-        SPMV_TRY(hll_alloc_arena(H));
+        if (max_bytes >= 0 && H->slots * (fits ? 10 : 12) > max_bytes) return SPMV_B200_OK;
+        SPMV_TRY(hll_alloc_arena(H, fits != 0));
         if (nb > 0) {
-            hll_fill_kernel<<<blocks_for((long long)nb * kHack, 256), 256, 0, stream>>>(ci.M, nb, row_ptr, col_idx, values,
-                                                                                       H->hack_off, H->JA, H->AS, mark);
+            const unsigned int g = blocks_for((long long)nb * kHack, 256);
+            const int mark = image ? kPadMark : 0;
+            if (fits)
+                hll_fill_kernel<<<g, 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx, values, H->hack_off, H->JA16, H->AS, mark);
+            else
+                hll_fill_kernel<<<g, 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx, values, H->hack_off, H->JA, H->AS, mark);
             SPMV_TRY_CUDA(cudaGetLastError());
         }
         SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
@@ -722,12 +802,13 @@ static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, int mark, lo
 }
 
 namespace spmv {
-int csr_image_build(const spmv_b200_csr *A, long long max_slots, cudaStream_t stream, spmv_b200_hll **out) {
+int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_bytes, cudaStream_t stream,
+                    spmv_b200_hll **out) {
     *out = nullptr;
     spmv_b200_hll *H = new (std::nothrow) spmv_b200_hll();
     if (!H) return fail(SPMV_B200_ERR_NOMEM, "csr image: out of host memory");
-    const int rc = hll_convert(A, stream, kPadMark, max_slots, H);
-    if (rc != SPMV_B200_OK || !H->JA) {
+    const int rc = hll_convert(A, stream, true, max_slots, max_bytes, H);
+    if (rc != SPMV_B200_OK || (!H->JA && !H->JA16)) {
         spmv_b200_hll_free(H);
         return rc;
     }
@@ -738,28 +819,30 @@ int csr_image_build(const spmv_b200_csr *A, long long max_slots, cudaStream_t st
     return SPMV_B200_OK;
 }
 
+long long csr_image_bytes(const spmv_b200_hll *H) { return H->slots * (H->JA16 ? 10 : 12); }
+
 int csr_image_default_form(const spmv_b200_hll *H) {
     return H->segments.count > 0 ? 64 + std::max(3, std::min(7, H->max_width)) : H->row_batch;
 }
 
-template <bool ACCUM>
-static int csr_image_launch_t(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
-                              cudaStream_t stream) {
-    const XPolicy keep = matrix_policy(H->JA, (size_t)H->slots * sizeof(int));
+template <bool ACCUM, typename I>
+static int csr_image_launch_t(const spmv_b200_hll *H, const I *JA, int form, int hack_begin, int hack_end, const double *x,
+                              double *y, cudaStream_t stream) {
+    const XPolicy keep = matrix_policy(JA, (size_t)H->slots * sizeof(I));
     const unsigned int g = blocks_for(hack_end - hack_begin, 8);
     if (form >= 64) {
         if (H->segments.count <= 0) return fail(SPMV_B200_ERR_INVALID, "csr image: not regular enough for the offset-free form");
-#define IROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, double, true, ACCUM>, g, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, H->AS, x, y, H->M)); break;
+#define IROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, double, true, ACCUM, I>, g, 256, 0, stream, keep, hack_begin, hack_end, H->segments, JA, H->AS, x, y, H->M)); break;
         switch (form - 64) {
             IROWU_CASE(3) IROWU_CASE(4) IROWU_CASE(6) IROWU_CASE(7)
-            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, double, true, ACCUM>, g, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, H->AS, x, y, H->M)); break;
+            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, double, true, ACCUM, I>, g, 256, 0, stream, keep, hack_begin, hack_end, H->segments, JA, H->AS, x, y, H->M)); break;
         }
 #undef IROWU_CASE
     } else {
-#define IROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, double, true, ACCUM>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, H->AS, x, y, H->M)); break;
+#define IROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, double, true, ACCUM, I>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, JA, H->AS, x, y, H->M)); break;
         switch (form) {
             IROW_CASE(2) IROW_CASE(3) IROW_CASE(5) IROW_CASE(6) IROW_CASE(7)
-            default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, double, true, ACCUM>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, H->AS, x, y, H->M)); break;
+            default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, double, true, ACCUM, I>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, JA, H->AS, x, y, H->M)); break;
         }
 #undef IROW_CASE
     }
@@ -770,8 +853,11 @@ static int csr_image_launch_t(const spmv_b200_hll *H, int form, int hack_begin, 
 int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
                      int accumulate, cudaStream_t stream) {
     if (hack_end <= hack_begin) return SPMV_B200_OK;
-    return accumulate ? csr_image_launch_t<true>(H, form, hack_begin, hack_end, x, y, stream)
-                      : csr_image_launch_t<false>(H, form, hack_begin, hack_end, x, y, stream);
+    if (H->JA16)
+        return accumulate ? csr_image_launch_t<true>(H, H->JA16, form, hack_begin, hack_end, x, y, stream)
+                          : csr_image_launch_t<false>(H, H->JA16, form, hack_begin, hack_end, x, y, stream);
+    return accumulate ? csr_image_launch_t<true>(H, H->JA, form, hack_begin, hack_end, x, y, stream)
+                      : csr_image_launch_t<false>(H, H->JA, form, hack_begin, hack_end, x, y, stream);
 }
 }  // namespace spmv
 
@@ -856,7 +942,7 @@ int spmv_b200_hll_from_csr(const spmv_b200_csr *A, void *stream_, spmv_b200_hll 
     cudaStream_t stream = as_stream(stream_);
     spmv_b200_hll *H = new (std::nothrow) spmv_b200_hll();
     if (!H) return fail(SPMV_B200_ERR_NOMEM, "hll_from_csr: out of host memory");
-    int rc = hll_convert(A, stream, 0, -1, H);
+    int rc = hll_convert(A, stream, false, -1, -1, H);
     if (rc == SPMV_B200_OK) rc = stream_plan_hll(H, stream);
     if (rc != SPMV_B200_OK) {
         spmv_b200_hll_free(H);
@@ -1121,6 +1207,7 @@ void spmv_b200_hll_free(spmv_b200_hll *H) {
     cudaFree(H->tiles);
     cudaFree(H->hack_off);
     cudaFree(H->JA);
+    cudaFree(H->JA16);
     cudaFree(H->AS);
     cudaFree(H->stage_x);
     cudaFree(H->stage_y);

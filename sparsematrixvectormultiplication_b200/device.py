@@ -302,11 +302,12 @@ class DeviceCSR:
         return self
 
     def image_form(self) -> str:
-        """Name of the kernel that multiplies the private image ("none" without one)."""
-        form = self.info().image_form
-        if form >= 64:
-            return f"hll_rowu_kernel<{form - 64},double,true>"
-        return f"hll_row_kernel<{form},double,true>" if form > 0 else "none"
+        """Name of the kernel that multiplies the private image, index type included ("none" without one)."""
+        i = self.info()
+        index = "uint16_t" if i.image_index_bytes == 2 else "int"
+        if i.image_form >= 64:
+            return f"hll_rowu_kernel<{i.image_form - 64},double,true,{index}>"
+        return f"hll_row_kernel<{i.image_form},double,true,{index}>" if i.image_form > 0 else "none"
 
     def spmv_rows(self, row_begin, row_end, x, y, stream=None):
         i = self.info()

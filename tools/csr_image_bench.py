@@ -8,10 +8,10 @@ plan's batch) and AUTO alternate: per repetition `launches` back-to-back product
 a warm-up of both.  Every working set exceeds the 126 MB L2.  Reported per workload: mean / min / max microseconds per
 product of each arm, the speed-up (ROW mean / AUTO mean), the chosen kernel, plan time (the synth call, timing included),
 the image's device bytes, the algorithmic bytes of the CSR product (12 nnz + 4 (M+1) + 8 M + 8 N) and the bytes the
-chosen kernel actually reads (image: 12 slots + 8 M + 8 N, no row_ptr), each over the AUTO time, and whether AUTO gives
-ALGO_ROW's bits (it must wherever AUTO is a serial-order kernel: the image, ROW, STREAM; uniform 32 per row is too long for
-the image and stays on the vector kernel, whose shuffle sums differ in the last bits).  The device name and power limit
-are read in the same run.
+chosen kernel actually reads (image: image_device_bytes + 8 M + 8 N, no row_ptr; 10 or 12 bytes per slot with a narrow
+or wide column field), each over the AUTO time, and whether AUTO gives ALGO_ROW's bits (it must wherever AUTO is a
+serial-order kernel: the image, ROW, STREAM; uniform 32 per row is too long for the image and stays on the vector kernel,
+whose shuffle sums differ in the last bits).  The device name and power limit are read in the same run.
 """
 from __future__ import annotations
 
@@ -84,7 +84,7 @@ def run(name, make, reps, launches):
         t_auto.append(arm_ms(A, x, y_auto, d.ALGO_AUTO, launches))
     on_image = i.auto_algo == d.ALGO_ROW_IMAGE
     alg = i.algorithmic_bytes
-    read = (i.image_bytes + 8 * i.M + 8 * i.N) if on_image else alg
+    read = (i.image_device_bytes + 8 * i.M + 8 * i.N) if on_image else alg
     auto_kernel = A.image_form() if on_image else (f"csr_row_kernel<{i.row_batch},double>" if i.auto_algo == d.ALGO_ROW
                                                    else d.ALGO_NAMES[i.auto_algo])
 
@@ -93,7 +93,7 @@ def run(name, make, reps, launches):
                 "spread_us": 1e3 * (max(ts) - min(ts))}
     out = {"M": i.M, "N": i.N, "nnz": i.nnz, "max_row_nnz": i.max_row_nnz, "plan_s": plan_s,
            "row_kernel": f"csr_row_kernel<{i.row_batch},double>", "auto_algo": i.auto_algo, "auto_kernel": auto_kernel,
-           "image_bytes": i.image_bytes, "csr_array_bytes": 12 * i.nnz + 4 * (i.M + 1),
+           "image_bytes": i.image_bytes, "image_device_bytes": i.image_device_bytes, "image_index_bytes": i.image_index_bytes, "csr_array_bytes": 12 * i.nnz + 4 * (i.M + 1),
            "algorithmic_bytes": alg, "read_bytes_auto": read,
            "row": stats(t_row), "auto": stats(t_auto), "speedup_row_over_auto": statistics.mean(t_row) / statistics.mean(t_auto),
            "algorithmic_TBps_auto": alg / (1e-3 * statistics.mean(t_auto)) / 1e12,

@@ -1,5 +1,6 @@
 """Survey of the multi-row forms of the row kernels (csr_rowm_kernel / hll_rowm_kernel) in the built library, and of the
-one-row kernels including the masked forms that multiply a CSR handle's private image: registers,
+one-row kernels including the masked forms that multiply a CSR handle's private image (accumulate or not, 4-byte `int` or
+narrow 2-byte `u16` column field): registers,
 spill bytes (csrc/build/*.ptxas.log) and how many of a step's loads ptxas issues ahead of the first multiply (cuobjdump
 -sass).  A form whose loads are split by a DMUL stalls on its first gather before the rest is requested.  No GPU needed.
 
@@ -36,10 +37,10 @@ def main():
     rows = []
     for body in re.split(r"Function : ", sass)[1:]:
         name = body.split()[0]
-        m = re.search(r"(csr|hll)_row(m|u?)_kernelILi(\d)E(?:Li(\d)ELi(\d)E)?([fd])(?:Lb([01]))?E", name)
+        m = re.search(r"(csr|hll)_row(m|u?)_kernelILi(\d)E(?:Li(\d)ELi(\d)E)?([fd])(?:Lb([01])E)?(?:Lb([01])E)?([it])?", name)
         if not m:
             continue
-        fmt, multi, batch, rows_per, ctas, v, masked = m.groups()
+        fmt, multi, batch, rows_per, ctas, v, masked, accum, index = m.groups()
         ops = re.findall(r"\b(LDG|DMUL)\b", body)
         ahead = 0
         for op in ops:
@@ -49,7 +50,8 @@ def main():
         total = ops.count("LDG")
         rec = info.get(name, {})
         rows.append((fmt, v, int(rows_per or 1), int(batch), int(ctas or 8), rec.get("regs"), rec.get("spill"), ahead, total,
-                     "row" + multi + (" masked" if masked == "1" else "")))
+                     "row" + multi + (" masked" if masked == "1" else "") + (" accum" if accum == "1" else "")
+                     + (" u16" if index == "t" else "")))
     print("format storage rows batch ctas/SM regs spill_bytes loads_ahead_of_first_DMUL/loads rows_in_flight/SM kernel")
     for r in sorted(rows):
         fmt, v, rp, b, c, regs, spill, ahead, total, kind = r
