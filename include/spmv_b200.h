@@ -78,9 +78,12 @@ typedef struct {
     long long image_bytes; /* size of the private image at 12 bytes per slot, as defined in version 102, whatever the
                               width of its column field (0: none, see spmv_b200_csr_set_image); image_device_bytes
                               is what it occupies */
-    int image_form;      /* its kernel: 64 + B hll_rowu_kernel<B,double,true>, B hll_row_kernel<B,double,true>, 0 none */
+    int image_form;      /* its kernel: 64 + B hll_rowu_kernel<B,double,true>, B hll_row_kernel<B,double,true>, 0 none
+                            (on the value codes when image_value_bytes is 1) */
     int image_index_bytes; /* bytes of its column field: 2 (col - row; every column within 2^14 of its row), 4, 0 none */
-    long long image_device_bytes; /* device bytes of its columns and values: (8 + image_index_bytes) per slot */
+    long long image_device_bytes; /* device bytes of its columns, values and value table:
+                                     (image_index_bytes + image_value_bytes) per slot, plus 8 per table entry */
+    int image_value_bytes; /* bytes of its value field: 8 (fp64), 1 (a code into a table of at most 256 doubles), 0 none */
 } spmv_b200_csr_info_t;
 
 typedef struct {
@@ -268,15 +271,22 @@ int spmv_b200_csr_interior_rows(const spmv_b200_csr *A, long long col_lo, long l
  * SPMV_B200_ALGO_ROW for every x, accumulate included).  When every slot's column lies within 2^14 of its row
  * (col - row in [-16384, 16383]: banded matrices, 2-D stencils up to a 16383-wide grid) the column field is 2 bytes,
  * col - row with bit 15 marking padding, and the image takes 10 bytes per slot; otherwise it is the column itself with
- * bit 31 marking padding, 12 bytes per slot.  The width follows from the matrix (image_index_bytes).  Its kernels need
- * no row_ptr load and find a hack's first slot by arithmetic, which makes them faster on stencils (lap2d 4096^2:
- * DESIGN.md section 3).  The plan keeps it only when it times faster than every other candidate and its padding adds at
- * most a quarter to nnz; then AUTO uses it.  Cost: about 10 or 12 bytes per nonzero on top of the CSR arrays (+839 MB
- * on lap2d 4096^2, narrow).
- * mode 0 drops the image (AUTO falls back to the plan's choice among ROW / STREAM); mode 1 builds it whenever the
- * matrix is eligible in structure (owned arrays, no row above 12 nonzeros, no long rows), whatever its size or timing,
- * narrow when the matrix qualifies, and returns SPMV_B200_ERR_INVALID otherwise.  replan decides again; remap_columns
- * drops it.  The fp32, SpMM, fused, row-range and host-buffer products do not use it. */
+ * bit 31 marking padding, 12 bytes per slot.  The width follows from the matrix (image_index_bytes).  The values are
+ * fp64, or -- when the matrix holds at most 256 distinct 64-bit value patterns (stencils, FEM assembly, unit-weight
+ * graphs; +0.0 and -0.0, and NaNs of different payloads, count apart) -- 1-byte codes into a table of those patterns,
+ * sorted as uint64; the kernels multiply by the stored double itself in the same order, so y keeps its bits
+ * (image_value_bytes 8 or 1) -- except that where two different NaNs meet in one row's sum (a NaN value or x entry and
+ * an invalid product such as 0 * Inf) the NaN that results may carry the other payload or sign.  Its kernels need no row_ptr load and find a hack's first slot by arithmetic, which makes them faster on stencils
+ * (lap2d 4096^2: DESIGN.md section 3).  The plan times the image with either value field and keeps it only when one
+ * times faster than every other candidate and its padding adds at most a quarter to nnz; then AUTO uses it.  Cost, on
+ * top of the CSR arrays, per slot: 2 or 4 bytes of column field plus 8 (fp64) or 1 (codes) -- +252 MB on lap2d 4096^2,
+ * narrow and coded; +839 MB with fp64 values.
+ * mode 0 drops the image (AUTO falls back to the plan's choice among ROW / STREAM); mode 1 builds it with fp64 values
+ * whenever the matrix is eligible in structure (owned arrays, no row above 12 nonzeros, no long rows), whatever its size
+ * or timing, narrow when the matrix qualifies, replacing a coded one, and returns SPMV_B200_ERR_INVALID otherwise; mode 2
+ * does the same with the value codes, and returns SPMV_B200_ERR_INVALID, leaving the handle as it was, on a matrix of
+ * more than 256 distinct value patterns.  replan decides again; remap_columns drops it.  The fp32, SpMM, fused,
+ * row-range and host-buffer products do not use it. */
 int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream);
 void spmv_b200_csr_free(spmv_b200_csr *A);
 

@@ -110,6 +110,17 @@ __device__ __forceinline__ int ldg_stream_u16(const uint16_t *p) {
     return (int)r;
 }
 
+// the 1-byte value code of the coded private image of a CSR handle (hll.cu), zero-extended into a 32-bit register
+__device__ __forceinline__ int ldg_stream_u8(const uint8_t *p) {
+    unsigned int r;
+#ifdef SPMV_STREAM_EVICT_FIRST
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(r) : "l"(p), "l"(policy_stream()));
+#else
+    asm volatile("ld.global.nc.L1::no_allocate.u8 %0, [%1];" : "=r"(r) : "l"(p));
+#endif
+    return (int)r;
+}
+
 // x is gathered through the read-only path (LDG.CONSTANT), allocating in L1: neighbouring rows of
 // banded matrices hit the same lines -- and, more important, a gather that misses needs an L1 line while it is in
 // flight: with L1::no_allocate the same kernels ran 3x slower on random columns (profiles/r01d_kernel_selection.md).

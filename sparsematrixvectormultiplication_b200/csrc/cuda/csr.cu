@@ -1071,33 +1071,42 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
         A->row_batch = forced_batch;
     } else if (A->max_row <= kRowKernelMaxLen && A->nnz >= kAutotuneMinNnz && env_int("SPMV_B200_AUTOTUNE", 1)) {
         // candidates: (0) the TMA stream kernel, the row kernel with batch 2..7 and, on a matrix that owns its arrays, the
-        // private image (csr_image_build) in each of its forms: 64 + B hll_rowu_kernel, 32 + B hll_row_kernel.  All give
-        // the same bits on such rows.  The image qualifies when its padding adds at most a quarter to nnz and it fits in a
-        // quarter of the free memory (10 or 12 bytes per slot: narrow or wide column field); it is freed again unless it wins.
+        // private image (csr_image_build) in each of its forms: 64 + B hll_rowu_kernel, 32 + B hll_row_kernel, each on
+        // the fp64 values and, when the matrix holds at most 256 distinct value patterns, on the 1-byte value codes
+        // (+ kImageCoded).  All give the same bits on such rows.  The image qualifies when its padding adds at most a
+        // quarter to nnz and it fits in a quarter of the free memory (2 or 4 bytes of column field per slot, plus 8 + 1
+        // for both value streams, or 1 for the codes alone where both do not fit); it is freed again unless it wins, and
+        // the losing value stream is freed when it does.
         if (A->owns && A->num_long == 0) {
             size_t free_bytes = 0, total_bytes = 0;
             if (cudaMemGetInfo(&free_bytes, &total_bytes) == cudaSuccess) {
                 const long long fit_bytes = (long long)(free_bytes / 4) - 8LL * ((long long)M / 32 + 2);
-                if (fit_bytes >= 0 && csr_image_build(A, A->nnz + A->nnz / 4, fit_bytes, stream, &A->image) != SPMV_B200_OK)
+                if (fit_bytes >= 0 &&
+                    csr_image_build(A, A->nnz + A->nnz / 4, fit_bytes, kImageBoth, stream, &A->image) != SPMV_B200_OK)
                     A->image = nullptr;
             }
             cudaGetLastError();
         }
-        int ids[16], n = 0, fallback = 0;
+        int ids[24], n = 0, fallback = 0;  // 7 plain + 6 + 6 image forms on an irregular image
         ids[n++] = 0;
         for (int batch = 2; batch <= 7; ++batch) {
             if (batch == A->row_batch) fallback = n;
             ids[n++] = batch;
         }
         const int plain = n;
-        for (int batch = 2; A->image && batch <= 7; ++batch)
-            if (A->image->segments.count == 0) ids[n++] = 32 + batch;
-            else if (batch >= 4) ids[n++] = 64 + batch;
-        float ms[16];
+        for (int coded = 0; A->image && coded <= 1; ++coded) {
+            const int flag = coded ? kImageCoded : 0;
+            if (coded ? !A->image->AC : !A->image->AS) continue;
+            for (int batch = 2; batch <= 7; ++batch)
+                if (A->image->segments.count == 0) ids[n++] = flag + 32 + batch;
+                else if (batch >= 4) ids[n++] = flag + 64 + batch;
+        }
+        auto image_form = [](int id) { return (id & kImageCoded) | ((id & ~kImageCoded) >= 64 ? id & ~kImageCoded : (id & ~kImageCoded) - 32); };
+        float ms[24];
         const int pick = tune_candidates(M, A->N, n, fallback, stream, [&](int i, double *x, double *y) {
             if (ids[i] == 0) return stream_launch_csr(A, x, y, 0, nullptr, stream);
             if (ids[i] < 16) return launch_rows(0, M, A->row_ptr, A->col_idx, A->values, x, y, ids[i], 0, stream);
-            return csr_image_launch(A->image, ids[i] >= 64 ? ids[i] : ids[i] - 32, 0, A->image->num_hacks, x, y, 0, stream);
+            return csr_image_launch(A->image, image_form(ids[i]), 0, A->image->num_hacks, x, y, 0, stream);
         }, ms);
         int best = fallback;  // the plain choice stays for ALGO_ROW and the other entry points even when the image wins
         for (int i = 0; i < plain; ++i)
@@ -1105,7 +1114,8 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
         if (ids[best] == 0) A->short_rows_stream = true;
         else A->row_batch = ids[best];
         if (pick >= plain) {
-            A->image_form = ids[pick] >= 64 ? ids[pick] : ids[pick] - 32;
+            A->image_form = image_form(ids[pick]);
+            csr_image_keep(A->image, (A->image_form & kImageCoded) != 0);
         } else {
             spmv_b200_hll_free(A->image);
             A->image = nullptr;
@@ -1703,9 +1713,10 @@ int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info) {
     info->flat_batch = A->flat_batch;
     info->flat_chunks = A->flat_chunks;
     info->image_bytes = A->image ? 12 * A->image->slots : 0;
-    info->image_form = A->image ? A->image_form : 0;
+    info->image_form = A->image ? A->image_form & ~kImageCoded : 0;
     info->image_index_bytes = !A->image ? 0 : A->image->JA16 ? 2 : 4;
     info->image_device_bytes = A->image ? csr_image_bytes(A->image) : 0;
+    info->image_value_bytes = A->image ? csr_image_value_bytes(A->image) : 0;
     return SPMV_B200_OK;
 }
 
@@ -1871,7 +1882,7 @@ int spmv_b200_csr_remap_columns(spmv_b200_csr *A, int nparts, const long long *s
 
 int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream) {
     if (!A) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: NULL matrix");
-    if (mode != 0 && mode != 1) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: unknown mode %d", mode);
+    if (mode < 0 || mode > 2) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: unknown mode %d", mode);
     if (mode == 0) {
         spmv_b200_hll_free(A->image);
         A->image = nullptr;
@@ -1882,8 +1893,12 @@ int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream) {
     if (A->max_row > kRowKernelMaxLen || A->num_long > 0)
         return fail(SPMV_B200_ERR_INVALID, "csr_set_image: rows of up to %d nonzeros and no long rows only (longest row: %d)",
                     kRowKernelMaxLen, A->max_row);
-    if (A->image) return SPMV_B200_OK;
-    SPMV_TRY(csr_image_build(A, -1, -1, as_stream(stream), &A->image));
+    const bool coded = mode == 2;
+    if (A->image && (coded ? A->image->AC != nullptr : A->image->AS != nullptr)) return SPMV_B200_OK;
+    spmv_b200_hll *image = nullptr;  // the held image stays until the new one is built (mode 2 fails on > 256 patterns)
+    SPMV_TRY(csr_image_build(A, -1, -1, coded ? kImageCodes : kImageF64, as_stream(stream), &image));
+    spmv_b200_hll_free(A->image);
+    A->image = image;
     A->image_form = csr_image_default_form(A->image);
     return SPMV_B200_OK;
 }

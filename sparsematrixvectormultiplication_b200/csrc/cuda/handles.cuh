@@ -242,8 +242,11 @@ struct spmv_b200_csr {
     // slots marked, multiplied by the masked hll_rowu / hll_row kernels -- bit for bit csr_row_kernel.  Narrow (JA16, 10
     // bytes per slot) when every slot's column lies within 2^14 of its row, else wide (JA, 12 bytes per slot).  Held only
     // when plan-time timing found it faster (or set_image asked for it); owned arrays only, dropped by remap_columns.
+    // Its values are fp64 (AS) or, when the matrix holds at most 256 distinct 64-bit patterns, 1-byte codes into a table
+    // (AC, table): 3 or 5 bytes per slot; the plan times both and keeps the faster.
     spmv_b200_hll *image = nullptr;
-    int image_form = 0;  // 64 + B: hll_rowu_kernel<B, double, true>; B: hll_row_kernel<B, double, true> (index type: JA16 / JA)
+    int image_form = 0;  // 64 + B: hll_rowu_kernel<B, double, true>; B: hll_row_kernel<B, double, true> (index type: JA16 / JA),
+                         // plus spmv::kImageCoded when it reads the value codes
     // staging vectors of the *_host entry points
     double *stage_x = nullptr;
     double *stage_y = nullptr;
@@ -272,6 +275,10 @@ struct spmv_b200_hll {
     uint16_t *JA16 = nullptr;       // device [slots]: the narrow column field of a CSR handle's private image (JA is then
                                     // NULL): bits 0-14 hold col - row as a 15-bit two's complement, bit 15 marks padding
     double *AS = nullptr;           // device [slots]
+    uint8_t *AC = nullptr;          // device [slots]: the value codes of a CSR handle's coded private image (AS is then NULL
+                                    // once the plan has decided): the slot's value is table[AC[slot]], padding holds code 0
+    double *table = nullptr;        // device [max(num_values, 1)]: the distinct 64-bit value patterns, ascending as uint64
+    int num_values = 0;             // K <= kMaxImageValues patterns in the table (0: no coded image)
     float *AS32 = nullptr;          // fp32 copy of AS (spmv_b200_hll_enable_f32)
     std::vector<long long> host_off;
     // stream kernel plan
@@ -316,9 +323,17 @@ int hll_launch_window(const spmv_b200_hll *H, HllPath path, int unit_begin, int 
 int env_int(const char *name, int fallback);
 // hll.cu: the private image of a CSR handle.  csr_image_build leaves *out NULL when the image would exceed max_slots
 // slots or its column and value arrays max_bytes bytes (< 0: no limit); forms as in spmv_b200_csr::image_form.
-int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_bytes, cudaStream_t stream,
+// values: which value streams it fills -- fp64 (AS), the 1-byte codes (AC + table; the build fails with
+// SPMV_B200_ERR_INVALID on a matrix of more than kMaxImageValues distinct patterns), or both where they fit (plan time:
+// both when they fit, else the codes alone, else fp64 alone).
+constexpr int kMaxImageValues = 256;
+constexpr int kImageCoded = 128;  // image_form flag: the kernel reads the value codes
+enum ImageValues { kImageF64 = 1, kImageCodes = 2, kImageBoth = 3 };
+int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_bytes, ImageValues values, cudaStream_t stream,
                     spmv_b200_hll **out);
-long long csr_image_bytes(const spmv_b200_hll *H);  // device bytes of JA / JA16 and AS: 10 or 12 per slot
+long long csr_image_bytes(const spmv_b200_hll *H);  // device bytes of JA / JA16, AS, AC and the table
+int csr_image_value_bytes(const spmv_b200_hll *H);  // 8 (fp64), 1 (codes) or 9 (both, during the plan's timing)
+void csr_image_keep(spmv_b200_hll *H, bool coded);  // frees the other value stream
 int csr_image_default_form(const spmv_b200_hll *H);
 int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
                      int accumulate, cudaStream_t stream);

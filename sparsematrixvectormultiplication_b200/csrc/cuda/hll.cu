@@ -19,6 +19,7 @@
 #include <cub/cub.cuh>
 
 #include <algorithm>
+#include <type_traits>
 #include <cstdlib>
 #include <cstring>
 #include <new>
@@ -59,6 +60,29 @@ template <typename I>
 __device__ __forceinline__ int image_past_width(int first) {
     if constexpr (sizeof(I) == 2) return first | kPadMark16;
     else return kPadMark;
+}
+
+// The value field of a slot: fp64 (or fp32 storage) as loaded, or a 1-byte code (S = uint8_t: the coded private image of a
+// CSR handle) into the CTA's copy of the image's value table (image_table, staged by stage_image_table).  The load returns
+// the code; the table is read at the multiply, so the step's global loads all go out ahead of it.
+template <typename S>
+using stored_t = typename std::conditional<sizeof(S) == 1, int, double>::type;
+__device__ __forceinline__ double ldg_stream_value(const double *p) { return ldg_stream_f64(p); }
+__device__ __forceinline__ double ldg_stream_value(const float *p) { return ldg_stream_f64(p); }
+__device__ __forceinline__ int ldg_stream_value(const uint8_t *p) { return ldg_stream_u8(p); }
+__device__ __forceinline__ double image_value(double v, const double *) { return v; }
+__device__ __forceinline__ double image_value(int code, const double *tab) { return tab[code]; }
+
+// the table of a coded image into shared memory (K >= 1 entries, dynamic shared memory of 8 K bytes); every thread of the
+// CTA calls it, ahead of the kernel's warp-uniform early return
+template <typename S>
+__device__ __forceinline__ const double *stage_image_table(const double *__restrict__ table, int K) {
+    extern __shared__ double image_table[];
+    if constexpr (sizeof(S) == 1) {
+        for (int i = threadIdx.x; i < K; i += blockDim.x) image_table[i] = __ldg(table + i);
+        __syncthreads();
+    }
+    return image_table;
 }
 
 __device__ __forceinline__ void ldg_stream_f64x4(const float *p, double (&v)[4]) {  // fp32 storage: one 128-bit load
@@ -126,12 +150,15 @@ hll_slice_kernel(int hack_begin, int hack_end, const long long *__restrict__ hac
 // 0 * x[c] would give NaN for an infinite x[c], and +0 turns an untouched -0.0 positive.)  The loads are never predicated
 // on the loaded column.  ACCUM is a template flag, not an argument: a y[row] load hoisted ahead of the step holds two of
 // the 32 registers and pushed two of the 15 loads of hll_rowu_kernel<5> behind the first multiply (cuobjdump,
-// tools/rowm_survey.py).
-template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false, typename I = int>
+// tools/rowm_survey.py).  S: the stored value type -- V, or uint8_t for the coded private image (codes into `table`, K
+// entries, staged in shared memory; table and K are unused otherwise).
+template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false, typename I = int, typename S = V>
 __global__ void __launch_bounds__(256, 8)
 hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_off, const I *__restrict__ JA,
-               const V *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M) {
+               const S *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M, const double *__restrict__ table, int K) {
     static_assert(sizeof(I) == 4 || (MASKED && sizeof(V) == 8), "the narrow index exists in the fp64 private image only");
+    static_assert(sizeof(S) == sizeof(V) || (MASKED && sizeof(V) == 8), "value codes exist in the fp64 private image only");
+    const double *tab = stage_image_table<S>(table, K);
     const int hack = hack_begin + blockIdx.x * 8 + (threadIdx.x >> 5);
     if (hack >= hack_end) return;  // warp-uniform
     const int lane = threadIdx.x & 31;
@@ -142,18 +169,19 @@ hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_
     double acc = ACCUM && row < M ? (double)y[row] : 0.0;
     for (int j = 0; j < width; j += BATCH) {
         int c[BATCH];
-        double v[BATCH], xv[BATCH];
+        stored_t<S> v[BATCH];
+        double xv[BATCH];
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)  // u = 0 is always within the width
             c[u] = j + u < width ? ldg_stream_index(JA + base + (long long)(j + u) * kHack) : (MASKED ? image_past_width<I>(u ? c[0] : 0) : -1);
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_f64(AS + base + (long long)(j + u) * kHack) : 0.0;
+        for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_value(AS + base + (long long)(j + u) * kHack) : 0;
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
             xv[u] = MASKED ? ldg_x(x, image_column<I>(c[u], (unsigned)row)) : (c[u] >= 0 ? ldg_x(x, c[u]) : 0.0);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
-            if (MASKED ? image_adds<I>(c[u]) : c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
+            if (MASKED ? image_adds<I>(c[u]) : c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(image_value(v[u], tab), xv[u]));
     }
     if (row < M) y[row] = (V)acc;
 }
@@ -224,12 +252,14 @@ hll_rowm_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack
 // other ways to shorten that trip on images that are NOT regular, tried and removed: the hack_off line of the CTA N CTAs
 // further on prefetched into L2 by one thread per CTA (141-142 us at every N from 148 to 9472: the same 3 %), and the
 // offset array held in the persisting L2 carve-out (194.6 us: the carve-out costs the gathers more than the trip saves).
-// MASKED / ACCUM / I: as in hll_row_kernel -- the private image of a CSR handle, bit for bit csr_row_kernel.
-template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false, typename I = int>
+// MASKED / ACCUM / I / S: as in hll_row_kernel -- the private image of a CSR handle, bit for bit csr_row_kernel.
+template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false, typename I = int, typename S = V>
 __global__ void __launch_bounds__(256, 8)
 hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegments seg, const I *__restrict__ JA,
-                const V *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M) {
+                const S *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M, const double *__restrict__ table, int K) {
     static_assert(sizeof(I) == 4 || (MASKED && sizeof(V) == 8), "the narrow index exists in the fp64 private image only");
+    static_assert(sizeof(S) == sizeof(V) || (MASKED && sizeof(V) == 8), "value codes exist in the fp64 private image only");
+    const double *tab = stage_image_table<S>(table, K);
     const int hack = hack_begin + blockIdx.x * 8 + (threadIdx.x >> 5);
     if (hack >= hack_end) return;  // warp-uniform
     const int lane = threadIdx.x & 31;
@@ -250,31 +280,33 @@ hll_rowu_kernel(int hack_begin, int hack_end, const __grid_constant__ HllSegment
         // ncu on the predicated loop alone (profiles/r02e_ncu_f32_summary.md): issue slots 70 % busy, SM throughput 84 %
         // -- without the offset trip this kernel is close to instruction-issue bound, so instructions count.
         int c[BATCH];
-        double v[BATCH], xv[BATCH];
+        stored_t<S> v[BATCH];
+        double xv[BATCH];
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) c[u] = ldg_stream_index(JA + off + (long long)u * kHack);
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) v[u] = ldg_stream_f64(AS + off + (long long)u * kHack);
+        for (int u = 0; u < BATCH; ++u) v[u] = ldg_stream_value(AS + off + (long long)u * kHack);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, MASKED ? image_column<I>(c[u], (unsigned)row) : c[u]);
         if (ACCUM && row < M) acc = y[row];  // after the step's loads: held from the start, it pushed the narrow form to spill
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
-            if (!MASKED || image_adds<I>(c[u])) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
+            if (!MASKED || image_adds<I>(c[u])) acc = __dadd_rn(acc, __dmul_rn(image_value(v[u], tab), xv[u]));
     } else
     for (int j = 0; j < width; j += BATCH) {
         int c[BATCH];
-        double v[BATCH], xv[BATCH];
+        stored_t<S> v[BATCH];
+        double xv[BATCH];
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)  // u = 0 is always within the width
             c[u] = j + u < width ? ldg_stream_index(JA + off + (long long)(j + u) * kHack) : (MASKED ? image_past_width<I>(u ? c[0] : 0) : 0);
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_f64(AS + off + (long long)(j + u) * kHack) : 0.0;
+        for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_value(AS + off + (long long)(j + u) * kHack) : 0;
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) xv[u] = ldg_x(x, MASKED ? image_column<I>(c[u], (unsigned)row) : c[u]);
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
-            if (j + u < width && (!MASKED || image_adds<I>(c[u]))) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
+            if (j + u < width && (!MASKED || image_adds<I>(c[u]))) acc = __dadd_rn(acc, __dmul_rn(image_value(v[u], tab), xv[u]));
     }
     if (row < M) y[row] = (V)acc;
 }
@@ -429,10 +461,24 @@ __device__ __forceinline__ void put_index(uint16_t *JA, long long slot, int col,
     JA[slot] = (uint16_t)(((unsigned long long)(col - row) & 0x7fffu) | (pad ? kPadMark16 : 0));
 }
 
+// the code of a value in the ascending table of the K distinct 64-bit patterns of a coded image (the pattern is there)
+__device__ __forceinline__ int value_code(const double *__restrict__ table, int K, double v) {
+    const unsigned long long k = (unsigned long long)__double_as_longlong(v);
+    int lo = 0, hi = K - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if ((unsigned long long)__double_as_longlong(table[mid]) < k) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// AS (fp64 values) and AC (1-byte codes into table[K]) are each filled when not NULL; a padding slot holds 0.0 / code 0
 template <typename I>
 __global__ void hll_fill_kernel(int M, int N, int num_hacks, const int *__restrict__ row_ptr, const int *__restrict__ col_idx,
                                 const double *__restrict__ values, const long long *__restrict__ hack_off,
-                                I *__restrict__ JA, double *__restrict__ AS, int mark) {
+                                I *__restrict__ JA, double *__restrict__ AS, uint8_t *__restrict__ AC,
+                                const double *__restrict__ table, int K, int mark) {
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= (long long)num_hacks * kHack) return;
     const int hack = (int)(r / kHack), lr = (int)(r % kHack);
@@ -451,10 +497,13 @@ __global__ void hll_fill_kernel(int M, int N, int num_hacks, const int *__restri
         if (j < len) {
             pad_col = col_idx[begin + j];
             put_index(JA, slot, pad_col, r, false, mark);
-            AS[slot] = values[begin + j];
+            const double v = values[begin + j];
+            if (AS) AS[slot] = v;
+            if (AC) AC[slot] = (uint8_t)value_code(table, K, v);
         } else {
             put_index(JA, slot, pad_col, r, true, mark);
-            AS[slot] = 0.0;
+            if (AS) AS[slot] = 0.0;
+            if (AC) AC[slot] = 0;
         }
     }
 }
@@ -478,6 +527,52 @@ __global__ void hll_narrow_check_kernel(int M, int N, int num_hacks, const int *
     }
     if (begin == end && widths[r / kHack] > 0) ok = r - (N - 1) <= -kDeltaMin;
     if (!ok) *fits = 0;
+}
+
+// The distinct 64-bit value patterns among the nonzeros (the table of a coded image): +0.0 and -0.0, and NaNs of different
+// payloads, are different patterns.  keys: an open-addressing set of kDictSlots entries, kDictEmpty when free; the pattern
+// kDictEmpty itself sets state[1].  state[0] counts the patterns and passes kMaxImageValues as soon as a 257th appears (or
+// a probe walks past kMaxImageValues occupied entries, which only more patterns can fill); every warp then stops.  A warp
+// first merges its lanes' equal patterns (__match_any_sync), and one lane per pattern probes with a plain load: a pattern
+// already in the set -- every one after the first few on a stencil -- costs no atomic.  An entry, once written, never
+// changes, so a stale load can only read kDictEmpty, and the compare-and-swap then tells the truth.
+constexpr int kDictSlots = 1024;
+constexpr unsigned long long kDictEmpty = ~0ULL;
+
+__device__ __forceinline__ void dict_insert(unsigned long long k, unsigned long long *keys, int *state) {
+    if (k == kDictEmpty) {
+        state[1] = 1;
+        return;
+    }
+    unsigned int h = (unsigned int)mix64(k) & (kDictSlots - 1);
+    for (int probe = 0; probe <= kMaxImageValues; ++probe) {
+        unsigned long long cur = keys[h];
+        if (cur == kDictEmpty) {
+            cur = atomicCAS(keys + h, kDictEmpty, k);
+            if (cur == kDictEmpty) {
+                atomicAdd(state, 1);
+                return;
+            }
+        }
+        if (cur == k) return;
+        h = (h + 1) & (kDictSlots - 1);
+    }
+    atomicMax(state, kMaxImageValues + 1);
+}
+
+__global__ void hll_value_dict_kernel(long long nnz, const double *__restrict__ values, unsigned long long *keys, int *state) {
+    const int lane = threadIdx.x & 31;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    int step = 0;
+    for (long long base = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < nnz; base += stride, ++step) {
+        if ((step & 63) == 0) {  // warp-uniform
+            int stop = lane == 0 ? *(volatile int *)state : 0;
+            if (__shfl_sync(0xffffffffu, stop, 0) > kMaxImageValues) return;
+        }
+        const unsigned long long k = (unsigned long long)__double_as_longlong(values[min(base + lane, nnz - 1)]);
+        const unsigned int same = __match_any_sync(0xffffffffu, k);
+        if (lane == __ffs(same) - 1) dict_insert(k, keys, state);
+    }
 }
 
 __global__ void max_int_kernel(const int *__restrict__ v, int n, int *__restrict__ out) {
@@ -512,10 +607,10 @@ static int hll_launch_rows_t(const spmv_b200_hll *H, const V *AS, int hack_begin
     if (uniform > 0) {
         if (H->segments.count <= 0) return fail(SPMV_B200_ERR_INVALID, "hll row kernel: the image is not regular enough for the offset-free form");
         const unsigned int gu = blocks_for(hack_end - hack_begin, 8);
-#define HROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, V>, gu, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, AS, d_x, d_y, H->M)); break;
+#define HROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, V>, gu, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, AS, d_x, d_y, H->M, nullptr, 0)); break;
         switch (uniform) {
             HROWU_CASE(3) HROWU_CASE(4) HROWU_CASE(6) HROWU_CASE(7)
-            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, V>, gu, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, AS, d_x, d_y, H->M)); break;
+            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, V>, gu, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, AS, d_x, d_y, H->M, nullptr, 0)); break;
         }
 #undef HROWU_CASE
         SPMV_TRY_CUDA(cudaGetLastError());
@@ -536,10 +631,10 @@ static int hll_launch_rows_t(const spmv_b200_hll *H, const V *AS, int hack_begin
         return SPMV_B200_OK;
     }
     const unsigned int g = blocks_for(hack_end - hack_begin, 8);
-#define HROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, V>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, AS, d_x, d_y, H->M)); break;
+#define HROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, V>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, AS, d_x, d_y, H->M, nullptr, 0)); break;
     switch (batch) {
         HROW_CASE(1) HROW_CASE(2) HROW_CASE(3) HROW_CASE(5) HROW_CASE(6) HROW_CASE(7) HROW_CASE(8)
-        default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, V>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, AS, d_x, d_y, H->M)); break;
+        default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, V>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, AS, d_x, d_y, H->M, nullptr, 0)); break;
     }
 #undef HROW_CASE
     SPMV_TRY_CUDA(cudaGetLastError());
@@ -612,11 +707,12 @@ static int hll_launch(const spmv_b200_hll *H, int hack_begin, int hack_end, cons
     return SPMV_B200_OK;
 }
 
-static int hll_alloc_arena(spmv_b200_hll *H, bool narrow = false) {
+static int hll_alloc_arena(spmv_b200_hll *H, bool narrow = false, bool f64 = true, bool codes = false) {
     const size_t n = (size_t)std::max<long long>(H->slots, 32);
     if (narrow) SPMV_TRY_CUDA(cudaMalloc(&H->JA16, n * sizeof(uint16_t)));
     else SPMV_TRY_CUDA(cudaMalloc(&H->JA, n * sizeof(int)));
-    SPMV_TRY_CUDA(cudaMalloc(&H->AS, n * sizeof(double)));
+    if (f64) SPMV_TRY_CUDA(cudaMalloc(&H->AS, n * sizeof(double)));
+    if (codes) SPMV_TRY_CUDA(cudaMalloc(&H->AC, n * sizeof(uint8_t)));
     return SPMV_B200_OK;
 }
 
@@ -728,22 +824,23 @@ static void hll_pick_row_batch(spmv_b200_hll *H, cudaStream_t stream) {
 }  // namespace spmv
 
 // CSR -> column-major image on the device: widths, scan, fill (spmv_b200_hll_from_csr and the private image of a CSR
-// handle).  image: the private image -- padding slots marked, and narrow (JA16) when every slot fits it.  max_slots /
-// max_bytes >= 0: an image of more slots or more bytes of JA and AS is not filled (H->JA and H->JA16 stay NULL, H->slots
-// tells its size).
+// handle).  image: the private image -- padding slots marked, and narrow (JA16) when every slot fits it.  values: the value
+// streams to fill (csr_image_build; the HLL format always has AS).  max_slots / max_bytes >= 0: an image of more slots or
+// more bytes of columns, values and table is not filled (H->JA and H->JA16 stay NULL, H->slots tells its size).
 static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, bool image, long long max_slots, long long max_bytes,
-                       spmv_b200_hll *H) {
+                       spmv_b200_hll *H, ImageValues values = kImageF64) {
     spmv_b200_csr_info_t ci;
     const int *row_ptr, *col_idx;
-    const double *values;
+    const double *values_ptr;
     SPMV_TRY(spmv_b200_csr_info(A, &ci));
-    SPMV_TRY(spmv_b200_csr_device_arrays(A, &row_ptr, &col_idx, &values));
+    SPMV_TRY(spmv_b200_csr_device_arrays(A, &row_ptr, &col_idx, &values_ptr));
     H->M = ci.M;
     H->N = ci.N;
     const int nb = H->num_hacks = (ci.M + kHack - 1) / kHack;
     long long *slots = nullptr;
     int *widths = nullptr, *d_max = nullptr;  // d_max[0]: widest hack; d_max[1]: every slot fits the narrow field
     void *temp = nullptr;
+    unsigned long long *keys = nullptr;  // the dictionary pass (hll_value_dict_kernel): keys[kDictSlots], then state[2]
     int fits = 0;
     auto body = [&]() -> int {
         SPMV_TRY_CUDA(cudaMalloc(&H->hack_off, ((size_t)nb + 1) * sizeof(long long)));
@@ -759,6 +856,16 @@ static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, bool image, 
                                                                                             widths, d_max + 1);
             SPMV_TRY_CUDA(cudaGetLastError());
         }
+        if (values & kImageCodes) {
+            SPMV_TRY_CUDA(cudaMalloc(&keys, kDictSlots * sizeof(unsigned long long) + 2 * sizeof(int)));
+            SPMV_TRY_CUDA(cudaMemsetAsync(keys, 0xff, kDictSlots * sizeof(unsigned long long), stream));
+            SPMV_TRY_CUDA(cudaMemsetAsync(keys + kDictSlots, 0, 2 * sizeof(int), stream));
+            if (ci.nnz > 0) {
+                hll_value_dict_kernel<<<std::min(blocks_for(ci.nnz, 256), 4096u), 256, 0, stream>>>(
+                    ci.nnz, values_ptr, keys, reinterpret_cast<int *>(keys + kDictSlots));
+                SPMV_TRY_CUDA(cudaGetLastError());
+            }
+        }
         size_t temp_bytes = 0;
         SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, slots, H->hack_off, nb + 1, stream));
         SPMV_TRY_CUDA(cudaMalloc(&temp, temp_bytes ? temp_bytes : 1));
@@ -772,22 +879,56 @@ static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, bool image, 
                                       cudaMemcpyDeviceToHost, stream));
         SPMV_TRY_CUDA(cudaMemcpyAsync(&H->max_width, d_max, sizeof(int), cudaMemcpyDeviceToHost, stream));
         SPMV_TRY_CUDA(cudaMemcpyAsync(&fits, d_max + 1, sizeof(int), cudaMemcpyDeviceToHost, stream));
+        std::vector<unsigned long long> dict;
+        int state[2] = {0, 0};
+        if (keys) {
+            dict.resize(kDictSlots);
+            SPMV_TRY_CUDA(cudaMemcpyAsync(dict.data(), keys, kDictSlots * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
+            SPMV_TRY_CUDA(cudaMemcpyAsync(state, keys + kDictSlots, sizeof state, cudaMemcpyDeviceToHost, stream));
+        }
         SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
+        // the table: the patterns ascending as uint64, so that the image does not depend on the order of the inserts
+        bool codes = keys != nullptr && state[0] <= kMaxImageValues;
+        if (codes) {
+            dict.erase(std::remove(dict.begin(), dict.end(), kDictEmpty), dict.end());
+            if (state[1]) dict.push_back(kDictEmpty);
+            std::sort(dict.begin(), dict.end());
+            codes = (int)dict.size() <= kMaxImageValues;
+        }
+        if (values == kImageCodes && !codes)
+            return fail(SPMV_B200_ERR_INVALID, "csr image: the values hold more than %d distinct 64-bit patterns", kMaxImageValues);
         H->slots = H->host_off[nb];
         // reference layout keeps the last block short: its padded rows do not exist there
         const int last_rows = nb > 0 ? ci.M - (nb - 1) * kHack : 0;
         H->ref_slots = H->slots;
         if (nb > 0) H->ref_slots -= ((H->host_off[nb] - H->host_off[nb - 1]) / kHack) * (kHack - last_rows);
         if (max_slots >= 0 && H->slots > max_slots) return SPMV_B200_OK;
-        if (max_bytes >= 0 && H->slots * (fits ? 10 : 12) > max_bytes) return SPMV_B200_OK;
-        SPMV_TRY(hll_alloc_arena(H, fits != 0));
+        // bytes per slot of each choice, largest first: both value streams (plan time), the codes alone, fp64 alone
+        const long long index = fits ? 2 : 4, table = codes ? 8LL * (long long)dict.size() : 0;
+        auto fit = [&](long long per_slot, long long extra) { return max_bytes < 0 || H->slots * per_slot + extra <= max_bytes; };
+        bool f64 = values != kImageCodes, use_codes = codes;
+        if (f64 && use_codes && !fit(index + 9, table)) f64 = false;  // plan time: the codes alone where both do not fit
+        if (!use_codes && !fit(index + 8, 0)) return SPMV_B200_OK;
+        if (use_codes && !fit(index + (f64 ? 9 : 1), table)) return SPMV_B200_OK;
+        SPMV_TRY(hll_alloc_arena(H, fits != 0, f64, use_codes));
+        if (use_codes) {
+            std::vector<double> tab(std::max<size_t>(dict.size(), 1), 0.0);  // at least one entry: padding reads code 0
+            std::memcpy(tab.data(), dict.data(), dict.size() * sizeof(double));
+            H->num_values = (int)dict.size();
+            SPMV_TRY_CUDA(cudaMalloc(&H->table, tab.size() * sizeof(double)));
+            SPMV_TRY_CUDA(cudaMemcpyAsync(H->table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, stream));
+            SPMV_TRY_CUDA(cudaStreamSynchronize(stream));  // tab is a local
+        }
         if (nb > 0) {
             const unsigned int g = blocks_for((long long)nb * kHack, 256);
             const int mark = image ? kPadMark : 0;
+            const int K = H->num_values;
             if (fits)
-                hll_fill_kernel<<<g, 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx, values, H->hack_off, H->JA16, H->AS, mark);
+                hll_fill_kernel<<<g, 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx, values_ptr, H->hack_off, H->JA16, H->AS, H->AC,
+                                                       H->table, K, mark);
             else
-                hll_fill_kernel<<<g, 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx, values, H->hack_off, H->JA, H->AS, mark);
+                hll_fill_kernel<<<g, 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx, values_ptr, H->hack_off, H->JA, H->AS, H->AC,
+                                                       H->table, K, mark);
             SPMV_TRY_CUDA(cudaGetLastError());
         }
         SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
@@ -798,16 +939,17 @@ static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, bool image, 
     cudaFree(widths);
     cudaFree(d_max);
     cudaFree(temp);
+    cudaFree(keys);
     return rc;
 }
 
 namespace spmv {
-int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_bytes, cudaStream_t stream,
+int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_bytes, ImageValues values, cudaStream_t stream,
                     spmv_b200_hll **out) {
     *out = nullptr;
     spmv_b200_hll *H = new (std::nothrow) spmv_b200_hll();
     if (!H) return fail(SPMV_B200_ERR_NOMEM, "csr image: out of host memory");
-    const int rc = hll_convert(A, stream, true, max_slots, max_bytes, H);
+    const int rc = hll_convert(A, stream, true, max_slots, max_bytes, H, values);
     if (rc != SPMV_B200_OK || (!H->JA && !H->JA16)) {
         spmv_b200_hll_free(H);
         return rc;
@@ -819,30 +961,49 @@ int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_b
     return SPMV_B200_OK;
 }
 
-long long csr_image_bytes(const spmv_b200_hll *H) { return H->slots * (H->JA16 ? 10 : 12); }
+int csr_image_value_bytes(const spmv_b200_hll *H) { return (H->AS ? 8 : 0) + (H->AC ? 1 : 0); }
 
-int csr_image_default_form(const spmv_b200_hll *H) {
-    return H->segments.count > 0 ? 64 + std::max(3, std::min(7, H->max_width)) : H->row_batch;
+long long csr_image_bytes(const spmv_b200_hll *H) {
+    return H->slots * ((H->JA16 ? 2 : 4) + csr_image_value_bytes(H)) + (H->AC ? 8LL * H->num_values : 0);
 }
 
-template <bool ACCUM, typename I>
-static int csr_image_launch_t(const spmv_b200_hll *H, const I *JA, int form, int hack_begin, int hack_end, const double *x,
-                              double *y, cudaStream_t stream) {
+void csr_image_keep(spmv_b200_hll *H, bool coded) {
+    if (coded) {
+        cudaFree(H->AS);
+        H->AS = nullptr;
+    } else {
+        cudaFree(H->AC);
+        cudaFree(H->table);
+        H->AC = nullptr;
+        H->table = nullptr;
+        H->num_values = 0;
+    }
+}
+
+int csr_image_default_form(const spmv_b200_hll *H) {
+    return (H->segments.count > 0 ? 64 + std::max(3, std::min(7, H->max_width)) : H->row_batch) | (H->AS ? 0 : kImageCoded);
+}
+
+template <bool ACCUM, typename I, typename S>
+static int csr_image_launch_t(const spmv_b200_hll *H, const I *JA, const S *AS, int form, int hack_begin, int hack_end,
+                              const double *x, double *y, cudaStream_t stream) {
     const XPolicy keep = matrix_policy(JA, (size_t)H->slots * sizeof(I));
     const unsigned int g = blocks_for(hack_end - hack_begin, 8);
+    const int K = std::max(H->num_values, 1);
+    const size_t smem = sizeof(S) == 1 ? (size_t)K * sizeof(double) : 0;  // the staged table of a coded image
     if (form >= 64) {
         if (H->segments.count <= 0) return fail(SPMV_B200_ERR_INVALID, "csr image: not regular enough for the offset-free form");
-#define IROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, double, true, ACCUM, I>, g, 256, 0, stream, keep, hack_begin, hack_end, H->segments, JA, H->AS, x, y, H->M)); break;
+#define IROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->segments, JA, AS, x, y, H->M, H->table, K)); break;
         switch (form - 64) {
             IROWU_CASE(3) IROWU_CASE(4) IROWU_CASE(6) IROWU_CASE(7)
-            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, double, true, ACCUM, I>, g, 256, 0, stream, keep, hack_begin, hack_end, H->segments, JA, H->AS, x, y, H->M)); break;
+            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->segments, JA, AS, x, y, H->M, H->table, K)); break;
         }
 #undef IROWU_CASE
     } else {
-#define IROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, double, true, ACCUM, I>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, JA, H->AS, x, y, H->M)); break;
+#define IROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->hack_off, JA, AS, x, y, H->M, H->table, K)); break;
         switch (form) {
             IROW_CASE(2) IROW_CASE(3) IROW_CASE(5) IROW_CASE(6) IROW_CASE(7)
-            default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, double, true, ACCUM, I>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, JA, H->AS, x, y, H->M)); break;
+            default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->hack_off, JA, AS, x, y, H->M, H->table, K)); break;
         }
 #undef IROW_CASE
     }
@@ -850,14 +1011,26 @@ static int csr_image_launch_t(const spmv_b200_hll *H, const I *JA, int form, int
     return SPMV_B200_OK;
 }
 
+template <typename I>
+static int csr_image_launch_i(const spmv_b200_hll *H, const I *JA, int form, int hack_begin, int hack_end, const double *x,
+                              double *y, int accumulate, cudaStream_t stream) {
+    if (form & kImageCoded) {
+        if (!H->AC) return fail(SPMV_B200_ERR_INVALID, "csr image: the image holds no value codes");
+        form &= ~kImageCoded;
+        return accumulate ? csr_image_launch_t<true>(H, JA, H->AC, form, hack_begin, hack_end, x, y, stream)
+                          : csr_image_launch_t<false>(H, JA, H->AC, form, hack_begin, hack_end, x, y, stream);
+    }
+    if (!H->AS) return fail(SPMV_B200_ERR_INVALID, "csr image: the image holds no fp64 values");
+    return accumulate ? csr_image_launch_t<true>(H, JA, H->AS, form, hack_begin, hack_end, x, y, stream)
+                      : csr_image_launch_t<false>(H, JA, H->AS, form, hack_begin, hack_end, x, y, stream);
+}
+
+// form: as in spmv_b200_csr::image_form -- kImageCoded selects the value codes
 int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
                      int accumulate, cudaStream_t stream) {
     if (hack_end <= hack_begin) return SPMV_B200_OK;
-    if (H->JA16)
-        return accumulate ? csr_image_launch_t<true>(H, H->JA16, form, hack_begin, hack_end, x, y, stream)
-                          : csr_image_launch_t<false>(H, H->JA16, form, hack_begin, hack_end, x, y, stream);
-    return accumulate ? csr_image_launch_t<true>(H, H->JA, form, hack_begin, hack_end, x, y, stream)
-                      : csr_image_launch_t<false>(H, H->JA, form, hack_begin, hack_end, x, y, stream);
+    if (H->JA16) return csr_image_launch_i(H, H->JA16, form, hack_begin, hack_end, x, y, accumulate, stream);
+    return csr_image_launch_i(H, H->JA, form, hack_begin, hack_end, x, y, accumulate, stream);
 }
 }  // namespace spmv
 
@@ -1209,6 +1382,8 @@ void spmv_b200_hll_free(spmv_b200_hll *H) {
     cudaFree(H->JA);
     cudaFree(H->JA16);
     cudaFree(H->AS);
+    cudaFree(H->AC);
+    cudaFree(H->table);
     cudaFree(H->stage_x);
     cudaFree(H->stage_y);
     host_pipe_free(H->pipe);

@@ -296,18 +296,23 @@ class DeviceCSR:
         return lo.value, hi.value
 
     def set_image(self, mode, stream=None):
-        """mode 0: drop the private column-major image; mode 1: build it on any matrix eligible in structure (owned arrays,
-        rows of at most 12 nonzeros), whatever its size or timing (spmv_b200_csr_set_image).  Raises SpmvError otherwise."""
+        """mode 0: drop the private column-major image; mode 1: build it with fp64 values on any matrix eligible in
+        structure (owned arrays, rows of at most 12 nonzeros), whatever its size or timing; mode 2: the same with 1-byte
+        value codes, on a matrix of at most 256 distinct value patterns (spmv_b200_csr_set_image).  Raises SpmvError
+        otherwise, and mode 2 then leaves the handle as it was."""
         N.check(N.lib().spmv_b200_csr_set_image(self._h, int(mode), _stream(stream)))
         return self
 
     def image_form(self) -> str:
-        """Name of the kernel that multiplies the private image, index type included ("none" without one)."""
+        """Name of the kernel that multiplies the private image, index type and, for the value codes, the stored value
+        type included ("none" without one)."""
         i = self.info()
-        index = "uint16_t" if i.image_index_bytes == 2 else "int"
+        args = "uint16_t" if i.image_index_bytes == 2 else "int"
+        if i.image_value_bytes == 1:
+            args += ",uint8_t"
         if i.image_form >= 64:
-            return f"hll_rowu_kernel<{i.image_form - 64},double,true,{index}>"
-        return f"hll_row_kernel<{i.image_form},double,true,{index}>" if i.image_form > 0 else "none"
+            return f"hll_rowu_kernel<{i.image_form - 64},double,true,{args}>"
+        return f"hll_row_kernel<{i.image_form},double,true,{args}>" if i.image_form > 0 else "none"
 
     def spmv_rows(self, row_begin, row_end, x, y, stream=None):
         i = self.info()

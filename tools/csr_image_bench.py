@@ -1,15 +1,16 @@
-"""The private image of a CSR handle against csr_row_kernel, alternating in one process.
+"""The private image of a CSR handle against its fp64 form and csr_row_kernel, alternating in one process.
 
     python tools/csr_image_bench.py --out FILE [--reps 12] [--launches 50] [--workloads lap2d_4096,lap3d_384,...]
 
 For each workload the handle is built as a user builds it (synth: owned arrays, plan-time timing on), so AUTO is whatever
-the plan chose -- the private image (SPMV_B200_ALGO_ROW_IMAGE) where it timed fastest.  Then ALGO_ROW (csr_row_kernel, the
-plan's batch) and AUTO alternate: per repetition `launches` back-to-back products of each arm between CUDA events, after
-a warm-up of both.  Every working set exceeds the 126 MB L2.  Reported per workload: mean / min / max microseconds per
+the plan chose -- the private image (SPMV_B200_ALGO_ROW_IMAGE) where it timed fastest, with fp64 values or 1-byte value
+codes.  A second handle of the same matrix holds the image with fp64 values (set_image(1)).  Then ALGO_ROW (csr_row_kernel,
+the plan's batch), AUTO and ROW_IMAGE on the fp64 image alternate: per repetition `launches` back-to-back products of each
+arm between CUDA events, after a warm-up of all.  Every working set exceeds the 126 MB L2.  Reported per workload: mean / min / max microseconds per
 product of each arm, the speed-up (ROW mean / AUTO mean), the chosen kernel, plan time (the synth call, timing included),
-the image's device bytes, the algorithmic bytes of the CSR product (12 nnz + 4 (M+1) + 8 M + 8 N) and the bytes the
-chosen kernel actually reads (image: image_device_bytes + 8 M + 8 N, no row_ptr; 10 or 12 bytes per slot with a narrow
-or wide column field), each over the AUTO time, and whether AUTO gives ALGO_ROW's bits (it must wherever AUTO is a
+the image's device bytes and value bytes, the algorithmic bytes of the CSR product (12 nnz + 4 (M+1) + 8 M + 8 N) and the
+bytes each image kernel actually reads (image_device_bytes + 8 M + 8 N, no row_ptr; 2 or 4 bytes of column field and 8 or 1
+of value per slot), each over its time, and whether AUTO and the fp64 image give ALGO_ROW's bits (it must wherever AUTO is a
 serial-order kernel: the image, ROW, STREAM; uniform 32 per row is too long for the image and stays on the vector kernel,
 whose shuffle sums differ in the last bits).  The device name and power limit are read in the same run.
 """
@@ -70,21 +71,28 @@ def run(name, make, reps, launches):
     torch.cuda.synchronize()
     plan_s = time.perf_counter() - t0
     i = A.info()
+    B = make()
+    B.set_image(1)  # the fp64 image, whatever the plan chose
+    ib = B.info()
     g = torch.Generator(device="cuda").manual_seed(11)
     x = torch.randn(i.N, dtype=torch.float64, device="cuda", generator=g)
     y_row = torch.empty(i.M, dtype=torch.float64, device="cuda")
     y_auto = torch.empty(i.M, dtype=torch.float64, device="cuda")
-    for algo, y in ((d.ALGO_ROW, y_row), (d.ALGO_AUTO, y_auto)):
-        arm_ms(A, x, y, algo, launches)
+    y_f64 = torch.empty(i.M, dtype=torch.float64, device="cuda")
+    arms = ((A, d.ALGO_ROW, y_row), (A, d.ALGO_AUTO, y_auto), (B, d.ALGO_ROW_IMAGE, y_f64))
+    for H, algo, y in arms:
+        arm_ms(H, x, y, algo, launches)
     torch.cuda.synchronize()
     bitwise = bool(torch.equal(y_row.view(torch.int64), y_auto.view(torch.int64)))
-    t_row, t_auto = [], []
+    bitwise_f64 = bool(torch.equal(y_row.view(torch.int64), y_f64.view(torch.int64)))
+    t_row, t_auto, t_f64 = [], [], []
     for _ in range(reps):
-        t_row.append(arm_ms(A, x, y_row, d.ALGO_ROW, launches))
-        t_auto.append(arm_ms(A, x, y_auto, d.ALGO_AUTO, launches))
+        for (H, algo, y), ts in zip(arms, (t_row, t_auto, t_f64)):
+            ts.append(arm_ms(H, x, y, algo, launches))
     on_image = i.auto_algo == d.ALGO_ROW_IMAGE
     alg = i.algorithmic_bytes
     read = (i.image_device_bytes + 8 * i.M + 8 * i.N) if on_image else alg
+    read_f64 = ib.image_device_bytes + 8 * i.M + 8 * i.N
     auto_kernel = A.image_form() if on_image else (f"csr_row_kernel<{i.row_batch},double>" if i.auto_algo == d.ALGO_ROW
                                                    else d.ALGO_NAMES[i.auto_algo])
 
@@ -93,16 +101,23 @@ def run(name, make, reps, launches):
                 "spread_us": 1e3 * (max(ts) - min(ts))}
     out = {"M": i.M, "N": i.N, "nnz": i.nnz, "max_row_nnz": i.max_row_nnz, "plan_s": plan_s,
            "row_kernel": f"csr_row_kernel<{i.row_batch},double>", "auto_algo": i.auto_algo, "auto_kernel": auto_kernel,
-           "image_bytes": i.image_bytes, "image_device_bytes": i.image_device_bytes, "image_index_bytes": i.image_index_bytes, "csr_array_bytes": 12 * i.nnz + 4 * (i.M + 1),
+           "image_bytes": i.image_bytes, "image_device_bytes": i.image_device_bytes, "image_index_bytes": i.image_index_bytes,
+           "image_value_bytes": i.image_value_bytes, "csr_array_bytes": 12 * i.nnz + 4 * (i.M + 1),
            "algorithmic_bytes": alg, "read_bytes_auto": read,
            "row": stats(t_row), "auto": stats(t_auto), "speedup_row_over_auto": statistics.mean(t_row) / statistics.mean(t_auto),
            "algorithmic_TBps_auto": alg / (1e-3 * statistics.mean(t_auto)) / 1e12,
            "read_TBps_auto": read / (1e-3 * statistics.mean(t_auto)) / 1e12,
-           "auto_bitwise_equal_row": bitwise}
+           "auto_bitwise_equal_row": bitwise,
+           "image_f64": {"kernel": B.image_form(), "image_device_bytes": ib.image_device_bytes, "read_bytes": read_f64,
+                         **stats(t_f64), "read_TBps": read_f64 / (1e-3 * statistics.mean(t_f64)) / 1e12,
+                         "speedup_over_auto": statistics.mean(t_f64) / statistics.mean(t_auto),
+                         "bitwise_equal_row": bitwise_f64}}
     print(f"[csr_image] {name}: row {out['row']['mean_us']:.1f} us, auto {out['auto']['mean_us']:.1f} us "
-          f"({auto_kernel}), x{out['speedup_row_over_auto']:.3f}, bitwise {bitwise}, plan {plan_s:.2f} s", flush=True)
+          f"({auto_kernel}), fp64 image {out['image_f64']['mean_us']:.1f} us ({B.image_form()}), "
+          f"x{out['speedup_row_over_auto']:.3f}, bitwise {bitwise}/{bitwise_f64}, plan {plan_s:.2f} s", flush=True)
     A.close()
-    del x, y_row, y_auto
+    B.close()
+    del x, y_row, y_auto, y_f64
     torch.cuda.empty_cache()
     return out
 

@@ -1,6 +1,6 @@
 """Survey of the multi-row forms of the row kernels (csr_rowm_kernel / hll_rowm_kernel) in the built library, and of the
 one-row kernels including the masked forms that multiply a CSR handle's private image (accumulate or not, 4-byte `int` or
-narrow 2-byte `u16` column field): registers,
+narrow 2-byte `u16` column field, fp64 values or 1-byte `u8` value codes): registers,
 spill bytes (csrc/build/*.ptxas.log) and how many of a step's loads ptxas issues ahead of the first multiply (cuobjdump
 -sass).  A form whose loads are split by a DMUL stalls on its first gather before the rest is requested.  No GPU needed.
 
@@ -37,10 +37,10 @@ def main():
     rows = []
     for body in re.split(r"Function : ", sass)[1:]:
         name = body.split()[0]
-        m = re.search(r"(csr|hll)_row(m|u?)_kernelILi(\d)E(?:Li(\d)ELi(\d)E)?([fd])(?:Lb([01])E)?(?:Lb([01])E)?([it])?", name)
+        m = re.search(r"(csr|hll)_row(m|u?)_kernelILi(\d)E(?:Li(\d)ELi(\d)E)?([fd])(?:Lb([01])E)?(?:Lb([01])E)?([it])?([dfh])?", name)
         if not m:
             continue
-        fmt, multi, batch, rows_per, ctas, v, masked, accum, index = m.groups()
+        fmt, multi, batch, rows_per, ctas, v, masked, accum, index, stored = m.groups()
         ops = re.findall(r"\b(LDG|DMUL)\b", body)
         ahead = 0
         for op in ops:
@@ -48,14 +48,21 @@ def main():
                 break
             ahead += 1
         total = ops.count("LDG")
+        # the most loads any path issues between two multiplies: the straight-line step of hll_rowu_kernel (width equal
+        # to the batch) may sit after the predicated loop in the code, where the first DMUL above finds the loop's
+        most, run = 0, 0
+        for op in ops:
+            run = 0 if op == "DMUL" else run + 1
+            most = max(most, run)
         rec = info.get(name, {})
-        rows.append((fmt, v, int(rows_per or 1), int(batch), int(ctas or 8), rec.get("regs"), rec.get("spill"), ahead, total,
+        rows.append((fmt, v, int(rows_per or 1), int(batch), int(ctas or 8), rec.get("regs"), rec.get("spill"), ahead, most, total,
                      "row" + multi + (" masked" if masked == "1" else "") + (" accum" if accum == "1" else "")
-                     + (" u16" if index == "t" else "")))
-    print("format storage rows batch ctas/SM regs spill_bytes loads_ahead_of_first_DMUL/loads rows_in_flight/SM kernel")
+                     + (" u16" if index == "t" else "") + (" u8" if stored == "h" else "")))
+    print("format storage rows batch ctas/SM regs spill_bytes loads_ahead_of_first_DMUL/loads most_loads_between_DMULs "
+          "rows_in_flight/SM kernel")
     for r in sorted(rows):
-        fmt, v, rp, b, c, regs, spill, ahead, total, kind = r
-        print(f"{fmt} {'f32' if v == 'f' else 'f64'} {rp} {b} {c} {regs} {spill} {ahead}/{total} {256 * c * rp} {kind}")
+        fmt, v, rp, b, c, regs, spill, ahead, most, total, kind = r
+        print(f"{fmt} {'f32' if v == 'f' else 'f64'} {rp} {b} {c} {regs} {spill} {ahead}/{total} {most} {256 * c * rp} {kind}")
 
 
 if __name__ == "__main__":
