@@ -372,6 +372,24 @@ int spmv_b200_csr_spmv_host_f32(spmv_b200_csr *A, const float *x, float *y);
 int spmv_b200_hll_enable_f32(spmv_b200_hll *H, void *stream);
 int spmv_b200_hll_spmv_f32(const spmv_b200_hll *H, const float *d_x, float *d_y, void *stream);
 int spmv_b200_hll_spmv_host_f32(spmv_b200_hll *H, const float *x, float *y);
+/* Multi-vector products on the float copy (spmv_b200_version() >= 105): X, Y and the values are float, the conventions
+ * those of spmv_b200_csr_spmm / spmv_b200_hll_spmm (row-major, ld >= k, 64-bit offsets, only rows < M and columns < k of
+ * Y written, no overlap, k = 0 and M = 0 no-ops, nnz = 0 gives zero or leaves Y with accumulate).  A widened float times
+ * a widened float is exact in double (24 + 24 significand bits), so the only roundings are the adds and the final store:
+ *   CSR, rows of at most info.long_threshold nonzeros: column c of Y is bit for bit spmv_b200_csr_spmv_f32(...,
+ *     SPMV_B200_ALGO_ROW) on column c of X -- the serial fp64 loop over the widened values and x, rounded once to float;
+ *     accumulate != 0 starts each sum from (double)Y[i,c].
+ *   CSR, longer rows: each fragment summed as the same fixed sub-ranges and tree as the fp64 product, in double, the
+ *     fragments added in order and rounded once; within ulp32(y) + (len + 2) 2^-53 sum_j |a_ij x_jc| of the exact sum,
+ *     identical bits from call to call, and the bits of a column do not depend on k, ldx, ldy or its position in X.
+ *   HLL, every row (hacks of any width): serial in j with the padding slots included, rounded once -- the bits of the
+ *     lane-per-row kernel hll_row_kernel<B,float>.  No accumulate flag.
+ * Without spmv_b200_{csr,hll}_enable_f32 on the handle they return SPMV_B200_ERR_INVALID and launch nothing; bad k, ld or
+ * NULL arguments are rejected as by the fp64 forms.  The CSR form shares the fp64 form's partials buffer. */
+int spmv_b200_csr_spmm_f32(const spmv_b200_csr *A, int k, const float *d_X, long long ldx, float *d_Y, long long ldy,
+                           int accumulate, void *stream);
+int spmv_b200_hll_spmm_f32(const spmv_b200_hll *H, int k, const float *d_X, long long ldx, float *d_Y, long long ldy,
+                           void *stream);
 /* Which form of the row kernel enable_f32 timed fastest for this matrix: 1..8 = csr_row_kernel / hll_row_kernel with that
  * many loads in flight per row; >= 16 = form (id - 16) of csr_rowm_kernel / hll_rowm_kernel (index-only predicates, so
  * that every load of a step is issued ahead of the first multiply; rows per thread, loads in flight per row and CTAs

@@ -19,6 +19,8 @@
 //   * hll_spmm_kernel<KT,BATCH>  -- the same lane mapping over the column-major HLL image: a warp covers 32/KT rows of a
 //       hack, slot loads JA/AS[off + 32 j + r] are contiguous across those rows, j runs in order and the padding slots
 //       (x 0.0) are included: column c is bit for bit spmv_hll_serial on column c (hll_row_kernel's order).
+// Every kernel takes the storage type V of values, X and Y: double, or float for the copy of enable_f32 (the *_spmm_f32
+// entry points).  Loads are widened to double, accumulators and fragment partials are double, and Y is rounded to V once.
 #include <algorithm>
 
 #include "common.cuh"
@@ -34,8 +36,11 @@ constexpr int kSpmmSubLen = kSpmmFragNnz / kSpmmSubRanges;
 // Column / value loads in flight per lane before the first gather, per format.  Swept over {2, 4, 8} with
 // tools/spmm_bench.py --batches on a B200 at 1000 W (profiles/r03a_spmm_batch_sweep.json): CSR 2 and 4 within 4 % of
 // each other and 8 slower; HLL 8 fastest on lap2d and on uniform for k >= 8.  SPMV_B200_SPMM_BATCH in {2, 4, 8}
-// overrides both (for such sweeps).
+// overrides both (for such sweeps).  The fp32 products, swept the same way (profiles/r03e_spmm_f32_batch_sweep.json): CSR 2
+// fastest on lap2d, on R-MAT and on uniform for k >= 8 (uniform k = 32: 9.03 ms against 11.20 at 4), within 7 % of 4
+// elsewhere; HLL 8 fastest for k >= 2, as in fp64.
 constexpr int kSpmmBatchCsr = 4;
+constexpr int kSpmmBatchCsr32 = 2;
 constexpr int kSpmmBatchHll = 8;
 
 // Lanes per row for a tile of `cols` columns: the smallest power of two >= cols (cols <= 32).
@@ -53,17 +58,17 @@ __device__ __forceinline__ int hll_load_col(const int *p) {
     if constexpr (KT == 1) return ldg_stream_s32(p);
     else return __ldg(p);
 }
-template <int KT>
-__device__ __forceinline__ double hll_load_val(const double *p) {
+template <int KT, typename V>
+__device__ __forceinline__ double hll_load_val(const V *p) {
     if constexpr (KT == 1) return ldg_stream_f64(p);
-    else return __ldg(p);
+    else return (double)__ldg(p);
 }
 
 // grid.x: blocks of 256/KT rows; grid.y: column tiles of KT columns starting at c0 + 32*blockIdx.y (cols <= KT live lanes)
-template <int KT, int BATCH>
+template <int KT, int BATCH, typename V>
 __global__ void __launch_bounds__(kSpmmThreads)
-csr_spmm_kernel(int M, const int *__restrict__ row_ptr, const int *__restrict__ col_idx, const double *__restrict__ values,
-                int long_threshold, int c0, int cols, const double *__restrict__ X, long long ldx, double *__restrict__ Y,
+csr_spmm_kernel(int M, const int *__restrict__ row_ptr, const int *__restrict__ col_idx, const V *__restrict__ values,
+                int long_threshold, int c0, int cols, const V *__restrict__ X, long long ldx, V *__restrict__ Y,
                 long long ldy, int accumulate) {
     const long long row = (long long)blockIdx.x * (kSpmmThreads / KT) + threadIdx.x / KT;
     const int c = (int)(threadIdx.x & (KT - 1));
@@ -71,34 +76,35 @@ csr_spmm_kernel(int M, const int *__restrict__ row_ptr, const int *__restrict__ 
     const int lo = __ldg(row_ptr + row), hi = __ldg(row_ptr + row + 1);
     if (hi - lo > long_threshold) return;  // a long row of the plan: the fragment kernels own it
     const int col = c0 + kSpmmTile * (int)blockIdx.y + c;
-    const double *__restrict__ xc = X + col;
-    double *__restrict__ yp = Y + row * ldy + col;
-    double acc = accumulate ? *yp : 0.0;
+    const V *__restrict__ xc = X + col;
+    V *__restrict__ yp = Y + row * ldy + col;
+    double acc = accumulate ? (double)*yp : 0.0;
     for (int k = lo; k < hi; k += BATCH) {
         int ci[BATCH];
         double v[BATCH], xv[BATCH];
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) ci[u] = k + u < hi ? __ldg(col_idx + k + u) : -1;
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) v[u] = k + u < hi ? __ldg(values + k + u) : 0.0;
+        for (int u = 0; u < BATCH; ++u) v[u] = k + u < hi ? (double)__ldg(values + k + u) : 0.0;
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) xv[u] = ci[u] >= 0 ? __ldg(xc + (long long)ci[u] * ldx) : 0.0;
+        for (int u = 0; u < BATCH; ++u) xv[u] = ci[u] >= 0 ? (double)__ldg(xc + (long long)ci[u] * ldx) : 0.0;
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
             if (ci[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));  // one lane, index order: the serial loop
     }
-    *yp = acc;
+    *yp = (V)acc;
 }
 
 // One CTA per (fragment f, column tile of `cols` <= 32 columns at c0).  The (sub-range s, column c) pairs p = s * cols + c
 // are dealt to the threads round-robin (p = t, t + 256, ...), so the lanes of a warp cover consecutive columns of one or
 // a few sub-ranges (broadcast column / value loads, contiguous gathers) and a narrow tile still keeps 128 threads busy.
 // Which thread sums a pair changes with cols; the sum itself does not.  partial[f * 32 + c] = tree over the sub-range
-// sums of column c.
+// sums of column c (in double whatever V is).
+template <typename V>
 __global__ void __launch_bounds__(kSpmmThreads)
 csr_spmm_fragment_kernel(const int *__restrict__ long_rows, const int *__restrict__ frag_first, int num_long,
-                         const int *__restrict__ row_ptr, const int *__restrict__ col_idx, const double *__restrict__ values,
-                         int c0, int cols, const double *__restrict__ X, long long ldx, double *__restrict__ partial) {
+                         const int *__restrict__ row_ptr, const int *__restrict__ col_idx, const V *__restrict__ values,
+                         int c0, int cols, const V *__restrict__ X, long long ldx, double *__restrict__ partial) {
     __shared__ double sub[kSpmmSubRanges][kSpmmTile];
     const int f = (int)blockIdx.x;
     int lo = 0, hi = num_long;  // last long row whose first fragment is <= f
@@ -113,7 +119,7 @@ csr_spmm_fragment_kernel(const int *__restrict__ long_rows, const int *__restric
     constexpr int kBatch = 4;
     for (int p = (int)threadIdx.x; p < kSpmmSubRanges * cols; p += kSpmmThreads) {
         const int s = p / cols, c = p - s * cols;
-        const double *__restrict__ xc = X + c0 + c;
+        const V *__restrict__ xc = X + c0 + c;
         const long long sb = begin + (long long)s * kSpmmSubLen;
         const long long se = sb + kSpmmSubLen < end ? sb + kSpmmSubLen : end;
         double acc = 0.0;
@@ -124,9 +130,9 @@ csr_spmm_fragment_kernel(const int *__restrict__ long_rows, const int *__restric
 #pragma unroll
                 for (int u = 0; u < kBatch; ++u) ci[u] = k + u < se ? __ldg(col_idx + k + u) : -1;
 #pragma unroll
-                for (int u = 0; u < kBatch; ++u) v[u] = k + u < se ? __ldg(values + k + u) : 0.0;
+                for (int u = 0; u < kBatch; ++u) v[u] = k + u < se ? (double)__ldg(values + k + u) : 0.0;
 #pragma unroll
-                for (int u = 0; u < kBatch; ++u) xv[u] = ci[u] >= 0 ? __ldg(xc + (long long)ci[u] * ldx) : 0.0;
+                for (int u = 0; u < kBatch; ++u) xv[u] = ci[u] >= 0 ? (double)__ldg(xc + (long long)ci[u] * ldx) : 0.0;
 #pragma unroll
                 for (int u = 0; u < kBatch; ++u)
                     if (ci[u] >= 0) acc = fma(v[u], xv[u], acc);
@@ -146,25 +152,26 @@ csr_spmm_fragment_kernel(const int *__restrict__ long_rows, const int *__restric
     if (threadIdx.x < (unsigned)cols) partial[(long long)f * kSpmmTile + threadIdx.x] = sub[0][threadIdx.x];
 }
 
-// One thread per (long row, column of the tile): Y (or 0) plus the row's fragments, in order.
+// One thread per (long row, column of the tile): Y (or 0) plus the row's fragments, in order, rounded to V once.
+template <typename V>
 __global__ void csr_spmm_combine_kernel(const int *__restrict__ long_rows, const int *__restrict__ frag_first, int num_long,
-                                        const double *__restrict__ partial, int c0, int cols, double *__restrict__ Y,
+                                        const double *__restrict__ partial, int c0, int cols, V *__restrict__ Y,
                                         long long ldy, int accumulate) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int i = (int)(t / kSpmmTile), c = (int)(t % kSpmmTile);
     if (i >= num_long || c >= cols) return;
-    double *yp = Y + (long long)long_rows[i] * ldy + c0 + c;
-    double acc = accumulate ? *yp : 0.0;
+    V *yp = Y + (long long)long_rows[i] * ldy + c0 + c;
+    double acc = accumulate ? (double)*yp : 0.0;
     for (int f = frag_first[i]; f < frag_first[i + 1]; ++f) acc += partial[(long long)f * kSpmmTile + c];  // fixed order
-    *yp = acc;
+    *yp = (V)acc;
 }
 
 // grid.x: blocks of 256/KT rows of the padded image (num_hacks * 32 rows); grid.y: column tiles as csr_spmm_kernel
-template <int KT, int BATCH>
+template <int KT, int BATCH, typename V>
 __global__ void __launch_bounds__(kSpmmThreads)
 hll_spmm_kernel(int M, int num_hacks, const long long *__restrict__ hack_off, const int *__restrict__ JA,
-                const double *__restrict__ AS, int c0, int cols, const double *__restrict__ X, long long ldx,
-                double *__restrict__ Y, long long ldy) {
+                const V *__restrict__ AS, int c0, int cols, const V *__restrict__ X, long long ldx,
+                V *__restrict__ Y, long long ldy) {
     const long long prow = (long long)blockIdx.x * (kSpmmThreads / KT) + threadIdx.x / KT;  // row of the padded image
     const int c = (int)(threadIdx.x & (KT - 1));
     const int hack = (int)(prow >> 5), r = (int)(prow & 31);
@@ -173,7 +180,7 @@ hll_spmm_kernel(int M, int num_hacks, const long long *__restrict__ hack_off, co
     const int width = (int)((__ldg(hack_off + hack + 1) - off) >> 5);
     const long long base = off + r;
     const int col = c0 + kSpmmTile * (int)blockIdx.y + c;
-    const double *__restrict__ xc = X + col;
+    const V *__restrict__ xc = X + col;
     double acc = 0.0;
     for (int j = 0; j < width; j += BATCH) {
         int ci[BATCH];
@@ -183,12 +190,12 @@ hll_spmm_kernel(int M, int num_hacks, const long long *__restrict__ hack_off, co
 #pragma unroll
         for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? hll_load_val<KT>(AS + base + (long long)(j + u) * 32) : 0.0;
 #pragma unroll
-        for (int u = 0; u < BATCH; ++u) xv[u] = ci[u] >= 0 ? __ldg(xc + (long long)ci[u] * ldx) : 0.0;
+        for (int u = 0; u < BATCH; ++u) xv[u] = ci[u] >= 0 ? (double)__ldg(xc + (long long)ci[u] * ldx) : 0.0;
 #pragma unroll
         for (int u = 0; u < BATCH; ++u)
             if (ci[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));  // padding slots included: 0.0 * x
     }
-    if (prow < M) Y[prow * ldy + col] = acc;
+    if (prow < M) Y[prow * ldy + col] = (V)acc;
 }
 
 static int spmm_batch(int fallback) {
@@ -244,13 +251,54 @@ struct HllSpmmLaunch {
     }
 };
 
-static int check_spmm_args(const char *what, const void *h, int k, const double *X, long long ldx, const double *Y,
+static int check_spmm_args(const char *what, const void *h, int k, const void *X, long long ldx, const void *Y,
                            long long ldy) {
     if (k < 0) return fail(SPMV_B200_ERR_INVALID, "%s: negative k (%d)", what, k);
     if (ldx < k || ldy < k)
         return fail(SPMV_B200_ERR_INVALID, "%s: leading dimensions must be >= k (k=%d ldx=%lld ldy=%lld)", what, k, ldx, ldy);
     if (k > 0 && (!h || !X || !Y)) return fail(SPMV_B200_ERR_INVALID, "%s: NULL argument", what);
     return SPMV_B200_OK;
+}
+
+// The products behind the entry points (arguments checked, k > 0, M > 0): V = double on the fp64 values, V = float on
+// the copy of enable_f32; every sum is formed in double either way.
+template <typename V>
+static int csr_spmm(const spmv_b200_csr *A, const V *values, int k, const V *d_X, long long ldx, V *d_Y, long long ldy,
+                    int accumulate, cudaStream_t stream) {
+    const int batch = spmm_batch(sizeof(V) == 4 ? kSpmmBatchCsr32 : kSpmmBatchCsr);
+    const int M = A->M;
+    const int acc = accumulate ? 1 : 0;
+    SPMV_TRY(spmm_tiles(k, [&](int kt, int c0, int cols, int tiles) {
+        const dim3 grid(blocks_for(M, kSpmmThreads / kt), (unsigned)tiles);
+        return spmm_dispatch<CsrSpmmLaunch>(kt, batch, grid, stream, M, (const int *)A->row_ptr, (const int *)A->col_idx,
+                                            values, A->long_threshold, c0, cols, d_X, ldx, d_Y, ldy, acc);
+    }));
+    if (A->num_long == 0) return SPMV_B200_OK;
+    // the long rows: one fragment + combine launch pair per column tile, through the handle's partials buffer
+    if (!A->spmm_partial) SPMV_TRY_CUDA(cudaMalloc(&A->spmm_partial, (size_t)A->num_frag * kSpmmTile * sizeof(double)));
+    for (int c0 = 0; c0 < k; c0 += kSpmmTile) {
+        const int cols = std::min(kSpmmTile, k - c0);
+        csr_spmm_fragment_kernel<V><<<A->num_frag, kSpmmThreads, 0, stream>>>(A->long_rows, A->frag_first, A->num_long,
+                                                                               A->row_ptr, A->col_idx, values, c0, cols,
+                                                                               d_X, ldx, A->spmm_partial);
+        SPMV_TRY_CUDA(cudaGetLastError());
+        csr_spmm_combine_kernel<V><<<blocks_for((long long)A->num_long * kSpmmTile, 128), 128, 0, stream>>>(
+            A->long_rows, A->frag_first, A->num_long, A->spmm_partial, c0, cols, d_Y, ldy, acc);
+        SPMV_TRY_CUDA(cudaGetLastError());
+    }
+    return SPMV_B200_OK;
+}
+
+template <typename V>
+static int hll_spmm(const spmv_b200_hll *H, const V *AS, int k, const V *d_X, long long ldx, V *d_Y, long long ldy,
+                    cudaStream_t stream) {
+    const int batch = spmm_batch(kSpmmBatchHll);
+    const long long rows = (long long)H->num_hacks * 32;
+    return spmm_tiles(k, [&](int kt, int c0, int cols, int tiles) {
+        const dim3 grid(blocks_for(rows, kSpmmThreads / kt), (unsigned)tiles);
+        return spmm_dispatch<HllSpmmLaunch>(kt, batch, grid, stream, H->M, H->num_hacks, (const long long *)H->hack_off,
+                                            (const int *)H->JA, AS, c0, cols, d_X, ldx, d_Y, ldy);
+    });
 }
 
 }  // namespace spmv
@@ -260,46 +308,33 @@ using namespace spmv;
 extern "C" {
 
 int spmv_b200_csr_spmm(const spmv_b200_csr *A, int k, const double *d_X, long long ldx, double *d_Y, long long ldy,
-                       int accumulate, void *stream_) {
+                       int accumulate, void *stream) {
     SPMV_TRY(check_spmm_args("csr_spmm", A, k, d_X, ldx, d_Y, ldy));
     if (k == 0 || A->M == 0) return SPMV_B200_OK;
-    const cudaStream_t stream = as_stream(stream_);
-    const int batch = spmm_batch(kSpmmBatchCsr);
-    const int M = A->M;
-    const int acc = accumulate ? 1 : 0;
-    SPMV_TRY(spmm_tiles(k, [&](int kt, int c0, int cols, int tiles) {
-        const dim3 grid(blocks_for(M, kSpmmThreads / kt), (unsigned)tiles);
-        return spmm_dispatch<CsrSpmmLaunch>(kt, batch, grid, stream, M, (const int *)A->row_ptr, (const int *)A->col_idx,
-                                            (const double *)A->values, A->long_threshold, c0, cols, d_X, ldx, d_Y, ldy, acc);
-    }));
-    if (A->num_long == 0) return SPMV_B200_OK;
-    // the long rows: one fragment + combine launch pair per column tile, through the handle's partials buffer
-    if (!A->spmm_partial) SPMV_TRY_CUDA(cudaMalloc(&A->spmm_partial, (size_t)A->num_frag * kSpmmTile * sizeof(double)));
-    for (int c0 = 0; c0 < k; c0 += kSpmmTile) {
-        const int cols = std::min(kSpmmTile, k - c0);
-        csr_spmm_fragment_kernel<<<A->num_frag, kSpmmThreads, 0, stream>>>(A->long_rows, A->frag_first, A->num_long,
-                                                                            A->row_ptr, A->col_idx, A->values, c0, cols,
-                                                                            d_X, ldx, A->spmm_partial);
-        SPMV_TRY_CUDA(cudaGetLastError());
-        csr_spmm_combine_kernel<<<blocks_for((long long)A->num_long * kSpmmTile, 128), 128, 0, stream>>>(
-            A->long_rows, A->frag_first, A->num_long, A->spmm_partial, c0, cols, d_Y, ldy, acc);
-        SPMV_TRY_CUDA(cudaGetLastError());
-    }
-    return SPMV_B200_OK;
+    return csr_spmm(A, (const double *)A->values, k, d_X, ldx, d_Y, ldy, accumulate, as_stream(stream));
+}
+
+int spmv_b200_csr_spmm_f32(const spmv_b200_csr *A, int k, const float *d_X, long long ldx, float *d_Y, long long ldy,
+                           int accumulate, void *stream) {
+    SPMV_TRY(check_spmm_args("csr_spmm_f32", A, k, d_X, ldx, d_Y, ldy));
+    if (A && !A->values32) return fail(SPMV_B200_ERR_INVALID, "csr_spmm_f32: call spmv_b200_csr_enable_f32 first");
+    if (k == 0 || A->M == 0) return SPMV_B200_OK;
+    return csr_spmm(A, (const float *)A->values32, k, d_X, ldx, d_Y, ldy, accumulate, as_stream(stream));
 }
 
 int spmv_b200_hll_spmm(const spmv_b200_hll *H, int k, const double *d_X, long long ldx, double *d_Y, long long ldy,
-                       void *stream_) {
+                       void *stream) {
     SPMV_TRY(check_spmm_args("hll_spmm", H, k, d_X, ldx, d_Y, ldy));
     if (k == 0 || H->M == 0 || H->num_hacks == 0) return SPMV_B200_OK;
-    const cudaStream_t stream = as_stream(stream_);
-    const int batch = spmm_batch(kSpmmBatchHll);
-    const long long rows = (long long)H->num_hacks * 32;
-    return spmm_tiles(k, [&](int kt, int c0, int cols, int tiles) {
-        const dim3 grid(blocks_for(rows, kSpmmThreads / kt), (unsigned)tiles);
-        return spmm_dispatch<HllSpmmLaunch>(kt, batch, grid, stream, H->M, H->num_hacks, (const long long *)H->hack_off,
-                                            (const int *)H->JA, (const double *)H->AS, c0, cols, d_X, ldx, d_Y, ldy);
-    });
+    return hll_spmm(H, (const double *)H->AS, k, d_X, ldx, d_Y, ldy, as_stream(stream));
+}
+
+int spmv_b200_hll_spmm_f32(const spmv_b200_hll *H, int k, const float *d_X, long long ldx, float *d_Y, long long ldy,
+                           void *stream) {
+    SPMV_TRY(check_spmm_args("hll_spmm_f32", H, k, d_X, ldx, d_Y, ldy));
+    if (H && !H->AS32) return fail(SPMV_B200_ERR_INVALID, "hll_spmm_f32: call spmv_b200_hll_enable_f32 first");
+    if (k == 0 || H->M == 0 || H->num_hacks == 0) return SPMV_B200_OK;
+    return hll_spmm(H, (const float *)H->AS32, k, d_X, ldx, d_Y, ldy, as_stream(stream));
 }
 
 }  // extern "C"

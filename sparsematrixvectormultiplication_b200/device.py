@@ -56,13 +56,13 @@ def _host_vectors(x, y, n, m, dtype):
     return x, y
 
 
-def _check_dense(t, rows, what):
-    """A row-major block of a multi-vector product: a 2-D float64 CUDA tensor of `rows` rows whose columns are
+def _check_dense(t, rows, what, dtype="float64"):
+    """A row-major block of a multi-vector product: a 2-D CUDA tensor of `dtype` with `rows` rows whose columns are
     adjacent (column stride 1) and whose row stride, the leading dimension, is at least the column count.  Strides
     of dimensions of size 1 do not matter, as in torch.  Returns (columns, leading dimension)."""
     import torch
-    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and t.dim() == 2):
-        raise ValueError(f"{what} must be a 2-D float64 CUDA tensor")
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == getattr(torch, dtype) and t.dim() == 2):
+        raise ValueError(f"{what} must be a 2-D {dtype} CUDA tensor")
     n, k = t.shape
     if n != rows:
         raise ValueError(f"{what} must have {rows} rows (got shape {tuple(t.shape)})")
@@ -74,29 +74,29 @@ def _check_dense(t, rows, what):
     return k, ld
 
 
-def _dense_overlap(a, lda, b, ldb, k):
-    """Do the row-major k-column blocks a (leading dimension lda) and b (ldb) share an element?  Exact when the
-    leading dimensions are equal (interleaved column slices of one buffer do not overlap), conservative otherwise:
-    then any intersection of the two address ranges counts."""
+def _dense_overlap(a, lda, b, ldb, k, size=8):
+    """Do the row-major k-column blocks a (leading dimension lda) and b (ldb) of `size`-byte elements share an element?
+    Exact when the leading dimensions are equal (interleaved column slices of one buffer do not overlap), conservative
+    otherwise: then any intersection of the two address ranges counts."""
     if k == 0 or a.numel() == 0 or b.numel() == 0:
         return False
     pa, pb = a.data_ptr(), b.data_ptr()
-    ea = pa + 8 * ((a.shape[0] - 1) * lda + k)
-    eb = pb + 8 * ((b.shape[0] - 1) * ldb + k)
+    ea = pa + size * ((a.shape[0] - 1) * lda + k)
+    eb = pb + size * ((b.shape[0] - 1) * ldb + k)
     if ea <= pb or eb <= pa:
         return False
-    if lda != ldb or (pb - pa) % 8:
+    if lda != ldb or (pb - pa) % size:
         return True
-    s = ((pb - pa) // 8) % lda  # b's columns sit at residues [s, s + k) modulo ld, a's at [0, k)
+    s = ((pb - pa) // size) % lda  # b's columns sit at residues [s, s + k) modulo ld, a's at [0, k)
     return s < k or s + k > lda
 
 
-def _spmm_operands(X, Y, M, N_):
-    k, ldx = _check_dense(X, N_, "X")
-    ky, ldy = _check_dense(Y, M, "Y")
+def _spmm_operands(X, Y, M, N_, dtype="float64"):
+    k, ldx = _check_dense(X, N_, "X", dtype)
+    ky, ldy = _check_dense(Y, M, "Y", dtype)
     if ky != k:
         raise ValueError(f"X and Y must have the same number of columns (got {k} and {ky})")
-    if _dense_overlap(X, ldx, Y, ldy, k):
+    if _dense_overlap(X, ldx, Y, ldy, k, X.element_size()):
         raise ValueError("Y must not overlap X")
     return k, ldx, ldy
 
@@ -349,6 +349,16 @@ class DeviceCSR:
         N.check(N.lib().spmv_b200_csr_spmv_f32(self._h, _ptr(x), _ptr(y), int(bool(accumulate)), algo, _stream(stream)))
         return y
 
+    def spmm_f32(self, X, Y, accumulate=False, stream=None):
+        """Y = A X (or Y += A X) as spmm, on float32 tensors through the float copy of enable_f32 (products and sums in
+        double, one rounding to float per element): on rows up to the long-row threshold each column is bit for bit
+        spmv_f32(algo=ALGO_ROW) on that column (spmv_b200_csr_spmm_f32).  SpmvError without enable_f32."""
+        i = self.info()
+        k, ldx, ldy = _spmm_operands(X, Y, i.M, i.N, "float32")
+        if k and i.M:
+            N.check(N.lib().spmv_b200_csr_spmm_f32(self._h, k, _ptr(X), ldx, _ptr(Y), ldy, int(bool(accumulate)), _stream(stream)))
+        return Y
+
     def spmv_host_f32(self, x, y=None):
         i = self.info()
         x, y = _host_vectors(x, y, i.N, i.M, np.float32)
@@ -450,6 +460,16 @@ class DeviceHLL:
         _check_vec(y, i.M, "y", "float32")
         N.check(N.lib().spmv_b200_hll_spmv_f32(self._h, _ptr(x), _ptr(y), _stream(stream)))
         return y
+
+    def spmm_f32(self, X, Y, stream=None):
+        """Y = A X as spmm, on float32 tensors through the float copy of enable_f32: each column bit for bit the
+        lane-per-row product in double, rounded once to float, on hacks of any width (spmv_b200_hll_spmm_f32).  No
+        accumulate flag; SpmvError without enable_f32."""
+        i = self.info()
+        k, ldx, ldy = _spmm_operands(X, Y, i.M, i.N, "float32")
+        if k and i.M:
+            N.check(N.lib().spmv_b200_hll_spmm_f32(self._h, k, _ptr(X), ldx, _ptr(Y), ldy, _stream(stream)))
+        return Y
 
     def spmv_host_f32(self, x, y=None):
         i = self.info()
