@@ -74,7 +74,8 @@ typedef struct {
     int auto_algo;       /* the SPMV_B200_ALGO_* that SPMV_B200_ALGO_AUTO resolves to        */
     int row_batch;       /* batch of the thread-per-row kernel (tuned at plan time)          */
     int fused_batch;     /* fused iterated product: 0 = fused stream kernel, else batch of the fused row kernel */
-    int flat_batch, flat_chunks; /* the FLAT fused row kernel of the two-launch iterated product (plan-time choice) */
+    int flat_batch;      /* batch of the FLAT fused row kernel of the two-launch iterated product (plan-time choice) */
+    int flat_chunks;     /* always 1: the FLAT kernel runs one CTA per 256 rows (kept for the layout of this struct) */
     long long image_bytes; /* size of the private image at 12 bytes per slot, as defined in version 102, whatever the
                               width of its column field (0: none, see spmv_b200_csr_set_image); image_device_bytes
                               is what it occupies */
@@ -95,7 +96,8 @@ typedef struct {
     long long algorithmic_bytes;   /* slots*12 + 8*(num_hacks+1) + 8*M + 8*N                 */
     int auto_kernel;        /* automatic choice: 0 slice, 1 stream, 2 rows                   */
     int row_batch;          /* batch of the lane-per-row kernel (tuned at plan time)         */
-    int fused_batch, flat_batch, flat_chunks; /* plan-time choices of the fused iterated product (grid-stride / FLAT) */
+    int fused_batch, flat_batch; /* plan-time choices of the fused iterated product (grid-stride / FLAT) */
+    int flat_chunks;        /* always 1: the FLAT kernel runs one CTA per 8 hacks (kept for the layout of this struct) */
 } spmv_b200_hll_info_t;
 
 /* ---- library / device ---------------------------------------------------------------- */

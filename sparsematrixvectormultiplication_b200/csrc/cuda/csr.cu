@@ -240,20 +240,12 @@ csr_vector4_kernel(int row_begin, int row_end, const int *__restrict__ row_ptr, 
     if (live && lane == 0) y[row] = (V)(accumulate ? (double)y[row] + acc : acc);
 }
 
-// One THREAD per row (stencil-like matrices, every row short).  Lane i walks row i: a warp's loads are strided by the
-// row length, so a sector is consumed over several iterations and must live in L1 in between -- plain read-only
-// loads that allocate, no shared memory (all 256 KB are L1), 8 CTAs x 256 threads per SM.  BATCH column/value loads
-// are issued before the first gather.  One lane, index order, mul and add rounded separately: every row is bit-identical
-// to the reference's serial loop (src/csr_matrix.c:134-138) -- and it is the reference's own thread-per-row idea
-// (cuda_src/csr_matrix_cuda.cu:122-146), which at 6.0 TB/s on lap2d 4096^2 is the kernel to beat on this chip.
+// The row loop of every thread-per-row CSR kernel: acc plus the products of row [lo, hi), BATCH column/value loads issued
+// before the first gather.  One lane, index order, mul and add rounded separately: every row is bit-identical to the
+// reference's serial loop (src/csr_matrix.c:134-138).
 template <int BATCH, typename V>
-__global__ void __launch_bounds__(256, 8)
-csr_row_kernel(int row_begin, int row_end, const int *__restrict__ row_ptr, const int *__restrict__ col_idx,
-               const V *__restrict__ values, const V *__restrict__ x, V *__restrict__ y, int accumulate) {
-    const long long row = row_begin + (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (row >= row_end) return;
-    const int lo = __ldg(row_ptr + row), hi = __ldg(row_ptr + row + 1);
-    double acc = accumulate ? (double)y[row] : 0.0;
+__device__ __forceinline__ double row_sum(int lo, int hi, const int *__restrict__ col_idx, const V *__restrict__ values,
+                                          const V *__restrict__ x, double acc) {
     for (int k = lo; k < hi; k += BATCH) {
         int c[BATCH];
         double v[BATCH], xv[BATCH];
@@ -267,7 +259,22 @@ csr_row_kernel(int row_begin, int row_end, const int *__restrict__ row_ptr, cons
         for (int u = 0; u < BATCH; ++u)
             if (c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
     }
-    y[row] = (V)acc;
+    return acc;
+}
+
+// One THREAD per row (stencil-like matrices, every row short).  Lane i walks row i: a warp's loads are strided by the
+// row length, so a sector is consumed over several iterations and must live in L1 in between -- plain read-only
+// loads that allocate, no shared memory (all 256 KB are L1), 8 CTAs x 256 threads per SM.  It is the reference's own
+// thread-per-row idea (cuda_src/csr_matrix_cuda.cu:122-146), which at 6.0 TB/s on lap2d 4096^2 is the kernel to beat on
+// this chip.
+template <int BATCH, typename V>
+__global__ void __launch_bounds__(256, 8)
+csr_row_kernel(int row_begin, int row_end, const int *__restrict__ row_ptr, const int *__restrict__ col_idx,
+               const V *__restrict__ values, const V *__restrict__ x, V *__restrict__ y, int accumulate) {
+    const long long row = row_begin + (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= row_end) return;
+    const int lo = __ldg(row_ptr + row), hi = __ldg(row_ptr + row + 1);
+    y[row] = (V)row_sum<BATCH>(lo, hi, col_idx, values, x, accumulate ? (double)y[row] : 0.0);
 }
 
 // csr_row_kernel in a second form (round 2e; candidates of the fp32 path): ROWS rows per thread, CTAS CTAs per SM, and --
@@ -365,19 +372,7 @@ csr_row_flat_kernel(int M, const int *__restrict__ row_ptr, const int *__restric
     double acc = 0.0;
     if (live) {
         const int lo = __ldg(row_ptr + row), hi = __ldg(row_ptr + row + 1);
-        for (int k = lo; k < hi; k += BATCH) {
-            int c[BATCH];
-            double v[BATCH], xv[BATCH];
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) c[u] = k + u < hi ? __ldg(col_idx + k + u) : -1;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) v[u] = k + u < hi ? __ldg(values + k + u) : 0.0;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) xv[u] = c[u] >= 0 ? __ldg(x + c[u]) : 0.0;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u)
-                if (c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
-        }
+        acc = row_sum<BATCH>(lo, hi, col_idx, values, x, 0.0);
         if (ep.inv_norm != nullptr) acc *= __ldg(ep.inv_norm);
         y[row] = acc;
         if (fused_chunk_is_boundary(ep, (long long)blockIdx.x * 256)) fused_peer_store(ep, row, acc);
@@ -419,20 +414,7 @@ csr_row_fused_kernel(int M, const int *__restrict__ row_ptr, const int *__restri
         const long long row = chunk_lo + threadIdx.x;
         if (row >= M) continue;
         const int lo = __ldg(row_ptr + row), hi = __ldg(row_ptr + row + 1);
-        double acc = 0.0;
-        for (int k = lo; k < hi; k += BATCH) {
-            int c[BATCH];
-            double v[BATCH], xv[BATCH];
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) c[u] = k + u < hi ? __ldg(col_idx + k + u) : -1;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) v[u] = k + u < hi ? __ldg(values + k + u) : 0.0;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) xv[u] = c[u] >= 0 ? __ldg(x + c[u]) : 0.0;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u)
-                if (c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
-        }
+        double acc = row_sum<BATCH>(lo, hi, col_idx, values, x, 0.0);
         if (scaled) acc *= inv_norm;
         sq = fma(acc, acc, sq);
         y[row] = acc;
@@ -521,20 +503,7 @@ csr_row_async_kernel(int M, const int *__restrict__ row_ptr, const int *__restri
         const long long row = (long long)chunk * 256 + threadIdx.x;
         if (row < M) {
             const int lo = __ldg(row_ptr + row), hi = __ldg(row_ptr + row + 1);
-            double acc = 0.0;
-            for (int e = lo; e < hi; e += BATCH) {
-                int c[BATCH];
-                double v[BATCH], xv[BATCH];
-#pragma unroll
-                for (int u = 0; u < BATCH; ++u) c[u] = e + u < hi ? __ldg(col_idx + e + u) : -1;
-#pragma unroll
-                for (int u = 0; u < BATCH; ++u) v[u] = e + u < hi ? __ldg(values + e + u) : 0.0;
-#pragma unroll
-                for (int u = 0; u < BATCH; ++u) xv[u] = c[u] >= 0 ? __ldg(x + c[u]) : 0.0;
-#pragma unroll
-                for (int u = 0; u < BATCH; ++u)
-                    if (c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
-            }
+            double acc = row_sum<BATCH>(lo, hi, col_idx, values, x, 0.0);
             acc *= scale;
             sq = fma(acc, acc, sq);
             y[row] = acc;
@@ -962,13 +931,10 @@ template <typename V>
 static int launch_rows(int row_begin, int row_end, const int *row_ptr, const int *col_idx, const V *values,
                        const V *x, V *y, int batch, int accumulate, cudaStream_t stream);
 static int safe_vector_nnz(const spmv_b200_csr *A);
-struct FlatChoice {
-    int batch, chunks;
-};
-static const FlatChoice kFlatCandidates[] = {{2, 1}, {3, 1}, {4, 1}, {5, 1}, {6, 1}, {7, 1}};
-static int flat_grid(long long M, int chunks_per_cta);
+static const int kFlatCandidates[] = {2, 3, 4, 5, 6, 7};
+static int flat_grid(long long M);
 static int launch_fused_flat(const spmv_b200_csr *A, const double *x, double *y, const Epilogue &ep, cudaStream_t stream,
-                             int batch, int chunks_per_cta);
+                             int batch);
 static int launch_fused(const spmv_b200_csr *A, const double *x, double *y, const Epilogue &ep, cudaStream_t stream, int batch);
 static int fused_row_grid(const spmv_b200_csr *A);
 
@@ -1134,19 +1100,18 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
             }
             cudaGetLastError();
             cudaFree(partials);
-            // the FLAT form (two-launch iterated product): batch x chunks per CTA
+            // the FLAT form (two-launch iterated product): its batch
             double *flat_partials = nullptr;
-            if (cudaMalloc(&flat_partials, (size_t)flat_grid(M, 1) * sizeof(double)) == cudaSuccess) {
+            if (cudaMalloc(&flat_partials, (size_t)flat_grid(M) * sizeof(double)) == cudaSuccess) {
                 Epilogue fe;
                 fe.partials = flat_partials;
+                fe.partials_total = flat_grid(M);
                 fe.inv_norm = flat_partials;  // any finite double will do for the timing
                 const int n = (int)(sizeof kFlatCandidates / sizeof kFlatCandidates[0]);
                 const int best = tune_candidates(M, A->N, n, 1, stream, [&](int i, double *x, double *y) {
-                    fe.partials_total = flat_grid(M, kFlatCandidates[i].chunks);
-                    return launch_fused_flat(A, x, y, fe, stream, kFlatCandidates[i].batch, kFlatCandidates[i].chunks);
+                    return launch_fused_flat(A, x, y, fe, stream, kFlatCandidates[i]);
                 });
-                A->flat_batch = kFlatCandidates[best].batch;
-                A->flat_chunks = kFlatCandidates[best].chunks;
+                A->flat_batch = kFlatCandidates[best];
             }
             cudaGetLastError();
             cudaFree(flat_partials);
@@ -1197,12 +1162,9 @@ static int launch_rows(int row_begin, int row_end, const int *row_ptr, const int
         return SPMV_B200_OK;
     }
     const unsigned int g = blocks_for(rows, 256);
-#define ROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(csr_row_kernel<B, V>, g, 256, 0, stream, keep, row_begin, row_end, row_ptr, col_idx, values, x, y, accumulate)); break;
-    switch (batch) {
-        ROW_CASE(1) ROW_CASE(2) ROW_CASE(3) ROW_CASE(5) ROW_CASE(6) ROW_CASE(7) ROW_CASE(8)
-        default: SPMV_TRY_CUDA(launch_x(csr_row_kernel<4, V>, g, 256, 0, stream, keep, row_begin, row_end, row_ptr, col_idx, values, x, y, accumulate)); break;
-    }
-#undef ROW_CASE
+    SPMV_TRY_CUDA((with_batch<4, 1, 2, 3, 5, 6, 7, 8>(batch, [&](auto B) {
+        return launch_x(csr_row_kernel<B, V>, g, 256, 0, stream, keep, row_begin, row_end, row_ptr, col_idx, values, x, y, accumulate);
+    })));
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
 }
@@ -1444,39 +1406,25 @@ static int launch_fused(const spmv_b200_csr *A, const double *x, double *y, cons
     if (batch < 0) batch = env_int("SPMV_B200_FUSED_BATCH", A->fused_batch);
     if (batch == 0) return stream_launch_csr(A, x, y, 0, &ep, stream);
     const int g = fused_row_grid(A);
-#define FROW_CASE(B) case B: csr_row_fused_kernel<B><<<g, 256, 0, stream>>>(A->M, A->row_ptr, A->col_idx, A->values, x, y, ep); break;
-    switch (batch) {
-        FROW_CASE(2) FROW_CASE(3) FROW_CASE(5) FROW_CASE(6) FROW_CASE(7)
-        default: csr_row_fused_kernel<4><<<g, 256, 0, stream>>>(A->M, A->row_ptr, A->col_idx, A->values, x, y, ep); break;
-    }
-#undef FROW_CASE
+    with_batch<4, 2, 3, 5, 6, 7>(batch, [&](auto B) {
+        csr_row_fused_kernel<B><<<g, 256, 0, stream>>>(A->M, A->row_ptr, A->col_idx, A->values, x, y, ep);
+    });
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
 }
 
 // ---- the FLAT form (two-launch iterated product): one CTA per 256 rows; the batch is timed at plan time ----
-static int flat_grid(long long M, int chunks_per_cta) {
-    (void)chunks_per_cta;
-    return (int)std::max<long long>(1, (M + 255) / 256);
-}
+static int flat_grid(long long M) { return (int)std::max<long long>(1, (M + 255) / 256); }
 
 static int launch_fused_flat(const spmv_b200_csr *A, const double *x, double *y, const Epilogue &ep, cudaStream_t stream,
-                             int batch, int chunks_per_cta) {
-    const int g = flat_grid(A->M, chunks_per_cta);
+                             int batch) {
+    const int g = flat_grid(A->M);
     const XPolicy keep = matrix_policy(A->row_ptr, (size_t)(A->M + 1) * sizeof(int));
-#define FLAT_CASE(B) case B: SPMV_TRY_CUDA(launch_x(csr_row_flat_kernel<B>, g, 256, 0, stream, keep, A->M, A->row_ptr, A->col_idx, A->values, x, y, ep)); break;
-    switch (batch) {
-        FLAT_CASE(2) FLAT_CASE(3) FLAT_CASE(5) FLAT_CASE(6) FLAT_CASE(7)
-        default: SPMV_TRY_CUDA(launch_x(csr_row_flat_kernel<4>, g, 256, 0, stream, keep, A->M, A->row_ptr, A->col_idx, A->values, x, y, ep)); break;
-    }
-#undef FLAT_CASE
+    SPMV_TRY_CUDA((with_batch<4, 2, 3, 5, 6, 7>(batch, [&](auto B) {
+        return launch_x(csr_row_flat_kernel<B>, g, 256, 0, stream, keep, A->M, A->row_ptr, A->col_idx, A->values, x, y, ep);
+    })));
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
-}
-
-static void flat_choice(const spmv_b200_csr *A, int &batch, int &chunks) {
-    batch = env_int("SPMV_B200_FLAT_BATCH", A->flat_batch);
-    chunks = std::max(1, env_int("SPMV_B200_FLAT_CHUNKS", A->flat_chunks));
 }
 
 int boundary_first_order(const spmv_b200_peers_t &peers, int M, ChunkOrder &order) {
@@ -1711,7 +1659,7 @@ int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info) {
     info->row_batch = A->row_batch;
     info->fused_batch = A->fused_batch;
     info->flat_batch = A->flat_batch;
-    info->flat_chunks = A->flat_chunks;
+    info->flat_chunks = 1;
     info->image_bytes = A->image ? 12 * A->image->slots : 0;
     info->image_form = A->image ? A->image_form & ~kImageCoded : 0;
     info->image_index_bytes = !A->image ? 0 : A->image->JA16 ? 2 : 4;
@@ -1771,9 +1719,7 @@ int spmv_b200_csr_spmv_fused(const spmv_b200_csr *A, const double *d_x, double *
 
 int spmv_b200_csr_flat_partials_count(const spmv_b200_csr *A) {
     if (!A) return 0;
-    int batch, chunks;
-    flat_choice(A, batch, chunks);
-    return flat_grid(A->M, chunks);
+    return flat_grid(A->M);
 }
 
 int spmv_b200_csr_spmv_fused_flat(const spmv_b200_csr *A, const double *d_x, double *d_y, const double *d_inv_norm,
@@ -1784,14 +1730,12 @@ int spmv_b200_csr_spmv_fused_flat(const spmv_b200_csr *A, const double *d_x, dou
     if (peers && (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS))
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_flat: bad peer count %d", peers->count);
     if (A->M == 0) return SPMV_B200_OK;
-    int batch, chunks;
-    flat_choice(A, batch, chunks);
     Epilogue ep;
     ep.inv_norm = d_inv_norm;
     ep.partials = d_partials;
-    ep.partials_total = flat_grid(A->M, chunks);
+    ep.partials_total = flat_grid(A->M);
     if (peers) ep.peers = *peers;
-    return launch_fused_flat(A, d_x, d_y, ep, as_stream(stream), batch, chunks);
+    return launch_fused_flat(A, d_x, d_y, ep, as_stream(stream), env_int("SPMV_B200_FLAT_BATCH", A->flat_batch));
 }
 
 int spmv_b200_csr_spmv_fused_mail(const spmv_b200_csr *A, const double *d_x, double *d_y, double *d_partials,
@@ -1844,12 +1788,9 @@ int spmv_b200_csr_spmv_fused_async(const spmv_b200_csr *A, const double *d_x, do
     args.peers = ps;
     args.as = *as;
     args.order = order;
-#define AROW_CASE(B) case B: csr_row_async_kernel<B><<<g, 256, 0, st>>>(A->M, A->row_ptr, A->col_idx, A->values, d_x, d_y, d_partials, args); break;
-    switch (A->fused_batch > 0 ? A->fused_batch : A->row_batch) {
-        AROW_CASE(2) AROW_CASE(3) AROW_CASE(5) AROW_CASE(6) AROW_CASE(7)
-        default: csr_row_async_kernel<4><<<g, 256, 0, st>>>(A->M, A->row_ptr, A->col_idx, A->values, d_x, d_y, d_partials, args); break;
-    }
-#undef AROW_CASE
+    with_batch<4, 2, 3, 5, 6, 7>(A->fused_batch > 0 ? A->fused_batch : A->row_batch, [&](auto B) {
+        csr_row_async_kernel<B><<<g, 256, 0, st>>>(A->M, A->row_ptr, A->col_idx, A->values, d_x, d_y, d_partials, args);
+    });
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
 }

@@ -1,6 +1,7 @@
 // handles.cuh -- the opaque handle types of include/spmv_b200.h (internal layout).
 #pragma once
 
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -233,7 +234,7 @@ struct spmv_b200_csr {
     int row_batch32 = 4; // the same for fp32 storage (tuned by spmv_b200_csr_enable_f32)
     bool short_rows_stream = false;  // plan-time timing found the stream kernel faster than every row-kernel batch
     int fused_batch = 0;             // fused iterated product: 0 = fused stream kernel, else batch of the fused row kernel
-    int flat_batch = 4, flat_chunks = 2;  // the FLAT fused row kernel (two-launch iterated product), timed at plan time
+    int flat_batch = 4;              // the FLAT fused row kernel (two-launch iterated product), timed at plan time
     // stream kernel launch shape
     int stages = spmv::kDefaultStages;
     int consumers = 12;
@@ -293,7 +294,7 @@ struct spmv_b200_hll {
     int row_form = 0;    // fp64 row path: 0 = hll_row_kernel<row_batch>; 64 + b = hll_rowu_kernel<b> (regular images, timed at plan time)
     int row_batch32 = 4; // the same for fp32 storage (tuned by spmv_b200_hll_enable_f32)
     int fused_batch = 0; // hll_row_fused_kernel batch (tuned at plan time; 0 = row_batch)
-    int flat_batch = 4, flat_chunks = 2;  // the FLAT form of hll_row_fused_kernel (two-launch iterated product)
+    int flat_batch = 4;  // the FLAT form of hll_row_fused_kernel (two-launch iterated product)
     bool narrow_stream = false;  // plan-time timing found the stream kernel faster than every row-kernel batch
     double *stage_x = nullptr;
     double *stage_y = nullptr;
@@ -366,6 +367,14 @@ inline cudaError_t launch_x(void (*kernel)(Params...), unsigned int grid, unsign
     cfg.attrs = const_cast<cudaLaunchAttribute *>(policy.attr);
     cfg.numAttrs = policy.count;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<Params>(args)...);
+}
+// Returns f(std::integral_constant<int, B>{}) for the B of Bs equal to batch, or for Default when none is: a launch site
+// names the batches its kernel is instantiated for and the one that any other batch runs.
+template <int Default, int B, int... Bs, class F>
+auto with_batch(int batch, F &&f) {
+    if (batch == B) return f(std::integral_constant<int, B>{});
+    if constexpr (sizeof...(Bs) == 0) return f(std::integral_constant<int, Default>{});
+    else return with_batch<Default, Bs...>(batch, f);
 }
 // Times launch(candidate) for candidate = first .. 7 on scratch vectors and returns the fastest (plan time, large
 // matrices).  Candidates 2..7 are batches of the row kernels; 0 (first = 0 only, 1 is skipped) stands for the stream kernel.

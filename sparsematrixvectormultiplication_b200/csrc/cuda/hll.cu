@@ -140,33 +140,18 @@ hll_slice_kernel(int hack_begin, int hack_end, const long long *__restrict__ hac
     }
 }
 
-// Row kernel for narrow hacks (stencils): one warp per hack, lane = row, the column-major image makes every load of a
-// warp one contiguous 128 B (JA) / 256 B (AS) segment -- no shared memory, no reliance on L1 for the stream.  BATCH
-// slots are requested before the first gather.  One lane per row, sequential in j, mul and add rounded separately:
-// bit-identical to the reference's spmv_hll_serial (src/hll_matrix.c:294-306), padding slots (x 0.0) included.
-// MASKED: the private image of a CSR handle (csr_image_build), whose padding slots carry bit 31 of the column (I = int) or
-// bit 15 of a row-relative 16-bit field (I = uint16_t, image_column).  Such a slot gathers its column like any other and
-// skips the add; ACCUM: the sum starts from y[row].  Bit-identical to csr_row_kernel for every x.  (Adding the padding's
-// 0 * x[c] would give NaN for an infinite x[c], and +0 turns an untouched -0.0 positive.)  The loads are never predicated
-// on the loaded column.  ACCUM is a template flag, not an argument: a y[row] load hoisted ahead of the step holds two of
-// the 32 registers and pushed two of the 15 loads of hll_rowu_kernel<5> behind the first multiply (cuobjdump,
-// tools/rowm_survey.py).  S: the stored value type -- V, or uint8_t for the coded private image (codes into `table`, K
-// entries, staged in shared memory; table and K are unused otherwise).
-template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false, typename I = int, typename S = V>
-__global__ void __launch_bounds__(256, 8)
-hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_off, const I *__restrict__ JA,
-               const S *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M, const double *__restrict__ table, int K) {
-    static_assert(sizeof(I) == 4 || (MASKED && sizeof(V) == 8), "the narrow index exists in the fp64 private image only");
-    static_assert(sizeof(S) == sizeof(V) || (MASKED && sizeof(V) == 8), "value codes exist in the fp64 private image only");
-    const double *tab = stage_image_table<S>(table, K);
-    const int hack = hack_begin + blockIdx.x * 8 + (threadIdx.x >> 5);
-    if (hack >= hack_end) return;  // warp-uniform
-    const int lane = threadIdx.x & 31;
-    const long long row = (long long)hack * kHack + lane;
-    const long long off = __ldg(hack_off + hack);
-    const int width = (int)((__ldg(hack_off + hack + 1) - off) >> 5);
-    const long long base = off + lane;
-    double acc = ACCUM && row < M ? (double)y[row] : 0.0;
+// The hack-row loop of every lane-per-row HLL kernel: acc plus the products of row `row` of a hack, whose slot j lies at
+// base + j * 32 (j < width), BATCH slots requested before the first gather.  One lane per row, sequential in j, mul and
+// add rounded separately: bit-identical to the reference's spmv_hll_serial (src/hll_matrix.c:294-306), padding slots
+// (x 0.0) included.  MASKED: the private image of a CSR handle (csr_image_build), whose padding slots carry bit 31 of the
+// column (I = int) or bit 15 of a row-relative 16-bit field (I = uint16_t, image_column).  Such a slot gathers its column
+// like any other and skips the add: bit-identical to csr_row_kernel for every x.  (Adding the padding's 0 * x[c] would
+// give NaN for an infinite x[c], and +0 turns an untouched -0.0 positive.)  The loads are never predicated on the loaded
+// column.  S: the stored value type -- V, or uint8_t for codes into `tab` (unused otherwise).
+template <int BATCH, typename V, bool MASKED = false, typename I = int, typename S = V>
+__device__ __forceinline__ double hack_row_sum(long long base, int width, long long row, const I *__restrict__ JA,
+                                               const S *__restrict__ AS, const V *__restrict__ x, const double *tab,
+                                               double acc) {
     for (int j = 0; j < width; j += BATCH) {
         int c[BATCH];
         stored_t<S> v[BATCH];
@@ -183,6 +168,29 @@ hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_
         for (int u = 0; u < BATCH; ++u)
             if (MASKED ? image_adds<I>(c[u]) : c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(image_value(v[u], tab), xv[u]));
     }
+    return acc;
+}
+
+// Row kernel for narrow hacks (stencils): one warp per hack, lane = row, the column-major image makes every load of a
+// warp one contiguous 128 B (JA) / 256 B (AS) segment -- no shared memory, no reliance on L1 for the stream.  MASKED, I
+// and S as in hack_row_sum; ACCUM: the sum starts from y[row].  ACCUM is a template flag, not an argument: a y[row] load
+// hoisted ahead of the step holds two of the 32 registers and pushed two of the 15 loads of hll_rowu_kernel<5> behind the
+// first multiply (cuobjdump, tools/rowm_survey.py).  The coded image's `table` (K entries) is staged in shared memory.
+template <int BATCH, typename V, bool MASKED = false, bool ACCUM = false, typename I = int, typename S = V>
+__global__ void __launch_bounds__(256, 8)
+hll_row_kernel(int hack_begin, int hack_end, const long long *__restrict__ hack_off, const I *__restrict__ JA,
+               const S *__restrict__ AS, const V *__restrict__ x, V *__restrict__ y, int M, const double *__restrict__ table, int K) {
+    static_assert(sizeof(I) == 4 || (MASKED && sizeof(V) == 8), "the narrow index exists in the fp64 private image only");
+    static_assert(sizeof(S) == sizeof(V) || (MASKED && sizeof(V) == 8), "value codes exist in the fp64 private image only");
+    const double *tab = stage_image_table<S>(table, K);
+    const int hack = hack_begin + blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (hack >= hack_end) return;  // warp-uniform
+    const int lane = threadIdx.x & 31;
+    const long long row = (long long)hack * kHack + lane;
+    const long long off = __ldg(hack_off + hack);
+    const int width = (int)((__ldg(hack_off + hack + 1) - off) >> 5);
+    const long long base = off + lane;
+    const double acc = hack_row_sum<BATCH, V, MASKED, I, S>(base, width, row, JA, AS, x, tab, ACCUM && row < M ? (double)y[row] : 0.0);
     if (row < M) y[row] = (V)acc;
 }
 
@@ -349,19 +357,7 @@ hll_row_flat_kernel(int num_hacks, const long long *__restrict__ hack_off, const
         const long long off = __ldg(hack_off + hack);
         const int width = (int)((__ldg(hack_off + hack + 1) - off) >> 5);
         const long long base = off + lane;
-        for (int j = 0; j < width; j += BATCH) {
-            int c[BATCH];
-            double v[BATCH], xv[BATCH];
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) c[u] = j + u < width ? ldg_stream_s32(JA + base + (long long)(j + u) * kHack) : -1;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_f64(AS + base + (long long)(j + u) * kHack) : 0.0;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) xv[u] = c[u] >= 0 ? __ldg(x + c[u]) : 0.0;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u)
-                if (c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
-        }
+        acc = hack_row_sum<BATCH, double>(base, width, row, JA, AS, x, nullptr, 0.0);
         if (row < M) {
             if (ep.inv_norm != nullptr) acc *= __ldg(ep.inv_norm);
             y[row] = acc;
@@ -410,20 +406,7 @@ hll_row_fused_kernel(int num_hacks, const long long *__restrict__ hack_off, cons
         const long long off = __ldg(hack_off + hack);
         const int width = (int)((__ldg(hack_off + hack + 1) - off) >> 5);
         const long long base = off + lane;
-        double acc = 0.0;
-        for (int j = 0; j < width; j += BATCH) {
-            int c[BATCH];
-            double v[BATCH], xv[BATCH];
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) c[u] = j + u < width ? ldg_stream_s32(JA + base + (long long)(j + u) * kHack) : -1;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) v[u] = j + u < width ? ldg_stream_f64(AS + base + (long long)(j + u) * kHack) : 0.0;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u) xv[u] = c[u] >= 0 ? __ldg(x + c[u]) : 0.0;
-#pragma unroll
-            for (int u = 0; u < BATCH; ++u)
-                if (c[u] >= 0) acc = __dadd_rn(acc, __dmul_rn(v[u], xv[u]));
-        }
+        double acc = hack_row_sum<BATCH, double>(base, width, chunk_lo + threadIdx.x, JA, AS, x, nullptr, 0.0);
         const long long row = chunk_lo + threadIdx.x;
         if (row >= M) continue;
         if (scaled) acc *= inv_norm;
@@ -607,12 +590,9 @@ static int hll_launch_rows_t(const spmv_b200_hll *H, const V *AS, int hack_begin
     if (uniform > 0) {
         if (H->segments.count <= 0) return fail(SPMV_B200_ERR_INVALID, "hll row kernel: the image is not regular enough for the offset-free form");
         const unsigned int gu = blocks_for(hack_end - hack_begin, 8);
-#define HROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, V>, gu, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, AS, d_x, d_y, H->M, nullptr, 0)); break;
-        switch (uniform) {
-            HROWU_CASE(3) HROWU_CASE(4) HROWU_CASE(6) HROWU_CASE(7)
-            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, V>, gu, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, AS, d_x, d_y, H->M, nullptr, 0)); break;
-        }
-#undef HROWU_CASE
+        SPMV_TRY_CUDA((with_batch<5, 3, 4, 6, 7>(uniform, [&](auto B) {
+            return launch_x(hll_rowu_kernel<B, V>, gu, 256, 0, stream, keep, hack_begin, hack_end, H->segments, H->JA, AS, d_x, d_y, H->M, nullptr, 0);
+        })));
         SPMV_TRY_CUDA(cudaGetLastError());
         return SPMV_B200_OK;
     }
@@ -631,12 +611,9 @@ static int hll_launch_rows_t(const spmv_b200_hll *H, const V *AS, int hack_begin
         return SPMV_B200_OK;
     }
     const unsigned int g = blocks_for(hack_end - hack_begin, 8);
-#define HROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, V>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, AS, d_x, d_y, H->M, nullptr, 0)); break;
-    switch (batch) {
-        HROW_CASE(1) HROW_CASE(2) HROW_CASE(3) HROW_CASE(5) HROW_CASE(6) HROW_CASE(7) HROW_CASE(8)
-        default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, V>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, AS, d_x, d_y, H->M, nullptr, 0)); break;
-    }
-#undef HROW_CASE
+    SPMV_TRY_CUDA((with_batch<4, 1, 2, 3, 5, 6, 7, 8>(batch, [&](auto B) {
+        return launch_x(hll_row_kernel<B, V>, g, 256, 0, stream, keep, hack_begin, hack_end, H->hack_off, H->JA, AS, d_x, d_y, H->M, nullptr, 0);
+    })));
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
 }
@@ -653,45 +630,28 @@ static int hll_launch_fused(const spmv_b200_hll *H, const double *d_x, double *d
                             int batch = -1) {
     if (batch < 0) batch = env_int("SPMV_B200_HLL_FUSED_BATCH", H->fused_batch > 0 ? H->fused_batch : H->row_batch);
     const int g = hll_fused_grid(H);
-#define HFUSED_CASE(B) case B: hll_row_fused_kernel<B><<<g, 256, 0, stream>>>(H->num_hacks, H->hack_off, H->JA, H->AS, d_x, d_y, H->M, ep); break;
-    switch (batch) {
-        HFUSED_CASE(2) HFUSED_CASE(3) HFUSED_CASE(5) HFUSED_CASE(6) HFUSED_CASE(7)
-        default: hll_row_fused_kernel<4><<<g, 256, 0, stream>>>(H->num_hacks, H->hack_off, H->JA, H->AS, d_x, d_y, H->M, ep); break;
-    }
-#undef HFUSED_CASE
+    with_batch<4, 2, 3, 5, 6, 7>(batch, [&](auto B) {
+        hll_row_fused_kernel<B><<<g, 256, 0, stream>>>(H->num_hacks, H->hack_off, H->JA, H->AS, d_x, d_y, H->M, ep);
+    });
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
 }
 
 // the FLAT form (two-launch iterated product): one CTA per 8 hacks; the batch is timed at plan time
-static int hll_flat_grid(long long M, int chunks_per_cta) {
-    (void)chunks_per_cta;
-    return (int)std::max<long long>(1, (M + 255) / 256);
-}
+static int hll_flat_grid(long long M) { return (int)std::max<long long>(1, (M + 255) / 256); }
 
 static int hll_launch_fused_flat(const spmv_b200_hll *H, const double *d_x, double *d_y, const Epilogue &ep, cudaStream_t stream,
-                                 int batch, int chunks_per_cta) {
-    const int g = hll_flat_grid(H->M, chunks_per_cta);
+                                 int batch) {
+    const int g = hll_flat_grid(H->M);
     const XPolicy keep = matrix_policy(H->JA, (size_t)H->slots * sizeof(int));
-#define HFLAT_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_flat_kernel<B>, g, 256, 0, stream, keep, H->num_hacks, H->hack_off, H->JA, H->AS, d_x, d_y, H->M, ep)); break;
-    switch (batch) {
-        HFLAT_CASE(2) HFLAT_CASE(3) HFLAT_CASE(5) HFLAT_CASE(6) HFLAT_CASE(7)
-        default: SPMV_TRY_CUDA(launch_x(hll_row_flat_kernel<4>, g, 256, 0, stream, keep, H->num_hacks, H->hack_off, H->JA, H->AS, d_x, d_y, H->M, ep)); break;
-    }
-#undef HFLAT_CASE
+    SPMV_TRY_CUDA((with_batch<4, 2, 3, 5, 6, 7>(batch, [&](auto B) {
+        return launch_x(hll_row_flat_kernel<B>, g, 256, 0, stream, keep, H->num_hacks, H->hack_off, H->JA, H->AS, d_x, d_y, H->M, ep);
+    })));
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
 }
 
-struct HllFlatChoice {
-    int batch, chunks;
-};
-static const HllFlatChoice kHllFlatCandidates[] = {{2, 1}, {3, 1}, {4, 1}, {5, 1}, {6, 1}, {7, 1}};
-
-static void hll_flat_choice(const spmv_b200_hll *H, int &batch, int &chunks) {
-    batch = env_int("SPMV_B200_HLL_FLAT_BATCH", H->flat_batch);
-    chunks = std::max(1, env_int("SPMV_B200_HLL_FLAT_CHUNKS", H->flat_chunks));
-}
+static const int kHllFlatCandidates[] = {2, 3, 4, 5, 6, 7};
 
 static int hll_launch_rows(const spmv_b200_hll *H, int hack_begin, int hack_end, const double *d_x, double *d_y,
                            cudaStream_t stream) {
@@ -805,17 +765,16 @@ static void hll_pick_row_batch(spmv_b200_hll *H, cudaStream_t stream) {
         cudaGetLastError();
         cudaFree(partials);
         partials = nullptr;
-        if (cudaMalloc(&partials, (size_t)hll_flat_grid(H->M, 1) * sizeof(double)) == cudaSuccess) {  // the FLAT form
+        if (cudaMalloc(&partials, (size_t)hll_flat_grid(H->M) * sizeof(double)) == cudaSuccess) {  // the FLAT form
             Epilogue fe;
             fe.partials = partials;
+            fe.partials_total = hll_flat_grid(H->M);
             fe.inv_norm = partials;  // any finite double will do for the timing
             const int n = (int)(sizeof kHllFlatCandidates / sizeof kHllFlatCandidates[0]);
             const int pick = tune_candidates(H->M, H->N, n, 1, stream, [&](int i, double *x, double *y) {
-                fe.partials_total = hll_flat_grid(H->M, kHllFlatCandidates[i].chunks);
-                return hll_launch_fused_flat(H, x, y, fe, stream, kHllFlatCandidates[i].batch, kHllFlatCandidates[i].chunks);
+                return hll_launch_fused_flat(H, x, y, fe, stream, kHllFlatCandidates[i]);
             });
-            H->flat_batch = kHllFlatCandidates[pick].batch;
-            H->flat_chunks = kHllFlatCandidates[pick].chunks;
+            H->flat_batch = kHllFlatCandidates[pick];
         }
         cudaGetLastError();
         cudaFree(partials);
@@ -993,19 +952,13 @@ static int csr_image_launch_t(const spmv_b200_hll *H, const I *JA, const S *AS, 
     const size_t smem = sizeof(S) == 1 ? (size_t)K * sizeof(double) : 0;  // the staged table of a coded image
     if (form >= 64) {
         if (H->segments.count <= 0) return fail(SPMV_B200_ERR_INVALID, "csr image: not regular enough for the offset-free form");
-#define IROWU_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->segments, JA, AS, x, y, H->M, H->table, K)); break;
-        switch (form - 64) {
-            IROWU_CASE(3) IROWU_CASE(4) IROWU_CASE(6) IROWU_CASE(7)
-            default: SPMV_TRY_CUDA(launch_x(hll_rowu_kernel<5, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->segments, JA, AS, x, y, H->M, H->table, K)); break;
-        }
-#undef IROWU_CASE
+        SPMV_TRY_CUDA((with_batch<5, 3, 4, 6, 7>(form - 64, [&](auto B) {
+            return launch_x(hll_rowu_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->segments, JA, AS, x, y, H->M, H->table, K);
+        })));
     } else {
-#define IROW_CASE(B) case B: SPMV_TRY_CUDA(launch_x(hll_row_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->hack_off, JA, AS, x, y, H->M, H->table, K)); break;
-        switch (form) {
-            IROW_CASE(2) IROW_CASE(3) IROW_CASE(5) IROW_CASE(6) IROW_CASE(7)
-            default: SPMV_TRY_CUDA(launch_x(hll_row_kernel<4, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->hack_off, JA, AS, x, y, H->M, H->table, K)); break;
-        }
-#undef IROW_CASE
+        SPMV_TRY_CUDA((with_batch<4, 2, 3, 5, 6, 7>(form, [&](auto B) {
+            return launch_x(hll_row_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->hack_off, JA, AS, x, y, H->M, H->table, K);
+        })));
     }
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
@@ -1139,7 +1092,7 @@ int spmv_b200_hll_info(const spmv_b200_hll *H, spmv_b200_hll_info_t *info) {
     info->row_batch = H->row_batch;
     info->fused_batch = H->fused_batch;
     info->flat_batch = H->flat_batch;
-    info->flat_chunks = H->flat_chunks;
+    info->flat_chunks = 1;
     return SPMV_B200_OK;
 }
 
@@ -1257,9 +1210,7 @@ int spmv_b200_hll_spmv_fused(const spmv_b200_hll *H, const double *d_x, double *
 
 int spmv_b200_hll_flat_partials_count(const spmv_b200_hll *H) {
     if (!H) return 0;
-    int batch, chunks;
-    hll_flat_choice(H, batch, chunks);
-    return hll_flat_grid(H->M, chunks);
+    return hll_flat_grid(H->M);
 }
 
 int spmv_b200_hll_spmv_fused_flat(const spmv_b200_hll *H, const double *d_x, double *d_y, const double *d_inv_norm,
@@ -1268,14 +1219,12 @@ int spmv_b200_hll_spmv_fused_flat(const spmv_b200_hll *H, const double *d_x, dou
     if (peers && (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS))
         return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused_flat: bad peer count %d", peers->count);
     if (H->M == 0) return SPMV_B200_OK;
-    int batch, chunks;
-    hll_flat_choice(H, batch, chunks);
     Epilogue ep;
     ep.inv_norm = d_inv_norm;
     ep.partials = d_partials;
-    ep.partials_total = hll_flat_grid(H->M, chunks);
+    ep.partials_total = hll_flat_grid(H->M);
     if (peers) ep.peers = *peers;
-    return hll_launch_fused_flat(H, d_x, d_y, ep, as_stream(stream), batch, chunks);
+    return hll_launch_fused_flat(H, d_x, d_y, ep, as_stream(stream), env_int("SPMV_B200_HLL_FLAT_BATCH", H->flat_batch));
 }
 
 int spmv_b200_hll_spmv_fused_mail(const spmv_b200_hll *H, const double *d_x, double *d_y, double *d_partials,

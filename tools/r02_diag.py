@@ -107,28 +107,6 @@ if "fusedgrid" in what:
         torch.cuda.empty_cache()
     os.environ.pop("SPMV_B200_FUSED_CTAS_PER_SM")
 
-if "flat" in what:
-    section("lap3d: fused row kernel, loop only: grid-stride vs C consecutive chunks per CTA")
-    for n in (512, 256):
-        A = device.DeviceCSR.synth(synth.SYNTH_LAP3D, n)
-        i = A.info()
-        x = torch.ones(i.N, dtype=torch.float64, device="cuda")
-        y = torch.empty(i.M, dtype=torch.float64, device="cuda")
-        for batch in (2, 5):
-            os.environ["SPMV_B200_ROW_BATCH"] = str(batch)
-            os.environ["SPMV_B200_FUSED_BATCH"] = str(batch)
-            A.replan()
-            line = f"n {n} batch {batch}: plain {timeit(lambda: A.spmv(x, y, algo=device.ALGO_ROW))*1e3:.1f} us | fused loop only:"
-            for flat in (0, 1, 2, 4, 8, 16, 64):
-                os.environ["SPMV_B200_FUSED_FLAT"] = str(flat)
-                line += f" C={flat or 'grid-stride'} {timeit(lambda: A.spmv_fused(x, y))*1e3:.1f}"
-            print(line, flush=True)
-        for k in ("SPMV_B200_ROW_BATCH", "SPMV_B200_FUSED_BATCH", "SPMV_B200_FUSED_FLAT"):
-            os.environ.pop(k, None)
-        A.close()
-        del x, y
-        torch.cuda.empty_cache()
-
 if "flatpick" in what:
     section("FLAT fused kernels: plan-time choice and every candidate, lap3d 512^3 and the 8-GPU rank size (512^3 / 8 rows)")
     for n, rows in ((512, None), (512, 512 ** 3 // 8)):
@@ -136,7 +114,7 @@ if "flatpick" in what:
         i = A.info()
         H = A.to_hll()
         hi = H.info()
-        print(f"rows {i.M}: CSR plan fused_batch {i.fused_batch} flat ({i.flat_batch}, {i.flat_chunks}); HLL plan row_batch {hi.row_batch} fused_batch {hi.fused_batch} flat ({hi.flat_batch}, {hi.flat_chunks})")
+        print(f"rows {i.M}: CSR plan fused_batch {i.fused_batch} flat_batch {i.flat_batch}; HLL plan row_batch {hi.row_batch} fused_batch {hi.fused_batch} flat_batch {hi.flat_batch}")
         x = torch.ones(i.N, dtype=torch.float64, device="cuda")
         y = torch.empty(i.M, dtype=torch.float64, device="cuda")
         ss = torch.ones(1, dtype=torch.float64, device="cuda")
@@ -144,15 +122,11 @@ if "flatpick" in what:
         print(f"  plain: CSR {timeit(lambda: A.spmv(x, y))*1e3:.1f} us, HLL {timeit(lambda: H.spmv(x, y))*1e3:.1f} us; "
               f"grid-stride fused: CSR {timeit(lambda: A.spmv_fused(x, y, prev_sumsq=ss, partials=part))*1e3:.1f} us, HLL {timeit(lambda: H.spmv_fused(x, y, prev_sumsq=ss, partials=part))*1e3:.1f} us")
         for batch in (2, 3, 4, 5, 6, 7):
-            line = f"  batch {batch}:"
-            for chunks in (1,):
-                os.environ["SPMV_B200_FLAT_BATCH"], os.environ["SPMV_B200_FLAT_CHUNKS"] = str(batch), str(chunks)
-                os.environ["SPMV_B200_HLL_FLAT_BATCH"], os.environ["SPMV_B200_HLL_FLAT_CHUNKS"] = str(batch), str(chunks)
-                a = timeit(lambda: A.spmv_fused_flat(x, y, inv_norm=ss, partials=part))
-                b = timeit(lambda: H.spmv_fused_flat(x, y, inv_norm=ss, partials=part))
-                line += f"  C={chunks}: CSR {a*1e3:.1f} HLL {b*1e3:.1f}"
-            print(line, flush=True)
-        for k in ("SPMV_B200_FLAT_BATCH", "SPMV_B200_FLAT_CHUNKS", "SPMV_B200_HLL_FLAT_BATCH", "SPMV_B200_HLL_FLAT_CHUNKS"):
+            os.environ["SPMV_B200_FLAT_BATCH"] = os.environ["SPMV_B200_HLL_FLAT_BATCH"] = str(batch)
+            a = timeit(lambda: A.spmv_fused_flat(x, y, inv_norm=ss, partials=part))
+            b = timeit(lambda: H.spmv_fused_flat(x, y, inv_norm=ss, partials=part))
+            print(f"  batch {batch}: CSR {a*1e3:.1f} HLL {b*1e3:.1f}", flush=True)
+        for k in ("SPMV_B200_FLAT_BATCH", "SPMV_B200_HLL_FLAT_BATCH"):
             os.environ.pop(k, None)
         H.close()
         A.close()
