@@ -49,7 +49,7 @@ extern "C" {
 #define SPMV_B200_ALGO_STREAM 3   /* persistent row-binned kernel, TMA bulk-copy pipeline    */
 #define SPMV_B200_ALGO_BINNED 4   /* rows binned by length: 1..32 lanes per row, longest rows split */
 #define SPMV_B200_ALGO_ROW 5      /* one thread per row, serial order (bit-identical to the reference loop) */
-#define SPMV_B200_ALGO_ROW_IMAGE 6 /* one lane per row on the handle's private column-major image (spmv_b200_csr_set_image);
+#define SPMV_B200_ALGO_ROW_IMAGE 6 /* one lane per row on the handle's private image, column-major or patterns (spmv_b200_csr_set_image);
                                       the same bits as ROW.  SPMV_B200_ERR_INVALID when the handle holds no image */
 
 /* synthetic CSR generators (BASELINE.json configs 2, 3, 5) */
@@ -85,6 +85,11 @@ typedef struct {
     long long image_device_bytes; /* device bytes of its columns, values and value table:
                                      (image_index_bytes + image_value_bytes) per slot, plus 8 per table entry */
     int image_value_bytes; /* bytes of its value field: 8 (fp64), 1 (a code into a table of at most 256 doubles), 0 none */
+    int image_patterns;  /* the pattern form (set_image mode 3; spmv_b200_version() >= 106): the number of distinct row
+                            patterns in its dictionary, 0 for the other forms or none.  For this form image_form is
+                            256 + W (csr_pattern_kernel<W>, W the longest row), image_bytes and image_device_bytes are
+                            M (one byte per row) plus the dictionary's 12 * W + 4 bytes per pattern, and
+                            image_index_bytes and image_value_bytes are 0 */
 } spmv_b200_csr_info_t;
 
 typedef struct {
@@ -253,7 +258,8 @@ int spmv_b200_csr_spmv_fused_async(const spmv_b200_csr *A, const double *d_x, do
                                    const spmv_b200_peers_t *peers, const spmv_b200_async_t *async, void *stream);
 
 /* product restricted to rows [row_begin,row_end) (the reference's per-thread row ranges,
- * src/csr_matrix.c:294-313); other rows of y are left untouched.  Vector kernel. */
+ * src/csr_matrix.c:294-313); other rows of y are left untouched.  Vector kernel; one thread per row when no row holds
+ * more than 12 nonzeros, on the pattern form of the private image when the handle holds it (same bits). */
 int spmv_b200_csr_spmv_rows(const spmv_b200_csr *A, int row_begin, int row_end, const double *d_x,
                             double *d_y, void *stream);
 /* ---- support for the literal "NCCL allgather of x" refresh (BASELINE config 5; no reference counterpart).  One
@@ -283,12 +289,21 @@ int spmv_b200_csr_interior_rows(const spmv_b200_csr *A, long long col_lo, long l
  * times faster than every other candidate and its padding adds at most a quarter to nnz; then AUTO uses it.  Cost, on
  * top of the CSR arrays, per slot: 2 or 4 bytes of column field plus 8 (fp64) or 1 (codes) -- +252 MB on lap2d 4096^2,
  * narrow and coded; +839 MB with fp64 values.
+ * Pattern form (spmv_b200_version() >= 106): when the rows hold at most 256 distinct patterns -- a pattern is the row's
+ * length, then col - row of each nonzero, then the 64-bit pattern of each value (+0.0 and -0.0, and NaN payloads, count
+ * apart) -- and the dictionary of those patterns takes at most 24 KB at 12 bytes per pattern and slot of the longest
+ * row, the image may instead be one byte per row naming its pattern (csr_pattern_kernel: lap2d 4096^2, 9 patterns:
+ * +16.8 MB; DESIGN.md section 3).  The same bits as ROW, with the same NaN-payload exception as the value codes.  The
+ * plan builds it alongside the column-major image under the same padding rule (M times the longest row at most 5/4 of
+ * nnz), times both and keeps one of them at most.
  * mode 0 drops the image (AUTO falls back to the plan's choice among ROW / STREAM); mode 1 builds it with fp64 values
  * whenever the matrix is eligible in structure (owned arrays, no row above 12 nonzeros, no long rows), whatever its size
  * or timing, narrow when the matrix qualifies, replacing a coded one, and returns SPMV_B200_ERR_INVALID otherwise; mode 2
  * does the same with the value codes, and returns SPMV_B200_ERR_INVALID, leaving the handle as it was, on a matrix of
- * more than 256 distinct value patterns.  replan decides again; remap_columns drops it.  The fp32, SpMM, fused,
- * row-range and host-buffer products do not use it. */
+ * more than 256 distinct value patterns; mode 3 builds the pattern form, replacing a column-major image, and returns
+ * SPMV_B200_ERR_INVALID, leaving the handle as it was, on a matrix that does not qualify for it.  replan decides again;
+ * remap_columns drops it.  The fp32, SpMM, fused and host-buffer products do not use it, nor does the row-range product
+ * (spmv_b200_csr_spmv_rows) use the column-major image. */
 int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream);
 void spmv_b200_csr_free(spmv_b200_csr *A);
 

@@ -909,6 +909,15 @@ static void free_bins(spmv_b200_csr *A) {
     A->bins = BinPlan();
 }
 
+// frees the private image in whichever form the handle holds
+static void drop_image(spmv_b200_csr *A) {
+    spmv_b200_hll_free(A->image);
+    csr_patterns_free(A->patterns);
+    A->image = nullptr;
+    A->patterns = nullptr;
+    A->image_form = 0;
+}
+
 static void free_plan(spmv_b200_csr *A) {
     free_bins(A);
     cudaFree(A->tiles);
@@ -922,9 +931,7 @@ static void free_plan(spmv_b200_csr *A) {
     A->frag_partial = nullptr;
     A->spmm_partial = nullptr;
     A->num_tiles = A->num_long = A->num_frag = 0;
-    spmv_b200_hll_free(A->image);
-    A->image = nullptr;
-    A->image_form = 0;
+    drop_image(A);
 }
 
 template <typename V>
@@ -1042,7 +1049,9 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
         // (+ kImageCoded).  All give the same bits on such rows.  The image qualifies when its padding adds at most a
         // quarter to nnz and it fits in a quarter of the free memory (2 or 4 bytes of column field per slot, plus 8 + 1
         // for both value streams, or 1 for the codes alone where both do not fit); it is freed again unless it wins, and
-        // the losing value stream is freed when it does.
+        // the losing value stream is freed when it does.  Alongside, under the same padding rule (M * max_row slots), the
+        // pattern form (csr_patterns_build, id kImagePatterns) when the rows hold at most 256 patterns; whichever image
+        // loses is freed.
         if (A->owns && A->num_long == 0) {
             size_t free_bytes = 0, total_bytes = 0;
             if (cudaMemGetInfo(&free_bytes, &total_bytes) == cudaSuccess) {
@@ -1050,10 +1059,13 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
                 if (fit_bytes >= 0 &&
                     csr_image_build(A, A->nnz + A->nnz / 4, fit_bytes, kImageBoth, stream, &A->image) != SPMV_B200_OK)
                     A->image = nullptr;
+                if ((long long)M * A->max_row <= A->nnz + A->nnz / 4 && (long long)M <= fit_bytes &&
+                    csr_patterns_build(A, stream, &A->patterns) != SPMV_B200_OK)
+                    A->patterns = nullptr;
             }
             cudaGetLastError();
         }
-        int ids[24], n = 0, fallback = 0;  // 7 plain + 6 + 6 image forms on an irregular image
+        int ids[25], n = 0, fallback = 0;  // 7 plain + 6 + 6 image forms on an irregular image + the pattern form
         ids[n++] = 0;
         for (int batch = 2; batch <= 7; ++batch) {
             if (batch == A->row_batch) fallback = n;
@@ -1067,11 +1079,13 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
                 if (A->image->segments.count == 0) ids[n++] = flag + 32 + batch;
                 else if (batch >= 4) ids[n++] = flag + 64 + batch;
         }
+        if (A->patterns) ids[n++] = kImagePatterns;
         auto image_form = [](int id) { return (id & kImageCoded) | ((id & ~kImageCoded) >= 64 ? id & ~kImageCoded : (id & ~kImageCoded) - 32); };
-        float ms[24];
+        float ms[25];
         const int pick = tune_candidates(M, A->N, n, fallback, stream, [&](int i, double *x, double *y) {
             if (ids[i] == 0) return stream_launch_csr(A, x, y, 0, nullptr, stream);
             if (ids[i] < 16) return launch_rows(0, M, A->row_ptr, A->col_idx, A->values, x, y, ids[i], 0, stream);
+            if (ids[i] == kImagePatterns) return csr_patterns_launch(A->patterns, 0, M, A->N, x, y, 0, stream);
             return csr_image_launch(A->image, image_form(ids[i]), 0, A->image->num_hacks, x, y, 0, stream);
         }, ms);
         int best = fallback;  // the plain choice stays for ALGO_ROW and the other entry points even when the image wins
@@ -1079,12 +1093,17 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
             if (ms[i] >= 0.0f && (ms[best] < 0.0f || ms[i] < ms[best])) best = i;
         if (ids[best] == 0) A->short_rows_stream = true;
         else A->row_batch = ids[best];
-        if (pick >= plain) {
+        if (pick >= plain && ids[pick] == kImagePatterns) {
+            spmv_b200_hll_free(A->image);
+            A->image = nullptr;
+            A->image_form = kImagePatterns + A->patterns->width;
+        } else if (pick >= plain) {
+            csr_patterns_free(A->patterns);
+            A->patterns = nullptr;
             A->image_form = image_form(ids[pick]);
             csr_image_keep(A->image, (A->image_form & kImageCoded) != 0);
         } else {
-            spmv_b200_hll_free(A->image);
-            A->image = nullptr;
+            drop_image(A);
         }
         // the fused iterated product (scale + |w|^2 partials in the tail): fused stream kernel (0) or fused row kernel
         if (A->num_long == 0) {
@@ -1367,7 +1386,7 @@ CsrPath csr_resolve(const spmv_b200_csr *A, int algo) {
         default:
             // every row short: one thread per row (serial order, so forced_tpr == 1 is honoured as well) -- on the
             // private image when the handle holds one
-            if (A->max_row <= kRowKernelMaxLen) return A->image ? kPathImage : A->short_rows_stream ? kPathStream : kPathRow;
+            if (A->max_row <= kRowKernelMaxLen) return A->image || A->patterns ? kPathImage : A->short_rows_stream ? kPathStream : kPathRow;
             if (A->forced_tpr == 1 || A->nnz <= (long long)kAutoStreamMaxAvg * A->M) return kPathStream;
             {   // longer rows: one lane count for all rows (vector kernel) only while the lengths are even; a longest row
                 // far above the mean (or above the long-row threshold) means skew -> lanes per row by length class
@@ -1383,6 +1402,7 @@ int csr_launch_window(const spmv_b200_csr *A, CsrPath path, int unit_begin, int 
     if (path == kPathBinned) return launch_binned<double>(A, A->values, x, y, accumulate, stream);  // whole matrix: rows are permuted
     if (path == kPathRow)
         return launch_rows(unit_begin, unit_end, A->row_ptr, A->col_idx, A->values, x, y, A->row_batch, accumulate, stream);
+    if (path == kPathImage && A->patterns) return csr_patterns_launch(A->patterns, unit_begin, unit_end, A->N, x, y, accumulate, stream);
     if (path == kPathImage)  // rows, in whole hacks: unit_begin must be a multiple of 32
         return csr_image_launch(A->image, A->image_form, unit_begin / 32, (unit_end + 31) / 32, x, y, accumulate, stream);
     if (path == kPathVector)
@@ -1665,6 +1685,11 @@ int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info) {
     info->image_index_bytes = !A->image ? 0 : A->image->JA16 ? 2 : 4;
     info->image_device_bytes = A->image ? csr_image_bytes(A->image) : 0;
     info->image_value_bytes = A->image ? csr_image_value_bytes(A->image) : 0;
+    info->image_patterns = A->patterns ? A->patterns->count : 0;
+    if (A->patterns) {  // the pattern form: one byte per row plus the dictionary
+        info->image_form = A->image_form;
+        info->image_bytes = info->image_device_bytes = A->M + csr_patterns_dict_bytes(A->patterns);
+    }
     return SPMV_B200_OK;
 }
 
@@ -1689,7 +1714,8 @@ int spmv_b200_csr_spmv(const spmv_b200_csr *A, const double *d_x, double *d_y, i
     if (!A || !d_y || (A->N > 0 && !d_x)) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: NULL argument");
     if (A->M == 0) return SPMV_B200_OK;
     if (algo < SPMV_B200_ALGO_AUTO || algo > SPMV_B200_ALGO_ROW_IMAGE) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: unknown algo %d", algo);
-    if (algo == SPMV_B200_ALGO_ROW_IMAGE && !A->image) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: the matrix holds no image (spmv_b200_csr_set_image)");
+    if (algo == SPMV_B200_ALGO_ROW_IMAGE && !A->image && !A->patterns)
+        return fail(SPMV_B200_ERR_INVALID, "csr_spmv: the matrix holds no image (spmv_b200_csr_set_image)");
     const CsrPath path = csr_resolve(A, algo);
     const bool by_rows = path == kPathVector || path == kPathRow || path == kPathImage;
     return csr_launch_window(A, path, 0, by_rows ? A->M : A->num_tiles, d_x, d_y, accumulate, as_stream(stream));
@@ -1814,31 +1840,38 @@ int spmv_b200_csr_remap_columns(spmv_b200_csr *A, int nparts, const long long *s
         SPMV_TRY_CUDA(cudaGetLastError());
     }
     A->N = (int)(nparts * stride);  // plans, tiles and the fp32 copy of the values do not depend on the column ids;
-    spmv_b200_hll_free(A->image);   // the private image does
-    A->image = nullptr;
-    A->image_form = 0;
+    drop_image(A);                  // the private image does
     SPMV_TRY_CUDA(cudaStreamSynchronize(as_stream(stream)));
     return SPMV_B200_OK;
 }
 
 int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream) {
     if (!A) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: NULL matrix");
-    if (mode < 0 || mode > 2) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: unknown mode %d", mode);
+    if (mode < 0 || mode > 3) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: unknown mode %d", mode);
     if (mode == 0) {
-        spmv_b200_hll_free(A->image);
-        A->image = nullptr;
-        A->image_form = 0;
+        drop_image(A);
         return SPMV_B200_OK;
     }
     if (!A->owns) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: the matrix wraps arrays it does not own");
     if (A->max_row > kRowKernelMaxLen || A->num_long > 0)
         return fail(SPMV_B200_ERR_INVALID, "csr_set_image: rows of up to %d nonzeros and no long rows only (longest row: %d)",
                     kRowKernelMaxLen, A->max_row);
+    if (mode == 3) {
+        if (A->patterns) return SPMV_B200_OK;
+        CsrPatterns *patterns = nullptr;  // the held image stays unless the pattern form can be built
+        if (csr_patterns_build(A, as_stream(stream), &patterns) != SPMV_B200_OK)
+            return fail(SPMV_B200_ERR_INVALID, "csr_set_image: the pattern form needs 1 to %d nonzeros per row, at most %d distinct "
+                        "rows and a dictionary of at most %d bytes", kRowKernelMaxLen, kMaxPatterns, kPatternDictMaxBytes);
+        drop_image(A);
+        A->patterns = patterns;
+        A->image_form = kImagePatterns + patterns->width;
+        return SPMV_B200_OK;
+    }
     const bool coded = mode == 2;
     if (A->image && (coded ? A->image->AC != nullptr : A->image->AS != nullptr)) return SPMV_B200_OK;
     spmv_b200_hll *image = nullptr;  // the held image stays until the new one is built (mode 2 fails on > 256 patterns)
     SPMV_TRY(csr_image_build(A, -1, -1, coded ? kImageCodes : kImageF64, as_stream(stream), &image));
-    spmv_b200_hll_free(A->image);
+    drop_image(A);
     A->image = image;
     A->image_form = csr_image_default_form(A->image);
     return SPMV_B200_OK;
@@ -1888,6 +1921,8 @@ int spmv_b200_csr_spmv_rows(const spmv_b200_csr *A, int row_begin, int row_end, 
     if (!A || !d_y || !d_x) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_rows: NULL argument");
     if (row_begin < 0 || row_end > A->M || row_begin > row_end)
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv_rows: range [%d,%d) outside [0,%d)", row_begin, row_end, A->M);
+    if (A->patterns)  // the pattern form of the private image: any row range, the same bits
+        return csr_patterns_launch(A->patterns, row_begin, row_end, A->N, d_x, d_y, 0, as_stream(stream));
     if (A->max_row <= kRowKernelMaxLen)  // stencils: the thread-per-row kernel with the batch tuned at plan time (serial order)
         return launch_rows(row_begin, row_end, A->row_ptr, A->col_idx, A->values, d_x, d_y, A->row_batch, 0, as_stream(stream));
     return launch_vector(row_begin, row_end, A->row_ptr, A->col_idx, A->values, d_x, d_y,

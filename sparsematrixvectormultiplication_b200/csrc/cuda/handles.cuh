@@ -203,6 +203,20 @@ int tune_candidates(long long M, long long N, int n, int fallback, cudaStream_t 
     cudaFree(y);
     return best;
 }
+
+// The pattern form of a CSR handle's private image (pattern.cu): a matrix whose rows hold at most kMaxPatterns distinct
+// patterns -- a pattern is the row's length, the col - row of each slot and the 64-bit pattern of each value -- stored
+// as one byte per row that names the row's pattern in a dictionary the kernel stages in shared memory.
+constexpr int kMaxPatterns = 256;
+constexpr int kPatternDictMaxBytes = 24 * 1024;  // P * W * 12: 8 CTAs of 256 threads stay resident per SM
+struct CsrPatterns {
+    int count = 0;          // P patterns, in the order of their (length, deltas, value bits)
+    int width = 0;          // W: the matrix's longest row
+    uint8_t *id = nullptr;  // device [M]: the pattern of each row
+    int *dict = nullptr;    // device: value[W][P] (fp64), delta[W][P] (int32), len[P] (int32); a slot at or past a
+                            // pattern's length holds delta 0 and value 0.0
+};
+inline long long csr_patterns_dict_bytes(const CsrPatterns *P) { return 12LL * P->width * P->count + 4LL * P->count; }
 }  // namespace spmv
 
 struct spmv_b200_csr {
@@ -247,7 +261,10 @@ struct spmv_b200_csr {
     // (AC, table): 3 or 5 bytes per slot; the plan times both and keeps the faster.
     spmv_b200_hll *image = nullptr;
     int image_form = 0;  // 64 + B: hll_rowu_kernel<B, double, true>; B: hll_row_kernel<B, double, true> (index type: JA16 / JA),
-                         // plus spmv::kImageCoded when it reads the value codes
+                         // plus spmv::kImageCoded when it reads the value codes; 256 + W: csr_pattern_kernel<W> on `patterns`
+    // the pattern form of the private image (spmv::CsrPatterns): held instead of `image` when the plan timed it faster or
+    // set_image mode 3 asked for it; same rules otherwise
+    spmv::CsrPatterns *patterns = nullptr;
     // staging vectors of the *_host entry points
     double *stage_x = nullptr;
     double *stage_y = nullptr;
@@ -338,6 +355,14 @@ void csr_image_keep(spmv_b200_hll *H, bool coded);  // frees the other value str
 int csr_image_default_form(const spmv_b200_hll *H);
 int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
                      int accumulate, cudaStream_t stream);
+// pattern.cu: builds the pattern form of A (owned arrays and no long rows assumed by the caller).  SPMV_B200_ERR_INVALID,
+// without a message (the plan tries every eligible matrix), when A does not qualify: no row or one above
+// kRowKernelMaxLen, more than kMaxPatterns patterns, or a dictionary above kPatternDictMaxBytes
+constexpr int kImagePatterns = 256;  // image_form of the pattern form: kImagePatterns + W
+int csr_patterns_build(const spmv_b200_csr *A, cudaStream_t stream, CsrPatterns **out);
+void csr_patterns_free(CsrPatterns *P);
+int csr_patterns_launch(const CsrPatterns *P, int row_begin, int row_end, int N, const double *x, double *y, int accumulate,
+                        cudaStream_t stream);  // any row range
 int hll_row_forms();                                             // hll.cu: forms of hll_rowm_kernel (spmv_b200_row_forms)
 int hll_row_form(int index, int *hacks, int *batch, int *ctas);  // 0 = ok
 int fused_ctas_per_sm();  // csr.cu: CTAs per SM in the grid of the fused row kernels (CSR and HLL use the same value)

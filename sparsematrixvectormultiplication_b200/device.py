@@ -14,7 +14,7 @@ from . import _native as N
 
 ALGO_AUTO, ALGO_VECTOR, ALGO_TILE, ALGO_STREAM, ALGO_BINNED, ALGO_ROW, ALGO_ROW_IMAGE = 0, 1, 2, 3, 4, 5, 6
 ALGO_NAMES = {0: "auto", 1: "csr_vector_kernel", 2: "csr_stream_kernel (ALGO_TILE is retired)", 3: "csr_stream_kernel", 4: "csr_binned_kernel", 5: "csr_row_kernel",
-              6: "hll_rowu_kernel / hll_row_kernel on the handle's private image (masked padding)"}
+              6: "hll_rowu_kernel / hll_row_kernel / csr_pattern_kernel on the handle's private image (masked padding)"}
 HLL_KERNEL_NAMES = {0: "hll_slice_kernel", 1: "hll_stream_kernel", 2: "hll_row_kernel"}
 SYNTH_LAP2D, SYNTH_LAP3D, SYNTH_UNIFORM = 1, 2, 3
 
@@ -298,8 +298,9 @@ class DeviceCSR:
     def set_image(self, mode, stream=None):
         """mode 0: drop the private column-major image; mode 1: build it with fp64 values on any matrix eligible in
         structure (owned arrays, rows of at most 12 nonzeros), whatever its size or timing; mode 2: the same with 1-byte
-        value codes, on a matrix of at most 256 distinct value patterns (spmv_b200_csr_set_image).  Raises SpmvError
-        otherwise, and mode 2 then leaves the handle as it was."""
+        value codes, on a matrix of at most 256 distinct value patterns; mode 3: the pattern form, one byte per row, on a
+        matrix of at most 256 distinct rows (spmv_b200_csr_set_image).  Raises SpmvError otherwise, and modes 2 and 3
+        then leave the handle as it was."""
         N.check(N.lib().spmv_b200_csr_set_image(self._h, int(mode), _stream(stream)))
         return self
 
@@ -307,6 +308,8 @@ class DeviceCSR:
         """Name of the kernel that multiplies the private image, index type and, for the value codes, the stored value
         type included ("none" without one)."""
         i = self.info()
+        if i.image_patterns > 0:
+            return f"csr_pattern_kernel<{i.image_form - 256}>"
         args = "uint16_t" if i.image_index_bytes == 2 else "int"
         if i.image_value_bytes == 1:
             args += ",uint8_t"

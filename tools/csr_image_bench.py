@@ -4,13 +4,14 @@
 
 For each workload the handle is built as a user builds it (synth: owned arrays, plan-time timing on), so AUTO is whatever
 the plan chose -- the private image (SPMV_B200_ALGO_ROW_IMAGE) where it timed fastest, with fp64 values or 1-byte value
-codes.  A second handle of the same matrix holds the image with fp64 values (set_image(1)).  Then ALGO_ROW (csr_row_kernel,
-the plan's batch), AUTO and ROW_IMAGE on the fp64 image alternate: per repetition `launches` back-to-back products of each
-arm between CUDA events, after a warm-up of all.  Every working set exceeds the 126 MB L2.  Reported per workload: mean / min / max microseconds per
+codes, or in the pattern form (one byte per row).  Further handles of the same matrix hold the image with fp64 values
+(set_image(1)), with value codes (set_image(2)) and in the pattern form (set_image(3)), each where the matrix qualifies.
+Then ALGO_ROW (csr_row_kernel, the plan's batch), AUTO and ROW_IMAGE on each of those handles alternate: per repetition
+`launches` back-to-back products of each arm between CUDA events, after a warm-up of all.  Every working set exceeds the 126 MB L2.  Reported per workload: mean / min / max microseconds per
 product of each arm, the speed-up (ROW mean / AUTO mean), the chosen kernel, plan time (the synth call, timing included),
 the image's device bytes and value bytes, the algorithmic bytes of the CSR product (12 nnz + 4 (M+1) + 8 M + 8 N) and the
 bytes each image kernel actually reads (image_device_bytes + 8 M + 8 N, no row_ptr; 2 or 4 bytes of column field and 8 or 1
-of value per slot), each over its time, and whether AUTO and the fp64 image give ALGO_ROW's bits (it must wherever AUTO is a
+of value per slot, or 1 byte per row), each over its time, and whether AUTO and each image give ALGO_ROW's bits (it must wherever AUTO is a
 serial-order kernel: the image, ROW, STREAM; uniform 32 per row is too long for the image and stays on the vector kernel,
 whose shuffle sums differ in the last bits).  The device name and power limit are read in the same run.
 """
@@ -71,28 +72,32 @@ def run(name, make, reps, launches):
     torch.cuda.synchronize()
     plan_s = time.perf_counter() - t0
     i = A.info()
-    B = make()
-    B.set_image(1)  # the fp64 image, whatever the plan chose
-    ib = B.info()
+    images = {}  # the image in each form, whatever the plan chose
+    for form, mode in (("f64", 1), ("coded", 2), ("patterns", 3)):
+        H = make()
+        try:
+            H.set_image(mode)
+            images[form] = H
+        except Exception:  # the matrix does not qualify for this form
+            H.close()
     g = torch.Generator(device="cuda").manual_seed(11)
     x = torch.randn(i.N, dtype=torch.float64, device="cuda", generator=g)
     y_row = torch.empty(i.M, dtype=torch.float64, device="cuda")
     y_auto = torch.empty(i.M, dtype=torch.float64, device="cuda")
-    y_f64 = torch.empty(i.M, dtype=torch.float64, device="cuda")
-    arms = ((A, d.ALGO_ROW, y_row), (A, d.ALGO_AUTO, y_auto), (B, d.ALGO_ROW_IMAGE, y_f64))
+    arms = [(A, d.ALGO_ROW, y_row), (A, d.ALGO_AUTO, y_auto)]
+    arms += [(H, d.ALGO_ROW_IMAGE, torch.empty(i.M, dtype=torch.float64, device="cuda")) for H in images.values()]
     for H, algo, y in arms:
         arm_ms(H, x, y, algo, launches)
     torch.cuda.synchronize()
     bitwise = bool(torch.equal(y_row.view(torch.int64), y_auto.view(torch.int64)))
-    bitwise_f64 = bool(torch.equal(y_row.view(torch.int64), y_f64.view(torch.int64)))
-    t_row, t_auto, t_f64 = [], [], []
+    times = [[] for _ in arms]
     for _ in range(reps):
-        for (H, algo, y), ts in zip(arms, (t_row, t_auto, t_f64)):
+        for (H, algo, y), ts in zip(arms, times):
             ts.append(arm_ms(H, x, y, algo, launches))
+    t_row, t_auto = times[0], times[1]
     on_image = i.auto_algo == d.ALGO_ROW_IMAGE
     alg = i.algorithmic_bytes
     read = (i.image_device_bytes + 8 * i.M + 8 * i.N) if on_image else alg
-    read_f64 = ib.image_device_bytes + 8 * i.M + 8 * i.N
     auto_kernel = A.image_form() if on_image else (f"csr_row_kernel<{i.row_batch},double>" if i.auto_algo == d.ALGO_ROW
                                                    else d.ALGO_NAMES[i.auto_algo])
 
@@ -107,17 +112,20 @@ def run(name, make, reps, launches):
            "row": stats(t_row), "auto": stats(t_auto), "speedup_row_over_auto": statistics.mean(t_row) / statistics.mean(t_auto),
            "algorithmic_TBps_auto": alg / (1e-3 * statistics.mean(t_auto)) / 1e12,
            "read_TBps_auto": read / (1e-3 * statistics.mean(t_auto)) / 1e12,
-           "auto_bitwise_equal_row": bitwise,
-           "image_f64": {"kernel": B.image_form(), "image_device_bytes": ib.image_device_bytes, "read_bytes": read_f64,
-                         **stats(t_f64), "read_TBps": read_f64 / (1e-3 * statistics.mean(t_f64)) / 1e12,
-                         "speedup_over_auto": statistics.mean(t_f64) / statistics.mean(t_auto),
-                         "bitwise_equal_row": bitwise_f64}}
-    print(f"[csr_image] {name}: row {out['row']['mean_us']:.1f} us, auto {out['auto']['mean_us']:.1f} us "
-          f"({auto_kernel}), fp64 image {out['image_f64']['mean_us']:.1f} us ({B.image_form()}), "
-          f"x{out['speedup_row_over_auto']:.3f}, bitwise {bitwise}/{bitwise_f64}, plan {plan_s:.2f} s", flush=True)
+           "auto_bitwise_equal_row": bitwise}
+    line = f"[csr_image] {name}: row {out['row']['mean_us']:.1f} us, auto {out['auto']['mean_us']:.1f} us ({auto_kernel})"
+    for (form, H), (_, _, y), ts in zip(images.items(), arms[2:], times[2:]):
+        ih = H.info()
+        rd = ih.image_device_bytes + 8 * i.M + 8 * i.N
+        out[f"image_{form}"] = {"kernel": H.image_form(), "image_device_bytes": ih.image_device_bytes, "read_bytes": rd,
+                                **stats(ts), "read_TBps": rd / (1e-3 * statistics.mean(ts)) / 1e12,
+                                "speedup_over_auto": statistics.mean(ts) / statistics.mean(t_auto),
+                                "bitwise_equal_row": bool(torch.equal(y_row.view(torch.int64), y.view(torch.int64)))}
+        line += f", {form} {1e3 * statistics.mean(ts):.1f} us ({H.image_form()})"
+        H.close()
+    print(line + f", x{out['speedup_row_over_auto']:.3f}, bitwise {bitwise}, plan {plan_s:.2f} s", flush=True)
     A.close()
-    B.close()
-    del x, y_row, y_auto, y_f64
+    del x, y_row, y_auto, arms
     torch.cuda.empty_cache()
     return out
 

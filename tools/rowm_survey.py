@@ -2,7 +2,9 @@
 one-row kernels including the masked forms that multiply a CSR handle's private image (accumulate or not, 4-byte `int` or
 narrow 2-byte `u16` column field, fp64 values or 1-byte `u8` value codes): registers,
 spill bytes (csrc/build/*.ptxas.log) and how many of a step's loads ptxas issues ahead of the first multiply (cuobjdump
--sass).  A form whose loads are split by a DMUL stalls on its first gather before the rest is requested.  No GPU needed.
+-sass).  A form whose loads are split by a DMUL stalls on its first gather before the rest is requested.  Then the
+same for csr_pattern_kernel<W, ACCUM> (the pattern form of the private image): its W gathers (64-bit LDGs) against the
+first DMUL.  No GPU needed.
 
     python tools/rowm_survey.py            # every rowm instantiation and, for comparison, the one-row kernels
 """
@@ -34,9 +36,16 @@ def ptxas_info():
 def main():
     info = ptxas_info()
     sass = subprocess.run(["cuobjdump", "-sass", str(PKG / "libspmv_b200.so")], capture_output=True, text=True).stdout
-    rows = []
+    rows, patterns = [], []
     for body in re.split(r"Function : ", sass)[1:]:
         name = body.split()[0]
+        p = re.search(r"csr_pattern_kernelILi(\d+)ELb([01])E", name)
+        if p:
+            ops = re.findall(r"\b(LDG\.E\.64|DMUL)\b", body)
+            first = ops.index("DMUL") if "DMUL" in ops else len(ops)
+            rec = info.get(name, {})
+            patterns.append((int(p.group(1)), int(p.group(2)), rec.get("regs"), rec.get("spill"), first, ops.count("LDG.E.64")))
+            continue
         m = re.search(r"(csr|hll)_row(m|u?)_kernelILi(\d)E(?:Li(\d)ELi(\d)E)?([fd])(?:Lb([01])E)?(?:Lb([01])E)?([it])?([dfh])?", name)
         if not m:
             continue
@@ -63,6 +72,9 @@ def main():
     for r in sorted(rows):
         fmt, v, rp, b, c, regs, spill, ahead, most, total, kind = r
         print(f"{fmt} {'f32' if v == 'f' else 'f64'} {rp} {b} {c} {regs} {spill} {ahead}/{total} {most} {256 * c * rp} {kind}")
+    print("\ncsr_pattern_kernel: W accum regs spill_bytes gathers_ahead_of_first_DMUL/gathers")
+    for w, accum, regs, spill, ahead, total in sorted(patterns):
+        print(f"csr_pattern_kernel {w} {accum} {regs} {spill} {ahead}/{total}")
 
 
 if __name__ == "__main__":
