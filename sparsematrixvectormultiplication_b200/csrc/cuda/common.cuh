@@ -99,7 +99,7 @@ __device__ __forceinline__ int ldg_stream_s32(const int *p) {
     return r;
 }
 
-// the 16-bit column field of the narrow private image of a CSR handle (hll.cu), zero-extended into a 32-bit register
+// the 16-bit column field of a CSR handle's narrow private image (image.cu, hll.cu), zero-extended into 32 bits
 __device__ __forceinline__ int ldg_stream_u16(const uint16_t *p) {
     unsigned int r;
 #ifdef SPMV_STREAM_EVICT_FIRST
@@ -110,7 +110,7 @@ __device__ __forceinline__ int ldg_stream_u16(const uint16_t *p) {
     return (int)r;
 }
 
-// the 1-byte value code of the coded private image of a CSR handle (hll.cu), zero-extended into a 32-bit register
+// a CSR handle's private image (image.cu, hll.cu): a 1-byte value code or pattern id, zero-extended into 32 bits
 __device__ __forceinline__ int ldg_stream_u8(const uint8_t *p) {
     unsigned int r;
 #ifdef SPMV_STREAM_EVICT_FIRST

@@ -909,15 +909,6 @@ static void free_bins(spmv_b200_csr *A) {
     A->bins = BinPlan();
 }
 
-// frees the private image in whichever form the handle holds
-static void drop_image(spmv_b200_csr *A) {
-    spmv_b200_hll_free(A->image);
-    csr_patterns_free(A->patterns);
-    A->image = nullptr;
-    A->patterns = nullptr;
-    A->image_form = 0;
-}
-
 static void free_plan(spmv_b200_csr *A) {
     free_bins(A);
     cudaFree(A->tiles);
@@ -931,7 +922,7 @@ static void free_plan(spmv_b200_csr *A) {
     A->frag_partial = nullptr;
     A->spmm_partial = nullptr;
     A->num_tiles = A->num_long = A->num_frag = 0;
-    drop_image(A);
+    image_free(A->image);
 }
 
 template <typename V>
@@ -1043,68 +1034,32 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
     if (forced_batch >= 1 && forced_batch <= 8) {
         A->row_batch = forced_batch;
     } else if (A->max_row <= kRowKernelMaxLen && A->nnz >= kAutotuneMinNnz && env_int("SPMV_B200_AUTOTUNE", 1)) {
-        // candidates: (0) the TMA stream kernel, the row kernel with batch 2..7 and, on a matrix that owns its arrays, the
-        // private image (csr_image_build) in each of its forms: 64 + B hll_rowu_kernel, 32 + B hll_row_kernel, each on
-        // the fp64 values and, when the matrix holds at most 256 distinct value patterns, on the 1-byte value codes
-        // (+ kImageCoded).  All give the same bits on such rows.  The image qualifies when its padding adds at most a
-        // quarter to nnz and it fits in a quarter of the free memory (2 or 4 bytes of column field per slot, plus 8 + 1
-        // for both value streams, or 1 for the codes alone where both do not fit); it is freed again unless it wins, and
-        // the losing value stream is freed when it does.  Alongside, under the same padding rule (M * max_row slots), the
-        // pattern form (csr_patterns_build, id kImagePatterns) when the rows hold at most 256 patterns; whichever image
-        // loses is freed.
-        if (A->owns && A->num_long == 0) {
-            size_t free_bytes = 0, total_bytes = 0;
-            if (cudaMemGetInfo(&free_bytes, &total_bytes) == cudaSuccess) {
-                const long long fit_bytes = (long long)(free_bytes / 4) - 8LL * ((long long)M / 32 + 2);
-                if (fit_bytes >= 0 &&
-                    csr_image_build(A, A->nnz + A->nnz / 4, fit_bytes, kImageBoth, stream, &A->image) != SPMV_B200_OK)
-                    A->image = nullptr;
-                if ((long long)M * A->max_row <= A->nnz + A->nnz / 4 && (long long)M <= fit_bytes &&
-                    csr_patterns_build(A, stream, &A->patterns) != SPMV_B200_OK)
-                    A->patterns = nullptr;
-            }
-            cudaGetLastError();
-        }
-        int ids[25], n = 0, fallback = 0;  // 7 plain + 6 + 6 image forms on an irregular image + the pattern form
+        // candidates: (0) the TMA stream kernel, the row kernel with batch 2..7 and, on a matrix that owns its arrays, every
+        // form of the private image it qualifies for (image.cu).  All give the same bits on such rows.  The image is held
+        // only when one of its forms wins, and then in that form alone.
+        CsrImage *image = nullptr;
+        const int forms = A->owns && A->num_long == 0 ? image_candidates(A, stream, &image) : 0;
+        int ids[7], n = 0, fallback = 0;
         ids[n++] = 0;
         for (int batch = 2; batch <= 7; ++batch) {
             if (batch == A->row_batch) fallback = n;
             ids[n++] = batch;
         }
-        const int plain = n;
-        for (int coded = 0; A->image && coded <= 1; ++coded) {
-            const int flag = coded ? kImageCoded : 0;
-            if (coded ? !A->image->AC : !A->image->AS) continue;
-            for (int batch = 2; batch <= 7; ++batch)
-                if (A->image->segments.count == 0) ids[n++] = flag + 32 + batch;
-                else if (batch >= 4) ids[n++] = flag + 64 + batch;
-        }
-        if (A->patterns) ids[n++] = kImagePatterns;
-        auto image_form = [](int id) { return (id & kImageCoded) | ((id & ~kImageCoded) >= 64 ? id & ~kImageCoded : (id & ~kImageCoded) - 32); };
-        float ms[25];
-        const int pick = tune_candidates(M, A->N, n, fallback, stream, [&](int i, double *x, double *y) {
+        const int plain = n, total = plain + forms;
+        std::vector<float> ms((size_t)total);
+        const int pick = tune_candidates(M, A->N, total, fallback, stream, [&](int i, double *x, double *y) {
+            if (i >= plain) return image_launch_candidate(image, i - plain, x, y, stream);
             if (ids[i] == 0) return stream_launch_csr(A, x, y, 0, nullptr, stream);
-            if (ids[i] < 16) return launch_rows(0, M, A->row_ptr, A->col_idx, A->values, x, y, ids[i], 0, stream);
-            if (ids[i] == kImagePatterns) return csr_patterns_launch(A->patterns, 0, M, A->N, x, y, 0, stream);
-            return csr_image_launch(A->image, image_form(ids[i]), 0, A->image->num_hacks, x, y, 0, stream);
-        }, ms);
+            return launch_rows(0, M, A->row_ptr, A->col_idx, A->values, x, y, ids[i], 0, stream);
+        }, ms.data());
         int best = fallback;  // the plain choice stays for ALGO_ROW and the other entry points even when the image wins
         for (int i = 0; i < plain; ++i)
             if (ms[i] >= 0.0f && (ms[best] < 0.0f || ms[i] < ms[best])) best = i;
         if (ids[best] == 0) A->short_rows_stream = true;
         else A->row_batch = ids[best];
-        if (pick >= plain && ids[pick] == kImagePatterns) {
-            spmv_b200_hll_free(A->image);
-            A->image = nullptr;
-            A->image_form = kImagePatterns + A->patterns->width;
-        } else if (pick >= plain) {
-            csr_patterns_free(A->patterns);
-            A->patterns = nullptr;
-            A->image_form = image_form(ids[pick]);
-            csr_image_keep(A->image, (A->image_form & kImageCoded) != 0);
-        } else {
-            drop_image(A);
-        }
+        if (pick >= plain) image_keep(image, pick - plain);
+        else image_free(image);
+        A->image = image;
         // the fused iterated product (scale + |w|^2 partials in the tail): fused stream kernel (0) or fused row kernel
         if (A->num_long == 0) {
             double *partials = nullptr;
@@ -1386,7 +1341,7 @@ CsrPath csr_resolve(const spmv_b200_csr *A, int algo) {
         default:
             // every row short: one thread per row (serial order, so forced_tpr == 1 is honoured as well) -- on the
             // private image when the handle holds one
-            if (A->max_row <= kRowKernelMaxLen) return A->image || A->patterns ? kPathImage : A->short_rows_stream ? kPathStream : kPathRow;
+            if (A->max_row <= kRowKernelMaxLen) return A->image ? kPathImage : A->short_rows_stream ? kPathStream : kPathRow;
             if (A->forced_tpr == 1 || A->nnz <= (long long)kAutoStreamMaxAvg * A->M) return kPathStream;
             {   // longer rows: one lane count for all rows (vector kernel) only while the lengths are even; a longest row
                 // far above the mean (or above the long-row threshold) means skew -> lanes per row by length class
@@ -1402,9 +1357,7 @@ int csr_launch_window(const spmv_b200_csr *A, CsrPath path, int unit_begin, int 
     if (path == kPathBinned) return launch_binned<double>(A, A->values, x, y, accumulate, stream);  // whole matrix: rows are permuted
     if (path == kPathRow)
         return launch_rows(unit_begin, unit_end, A->row_ptr, A->col_idx, A->values, x, y, A->row_batch, accumulate, stream);
-    if (path == kPathImage && A->patterns) return csr_patterns_launch(A->patterns, unit_begin, unit_end, A->N, x, y, accumulate, stream);
-    if (path == kPathImage)  // rows, in whole hacks: unit_begin must be a multiple of 32
-        return csr_image_launch(A->image, A->image_form, unit_begin / 32, (unit_end + 31) / 32, x, y, accumulate, stream);
+    if (path == kPathImage) return image_launch(A->image, unit_begin, unit_end, x, y, accumulate, stream);
     if (path == kPathVector)
         return launch_vector(unit_begin, unit_end, A->row_ptr, A->col_idx, A->values, x, y, pick_vector_width(A->nnz, A->M),
                              accumulate, stream, (size_t)A->N * sizeof(double), safe_vector_nnz(A));
@@ -1680,16 +1633,7 @@ int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info) {
     info->fused_batch = A->fused_batch;
     info->flat_batch = A->flat_batch;
     info->flat_chunks = 1;
-    info->image_bytes = A->image ? 12 * A->image->slots : 0;
-    info->image_form = A->image ? A->image_form & ~kImageCoded : 0;
-    info->image_index_bytes = !A->image ? 0 : A->image->JA16 ? 2 : 4;
-    info->image_device_bytes = A->image ? csr_image_bytes(A->image) : 0;
-    info->image_value_bytes = A->image ? csr_image_value_bytes(A->image) : 0;
-    info->image_patterns = A->patterns ? A->patterns->count : 0;
-    if (A->patterns) {  // the pattern form: one byte per row plus the dictionary
-        info->image_form = A->image_form;
-        info->image_bytes = info->image_device_bytes = A->M + csr_patterns_dict_bytes(A->patterns);
-    }
+    image_info(A->image, info);
     return SPMV_B200_OK;
 }
 
@@ -1714,7 +1658,7 @@ int spmv_b200_csr_spmv(const spmv_b200_csr *A, const double *d_x, double *d_y, i
     if (!A || !d_y || (A->N > 0 && !d_x)) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: NULL argument");
     if (A->M == 0) return SPMV_B200_OK;
     if (algo < SPMV_B200_ALGO_AUTO || algo > SPMV_B200_ALGO_ROW_IMAGE) return fail(SPMV_B200_ERR_INVALID, "csr_spmv: unknown algo %d", algo);
-    if (algo == SPMV_B200_ALGO_ROW_IMAGE && !A->image && !A->patterns)
+    if (algo == SPMV_B200_ALGO_ROW_IMAGE && !A->image)
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv: the matrix holds no image (spmv_b200_csr_set_image)");
     const CsrPath path = csr_resolve(A, algo);
     const bool by_rows = path == kPathVector || path == kPathRow || path == kPathImage;
@@ -1840,7 +1784,7 @@ int spmv_b200_csr_remap_columns(spmv_b200_csr *A, int nparts, const long long *s
         SPMV_TRY_CUDA(cudaGetLastError());
     }
     A->N = (int)(nparts * stride);  // plans, tiles and the fp32 copy of the values do not depend on the column ids;
-    drop_image(A);                  // the private image does
+    image_free(A->image);           // the private image does
     SPMV_TRY_CUDA(cudaStreamSynchronize(as_stream(stream)));
     return SPMV_B200_OK;
 }
@@ -1849,32 +1793,10 @@ int spmv_b200_csr_set_image(spmv_b200_csr *A, int mode, void *stream) {
     if (!A) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: NULL matrix");
     if (mode < 0 || mode > 3) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: unknown mode %d", mode);
     if (mode == 0) {
-        drop_image(A);
+        image_free(A->image);
         return SPMV_B200_OK;
     }
-    if (!A->owns) return fail(SPMV_B200_ERR_INVALID, "csr_set_image: the matrix wraps arrays it does not own");
-    if (A->max_row > kRowKernelMaxLen || A->num_long > 0)
-        return fail(SPMV_B200_ERR_INVALID, "csr_set_image: rows of up to %d nonzeros and no long rows only (longest row: %d)",
-                    kRowKernelMaxLen, A->max_row);
-    if (mode == 3) {
-        if (A->patterns) return SPMV_B200_OK;
-        CsrPatterns *patterns = nullptr;  // the held image stays unless the pattern form can be built
-        if (csr_patterns_build(A, as_stream(stream), &patterns) != SPMV_B200_OK)
-            return fail(SPMV_B200_ERR_INVALID, "csr_set_image: the pattern form needs 1 to %d nonzeros per row, at most %d distinct "
-                        "rows and a dictionary of at most %d bytes", kRowKernelMaxLen, kMaxPatterns, kPatternDictMaxBytes);
-        drop_image(A);
-        A->patterns = patterns;
-        A->image_form = kImagePatterns + patterns->width;
-        return SPMV_B200_OK;
-    }
-    const bool coded = mode == 2;
-    if (A->image && (coded ? A->image->AC != nullptr : A->image->AS != nullptr)) return SPMV_B200_OK;
-    spmv_b200_hll *image = nullptr;  // the held image stays until the new one is built (mode 2 fails on > 256 patterns)
-    SPMV_TRY(csr_image_build(A, -1, -1, coded ? kImageCodes : kImageF64, as_stream(stream), &image));
-    drop_image(A);
-    A->image = image;
-    A->image_form = csr_image_default_form(A->image);
-    return SPMV_B200_OK;
+    return image_build(A, mode, as_stream(stream));
 }
 
 int spmv_b200_csr_interior_rows(const spmv_b200_csr *A, long long col_lo, long long col_hi, int *row_lo, int *row_hi,
@@ -1921,8 +1843,8 @@ int spmv_b200_csr_spmv_rows(const spmv_b200_csr *A, int row_begin, int row_end, 
     if (!A || !d_y || !d_x) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_rows: NULL argument");
     if (row_begin < 0 || row_end > A->M || row_begin > row_end)
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv_rows: range [%d,%d) outside [0,%d)", row_begin, row_end, A->M);
-    if (A->patterns)  // the pattern form of the private image: any row range, the same bits
-        return csr_patterns_launch(A->patterns, row_begin, row_end, A->N, d_x, d_y, 0, as_stream(stream));
+    if (A->image && image_any_rows(A->image))  // the private image where it takes any row range: the same bits
+        return image_launch(A->image, row_begin, row_end, d_x, d_y, 0, as_stream(stream));
     if (A->max_row <= kRowKernelMaxLen)  // stencils: the thread-per-row kernel with the batch tuned at plan time (serial order)
         return launch_rows(row_begin, row_end, A->row_ptr, A->col_idx, A->values, d_x, d_y, A->row_batch, 0, as_stream(stream));
     return launch_vector(row_begin, row_end, A->row_ptr, A->col_idx, A->values, d_x, d_y,

@@ -204,19 +204,7 @@ int tune_candidates(long long M, long long N, int n, int fallback, cudaStream_t 
     return best;
 }
 
-// The pattern form of a CSR handle's private image (pattern.cu): a matrix whose rows hold at most kMaxPatterns distinct
-// patterns -- a pattern is the row's length, the col - row of each slot and the 64-bit pattern of each value -- stored
-// as one byte per row that names the row's pattern in a dictionary the kernel stages in shared memory.
-constexpr int kMaxPatterns = 256;
-constexpr int kPatternDictMaxBytes = 24 * 1024;  // P * W * 12: 8 CTAs of 256 threads stay resident per SM
-struct CsrPatterns {
-    int count = 0;          // P patterns, in the order of their (length, deltas, value bits)
-    int width = 0;          // W: the matrix's longest row
-    uint8_t *id = nullptr;  // device [M]: the pattern of each row
-    int *dict = nullptr;    // device: value[W][P] (fp64), delta[W][P] (int32), len[P] (int32); a slot at or past a
-                            // pattern's length holds delta 0 and value 0.0
-};
-inline long long csr_patterns_dict_bytes(const CsrPatterns *P) { return 12LL * P->width * P->count + 4LL * P->count; }
+struct CsrImage;  // image.cu: the private image of a CSR handle
 }  // namespace spmv
 
 struct spmv_b200_csr {
@@ -253,18 +241,9 @@ struct spmv_b200_csr {
     int stages = spmv::kDefaultStages;
     int consumers = 12;
     int stream_grid = 0;
-    // private column-major image of the matrix (csr_image_build, spmv_b200_csr_set_image): HLL layout with the padding
-    // slots marked, multiplied by the masked hll_rowu / hll_row kernels -- bit for bit csr_row_kernel.  Narrow (JA16, 10
-    // bytes per slot) when every slot's column lies within 2^14 of its row, else wide (JA, 12 bytes per slot).  Held only
-    // when plan-time timing found it faster (or set_image asked for it); owned arrays only, dropped by remap_columns.
-    // Its values are fp64 (AS) or, when the matrix holds at most 256 distinct 64-bit patterns, 1-byte codes into a table
-    // (AC, table): 3 or 5 bytes per slot; the plan times both and keeps the faster.
-    spmv_b200_hll *image = nullptr;
-    int image_form = 0;  // 64 + B: hll_rowu_kernel<B, double, true>; B: hll_row_kernel<B, double, true> (index type: JA16 / JA),
-                         // plus spmv::kImageCoded when it reads the value codes; 256 + W: csr_pattern_kernel<W> on `patterns`
-    // the pattern form of the private image (spmv::CsrPatterns): held instead of `image` when the plan timed it faster or
-    // set_image mode 3 asked for it; same rules otherwise
-    spmv::CsrPatterns *patterns = nullptr;
+    // private image of the matrix (image.cu), column-major or patterns: held only when plan-time timing found it faster
+    // (or set_image asked for it); owned arrays only, dropped by remap_columns
+    spmv::CsrImage *image = nullptr;
     // staging vectors of the *_host entry points
     double *stage_x = nullptr;
     double *stage_y = nullptr;
@@ -290,13 +269,7 @@ struct spmv_b200_hll {
     long long slots = 0, ref_slots = 0;
     long long *hack_off = nullptr;  // device [num_hacks+1]
     int *JA = nullptr;              // device [slots]
-    uint16_t *JA16 = nullptr;       // device [slots]: the narrow column field of a CSR handle's private image (JA is then
-                                    // NULL): bits 0-14 hold col - row as a 15-bit two's complement, bit 15 marks padding
     double *AS = nullptr;           // device [slots]
-    uint8_t *AC = nullptr;          // device [slots]: the value codes of a CSR handle's coded private image (AS is then NULL
-                                    // once the plan has decided): the slot's value is table[AC[slot]], padding holds code 0
-    double *table = nullptr;        // device [max(num_values, 1)]: the distinct 64-bit value patterns, ascending as uint64
-    int num_values = 0;             // K <= kMaxImageValues patterns in the table (0: no coded image)
     float *AS32 = nullptr;          // fp32 copy of AS (spmv_b200_hll_enable_f32)
     std::vector<long long> host_off;
     // stream kernel plan
@@ -339,30 +312,40 @@ HllPath hll_resolve(const spmv_b200_hll *H);
 int hll_launch_window(const spmv_b200_hll *H, HllPath path, int unit_begin, int unit_end, const double *x, double *y,
                       cudaStream_t stream);  // units: tiles (stream kernel) or hacks (slice and row kernels)
 int env_int(const char *name, int fallback);
-// hll.cu: the private image of a CSR handle.  csr_image_build leaves *out NULL when the image would exceed max_slots
-// slots or its column and value arrays max_bytes bytes (< 0: no limit); forms as in spmv_b200_csr::image_form.
-// values: which value streams it fills -- fp64 (AS), the 1-byte codes (AC + table; the build fails with
-// SPMV_B200_ERR_INVALID on a matrix of more than kMaxImageValues distinct patterns), or both where they fit (plan time:
-// both when they fit, else the codes alone, else fp64 alone).
-constexpr int kMaxImageValues = 256;
-constexpr int kImageCoded = 128;  // image_form flag: the kernel reads the value codes
-enum ImageValues { kImageF64 = 1, kImageCodes = 2, kImageBoth = 3 };
-int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_bytes, ImageValues values, cudaStream_t stream,
-                    spmv_b200_hll **out);
-long long csr_image_bytes(const spmv_b200_hll *H);  // device bytes of JA / JA16, AS, AC and the table
-int csr_image_value_bytes(const spmv_b200_hll *H);  // 8 (fp64), 1 (codes) or 9 (both, during the plan's timing)
-void csr_image_keep(spmv_b200_hll *H, bool coded);  // frees the other value stream
-int csr_image_default_form(const spmv_b200_hll *H);
-int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
-                     int accumulate, cudaStream_t stream);
-// pattern.cu: builds the pattern form of A (owned arrays and no long rows assumed by the caller).  SPMV_B200_ERR_INVALID,
-// without a message (the plan tries every eligible matrix), when A does not qualify: no row or one above
-// kRowKernelMaxLen, more than kMaxPatterns patterns, or a dictionary above kPatternDictMaxBytes
-constexpr int kImagePatterns = 256;  // image_form of the pattern form: kImagePatterns + W
-int csr_patterns_build(const spmv_b200_csr *A, cudaStream_t stream, CsrPatterns **out);
-void csr_patterns_free(CsrPatterns *P);
-int csr_patterns_launch(const CsrPatterns *P, int row_begin, int row_end, int N, const double *x, double *y, int accumulate,
-                        cudaStream_t stream);  // any row range
+// hll.cu: the column-major layout, its fill and the masked kernels, for spmv_b200_hll_from_csr and the private image of a
+// CSR handle (image.cu).  hll_layout: the hack widths of M rows, scanned into hack_off (device [num_hacks + 1], allocated
+// here), its host copy, the widest hack and, unless narrow is NULL, whether every slot fits the image's narrow column
+// field (col - row within 2^14, padding included).  The column field is JA, or JA16 (the narrow field) when that is not
+// NULL.  hll_fill fills it and each value stream that is not NULL: fp64 (AS), 1-byte codes into table[K] (AC); masked: a
+// padding slot is marked as such (always so in the narrow field).  hll_masked_launch: y = A x (or y += A x) over hacks
+// [hack_begin, hack_end) by the masked hll_rowu_kernel<batch> (offset_free; regular layouts) or hll_row_kernel<batch>,
+// on the codes when AC is not NULL (K >= 1), else on AS.
+int hll_layout(int M, int N, const int *row_ptr, const int *col_idx, cudaStream_t stream, long long **hack_off,
+               std::vector<long long> &host_off, int *max_width, bool *narrow);
+HllSegments hll_find_segments(const std::vector<long long> &host_off, int num_hacks);
+int hll_fill(int M, int N, const int *row_ptr, const int *col_idx, const double *values, int num_hacks,
+             const long long *hack_off, int *JA, uint16_t *JA16, double *AS, uint8_t *AC, const double *table, int K,
+             bool masked, cudaStream_t stream);
+int hll_masked_launch(int hack_begin, int hack_end, int M, const long long *hack_off, const HllSegments &seg, const int *JA,
+                      const uint16_t *JA16, long long slots, const double *AS, const uint8_t *AC, const double *table, int K,
+                      int batch, bool offset_free, int accumulate, const double *x, double *y, cudaStream_t stream);
+// image.cu: the private image of a CSR handle.  Plan time (A owns its arrays and has no long rows: the plan checks):
+// image_candidates builds every form A qualifies for and returns their number (*out NULL when none),
+// image_launch_candidate multiplies scratch vectors with candidate i (y = A x over all rows), and image_keep holds
+// candidate i and frees every other stream -- or image_free frees them all (and sets img to NULL).
+int image_candidates(const spmv_b200_csr *A, cudaStream_t stream, CsrImage **out);
+int image_launch_candidate(const CsrImage *img, int i, const double *x, double *y, cudaStream_t stream);
+void image_keep(CsrImage *img, int i);
+void image_free(CsrImage *&img);
+// spmv_b200_csr_set_image modes 1 (column-major, fp64 values), 2 (column-major, value codes) and 3 (patterns): replaces
+// A->image by that form unless it holds it already; on failure (also: arrays not owned, long rows) A->image stays
+int image_build(spmv_b200_csr *A, int mode, cudaStream_t stream);
+// the held form over rows [row_begin, row_end): the column-major form runs whole hacks (row_begin a multiple of 32), the
+// pattern form any row range (image_any_rows)
+int image_launch(const CsrImage *img, int row_begin, int row_end, const double *x, double *y, int accumulate,
+                 cudaStream_t stream);
+bool image_any_rows(const CsrImage *img);
+void image_info(const CsrImage *img, spmv_b200_csr_info_t *info);  // the image_* fields (all 0 for NULL)
 int hll_row_forms();                                             // hll.cu: forms of hll_rowm_kernel (spmv_b200_row_forms)
 int hll_row_form(int index, int *hacks, int *batch, int *ctas);  // 0 = ok
 int fused_ctas_per_sm();  // csr.cu: CTAs per SM in the grid of the fused row kernels (CSR and HLL use the same value)

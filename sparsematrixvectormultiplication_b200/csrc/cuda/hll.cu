@@ -143,7 +143,7 @@ hll_slice_kernel(int hack_begin, int hack_end, const long long *__restrict__ hac
 // The hack-row loop of every lane-per-row HLL kernel: acc plus the products of row `row` of a hack, whose slot j lies at
 // base + j * 32 (j < width), BATCH slots requested before the first gather.  One lane per row, sequential in j, mul and
 // add rounded separately: bit-identical to the reference's spmv_hll_serial (src/hll_matrix.c:294-306), padding slots
-// (x 0.0) included.  MASKED: the private image of a CSR handle (csr_image_build), whose padding slots carry bit 31 of the
+// (x 0.0) included.  MASKED: the private image of a CSR handle (image.cu), whose padding slots carry bit 31 of the
 // column (I = int) or bit 15 of a row-relative 16-bit field (I = uint16_t, image_column).  Such a slot gathers its column
 // like any other and skips the add: bit-identical to csr_row_kernel for every x.  (Adding the padding's 0 * x[c] would
 // give NaN for an infinite x[c], and +0 turns an untouched -0.0 positive.)  The loads are never predicated on the loaded
@@ -418,8 +418,7 @@ hll_row_fused_kernel(int num_hacks, const long long *__restrict__ hack_off, cons
 }
 
 // ---- CSR -> HLL on the device ----------------------------------------------------------------------
-__global__ void hll_width_kernel(int M, int num_hacks, const int *__restrict__ row_ptr, long long *__restrict__ slots,
-                                 int *__restrict__ widths) {
+__global__ void hll_width_kernel(int M, int num_hacks, const int *__restrict__ row_ptr, long long *__restrict__ slots) {
     const int hack = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (hack > num_hacks) return;
     const int lane = threadIdx.x & 31;
@@ -430,10 +429,7 @@ __global__ void hll_width_kernel(int M, int num_hacks, const int *__restrict__ r
     }
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) len = max(len, __shfl_xor_sync(0xffffffffu, len, off));
-    if (lane == 0) {
-        slots[hack] = (long long)len * kHack;  // slots[num_hacks] = 0: the scan ends with the total
-        if (hack < num_hacks) widths[hack] = len;
-    }
+    if (lane == 0) slots[hack] = (long long)len * kHack;  // slots[num_hacks] = 0: the scan ends with the total
 }
 
 // the column field of a slot (mark: OR'ed into a padding slot's column of the wide image; the narrow one is always masked)
@@ -492,10 +488,11 @@ __global__ void hll_fill_kernel(int M, int N, int num_hacks, const int *__restri
 }
 
 // Does every slot of the image fit the narrow field (col - row in [kDeltaMin, kDeltaMax])?  One thread per row of the
-// padded image, after hll_width_kernel: a real slot holds col - row, a padding slot repeats the delta of its row's last
-// real column or, in a row without one that still has slots, gathers min(row, N - 1) (hll_fill_kernel).  Clears *fits.
+// padded image: a real slot holds col - row, a padding slot repeats the delta of its row's last real column or, in a row
+// without one that still has slots, gathers min(row, N - 1) (hll_fill_kernel).  Clears *fits.
 __global__ void hll_narrow_check_kernel(int M, int N, int num_hacks, const int *__restrict__ row_ptr,
-                                        const int *__restrict__ col_idx, const int *__restrict__ widths, int *__restrict__ fits) {
+                                        const int *__restrict__ col_idx, const long long *__restrict__ hack_off,
+                                        int *__restrict__ fits) {
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= (long long)num_hacks * kHack) return;
     int begin = 0, end = 0;
@@ -508,69 +505,12 @@ __global__ void hll_narrow_check_kernel(int M, int N, int num_hacks, const int *
         const long long d = col_idx[k] - r;
         ok = ok && d >= kDeltaMin && d <= kDeltaMax;
     }
-    if (begin == end && widths[r / kHack] > 0) ok = r - (N - 1) <= -kDeltaMin;
+    if (begin == end && hack_off[r / kHack + 1] > hack_off[r / kHack]) ok = r - (N - 1) <= -kDeltaMin;
     if (!ok) *fits = 0;
-}
-
-// The distinct 64-bit value patterns among the nonzeros (the table of a coded image): +0.0 and -0.0, and NaNs of different
-// payloads, are different patterns.  keys: an open-addressing set of kDictSlots entries, kDictEmpty when free; the pattern
-// kDictEmpty itself sets state[1].  state[0] counts the patterns and passes kMaxImageValues as soon as a 257th appears (or
-// a probe walks past kMaxImageValues occupied entries, which only more patterns can fill); every warp then stops.  A warp
-// first merges its lanes' equal patterns (__match_any_sync), and one lane per pattern probes with a plain load: a pattern
-// already in the set -- every one after the first few on a stencil -- costs no atomic.  An entry, once written, never
-// changes, so a stale load can only read kDictEmpty, and the compare-and-swap then tells the truth.
-constexpr int kDictSlots = 1024;
-constexpr unsigned long long kDictEmpty = ~0ULL;
-
-__device__ __forceinline__ void dict_insert(unsigned long long k, unsigned long long *keys, int *state) {
-    if (k == kDictEmpty) {
-        state[1] = 1;
-        return;
-    }
-    unsigned int h = (unsigned int)mix64(k) & (kDictSlots - 1);
-    for (int probe = 0; probe <= kMaxImageValues; ++probe) {
-        unsigned long long cur = keys[h];
-        if (cur == kDictEmpty) {
-            cur = atomicCAS(keys + h, kDictEmpty, k);
-            if (cur == kDictEmpty) {
-                atomicAdd(state, 1);
-                return;
-            }
-        }
-        if (cur == k) return;
-        h = (h + 1) & (kDictSlots - 1);
-    }
-    atomicMax(state, kMaxImageValues + 1);
-}
-
-__global__ void hll_value_dict_kernel(long long nnz, const double *__restrict__ values, unsigned long long *keys, int *state) {
-    const int lane = threadIdx.x & 31;
-    const long long stride = (long long)gridDim.x * blockDim.x;
-    int step = 0;
-    for (long long base = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); base < nnz; base += stride, ++step) {
-        if ((step & 63) == 0) {  // warp-uniform
-            int stop = lane == 0 ? *(volatile int *)state : 0;
-            if (__shfl_sync(0xffffffffu, stop, 0) > kMaxImageValues) return;
-        }
-        const unsigned long long k = (unsigned long long)__double_as_longlong(values[min(base + lane, nnz - 1)]);
-        const unsigned int same = __match_any_sync(0xffffffffu, k);
-        if (lane == __ffs(same) - 1) dict_insert(k, keys, state);
-    }
-}
-
-__global__ void max_int_kernel(const int *__restrict__ v, int n, int *__restrict__ out) {
-    int m = 0;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) m = max(m, v[i]);
-    atomicMax(out, m);  // integer max: order independent
 }
 
 }  // namespace spmv
 
-
-// csr.cu
-extern "C" int spmv_b200_csr_device_arrays(const spmv_b200_csr *A, const int **d_row_ptr, const int **d_col_idx,
-                                           const double **d_values);
-extern "C" int spmv_b200_csr_info(const spmv_b200_csr *A, spmv_b200_csr_info_t *info);
 
 using namespace spmv;
 
@@ -667,12 +607,10 @@ static int hll_launch(const spmv_b200_hll *H, int hack_begin, int hack_end, cons
     return SPMV_B200_OK;
 }
 
-static int hll_alloc_arena(spmv_b200_hll *H, bool narrow = false, bool f64 = true, bool codes = false) {
+static int hll_alloc_arena(spmv_b200_hll *H) {
     const size_t n = (size_t)std::max<long long>(H->slots, 32);
-    if (narrow) SPMV_TRY_CUDA(cudaMalloc(&H->JA16, n * sizeof(uint16_t)));
-    else SPMV_TRY_CUDA(cudaMalloc(&H->JA, n * sizeof(int)));
-    if (f64) SPMV_TRY_CUDA(cudaMalloc(&H->AS, n * sizeof(double)));
-    if (codes) SPMV_TRY_CUDA(cudaMalloc(&H->AC, n * sizeof(uint8_t)));
+    SPMV_TRY_CUDA(cudaMalloc(&H->JA, n * sizeof(int)));
+    SPMV_TRY_CUDA(cudaMalloc(&H->AS, n * sizeof(double)));
     return SPMV_B200_OK;
 }
 
@@ -693,11 +631,10 @@ int hll_launch_window(const spmv_b200_hll *H, HllPath path, int unit_begin, int 
 
 // batch of the lane-per-row kernel: the hack width when it is uniform and small; timed at plan time on large images
 // runs of hacks of equal width, from the host copy of the offsets (HllSegments, handles.cuh)
-static void hll_find_segments(spmv_b200_hll *H) {
+HllSegments hll_find_segments(const std::vector<long long> &off, int num_hacks) {
     HllSegments seg;
-    const std::vector<long long> &off = H->host_off;
-    bool regular = (int)off.size() == H->num_hacks + 1 && H->num_hacks > 0;
-    for (int h = 0; regular && h < H->num_hacks; ++h) {
+    bool regular = (int)off.size() == num_hacks + 1 && num_hacks > 0;
+    for (int h = 0; regular && h < num_hacks; ++h) {
         const int w = (int)((off[h + 1] - off[h]) / kHack);
         if (seg.count > 0 && seg.width[seg.count - 1] == w) continue;
         if (seg.count == kMaxHllSegments) {
@@ -711,14 +648,14 @@ static void hll_find_segments(spmv_b200_hll *H) {
     }
     if (!regular) seg = HllSegments();
     else {
-        seg.begin[seg.count] = H->num_hacks;
+        seg.begin[seg.count] = num_hacks;
         for (int s = seg.count + 1; s <= kMaxHllSegments; ++s) seg.begin[s] = 0x7fffffff;  // never reached: the kernel tests no count
     }
-    H->segments = seg;
+    return seg;
 }
 
 static void hll_pick_row_batch(spmv_b200_hll *H, cudaStream_t stream) {
-    hll_find_segments(H);
+    H->segments = hll_find_segments(H->host_off, H->num_hacks);
     const int forced = env_int("SPMV_B200_HLL_ROW_BATCH", 0);
     H->narrow_stream = false;
     H->row_form = 0;
@@ -780,212 +717,102 @@ static void hll_pick_row_batch(spmv_b200_hll *H, cudaStream_t stream) {
         cudaFree(partials);
     }
 }
-}  // namespace spmv
 
-// CSR -> column-major image on the device: widths, scan, fill (spmv_b200_hll_from_csr and the private image of a CSR
-// handle).  image: the private image -- padding slots marked, and narrow (JA16) when every slot fits it.  values: the value
-// streams to fill (csr_image_build; the HLL format always has AS).  max_slots / max_bytes >= 0: an image of more slots or
-// more bytes of columns, values and table is not filled (H->JA and H->JA16 stay NULL, H->slots tells its size).
-static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, bool image, long long max_slots, long long max_bytes,
-                       spmv_b200_hll *H, ImageValues values = kImageF64) {
-    spmv_b200_csr_info_t ci;
-    const int *row_ptr, *col_idx;
-    const double *values_ptr;
-    SPMV_TRY(spmv_b200_csr_info(A, &ci));
-    SPMV_TRY(spmv_b200_csr_device_arrays(A, &row_ptr, &col_idx, &values_ptr));
-    H->M = ci.M;
-    H->N = ci.N;
-    const int nb = H->num_hacks = (ci.M + kHack - 1) / kHack;
+int hll_layout(int M, int N, const int *row_ptr, const int *col_idx, cudaStream_t stream, long long **hack_off,
+               std::vector<long long> &host_off, int *max_width, bool *narrow) {
+    const int nb = (M + kHack - 1) / kHack;
     long long *slots = nullptr;
-    int *widths = nullptr, *d_max = nullptr;  // d_max[0]: widest hack; d_max[1]: every slot fits the narrow field
     void *temp = nullptr;
-    unsigned long long *keys = nullptr;  // the dictionary pass (hll_value_dict_kernel): keys[kDictSlots], then state[2]
-    int fits = 0;
+    int *d_fits = nullptr, fits = 1;
     auto body = [&]() -> int {
-        SPMV_TRY_CUDA(cudaMalloc(&H->hack_off, ((size_t)nb + 1) * sizeof(long long)));
+        SPMV_TRY_CUDA(cudaMalloc(hack_off, ((size_t)nb + 1) * sizeof(long long)));
         SPMV_TRY_CUDA(cudaMalloc(&slots, ((size_t)nb + 1) * sizeof(long long)));
-        SPMV_TRY_CUDA(cudaMalloc(&widths, (size_t)std::max(nb, 1) * sizeof(int)));
-        SPMV_TRY_CUDA(cudaMalloc(&d_max, 2 * sizeof(int)));
-        const int init[2] = {0, image ? 1 : 0};
-        SPMV_TRY_CUDA(cudaMemcpyAsync(d_max, init, sizeof init, cudaMemcpyHostToDevice, stream));
-        hll_width_kernel<<<blocks_for(nb + 1, 8), 256, 0, stream>>>(ci.M, nb, row_ptr, slots, widths);
+        hll_width_kernel<<<blocks_for(nb + 1, 8), 256, 0, stream>>>(M, nb, row_ptr, slots);
         SPMV_TRY_CUDA(cudaGetLastError());
-        if (image && nb > 0) {
-            hll_narrow_check_kernel<<<blocks_for((long long)nb * kHack, 256), 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx,
-                                                                                            widths, d_max + 1);
-            SPMV_TRY_CUDA(cudaGetLastError());
-        }
-        if (values & kImageCodes) {
-            SPMV_TRY_CUDA(cudaMalloc(&keys, kDictSlots * sizeof(unsigned long long) + 2 * sizeof(int)));
-            SPMV_TRY_CUDA(cudaMemsetAsync(keys, 0xff, kDictSlots * sizeof(unsigned long long), stream));
-            SPMV_TRY_CUDA(cudaMemsetAsync(keys + kDictSlots, 0, 2 * sizeof(int), stream));
-            if (ci.nnz > 0) {
-                hll_value_dict_kernel<<<std::min(blocks_for(ci.nnz, 256), 4096u), 256, 0, stream>>>(
-                    ci.nnz, values_ptr, keys, reinterpret_cast<int *>(keys + kDictSlots));
-                SPMV_TRY_CUDA(cudaGetLastError());
-            }
-        }
         size_t temp_bytes = 0;
-        SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, slots, H->hack_off, nb + 1, stream));
+        SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, slots, *hack_off, nb + 1, stream));
         SPMV_TRY_CUDA(cudaMalloc(&temp, temp_bytes ? temp_bytes : 1));
-        SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, slots, H->hack_off, nb + 1, stream));
-        if (nb > 0) {
-            max_int_kernel<<<std::min(blocks_for(nb, 256), 1024u), 256, 0, stream>>>(widths, nb, d_max);
+        SPMV_TRY_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, slots, *hack_off, nb + 1, stream));
+        if (narrow && nb > 0) {
+            SPMV_TRY_CUDA(cudaMalloc(&d_fits, sizeof(int)));
+            SPMV_TRY_CUDA(cudaMemcpyAsync(d_fits, &fits, sizeof(int), cudaMemcpyHostToDevice, stream));
+            hll_narrow_check_kernel<<<blocks_for((long long)nb * kHack, 256), 256, 0, stream>>>(M, N, nb, row_ptr, col_idx,
+                                                                                            *hack_off, d_fits);
             SPMV_TRY_CUDA(cudaGetLastError());
+            SPMV_TRY_CUDA(cudaMemcpyAsync(&fits, d_fits, sizeof(int), cudaMemcpyDeviceToHost, stream));
         }
-        H->host_off.resize((size_t)nb + 1);
-        SPMV_TRY_CUDA(cudaMemcpyAsync(H->host_off.data(), H->hack_off, ((size_t)nb + 1) * sizeof(long long),
-                                      cudaMemcpyDeviceToHost, stream));
-        SPMV_TRY_CUDA(cudaMemcpyAsync(&H->max_width, d_max, sizeof(int), cudaMemcpyDeviceToHost, stream));
-        SPMV_TRY_CUDA(cudaMemcpyAsync(&fits, d_max + 1, sizeof(int), cudaMemcpyDeviceToHost, stream));
-        std::vector<unsigned long long> dict;
-        int state[2] = {0, 0};
-        if (keys) {
-            dict.resize(kDictSlots);
-            SPMV_TRY_CUDA(cudaMemcpyAsync(dict.data(), keys, kDictSlots * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
-            SPMV_TRY_CUDA(cudaMemcpyAsync(state, keys + kDictSlots, sizeof state, cudaMemcpyDeviceToHost, stream));
-        }
-        SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
-        // the table: the patterns ascending as uint64, so that the image does not depend on the order of the inserts
-        bool codes = keys != nullptr && state[0] <= kMaxImageValues;
-        if (codes) {
-            dict.erase(std::remove(dict.begin(), dict.end(), kDictEmpty), dict.end());
-            if (state[1]) dict.push_back(kDictEmpty);
-            std::sort(dict.begin(), dict.end());
-            codes = (int)dict.size() <= kMaxImageValues;
-        }
-        if (values == kImageCodes && !codes)
-            return fail(SPMV_B200_ERR_INVALID, "csr image: the values hold more than %d distinct 64-bit patterns", kMaxImageValues);
-        H->slots = H->host_off[nb];
-        // reference layout keeps the last block short: its padded rows do not exist there
-        const int last_rows = nb > 0 ? ci.M - (nb - 1) * kHack : 0;
-        H->ref_slots = H->slots;
-        if (nb > 0) H->ref_slots -= ((H->host_off[nb] - H->host_off[nb - 1]) / kHack) * (kHack - last_rows);
-        if (max_slots >= 0 && H->slots > max_slots) return SPMV_B200_OK;
-        // bytes per slot of each choice, largest first: both value streams (plan time), the codes alone, fp64 alone
-        const long long index = fits ? 2 : 4, table = codes ? 8LL * (long long)dict.size() : 0;
-        auto fit = [&](long long per_slot, long long extra) { return max_bytes < 0 || H->slots * per_slot + extra <= max_bytes; };
-        bool f64 = values != kImageCodes, use_codes = codes;
-        if (f64 && use_codes && !fit(index + 9, table)) f64 = false;  // plan time: the codes alone where both do not fit
-        if (!use_codes && !fit(index + 8, 0)) return SPMV_B200_OK;
-        if (use_codes && !fit(index + (f64 ? 9 : 1), table)) return SPMV_B200_OK;
-        SPMV_TRY(hll_alloc_arena(H, fits != 0, f64, use_codes));
-        if (use_codes) {
-            std::vector<double> tab(std::max<size_t>(dict.size(), 1), 0.0);  // at least one entry: padding reads code 0
-            std::memcpy(tab.data(), dict.data(), dict.size() * sizeof(double));
-            H->num_values = (int)dict.size();
-            SPMV_TRY_CUDA(cudaMalloc(&H->table, tab.size() * sizeof(double)));
-            SPMV_TRY_CUDA(cudaMemcpyAsync(H->table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, stream));
-            SPMV_TRY_CUDA(cudaStreamSynchronize(stream));  // tab is a local
-        }
-        if (nb > 0) {
-            const unsigned int g = blocks_for((long long)nb * kHack, 256);
-            const int mark = image ? kPadMark : 0;
-            const int K = H->num_values;
-            if (fits)
-                hll_fill_kernel<<<g, 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx, values_ptr, H->hack_off, H->JA16, H->AS, H->AC,
-                                                       H->table, K, mark);
-            else
-                hll_fill_kernel<<<g, 256, 0, stream>>>(ci.M, ci.N, nb, row_ptr, col_idx, values_ptr, H->hack_off, H->JA, H->AS, H->AC,
-                                                       H->table, K, mark);
-            SPMV_TRY_CUDA(cudaGetLastError());
-        }
+        host_off.resize((size_t)nb + 1);
+        SPMV_TRY_CUDA(cudaMemcpyAsync(host_off.data(), *hack_off, ((size_t)nb + 1) * sizeof(long long), cudaMemcpyDeviceToHost,
+                                      stream));
         SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
         return SPMV_B200_OK;
     };
     const int rc = body();
     cudaFree(slots);
-    cudaFree(widths);
-    cudaFree(d_max);
     cudaFree(temp);
-    cudaFree(keys);
+    cudaFree(d_fits);
+    if (narrow) *narrow = fits != 0;
+    *max_width = 0;
+    for (int h = 0; rc == SPMV_B200_OK && h < nb; ++h) *max_width = std::max(*max_width, (int)((host_off[h + 1] - host_off[h]) / kHack));
     return rc;
 }
 
-namespace spmv {
-int csr_image_build(const spmv_b200_csr *A, long long max_slots, long long max_bytes, ImageValues values, cudaStream_t stream,
-                    spmv_b200_hll **out) {
-    *out = nullptr;
-    spmv_b200_hll *H = new (std::nothrow) spmv_b200_hll();
-    if (!H) return fail(SPMV_B200_ERR_NOMEM, "csr image: out of host memory");
-    const int rc = hll_convert(A, stream, true, max_slots, max_bytes, H, values);
-    if (rc != SPMV_B200_OK || (!H->JA && !H->JA16)) {
-        spmv_b200_hll_free(H);
-        return rc;
-    }
-    hll_find_segments(H);
-    const long long mean = H->num_hacks > 0 ? (H->slots / 32 + H->num_hacks - 1) / H->num_hacks : 4;
-    H->row_batch = (int)std::max<long long>(2, std::min<long long>(7, mean));
-    *out = H;
-    return SPMV_B200_OK;
-}
-
-int csr_image_value_bytes(const spmv_b200_hll *H) { return (H->AS ? 8 : 0) + (H->AC ? 1 : 0); }
-
-long long csr_image_bytes(const spmv_b200_hll *H) {
-    return H->slots * ((H->JA16 ? 2 : 4) + csr_image_value_bytes(H)) + (H->AC ? 8LL * H->num_values : 0);
-}
-
-void csr_image_keep(spmv_b200_hll *H, bool coded) {
-    if (coded) {
-        cudaFree(H->AS);
-        H->AS = nullptr;
-    } else {
-        cudaFree(H->AC);
-        cudaFree(H->table);
-        H->AC = nullptr;
-        H->table = nullptr;
-        H->num_values = 0;
-    }
-}
-
-int csr_image_default_form(const spmv_b200_hll *H) {
-    return (H->segments.count > 0 ? 64 + std::max(3, std::min(7, H->max_width)) : H->row_batch) | (H->AS ? 0 : kImageCoded);
-}
-
-template <bool ACCUM, typename I, typename S>
-static int csr_image_launch_t(const spmv_b200_hll *H, const I *JA, const S *AS, int form, int hack_begin, int hack_end,
-                              const double *x, double *y, cudaStream_t stream) {
-    const XPolicy keep = matrix_policy(JA, (size_t)H->slots * sizeof(I));
-    const unsigned int g = blocks_for(hack_end - hack_begin, 8);
-    const int K = std::max(H->num_values, 1);
-    const size_t smem = sizeof(S) == 1 ? (size_t)K * sizeof(double) : 0;  // the staged table of a coded image
-    if (form >= 64) {
-        if (H->segments.count <= 0) return fail(SPMV_B200_ERR_INVALID, "csr image: not regular enough for the offset-free form");
-        SPMV_TRY_CUDA((with_batch<5, 3, 4, 6, 7>(form - 64, [&](auto B) {
-            return launch_x(hll_rowu_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->segments, JA, AS, x, y, H->M, H->table, K);
-        })));
-    } else {
-        SPMV_TRY_CUDA((with_batch<4, 2, 3, 5, 6, 7>(form, [&](auto B) {
-            return launch_x(hll_row_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, H->hack_off, JA, AS, x, y, H->M, H->table, K);
-        })));
-    }
+int hll_fill(int M, int N, const int *row_ptr, const int *col_idx, const double *values, int num_hacks,
+             const long long *hack_off, int *JA, uint16_t *JA16, double *AS, uint8_t *AC, const double *table, int K,
+             bool masked, cudaStream_t stream) {
+    if (num_hacks == 0) return SPMV_B200_OK;
+    const unsigned int g = blocks_for((long long)num_hacks * kHack, 256);
+    if (JA16) hll_fill_kernel<<<g, 256, 0, stream>>>(M, N, num_hacks, row_ptr, col_idx, values, hack_off, JA16, AS, AC, table, K, 0);
+    else hll_fill_kernel<<<g, 256, 0, stream>>>(M, N, num_hacks, row_ptr, col_idx, values, hack_off, JA, AS, AC, table, K, masked ? kPadMark : 0);
     SPMV_TRY_CUDA(cudaGetLastError());
     return SPMV_B200_OK;
 }
 
-template <typename I>
-static int csr_image_launch_i(const spmv_b200_hll *H, const I *JA, int form, int hack_begin, int hack_end, const double *x,
-                              double *y, int accumulate, cudaStream_t stream) {
-    if (form & kImageCoded) {
-        if (!H->AC) return fail(SPMV_B200_ERR_INVALID, "csr image: the image holds no value codes");
-        form &= ~kImageCoded;
-        return accumulate ? csr_image_launch_t<true>(H, JA, H->AC, form, hack_begin, hack_end, x, y, stream)
-                          : csr_image_launch_t<false>(H, JA, H->AC, form, hack_begin, hack_end, x, y, stream);
-    }
-    if (!H->AS) return fail(SPMV_B200_ERR_INVALID, "csr image: the image holds no fp64 values");
-    return accumulate ? csr_image_launch_t<true>(H, JA, H->AS, form, hack_begin, hack_end, x, y, stream)
-                      : csr_image_launch_t<false>(H, JA, H->AS, form, hack_begin, hack_end, x, y, stream);
-}
-
-// form: as in spmv_b200_csr::image_form -- kImageCoded selects the value codes
-int csr_image_launch(const spmv_b200_hll *H, int form, int hack_begin, int hack_end, const double *x, double *y,
-                     int accumulate, cudaStream_t stream) {
+int hll_masked_launch(int hack_begin, int hack_end, int M, const long long *hack_off, const HllSegments &seg, const int *JA,
+                      const uint16_t *JA16, long long slots, const double *AS, const uint8_t *AC, const double *table, int K,
+                      int batch, bool offset_free, int accumulate, const double *x, double *y, cudaStream_t stream) {
     if (hack_end <= hack_begin) return SPMV_B200_OK;
-    if (H->JA16) return csr_image_launch_i(H, H->JA16, form, hack_begin, hack_end, x, y, accumulate, stream);
-    return csr_image_launch_i(H, H->JA, form, hack_begin, hack_end, x, y, accumulate, stream);
+    if (offset_free && seg.count <= 0) return fail(SPMV_B200_ERR_INVALID, "csr image: not regular enough for the offset-free form");
+    const unsigned int g = blocks_for(hack_end - hack_begin, 8);
+    auto launch = [&](auto accum, const auto *ja, const auto *as) {
+        constexpr bool ACCUM = decltype(accum)::value;
+        using I = std::remove_cv_t<std::remove_reference_t<decltype(*ja)>>;
+        using S = std::remove_cv_t<std::remove_reference_t<decltype(*as)>>;
+        const XPolicy keep = matrix_policy(ja, (size_t)slots * sizeof(I));
+        const size_t smem = sizeof(S) == 1 ? (size_t)K * sizeof(double) : 0;  // the staged table of a coded image
+        if (offset_free)
+            return with_batch<5, 3, 4, 6, 7>(batch, [&](auto B) {
+                return launch_x(hll_rowu_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, seg, ja, as, x, y, M, table, K);
+            });
+        return with_batch<4, 2, 3, 5, 6, 7>(batch, [&](auto B) {
+            return launch_x(hll_row_kernel<B, double, true, ACCUM, I, S>, g, 256, smem, stream, keep, hack_begin, hack_end, hack_off, ja, as, x, y, M, table, K);
+        });
+    };
+    auto values = [&](auto accum, const auto *ja) { return AC ? launch(accum, ja, AC) : launch(accum, ja, AS); };
+    auto columns = [&](auto accum) { return JA16 ? values(accum, JA16) : values(accum, JA); };
+    SPMV_TRY_CUDA(accumulate ? columns(std::true_type{}) : columns(std::false_type{}));
+    SPMV_TRY_CUDA(cudaGetLastError());
+    return SPMV_B200_OK;
 }
 }  // namespace spmv
+
+// CSR -> HLL on the device (spmv_b200_hll_from_csr): the layout, then the column and value streams
+static int hll_convert(const spmv_b200_csr *A, cudaStream_t stream, spmv_b200_hll *H) {
+    H->M = A->M;
+    H->N = A->N;
+    const int nb = H->num_hacks = (A->M + kHack - 1) / kHack;
+    SPMV_TRY(hll_layout(A->M, A->N, A->row_ptr, A->col_idx, stream, &H->hack_off, H->host_off, &H->max_width, nullptr));
+    H->slots = H->host_off[nb];
+    // reference layout keeps the last block short: its padded rows do not exist there
+    const int last_rows = nb > 0 ? A->M - (nb - 1) * kHack : 0;
+    H->ref_slots = H->slots;
+    if (nb > 0) H->ref_slots -= ((H->host_off[nb] - H->host_off[nb - 1]) / kHack) * (kHack - last_rows);
+    SPMV_TRY(hll_alloc_arena(H));
+    SPMV_TRY(hll_fill(A->M, A->N, A->row_ptr, A->col_idx, A->values, nb, H->hack_off, H->JA, nullptr, H->AS, nullptr, nullptr, 0,
+                      false, stream));
+    SPMV_TRY_CUDA(cudaStreamSynchronize(stream));
+    return SPMV_B200_OK;
+}
 
 extern "C" {
 
@@ -1068,7 +895,7 @@ int spmv_b200_hll_from_csr(const spmv_b200_csr *A, void *stream_, spmv_b200_hll 
     cudaStream_t stream = as_stream(stream_);
     spmv_b200_hll *H = new (std::nothrow) spmv_b200_hll();
     if (!H) return fail(SPMV_B200_ERR_NOMEM, "hll_from_csr: out of host memory");
-    int rc = hll_convert(A, stream, false, -1, -1, H);
+    int rc = hll_convert(A, stream, H);
     if (rc == SPMV_B200_OK) rc = stream_plan_hll(H, stream);
     if (rc != SPMV_B200_OK) {
         spmv_b200_hll_free(H);
@@ -1329,10 +1156,7 @@ void spmv_b200_hll_free(spmv_b200_hll *H) {
     cudaFree(H->tiles);
     cudaFree(H->hack_off);
     cudaFree(H->JA);
-    cudaFree(H->JA16);
     cudaFree(H->AS);
-    cudaFree(H->AC);
-    cudaFree(H->table);
     cudaFree(H->stage_x);
     cudaFree(H->stage_y);
     host_pipe_free(H->pipe);

@@ -349,7 +349,7 @@ extern "C" {
 int spmv_b200_csr_spmv_host(spmv_b200_csr *A, const double *x, double *y, int accumulate, int algo) {
     if (!A || (A->M > 0 && !y) || (A->N > 0 && A->nnz > 0 && !x)) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_host: NULL argument");
     if (algo < SPMV_B200_ALGO_AUTO || algo > SPMV_B200_ALGO_ROW_IMAGE) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_host: unknown algo %d", algo);
-    if (algo == SPMV_B200_ALGO_ROW_IMAGE && !A->image && !A->patterns) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_host: the matrix holds no image");
+    if (algo == SPMV_B200_ALGO_ROW_IMAGE && !A->image) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_host: the matrix holds no image");
     if (A->M == 0) return SPMV_B200_OK;
     if (!A->stage_x) SPMV_TRY_CUDA(cudaMalloc(&A->stage_x, std::max<size_t>(A->N, 1) * sizeof(double)));
     if (!A->stage_y) SPMV_TRY_CUDA(cudaMalloc(&A->stage_y, std::max<size_t>(A->M, 1) * sizeof(double)));
