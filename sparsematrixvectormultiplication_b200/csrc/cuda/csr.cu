@@ -1057,7 +1057,11 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
             if (ms[i] >= 0.0f && (ms[best] < 0.0f || ms[i] < ms[best])) best = i;
         if (ids[best] == 0) A->short_rows_stream = true;
         else A->row_batch = ids[best];
-        if (pick >= plain) image_keep(image, pick - plain);
+        // SPMV_B200_IMAGE_CANDIDATE=i >= 0 keeps image candidate i (image_candidates' order) instead of the fastest, and no
+        // image when i >= forms: the timing picks a form per machine and run, so tests walk every form the plan offers
+        const int forced_image = env_int("SPMV_B200_IMAGE_CANDIDATE", -1);
+        const int keep = forced_image < 0 ? pick - plain : forced_image < forms ? forced_image : -1;
+        if (keep >= 0) image_keep(image, keep);
         else image_free(image);
         A->image = image;
         // the fused iterated product (scale + |w|^2 partials in the tail): fused stream kernel (0) or fused row kernel

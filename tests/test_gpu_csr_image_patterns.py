@@ -81,13 +81,14 @@ def banded_pool(M, N, pool, seed):
     return np.array(rp, np.int32), np.array(ci, np.int32), np.array(va, np.float64)
 
 
-def make_pool(count, seed, span=40):
-    """count patterns of 1-12 sorted distinct deltas in [-span, span] and values from a small set with stored zeros."""
+def make_pool(count, seed, span=40, lengths=(1, 12)):
+    """count patterns of lengths[0]-lengths[1] sorted distinct deltas in [-span, span] and values from a small set with
+    stored zeros."""
     rng = np.random.default_rng(seed)
     choices = np.array([1.0, -1.0, 4.0, 0.0, -0.0, 0.25, 3.0e-300, -7.5])
     pool = []
     for _ in range(count):
-        n = int(rng.integers(1, 13))
+        n = int(rng.integers(lengths[0], lengths[1] + 1))
         deltas = sorted(rng.choice(np.arange(-span, span + 1), size=n, replace=False).tolist())
         pool.append((deltas, rng.choice(choices, size=n).tolist()))
     return pool
@@ -126,6 +127,16 @@ def count_matrix(count, M=2000):
     ci = np.arange(M, dtype=np.int32)
     va = 1.0 + np.arange(M) % count
     return rp, ci, va
+
+
+def wide_count_matrix(count, W, M=2000):
+    """Rows of W nonzeros at col - row = 0 .. W - 1 with `count` distinct first values: exactly `count` patterns of
+    width W, every column in [0, M + W - 1)."""
+    rp = np.arange(M + 1, dtype=np.int32) * W
+    ci = (np.arange(M, dtype=np.int32)[:, None] + np.arange(W, dtype=np.int32)[None, :]).ravel()
+    va = np.tile(np.linspace(-1.0, 0.5, W), (M, 1))
+    va[:, 0] = 1.0 + np.arange(M) % count
+    return rp, ci, va.ravel()
 
 
 def test_pattern_model_limits():
@@ -215,13 +226,19 @@ def test_patterns_on_stencils(kind, n):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("M,N", [(1000, 777), (33, 5), (31, 1), (4900, 4900), (700, 1400)])
-def test_patterns_on_irregular_rows(M, N):
-    """M > N and M < N, empty rows, rows of 1-12 nonzeros from a pool, stored +-0.0; x with +-Inf and NaN."""
+@pytest.mark.parametrize("M,N,W", [(1000, 777, None), (33, 5, None), (31, 1, None), (4900, 4900, None), (700, 1400, None)]
+                         + [(1500 + 37 * w, 1300, w) for w in range(1, 13)],
+                         ids=["1000-777", "33-5", "31-1", "4900-4900", "700-1400"] + [f"W{w}" for w in range(1, 13)])
+def test_patterns_on_irregular_rows(M, N, W):
+    """M > N and M < N, empty rows, rows of 1-12 nonzeros from a pool, stored +-0.0; x with +-Inf and NaN.  W: every
+    width of csr_pattern_kernel, on M > N with rows of 1 to W nonzeros."""
     d = dev()
-    rp, ci, va = banded_pool(M, N, make_pool(60, M), M + N)
+    pool = make_pool(60, M)
+    if W is not None:  # rows of 1 to W nonzeros, one pattern of exactly W
+        pool = make_pool(40, M, span=20, lengths=(1, W)) + [(list(range(-(W // 2), W - W // 2)), [2.0] * W)]
+    rp, ci, va = banded_pool(M, N, pool, M + N)
     pats = row_patterns(rp, ci, va)
-    assert pats is not None
+    assert pats is not None and pats[0] == (W or pats[0])
     A = d.DeviceCSR.upload(M, N, rp, ci, va)
     A.set_image(3)
     last = [ci[rp[r + 1] - 1] for r in range(M) if rp[r + 1] > rp[r]]
@@ -240,19 +257,24 @@ def test_equal_deltas_or_equal_values():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("count", [256, 257])
-def test_pattern_count_boundary(count):
-    """256 patterns build; 257 fail with SpmvError and leave the held image (here the fp64 column-major one) as it was."""
+@pytest.mark.parametrize("count,W", [(256, 1), (257, 1), (170, 12), (171, 12), (186, 11), (187, 11)],
+                         ids=["256", "257", "W12-170", "W12-171", "W11-186", "W11-187"])
+def test_pattern_count_boundary(count, W):
+    """256 patterns build; 257 fail with SpmvError and leave the held image (here the fp64 column-major one) as it was.
+    The dictionary's bytes bound it too: 12 W P <= 24576, so W = 12 holds 170 patterns (24480 bytes, the largest
+    dictionary) and not 171, W = 11 holds 186 and not 187."""
     import torch
     from sparsematrixvectormultiplication_b200 import _native as NN
     d = dev()
-    rp, ci, va = count_matrix(count)
-    M = len(rp) - 1
-    A = d.DeviceCSR.upload(M, M, rp, ci, va)
-    x = special_x(M, ci[::37], seed=count)
-    if count <= MAX_PATTERNS:
+    rp, ci, va = count_matrix(count) if W == 1 else wide_count_matrix(count, W)
+    M, N = len(rp) - 1, int(ci.max()) + 1
+    builds = count <= MAX_PATTERNS and 12 * W * count <= DICT_BYTES
+    assert (row_patterns(rp, ci, va) is not None) == builds
+    A = d.DeviceCSR.upload(M, N, rp, ci, va)
+    x = special_x(N, ci[::37], seed=count)
+    if builds:
         A.set_image(3)
-        check_pattern_form(A, M, M, 1, count, x)
+        check_pattern_form(A, M, N, W, count, x)
     else:
         A.set_image(1)
         before = A.info()

@@ -64,9 +64,10 @@ def coded_product(hacks, table, M, x, y0=None):
 
 
 def special_values():
-    """+-0.0, +-Inf, NaNs of two payloads, subnormals and a few normal numbers."""
+    """+-0.0, +-Inf, NaNs of two payloads, the all-ones pattern (a NaN, and the empty mark of the library's distinct-value
+    set), subnormals and a few normal numbers."""
     pats = np.array([0x0000000000000000, 0x8000000000000000, 0x7FF0000000000000, 0xFFF0000000000000,
-                     0x7FF8000000000000, 0x7FF8000000000123, 0x0000000000000001, 0x800FFFFFFFFFFFFF],
+                     0x7FF8000000000000, 0x7FF8000000000123, 0xFFFFFFFFFFFFFFFF, 0x0000000000000001, 0x800FFFFFFFFFFFFF],
                     np.uint64).view(np.float64)
     return np.concatenate([pats, [1.0, -2.5, 4.0, -1.0]])
 
@@ -220,22 +221,29 @@ def test_coded_image_on_irregular_rows(M, N):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("count", [256, 257])
-def test_value_count_boundary(count):
+@pytest.mark.parametrize("count,all_ones", [(256, False), (257, False), (256, True), (257, True)],
+                         ids=["256", "257", "256-all-ones", "257-all-ones"])
+def test_value_count_boundary(count, all_ones):
     """Exactly 256 patterns gets the coded image; 257 raises and leaves the handle as it was (no image, then the fp64
-    image)."""
+    image).  With the all-ones pattern among them -- counted on the host, not in the device's set -- 256 patterns build
+    with it as code 255, and 257 fail where the device counts 256."""
     import torch
     d = dev()
     from sparsematrixvectormultiplication_b200 import _native as NN
     pool = np.random.default_rng(count).standard_normal(count)
+    if all_ones:
+        pool[-1] = np.array([0xFFFFFFFFFFFFFFFF], np.uint64).view(np.float64)[0]
     M = N = 2000
     rp, ci, va = irregular(M, N, pool, count)
     assert len(np.unique(va.view(np.uint64))) == count
     A = d.DeviceCSR.upload(M, N, rp, ci, va)
     x = special_x(N, [], seed=count)
+    if all_ones:  # no NaN of another payload in x to meet the all-ones one in a sum
+        x = torch.nan_to_num(x, nan=float("-inf"), posinf=float("inf"), neginf=float("-inf"))
     if count <= MAX_VALUES:
         A.set_image(2)
         check_coded(A, rp, ci, va, N)
+        assert value_table(va)[-1] == 0xFFFFFFFFFFFFFFFF or not all_ones
         check_products(A, x, M)
     else:
         before = A.info()
