@@ -178,7 +178,7 @@ int spmv_b200_csr_spmv_host(spmv_b200_csr *A, const double *x, double *y, int ac
 typedef struct {
     int count;
     double *dst[SPMV_B200_MAX_PEERS]; /* peer pointer that corresponds to local row 0 of y            */
-    int lo[SPMV_B200_MAX_PEERS];      /* local row range [lo,hi) the peer needs                       */
+    int lo[SPMV_B200_MAX_PEERS];      /* local row range [lo,hi) the peer needs, 0 <= lo <= hi <= M   */
     int hi[SPMV_B200_MAX_PEERS];
 } spmv_b200_peers_t;
 int spmv_b200_csr_partials_count(const spmv_b200_csr *A);

@@ -1404,14 +1404,21 @@ static int launch_fused_flat(const spmv_b200_csr *A, const double *x, double *y,
     return SPMV_B200_OK;
 }
 
+int check_peers(const spmv_b200_peers_t *peers, int M, const char *what) {
+    if (!peers) return SPMV_B200_OK;
+    if (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS) return fail(SPMV_B200_ERR_INVALID, "%s: bad peer count %d", what, peers->count);
+    for (int p = 0; p < peers->count; ++p)
+        if (peers->lo[p] < 0 || peers->hi[p] > M || peers->lo[p] > peers->hi[p])
+            return fail(SPMV_B200_ERR_INVALID, "%s: peer %d: bad row range [%d,%d) of %d rows", what, p, peers->lo[p], peers->hi[p], M);
+    return SPMV_B200_OK;
+}
+
 int boundary_first_order(const spmv_b200_peers_t &peers, int M, ChunkOrder &order) {
     order = ChunkOrder();
+    SPMV_TRY(check_peers(&peers, M, "fused product"));
     std::vector<std::pair<int, int>> iv;
-    for (int p = 0; p < peers.count; ++p) {
-        if (peers.lo[p] < 0 || peers.hi[p] > M || peers.lo[p] > peers.hi[p])
-            return fail(SPMV_B200_ERR_INVALID, "fused product: peer %d: bad row range [%d,%d) of %d rows", p, peers.lo[p], peers.hi[p], M);
+    for (int p = 0; p < peers.count; ++p)
         if (peers.hi[p] > peers.lo[p]) iv.emplace_back(peers.lo[p] >> 8, (peers.hi[p] + 255) >> 8);
-    }
     std::sort(iv.begin(), iv.end());
     for (const auto &r : iv) {
         if (order.count > 0 && r.first <= order.hi[order.count - 1]) {
@@ -1679,8 +1686,7 @@ int spmv_b200_csr_spmv_fused(const spmv_b200_csr *A, const double *d_x, double *
     if (!A || !d_y || (A->N > 0 && !d_x)) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused: NULL argument");
     if (A->num_long > 0)
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused: %d rows exceed the long-row threshold; use csr_spmv", A->num_long);
-    if (peers && (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS))
-        return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused: bad peer count %d", peers->count);
+    SPMV_TRY(check_peers(peers, A->M, "csr_spmv_fused"));
     Epilogue ep;
     ep.prev_sumsq = d_prev_sumsq;
     ep.partials = d_partials;
@@ -1701,8 +1707,7 @@ int spmv_b200_csr_spmv_fused_flat(const spmv_b200_csr *A, const double *d_x, dou
     if (!A || !d_y || (A->N > 0 && !d_x)) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_flat: NULL argument");
     if (A->max_row > kRowKernelMaxLen)
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_flat: rows of up to %d nonzeros only (longest row: %d)", kRowKernelMaxLen, A->max_row);
-    if (peers && (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS))
-        return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_flat: bad peer count %d", peers->count);
+    SPMV_TRY(check_peers(peers, A->M, "csr_spmv_fused_flat"));
     if (A->M == 0) return SPMV_B200_OK;
     Epilogue ep;
     ep.inv_norm = d_inv_norm;
@@ -1718,8 +1723,7 @@ int spmv_b200_csr_spmv_fused_mail(const spmv_b200_csr *A, const double *d_x, dou
     if (A->num_long > 0)
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_mail: %d rows exceed the long-row threshold; use csr_spmv", A->num_long);
     if (A->M == 0 || A->num_tiles == 0) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_mail: a rank without rows cannot take part in the exchange");
-    if (peers && (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS))
-        return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_mail: bad peer count %d", peers->count);
+    SPMV_TRY(check_peers(peers, A->M, "csr_spmv_fused_mail"));
     if (mail->world < 1 || mail->world > SPMV_B200_MAX_RANKS || mail->rank < 0 || mail->rank >= mail->world || !mail->counter ||
         !mail->status)
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_mail: bad mailbox description (world %d, rank %d)", mail->world, mail->rank);
@@ -1744,10 +1748,13 @@ int spmv_b200_csr_spmv_fused_async(const spmv_b200_csr *A, const double *d_x, do
         return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_async: bad exchange description (world %d, rank %d)", as->world, as->rank);
     for (int r = 0; r < as->world; ++r)
         if (!as->box[r]) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_async: mailbox of rank %d is NULL", r);
+    for (int i = 0; i < as->num_recv; ++i)  // a halo tag is read at box[rank] + 8 world + recv_from[i]
+        if (as->recv_from[i] < 0 || as->recv_from[i] >= as->world)
+            return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_async: sender %d: bad rank %d", i, as->recv_from[i]);
+    SPMV_TRY(check_peers(peers, A->M, "csr_spmv_fused_async"));
     spmv_b200_peers_t ps;
     ps.count = 0;
     if (peers) ps = *peers;
-    if (ps.count < 0 || ps.count > SPMV_B200_MAX_PEERS) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_async: bad peer count %d", ps.count);
     ChunkOrder order;
     for (int p = 0; p < ps.count; ++p)
         if (as->send_to[p] < 0 || as->send_to[p] >= as->world) return fail(SPMV_B200_ERR_INVALID, "csr_spmv_fused_async: peer %d: bad rank", p);

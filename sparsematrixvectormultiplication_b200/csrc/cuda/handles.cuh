@@ -54,7 +54,10 @@ struct Epilogue {                 // optional fused tail of the CSR stream / row
     ChunkOrder order;             // row kernels only: boundary chunks first (filled by boundary_first_order)
 };
 
-// the union of the peers' row ranges in 256-row chunks, ascending and disjoint (host side)
+// the peers of a fused launch on M rows: a count in [0, SPMV_B200_MAX_PEERS] and row ranges 0 <= lo <= hi <= M (a range
+// that reaches past the matrix would silently leave rows out of a neighbour's x); NULL = none (host side)
+int check_peers(const spmv_b200_peers_t *peers, int M, const char *what);
+// the union of the peers' row ranges in 256-row chunks, ascending and disjoint (host side; peers passed check_peers)
 int boundary_first_order(const spmv_b200_peers_t &peers, int M, ChunkOrder &order);
 
 // entries of the partials buffer that this launch does not write (the buffer is sized for the largest fused grid)

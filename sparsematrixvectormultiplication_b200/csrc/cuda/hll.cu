@@ -1023,8 +1023,7 @@ int spmv_b200_hll_partials_count(const spmv_b200_hll *H) { return H ? hll_fused_
 int spmv_b200_hll_spmv_fused(const spmv_b200_hll *H, const double *d_x, double *d_y, const double *d_prev_sumsq,
                              double *d_partials, const spmv_b200_peers_t *peers, void *stream) {
     if (!H || !d_y || (H->N > 0 && !d_x)) return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused: NULL argument");
-    if (peers && (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS))
-        return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused: bad peer count %d", peers->count);
+    SPMV_TRY(check_peers(peers, H->M, "hll_spmv_fused"));
     if (H->M == 0) return SPMV_B200_OK;
     Epilogue ep;
     ep.prev_sumsq = d_prev_sumsq;
@@ -1043,8 +1042,7 @@ int spmv_b200_hll_flat_partials_count(const spmv_b200_hll *H) {
 int spmv_b200_hll_spmv_fused_flat(const spmv_b200_hll *H, const double *d_x, double *d_y, const double *d_inv_norm,
                                   double *d_partials, const spmv_b200_peers_t *peers, void *stream) {
     if (!H || !d_y || (H->N > 0 && !d_x)) return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused_flat: NULL argument");
-    if (peers && (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS))
-        return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused_flat: bad peer count %d", peers->count);
+    SPMV_TRY(check_peers(peers, H->M, "hll_spmv_fused_flat"));
     if (H->M == 0) return SPMV_B200_OK;
     Epilogue ep;
     ep.inv_norm = d_inv_norm;
@@ -1058,8 +1056,7 @@ int spmv_b200_hll_spmv_fused_mail(const spmv_b200_hll *H, const double *d_x, dou
                                   const spmv_b200_peers_t *peers, const spmv_b200_mail_t *mail, void *stream) {
     if (!H || !d_y || !d_partials || !mail || (H->N > 0 && !d_x)) return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused_mail: NULL argument");
     if (H->M == 0) return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused_mail: a rank without rows cannot take part in the exchange");
-    if (peers && (peers->count < 0 || peers->count > SPMV_B200_MAX_PEERS))
-        return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused_mail: bad peer count %d", peers->count);
+    SPMV_TRY(check_peers(peers, H->M, "hll_spmv_fused_mail"));
     if (mail->world < 1 || mail->world > SPMV_B200_MAX_RANKS || mail->rank < 0 || mail->rank >= mail->world || !mail->counter ||
         !mail->status)
         return fail(SPMV_B200_ERR_INVALID, "hll_spmv_fused_mail: bad mailbox description (world %d, rank %d)", mail->world, mail->rank);

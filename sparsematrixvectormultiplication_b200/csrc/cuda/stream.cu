@@ -186,6 +186,8 @@ csr_stream_kernel(const int2 *__restrict__ tiles, int num_tiles, const int *__re
         fence_mbar_init();
     }
     __syncthreads();
+    // before the producer warp leaves: zero_partials_tail strides over every thread of the CTA
+    if constexpr (kFused) zero_partials_tail(ep);
 
     if (warp == kConsumerWarps) {
         // ---------------- producer: one elected lane streams the CTA's tiles into the ring ----------------
@@ -237,7 +239,6 @@ csr_stream_kernel(const int2 *__restrict__ tiles, int num_tiles, const int *__re
         }
     }
     const double inv_norm = 1.0 / prev_norm;  // one division per thread, one multiplication per row (1 ulp from a division)
-    if constexpr (kFused) zero_partials_tail(ep);
     double sq = 0.0;  // sum of the squares of the rows this lane produced
     // y[row] = v; the fused instantiation scales it first, accumulates v^2 and mirrors boundary rows into the peers
     auto emit = [&](int row, double v) {
