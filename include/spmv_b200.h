@@ -90,6 +90,10 @@ typedef struct {
                             256 + W (csr_pattern_kernel<W>, W the longest row), image_bytes and image_device_bytes are
                             M (one byte per row) plus the dictionary's 12 * W + 4 bytes per pattern, and
                             image_index_bytes and image_value_bytes are 0 */
+    int image_windows;   /* the pattern form (spmv_b200_version() >= 107): the windows of x a tile of 1024 rows stages
+                            in shared memory -- one per cluster of the patterns' col - row, at most min(W, 3) of them --
+                            or 0 when its kernel gathers x from global memory (scattered col - row); 0 for the other
+                            forms.  The bytes of the image do not change with it */
 } spmv_b200_csr_info_t;
 
 typedef struct {

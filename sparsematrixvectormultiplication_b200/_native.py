@@ -63,7 +63,8 @@ class CsrInfo(C.Structure):  # include/spmv_b200.h spmv_b200_csr_info_t
                 ("max_row_nnz", C.c_int), ("auto_algo", C.c_int), ("row_batch", C.c_int), ("fused_batch", C.c_int),
                 ("flat_batch", C.c_int), ("flat_chunks", C.c_int), ("image_bytes", C.c_longlong), ("image_form", C.c_int),
                 ("image_index_bytes", C.c_int), ("image_device_bytes", C.c_longlong),
-                ("image_value_bytes", C.c_int), ("image_patterns", C.c_int)]
+                ("image_value_bytes", C.c_int), ("image_patterns", C.c_int),
+                ("image_windows", C.c_int)]
 
 
 class HllInfo(C.Structure):  # include/spmv_b200.h spmv_b200_hll_info_t

@@ -25,8 +25,26 @@ namespace spmv {
 constexpr int kMaxDistinct = 256;                // value patterns of the coded form, row patterns of the pattern form
 constexpr int kPatternDictMaxBytes = 24 * 1024;  // P * W * 12: 8 CTAs of 256 threads stay resident per SM
 
+// The tiled pattern kernel (csr_pattern_tile_kernel): a CTA of kTileThreads threads multiplies kTileRows rows from windows
+// of x staged in shared memory, one window per cluster of the patterns' deltas
+constexpr int kTileRows = 1024;     // 4 rows per thread, strided by kTileThreads: consecutive lanes read consecutive words
+constexpr int kTileThreads = 256;
+constexpr int kWindowGap = 32;      // sorted deltas less than this apart share a window
+constexpr int kWindowMaxSpan = 256; // hi - lo of one window: a window stages kTileRows + span + 2 doubles at most
+// Slot records and windows: with the kTileRows ids, 8 CTAs (+ 1 KB reserved each) fit an SM's 228 KB, as the kernel needs
+// all 2048 threads of an SM to hide its load phase.  Measured on lap3d 384^3 (B200): 5 windows (44 KB, 5 CTAs per SM)
+// took 498 us against 422 us for csr_pattern_kernel, while lap2d's 3 windows (25 KB, 8 CTAs) gained.
+constexpr int kWindowSmemMax = 26 * 1024;
+constexpr int kMaxWindows = 3;      // and at most W; a fourth window of a 1024-row tile exceeds kWindowSmemMax
+
+struct PatternWindows {
+    int count = 0;                           // windows a tile stages; 0: csr_pattern_kernel gathers x from global memory
+    int lo[kMaxWindows] = {}, hi[kMaxWindows] = {};  // the deltas each window covers
+    int base[kMaxWindows + 1] = {};          // its first double in shared memory, after the slot records; base[count]: end
+};
+
 struct ImageForm {
-    bool patterns = false;     // csr_pattern_kernel<W>; otherwise the column-major form, run by
+    bool patterns = false;     // csr_pattern_tile_kernel<W> or csr_pattern_kernel<W>; otherwise the column-major form, run by
     bool offset_free = false;  // hll_rowu_kernel<batch> (regular layouts) or hll_row_kernel<batch>
     int batch = 0;
     bool coded = false;        // on the value codes, else on the fp64 values
@@ -51,6 +69,7 @@ struct CsrPatterns {
     uint8_t *id = nullptr;  // device [M]: the pattern of each row
     int *dict = nullptr;    // device: value[W][P] (fp64), delta[W][P] (int32), len[P] (int32); a slot at or past a
                             // pattern's length holds delta 0 and value 0.0
+    PatternWindows windows; // planned from the dictionary at build time
 };
 static long long dict_bytes(const CsrPatterns &P) { return 12LL * P.width * P.count + 4LL * P.count; }
 
@@ -96,12 +115,149 @@ csr_pattern_kernel(int row_begin, int row_end, const uint8_t *__restrict__ id, c
     y[row] = acc;
 }
 
+// ---- the tiled product of the pattern form ---------------------------------------------------------------------------
+// csr_pattern_kernel waits on three dependent round trips per row (dictionary, id, gathers) with one row per thread in
+// flight.  When the patterns' deltas fall into a few narrow clusters (PatternWindows: lap2d {-n}, {-1..1}, {+n}), a CTA
+// instead issues every load of kTileRows rows at once -- each cluster's window of x as 16-byte cp.async, the ids and the
+// dictionary -- waits once, and computes the rows from shared memory (under ACCUM after a load of y).  The adds are
+// csr_pattern_kernel's (same values, same x words, same order), so y keeps its bits.
+struct alignas(16) PatternSlot {  // one slot of one pattern, read with one 16-byte shared-memory load
+    double value;
+    int offset;       // x[row + delta] is tile[offset + row - r0]
+    int real;         // the slot lies below the pattern's length
+};
+
+__device__ __forceinline__ void cp_async16(double *dst, const double *src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
+}
+
+// bytes 0 zero-fills the word without reading src
+__device__ __forceinline__ void cp_async8(double *dst, const double *src, int bytes) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src), "r"(bytes)
+                 : "memory");
+}
+
+// Window c of the tile at r0 starts at x[r0 + lo[c] - a], a = 0 or 1 so that its address is 16-byte aligned whatever the
+// alignment of x (a caller may pass x + 1); 64-bit, as r0 + lo reaches past 2^31 on lap3d 512^3.  Words outside [0, N)
+// are zero-filled: only padding slots and rows past row_end could point there, and neither adds them.
+__device__ __forceinline__ long long window_start(const double *x, long long r0, int lo) {
+    const long long g = r0 + lo;
+    return g - (long long)((((unsigned long long)x >> 3) + (unsigned long long)g) & 1);
+}
+
+template <int W, bool ACCUM>
+__global__ void __launch_bounds__(kTileThreads, 8)
+csr_pattern_tile_kernel(int row_begin, int row_end, const uint8_t *__restrict__ id, const int *__restrict__ dict, int P,
+                        const PatternWindows win, const double *__restrict__ x, double *__restrict__ y, int N) {
+    extern __shared__ __align__(16) double tile[];
+    PatternSlot *slot = reinterpret_cast<PatternSlot *>(tile);  // [W][P], then the windows from win.base[0]
+    __shared__ uint8_t ids[kTileRows];
+    const int t = threadIdx.x;
+    const long long r0 = row_begin + (long long)blockIdx.x * kTileRows;
+#pragma unroll
+    for (int c = 0; c < kMaxWindows; ++c) {
+        if (c >= win.count) break;
+        const long long start = window_start(x, r0, win.lo[c]);
+        double *dst = tile + win.base[c];
+        const int vecs = (win.base[c + 1] - win.base[c]) / 2;
+        for (int v = t; v < vecs; v += kTileThreads) {
+            const long long e = start + 2 * v;
+            if (e >= 0 && e + 2 <= N) {
+                cp_async16(dst + 2 * v, x + e);
+            } else {
+                const bool in0 = e >= 0 && e < N, in1 = e + 1 >= 0 && e + 1 < N;
+                cp_async8(dst + 2 * v, in0 ? x + e : x, in0 ? 8 : 0);
+                cp_async8(dst + 2 * v + 1, in1 ? x + e + 1 : x, in1 ? 8 : 0);
+            }
+        }
+    }
+    // the ids go through shared memory: held in registers, ptxas sank their loads below the barrier
+#pragma unroll
+    for (int k = 0; k < kTileRows / kTileThreads; ++k) {
+        const long long row = r0 + t + k * kTileThreads;
+        ids[t + k * kTileThreads] = (uint8_t)(row < row_end ? ldg_stream_u8(id + row) : 0);
+    }
+    const double *value = reinterpret_cast<const double *>(dict);
+    const int *delta = dict + 2 * W * P, *len = delta + W * P;
+    for (int i = t; i < W * P; i += kTileThreads) {
+        const int s = i / P, d = __ldg(delta + i);
+        int offset = win.base[0];  // a padding slot's delta 0 may lie in no window: any word of the tile will do
+#pragma unroll
+        for (int c = 0; c < kMaxWindows; ++c)
+            if (c < win.count && d >= win.lo[c] && d <= win.hi[c])
+                offset = win.base[c] + (int)(r0 + d - window_start(x, r0, win.lo[c]));
+        slot[i] = PatternSlot{__ldg(value + i), offset, s < __ldg(len + (i - s * P))};
+    }
+    asm volatile("cp.async.wait_all;" ::: "memory");
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < kTileRows / kTileThreads; ++k) {
+        const int i = t + k * kTileThreads;
+        if (r0 + i >= row_end) break;
+        double acc = ACCUM ? y[r0 + i] : 0.0;  // not held across the barrier: 4 rows of it spilled at 32 registers
+        int4 sl[W];  // a PatternSlot as one LDS.128: value in x (low) and y (high), offset in z, real in w
+        double xv[W];
+#pragma unroll
+        for (int s = 0; s < W; ++s) sl[s] = reinterpret_cast<const int4 *>(slot)[s * P + ids[i]];
+#pragma unroll
+        for (int s = 0; s < W; ++s) xv[s] = tile[sl[s].z + i];
+#pragma unroll
+        for (int s = 0; s < W; ++s)
+            if (sl[s].w) acc = __dadd_rn(acc, __dmul_rn(__hiloint2double(sl[s].y, sl[s].x), xv[s]));
+        y[r0 + i] = acc;
+    }
+}
+
+// The windows of the tiled kernel, planned from the host copy of the dictionary: the distinct deltas of the real slots,
+// sorted, clustered where neighbours lie less than kWindowGap apart.  count stays 0 (csr_pattern_kernel runs) unless there
+// are at most min(W, kMaxWindows) clusters, none spans more than kWindowMaxSpan, and records and windows fit
+// kWindowSmemMax.
+static PatternWindows plan_windows(int W, int P, const int *delta, const int *len) {
+    std::vector<int> d;
+    for (int p = 0; p < P; ++p)
+        for (int s = 0; s < len[p]; ++s) d.push_back(delta[s * P + p]);
+    std::sort(d.begin(), d.end());
+    d.erase(std::unique(d.begin(), d.end()), d.end());
+    PatternWindows w;
+    int n = 0;
+    for (size_t k = 0; k < d.size(); ++k) {
+        if (k > 0 && (long long)d[k] - d[k - 1] < kWindowGap) {
+            w.hi[n - 1] = d[k];
+            continue;
+        }
+        if (n == std::min(W, kMaxWindows)) return PatternWindows();
+        w.lo[n] = w.hi[n] = d[k];
+        ++n;
+    }
+    long long end = 2LL * W * P;  // the slot records: 16 bytes each
+    for (int c = 0; c < n; ++c) {
+        const long long span = (long long)w.hi[c] - w.lo[c];
+        if (span > kWindowMaxSpan) return PatternWindows();
+        w.base[c] = (int)end;
+        end += (kTileRows + span + 3) & ~1LL;  // kTileRows + span + 1 words from a 16-byte boundary, whole vectors
+    }
+    if (n == 0 || 8 * end > kWindowSmemMax) return PatternWindows();
+    w.base[n] = (int)end;
+    w.count = n;
+    return w;
+}
+
 static int launch_patterns(const CsrPatterns &P, int row_begin, int row_end, int N, const double *x, double *y, int accumulate,
                            cudaStream_t stream) {
     if (row_end <= row_begin) return SPMV_B200_OK;
-    const unsigned int g = blocks_for(row_end - row_begin, 256);
-    const size_t smem = (size_t)dict_bytes(P);
+    const PatternWindows &win = P.windows;
     SPMV_TRY_CUDA((with_batch<12, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11>(P.width, [&](auto W) {
+        if (win.count > 0) {
+            const unsigned int g = blocks_for(row_end - row_begin, kTileRows);
+            const size_t smem = 8 * (size_t)win.base[win.count];
+            if (accumulate)
+                csr_pattern_tile_kernel<W, true><<<g, kTileThreads, smem, stream>>>(row_begin, row_end, P.id, P.dict, P.count, win, x, y, N);
+            else
+                csr_pattern_tile_kernel<W, false><<<g, kTileThreads, smem, stream>>>(row_begin, row_end, P.id, P.dict, P.count, win, x, y, N);
+            return cudaGetLastError();
+        }
+        const unsigned int g = blocks_for(row_end - row_begin, 256);
+        const size_t smem = (size_t)dict_bytes(P);
         if (accumulate) csr_pattern_kernel<W, true><<<g, 256, smem, stream>>>(row_begin, row_end, P.id, P.dict, P.count, x, y, N);
         else csr_pattern_kernel<W, false><<<g, 256, smem, stream>>>(row_begin, row_end, P.id, P.dict, P.count, x, y, N);
         return cudaGetLastError();
@@ -316,6 +472,7 @@ static int build_patterns(const spmv_b200_csr *A, cudaStream_t stream, CsrPatter
                 std::memcpy(value + s * n + p, c + 1 + W + s, sizeof(double));
             }
         }
+        P.windows = plan_windows(W, n, delta, len);
         SPMV_TRY_CUDA(cudaMalloc(&P.dict, bytes));
         SPMV_TRY_CUDA(cudaMalloc(&P.id, (size_t)M));
         SPMV_TRY_CUDA(cudaMalloc(&slot_id_d, kSetSlots));
@@ -523,12 +680,13 @@ int image_build(spmv_b200_csr *A, int mode, cudaStream_t stream) {
 
 void image_info(const CsrImage *img, spmv_b200_csr_info_t *info) {
     info->image_bytes = info->image_device_bytes = 0;
-    info->image_form = info->image_index_bytes = info->image_value_bytes = info->image_patterns = 0;
+    info->image_form = info->image_index_bytes = info->image_value_bytes = info->image_patterns = info->image_windows = 0;
     if (!img) return;
     if (img->form.patterns) {  // one byte per row plus the dictionary
-        info->image_form = 256 + img->patterns.width;  // csr_pattern_kernel<W>
+        info->image_form = 256 + img->patterns.width;  // csr_pattern_kernel<W> or csr_pattern_tile_kernel<W>
         info->image_bytes = info->image_device_bytes = img->M + dict_bytes(img->patterns);
         info->image_patterns = img->patterns.count;
+        info->image_windows = img->patterns.windows.count;
         return;
     }
     const ColumnImage &C = img->cols;

@@ -4,7 +4,9 @@ narrow 2-byte `u16` column field, fp64 values or 1-byte `u8` value codes): regis
 spill bytes (csrc/build/*.ptxas.log) and how many of a step's loads ptxas issues ahead of the first multiply (cuobjdump
 -sass).  A form whose loads are split by a DMUL stalls on its first gather before the rest is requested.  Then the
 same for csr_pattern_kernel<W, ACCUM> (the pattern form of the private image): its W gathers (64-bit LDGs) against the
-first DMUL.  No GPU needed.
+first DMUL.  And for csr_pattern_tile_kernel<W, ACCUM> (its tiled kernel): the global loads (LDG and the LDGSTS of
+cp.async) ptxas places ahead of the tile's one BAR.SYNC, which should be all of them, and the shared-memory loads of
+the rows after it.  No GPU needed.
 
     python tools/rowm_survey.py            # every rowm instantiation and, for comparison, the one-row kernels
 """
@@ -36,9 +38,18 @@ def ptxas_info():
 def main():
     info = ptxas_info()
     sass = subprocess.run(["cuobjdump", "-sass", str(PKG / "libspmv_b200.so")], capture_output=True, text=True).stdout
-    rows, patterns = [], []
+    rows, patterns, tiles = [], [], []
     for body in re.split(r"Function : ", sass)[1:]:
         name = body.split()[0]
+        t = re.search(r"csr_pattern_tile_kernelILi(\d+)ELb([01])E", name)
+        if t:
+            ops = re.findall(r"(?<!@!PT )\b(LDGSTS|LDG|BAR\.SYNC|LDS)\b", body)  # @!PT LDS: never-issued padding
+            bar = ops.index("BAR.SYNC") if "BAR.SYNC" in ops else len(ops)
+            loads = sum(op in ("LDG", "LDGSTS") for op in ops)
+            rec = info.get(name, {})
+            tiles.append((int(t.group(1)), int(t.group(2)), rec.get("regs"), rec.get("spill"),
+                          sum(op in ("LDG", "LDGSTS") for op in ops[:bar]), loads, ops.count("LDS")))
+            continue
         p = re.search(r"csr_pattern_kernelILi(\d+)ELb([01])E", name)
         if p:
             ops = re.findall(r"\b(LDG\.E\.64|DMUL)\b", body)
@@ -75,6 +86,9 @@ def main():
     print("\ncsr_pattern_kernel: W accum regs spill_bytes gathers_ahead_of_first_DMUL/gathers")
     for w, accum, regs, spill, ahead, total in sorted(patterns):
         print(f"csr_pattern_kernel {w} {accum} {regs} {spill} {ahead}/{total}")
+    print("\ncsr_pattern_tile_kernel: W accum regs spill_bytes global_loads_ahead_of_BAR.SYNC/global_loads shared_loads")
+    for w, accum, regs, spill, ahead, total, lds in sorted(tiles):
+        print(f"csr_pattern_tile_kernel {w} {accum} {regs} {spill} {ahead}/{total} {lds}")
 
 
 if __name__ == "__main__":
