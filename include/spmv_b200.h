@@ -382,6 +382,25 @@ int spmv_b200_csr_spmm(const spmv_b200_csr *A, int k, const double *d_X, long lo
                        int accumulate, void *stream);
 int spmv_b200_hll_spmm(const spmv_b200_hll *H, int k, const double *d_X, long long ldx, double *d_Y, long long ldy,
                        void *stream);
+/* Host-buffer twins (spmv_b200_version() >= 108): host X -> device, Y = A X (or Y += A X), device -> host Y; one
+ * synchronous call, with the conventions of spmv_b200_csr_spmm / spmv_b200_hll_spmm above (row-major, ldx >= k and
+ * ldy >= k, 64-bit offsets, only rows < M and columns < k of Y written -- the elements between k and ldy are never
+ * touched, not even by a zero-copy store -- no overlap of X and Y, k = 0 and M = 0 no-ops, nnz = 0 gives zero or leaves
+ * Y with accumulate, bad k, ld or a NULL pointer SPMV_B200_ERR_INVALID before anything is launched, accumulate on CSR
+ * only).  Every column of Y has the bits spmv_b200_{csr,hll}_spmm gives on the same handle for the same X, whatever k,
+ * ldx, ldy, the window count or column-block width, pinned or pageable buffers, zero-copy or staged Y, long rows or not.
+ * As spmv_b200_csr_spmv_host does for one vector, the call cuts the rows into up to 16 windows (rows for CSR, hacks for
+ * HLL) and overlaps the upload of X in pieces, the products of the windows and the download of Y on three streams
+ * (hostpath.cu); the long rows of a CSR plan run after the last piece.  Y is stored by the kernels straight into a
+ * pinned or cudaHostRegister'ed buffer when ldy > k or a row of Y holds at most 16 bytes (measured, DESIGN.md section
+ * 3, "Host buffers"); it is staged and downloaded otherwise, and always with accumulate.  SPMV_B200_HOST_ZEROCOPY=0 forces staging.  Pinned buffers give the overlap; pageable ones work but
+ * serialise.
+ * Device memory: the handle keeps a staging buffer for N x kc elements of X (plus M x kc of Y when Y is staged), kc = k
+ * when that fits half of the free device memory, else column blocks of the largest kc that does; it is reused and grown
+ * by later calls and freed with the handle (spmv_b200_csr_free / spmv_b200_hll_free), as are the window plan, streams
+ * and events of these calls, made by the first one. */
+int spmv_b200_csr_spmm_host(spmv_b200_csr *A, int k, const double *X, long long ldx, double *Y, long long ldy, int accumulate);
+int spmv_b200_hll_spmm_host(spmv_b200_hll *H, int k, const double *X, long long ldx, double *Y, long long ldy);
 
 /* ---- fp32 storage with fp64 arithmetic (BASELINE.json: y within 1e-5 relative of the serial fp64 product).  The value
  * stream, x and y are float (algorithmic bytes 8 nnz + 4 (M+1) + 4 M + 4 N instead of 12 nnz + ...); every product is
@@ -411,6 +430,10 @@ int spmv_b200_csr_spmm_f32(const spmv_b200_csr *A, int k, const float *d_X, long
                            int accumulate, void *stream);
 int spmv_b200_hll_spmm_f32(const spmv_b200_hll *H, int k, const float *d_X, long long ldx, float *d_Y, long long ldy,
                            void *stream);
+/* Host-buffer twins of the two above (spmv_b200_version() >= 108), as spmv_b200_csr_spmm_host / _hll_spmm_host: the
+ * bits of spmv_b200_{csr,hll}_spmm_f32 on the same handle.  They call spmv_b200_{csr,hll}_enable_f32 themselves. */
+int spmv_b200_csr_spmm_host_f32(spmv_b200_csr *A, int k, const float *X, long long ldx, float *Y, long long ldy, int accumulate);
+int spmv_b200_hll_spmm_host_f32(spmv_b200_hll *H, int k, const float *X, long long ldx, float *Y, long long ldy);
 /* Which form of the row kernel enable_f32 timed fastest for this matrix: 1..8 = csr_row_kernel / hll_row_kernel with that
  * many loads in flight per row; >= 16 = form (id - 16) of csr_rowm_kernel / hll_rowm_kernel (index-only predicates, so
  * that every load of a step is issued ahead of the first multiply; rows per thread, loads in flight per row and CTAs

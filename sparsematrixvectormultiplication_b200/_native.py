@@ -175,6 +175,10 @@ SIGNATURES = {
     "spmv_b200_hll_spmm": (_I, [_V, _I, _V, _LL, _V, _LL, _V]),
     "spmv_b200_csr_spmm_f32": (_I, [_V, _I, _V, _LL, _V, _LL, _I, _V]),
     "spmv_b200_hll_spmm_f32": (_I, [_V, _I, _V, _LL, _V, _LL, _V]),
+    "spmv_b200_csr_spmm_host": (_I, [_V, _I, _V, _LL, _V, _LL, _I]),
+    "spmv_b200_hll_spmm_host": (_I, [_V, _I, _V, _LL, _V, _LL]),
+    "spmv_b200_csr_spmm_host_f32": (_I, [_V, _I, _V, _LL, _V, _LL, _I]),
+    "spmv_b200_hll_spmm_host_f32": (_I, [_V, _I, _V, _LL, _V, _LL]),
     "spmv_b200_hll_partials_count": (_I, [_V]),
     "spmv_b200_hll_spmv_fused": (_I, [_V, _V, _V, _V, _V, C.POINTER(Peers), _V]),
     "spmv_b200_hll_spmv_fused_mail": (_I, [_V, _V, _V, _V, C.POINTER(Peers), C.POINTER(Mail), _V]),

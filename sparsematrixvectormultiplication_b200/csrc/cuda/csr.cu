@@ -940,6 +940,8 @@ static int build_plan(spmv_b200_csr *A, cudaStream_t stream) {
     free_plan(A);
     host_pipe_free(A->pipe);  // the row windows of the host entry point follow the tiles
     A->pipe = nullptr;
+    host_pipe_free(A->spmm_pipe);  // its multi-vector windows know which hold long rows
+    A->spmm_pipe = nullptr;
     const int M = A->M;
     if (M == 0) return SPMV_B200_OK;
     unsigned char *boundary = nullptr, *is_long = nullptr;
@@ -1795,7 +1797,9 @@ int spmv_b200_csr_remap_columns(spmv_b200_csr *A, int nparts, const long long *s
         SPMV_TRY_CUDA(cudaGetLastError());
     }
     A->N = (int)(nparts * stride);  // plans, tiles and the fp32 copy of the values do not depend on the column ids;
-    image_free(A->image);           // the private image does
+    image_free(A->image);           // the private image does, and so do the pieces of X the multi-vector host
+    host_pipe_free(A->spmm_pipe);   // product uploads
+    A->spmm_pipe = nullptr;
     SPMV_TRY_CUDA(cudaStreamSynchronize(as_stream(stream)));
     return SPMV_B200_OK;
 }
@@ -1973,6 +1977,7 @@ void spmv_b200_csr_free(spmv_b200_csr *A) {
     cudaFree(A->stage_y);
     cudaFree(A->values32);
     host_pipe_free(A->pipe);
+    host_pipe_free(A->spmm_pipe);
     delete A;
 }
 

@@ -149,7 +149,7 @@ struct BinPlan {                 // csr.cu: row-binned vector kernel for skewed 
     bool built = false;
 };
 
-struct HostPipe;  // hostpath.cu: streams, events and the row-window plan of the *_spmv_host entry points
+struct HostPipe;  // hostpath.cu: streams, events and the row-window plan of the *_spmv_host / *_spmm_host entry points
 void host_pipe_free(HostPipe *p);
 
 struct HllTile {      // tiles[t] = first hack of tile t and its first slot; tiles[num_tiles] = {num_hacks, slots}
@@ -251,6 +251,7 @@ struct spmv_b200_csr {
     double *stage_x = nullptr;
     double *stage_y = nullptr;
     spmv::HostPipe *pipe = nullptr;
+    spmv::HostPipe *spmm_pipe = nullptr;  // the *_spmm_host entry points: their own windows and staging (hostpath.cu)
 };
 
 namespace spmv {
@@ -292,6 +293,7 @@ struct spmv_b200_hll {
     double *stage_x = nullptr;
     double *stage_y = nullptr;
     spmv::HostPipe *pipe = nullptr;
+    spmv::HostPipe *spmm_pipe = nullptr;  // the *_spmm_host entry points: their own windows and staging (hostpath.cu)
 };
 
 namespace spmv {
@@ -400,4 +402,18 @@ int tune_batch(long long M, long long N, int fallback, cudaStream_t stream, Laun
     const int pick = tune_candidates(M, N, n, fallback_index, stream, [&](int i, double *x, double *y) { return launch(ids[i], x, y); });
     return ids[pick] == fallback || pick != fallback_index ? ids[pick] : fallback;
 }
+
+// spmm.cu: the multi-vector launches of a window (V = double, or float on the enable_f32 copy; X and Y at row 0 of the
+// matrix, arguments checked by check_spmm_args).  csr_spmm_rows: rows [r0, r1), leaving out the plan's long rows;
+// csr_spmm_long: those long rows; hll_spmm_hacks: hacks [h0, h1).
+int check_spmm_args(const char *what, const void *h, int k, const void *X, long long ldx, const void *Y, long long ldy);
+template <typename V>
+int csr_spmm_rows(const spmv_b200_csr *A, const V *values, long long r0, long long r1, int k, const V *d_X, long long ldx,
+                  V *d_Y, long long ldy, int accumulate, cudaStream_t stream);
+template <typename V>
+int csr_spmm_long(const spmv_b200_csr *A, const V *values, int k, const V *d_X, long long ldx, V *d_Y, long long ldy,
+                  int accumulate, cudaStream_t stream);
+template <typename V>
+int hll_spmm_hacks(const spmv_b200_hll *H, const V *AS, int h0, int h1, int k, const V *d_X, long long ldx, V *d_Y,
+                   long long ldy, cudaStream_t stream);
 }  // namespace spmv

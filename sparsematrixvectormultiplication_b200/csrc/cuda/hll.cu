@@ -1157,6 +1157,7 @@ void spmv_b200_hll_free(spmv_b200_hll *H) {
     cudaFree(H->stage_x);
     cudaFree(H->stage_y);
     host_pipe_free(H->pipe);
+    host_pipe_free(H->spmm_pipe);
     delete H;
 }
 

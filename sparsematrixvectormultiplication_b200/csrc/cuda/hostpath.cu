@@ -25,6 +25,13 @@
 //   * tapered windows (small first / last windows, 32 MiB in the middle) are SLOWER, 3.36 ms with copies and 3.58 ms
 //     zero-copy: large windows serialise the two directions more than the small ends save (SPMV_B200_HOST_TAPER=1/2
 //     keeps them for experiments).
+//
+// The multi-vector products spmv_b200_{csr,hll}_spmm_host[_f32] run the same pass over k columns (run_pipeline with
+// HostCols): windows of rows (CSR) or hacks (HLL) planned once per handle in a HostPipe of their own, piece w of X ending
+// at need[w] rows (aligned to 256 KB of the staged block), the SpMM kernels of spmm.cu launched per window on shifted
+// base pointers, the CSR long rows (csr_spmm_long) after a block's last piece.  X, and Y when it is staged, are staged
+// in blocks of kc columns (all k when they fit half of the free device memory); a block's pieces and downloads are 2-D
+// copies unless the block is contiguous on both sides.
 #include <algorithm>
 #include <vector>
 
@@ -46,6 +53,8 @@ struct HostPipe {
     std::vector<cudaEvent_t> landed;  // chunk c of x is on the device
     std::vector<cudaEvent_t> done;    // window w is computed
     cudaEvent_t y_landed = nullptr;   // accumulate: the old y is on the device
+    cudaEvent_t x_free = nullptr;     // column blocks: the last kernel of the previous block has read the staged X
+    cudaEvent_t y_free = nullptr;     // column blocks: the staged Y of the previous block is downloaded
     // window plan (valid for `path` only)
     int path = -1;
     int windows = 0;
@@ -53,6 +62,9 @@ struct HostPipe {
     std::vector<long long> row;   // W+1: first row of every window
     std::vector<long long> need;  // W: doubles of x that must be resident before window w starts (running maximum)
     std::vector<long long> piece; // W: upload piece w ends here (need[w] rounded up to kPieceAlign, <= N; non-decreasing)
+    std::vector<char> tail_window;  // multi-vector CSR with long rows: W flags, window w holds a long row
+    void *stage = nullptr;          // multi-vector products: the staged column block of X, then of Y
+    size_t stage_bytes = 0;
 };
 
 void host_pipe_free(HostPipe *p) {
@@ -60,6 +72,9 @@ void host_pipe_free(HostPipe *p) {
     for (cudaEvent_t e : p->landed) cudaEventDestroy(e);
     for (cudaEvent_t e : p->done) cudaEventDestroy(e);
     if (p->y_landed) cudaEventDestroy(p->y_landed);
+    if (p->x_free) cudaEventDestroy(p->x_free);
+    if (p->y_free) cudaEventDestroy(p->y_free);
+    cudaFree(p->stage);
     if (p->up) cudaStreamDestroy(p->up);
     if (p->compute) cudaStreamDestroy(p->compute);
     if (p->down) cudaStreamDestroy(p->down);
@@ -74,6 +89,8 @@ static int pipe_create(HostPipe **out) {
         SPMV_TRY_CUDA(cudaStreamCreateWithFlags(&p->compute, cudaStreamNonBlocking));
         SPMV_TRY_CUDA(cudaStreamCreateWithFlags(&p->down, cudaStreamNonBlocking));
         SPMV_TRY_CUDA(cudaEventCreateWithFlags(&p->y_landed, cudaEventDisableTiming));
+        SPMV_TRY_CUDA(cudaEventCreateWithFlags(&p->x_free, cudaEventDisableTiming));
+        SPMV_TRY_CUDA(cudaEventCreateWithFlags(&p->y_free, cudaEventDisableTiming));
         p->landed.resize(kMaxWindows, nullptr);
         p->done.resize(kMaxWindows, nullptr);
         for (int i = 0; i < kMaxWindows; ++i) {
@@ -135,12 +152,15 @@ static int plan_needs(HostPipe *p, const int *d_idx, const std::vector<long long
     return SPMV_B200_OK;
 }
 
-// upload pieces: piece w ends where window w's referenced prefix of x ends, rounded up to a 256 KB boundary
-static void plan_pieces(HostPipe *p, long long N) {
-    p->piece.assign(p->windows, 0);
-    for (int w = 0; w < p->windows; ++w)
-        p->piece[w] = std::min(N, (p->need[w] + kPieceAlign - 1) / kPieceAlign * kPieceAlign);
+// upload pieces: piece w ends where window w's referenced prefix of x ends, rounded up to `align` rows
+static std::vector<long long> pieces_of(const HostPipe *p, long long N, long long align) {
+    std::vector<long long> piece(p->windows, 0);
+    for (int w = 0; w < p->windows; ++w) piece[w] = std::min(N, (p->need[w] + align - 1) / align * align);
+    return piece;
 }
+
+// one vector: on 256 KB boundaries of x
+static void plan_pieces(HostPipe *p, long long N) { p->piece = pieces_of(p, N, kPieceAlign); }
 
 static int pick_windows(long long M, long long N, int units) {
     const int forced = env_int("SPMV_B200_HOST_WINDOWS", 0);
@@ -190,58 +210,104 @@ static std::vector<long long> window_rows(long long M, long long N, int units) {
 
 // A host y that the device can address (pinned or registered, unified addressing): the products can store their rows
 // straight into it over PCIe and the download copies -- with their event hand-overs -- disappear.
-static double *device_alias_of_host(double *y) {
+template <class V>
+static V *device_alias_of_host(V *y) {
     cudaPointerAttributes attr;
     if (cudaPointerGetAttributes(&attr, y) != cudaSuccess) {
         cudaGetLastError();
         return nullptr;
     }
     if (attr.type != cudaMemoryTypeHost || attr.devicePointer == nullptr) return nullptr;
-    return static_cast<double *>(attr.devicePointer);
+    return static_cast<V *>(attr.devicePointer);
 }
 
-// The pass itself.  launch(w, y_base) enqueues the kernel(s) of window w on p->compute; they write rows r of the matrix
-// to y_base[r].  zero_copy_ok: every row is written exactly once and never read back by the kernels of this path.
-template <class Launch>
-static int run_pipeline(HostPipe *p, long long M, long long N, const double *x, double *y, double *d_x, double *d_y,
-                        bool accumulate, bool zero_copy_ok, Launch launch) {
+// SPMV_B200_HOST_ZEROCOPY (default on; 0 forces it off): kernels store y directly into the caller's pinned buffer
+template <class V>
+static V *zero_copy_alias(bool zero_copy_ok, bool accumulate, long long M, V *y) {
+    return (zero_copy_ok && !accumulate && M && env_int("SPMV_B200_HOST_ZEROCOPY", kZeroCopyDefault)) ? device_alias_of_host(y) : nullptr;
+}
+
+// The columns of a pass: x is N x k with leading dimension ldx and y is M x k with ldy, in elements; one vector is
+// k = kc = ldx = ldy = 1.  They travel in blocks of kc columns: the device holds one block of x (and of y when y is
+// staged) at a time, with leading dimension kc.
+struct HostCols {
+    int k = 1, kc = 1;
+    long long ldx = 1, ldy = 1;
+};
+
+// rows x cols elements between two row-major blocks: one 1-D copy when both are contiguous, one 2-D copy otherwise
+template <class V>
+static int copy_rows(V *dst, long long ldd, const V *src, long long lds, int cols, long long rows, cudaMemcpyKind kind,
+                     cudaStream_t stream) {
+    if (ldd == cols && lds == cols)
+        SPMV_TRY_CUDA(cudaMemcpyAsync(dst, src, (size_t)rows * cols * sizeof(V), kind, stream));
+    else
+        SPMV_TRY_CUDA(cudaMemcpy2DAsync(dst, (size_t)ldd * sizeof(V), src, (size_t)lds * sizeof(V), (size_t)cols * sizeof(V),
+                                        (size_t)rows, kind, stream));
+    return SPMV_B200_OK;
+}
+
+// The pass itself.  launch(w, y_base, ld, cols) enqueues the kernel(s) of window w on p->compute for the `cols` columns
+// of the current block (x staged at d_x with leading dimension kc); they write row r, column c of the block to
+// y_base[r * ld + c].  zero_copy_ok: every element is written exactly once and never read back by the kernels of this
+// path.  tail(y_base, ld, cols) runs after the last window of a block (the CSR long rows); the downloads of the windows
+// flagged in p->tail_window wait for it.  piece: the W upload pieces of a block, in rows of x.
+template <class V, class Launch, class Tail>
+static int run_pipeline(HostPipe *p, long long M, long long N, const V *x, V *y, V *d_x, V *d_y, bool accumulate,
+                        bool zero_copy_ok, const std::vector<long long> &piece, const HostCols &c, Launch launch, Tail tail) {
     const int W = p->windows;
-    // SPMV_B200_HOST_ZEROCOPY (default on): kernels store y directly into the caller's pinned buffer
-    double *y_alias = (zero_copy_ok && !accumulate && M && env_int("SPMV_B200_HOST_ZEROCOPY", kZeroCopyDefault)) ? device_alias_of_host(y) : nullptr;
-    double *y_base = y_alias ? y_alias : d_y;
-    // (1) uploads: the old y first (accumulate), then x in W chunks
-    if (accumulate && M) {
-        SPMV_TRY_CUDA(cudaMemcpyAsync(d_y, y, (size_t)M * sizeof(double), cudaMemcpyHostToDevice, p->up));
-        SPMV_TRY_CUDA(cudaEventRecord(p->y_landed, p->up));
-    }
-    // piece w of x ends where window w's columns end; a window that needs nothing new reuses the previous event.
-    // Columns no window references are never uploaded.
-    std::vector<int> gate(W, -1);
-    long long at = 0;
-    int last = -1;
-    for (int w = 0; w < W; ++w) {
-        const long long upto = std::min(N, p->piece[w]);
-        if (upto > at) {
-            SPMV_TRY_CUDA(cudaMemcpyAsync(d_x + at, x + at, (size_t)(upto - at) * sizeof(double), cudaMemcpyHostToDevice, p->up));
-            SPMV_TRY_CUDA(cudaEventRecord(p->landed[w], p->up));
-            last = w;
-            at = upto;
+    V *y_alias = zero_copy_alias(zero_copy_ok, accumulate, M, y);
+    const bool tails = !p->tail_window.empty();
+    for (int c0 = 0; c0 < c.k; c0 += c.kc) {
+        const int cw = std::min(c.kc, c.k - c0);
+        const bool first = c0 == 0, more = c0 + c.kc < c.k;
+        V *y_base = y_alias ? y_alias + c0 : d_y;
+        const long long ld_y = y_alias ? c.ldy : c.kc;
+        // (1) uploads: the old y first (accumulate), then x in W chunks.  A later block overwrites the staging of the
+        // previous one: its x waits for that block's last kernel, its old y for that block's downloads.
+        if (!first) SPMV_TRY_CUDA(cudaStreamWaitEvent(p->up, p->x_free, 0));
+        if (accumulate && M) {
+            if (!first) SPMV_TRY_CUDA(cudaStreamWaitEvent(p->up, p->y_free, 0));
+            SPMV_TRY(copy_rows(d_y, c.kc, y + c0, c.ldy, cw, M, cudaMemcpyHostToDevice, p->up));
+            SPMV_TRY_CUDA(cudaEventRecord(p->y_landed, p->up));
         }
-        gate[w] = last;
-    }
-    // (2) products: window w waits for its piece
-    for (int w = 0; w < W; ++w) {
-        if (accumulate && M && w == 0) SPMV_TRY_CUDA(cudaStreamWaitEvent(p->compute, p->y_landed, 0));
-        if (gate[w] >= 0 && (w == 0 || gate[w] != gate[w - 1])) SPMV_TRY_CUDA(cudaStreamWaitEvent(p->compute, p->landed[gate[w]], 0));
-        SPMV_TRY(launch(w, y_base));
-        if (!y_alias) SPMV_TRY_CUDA(cudaEventRecord(p->done[w], p->compute));
-    }
-    // (3) downloads, window by window (none when the kernels wrote into the host buffer themselves)
-    for (int w = 0; w < W && !y_alias; ++w) {
-        const long long r0 = p->row[w], r1 = p->row[w + 1];
-        if (r1 <= r0) continue;
-        SPMV_TRY_CUDA(cudaStreamWaitEvent(p->down, p->done[w], 0));
-        SPMV_TRY_CUDA(cudaMemcpyAsync(y + r0, d_y + r0, (size_t)(r1 - r0) * sizeof(double), cudaMemcpyDeviceToHost, p->down));
+        // piece w of x ends where window w's columns end; a window that needs nothing new reuses the previous event.
+        // Columns no window references are never uploaded.
+        std::vector<int> gate(W, -1);
+        long long at = 0;
+        int last = -1;
+        for (int w = 0; w < W; ++w) {
+            const long long upto = std::min(N, piece[w]);
+            if (upto > at) {
+                SPMV_TRY(copy_rows(d_x + at * c.kc, c.kc, x + at * c.ldx + c0, c.ldx, cw, upto - at, cudaMemcpyHostToDevice, p->up));
+                SPMV_TRY_CUDA(cudaEventRecord(p->landed[w], p->up));
+                last = w;
+                at = upto;
+            }
+            gate[w] = last;
+        }
+        // (2) products: window w waits for its piece (and a later block's first window for the staged y to be free)
+        for (int w = 0; w < W; ++w) {
+            if (!first && !y_alias && w == 0) SPMV_TRY_CUDA(cudaStreamWaitEvent(p->compute, p->y_free, 0));
+            if (accumulate && M && w == 0) SPMV_TRY_CUDA(cudaStreamWaitEvent(p->compute, p->y_landed, 0));
+            if (gate[w] >= 0 && (w == 0 || gate[w] != gate[w - 1])) SPMV_TRY_CUDA(cudaStreamWaitEvent(p->compute, p->landed[gate[w]], 0));
+            SPMV_TRY(launch(w, y_base, ld_y, cw));
+            if (!y_alias && !(tails && p->tail_window[w])) SPMV_TRY_CUDA(cudaEventRecord(p->done[w], p->compute));
+        }
+        SPMV_TRY(tail(y_base, ld_y, cw));
+        for (int w = 0; tails && !y_alias && w < W; ++w)
+            if (p->tail_window[w]) SPMV_TRY_CUDA(cudaEventRecord(p->done[w], p->compute));
+        if (more) SPMV_TRY_CUDA(cudaEventRecord(p->x_free, p->compute));
+        // (3) downloads, window by window, those the tail writes into last (none when the kernels wrote into the host
+        // buffer themselves)
+        for (int pass = 0; pass < (tails ? 2 : 1) && !y_alias; ++pass)
+            for (int w = 0; w < W; ++w) {
+                const long long r0 = p->row[w], r1 = p->row[w + 1];
+                if (r1 <= r0 || (tails && p->tail_window[w] != pass)) continue;
+                SPMV_TRY_CUDA(cudaStreamWaitEvent(p->down, p->done[w], 0));
+                SPMV_TRY(copy_rows(y + r0 * c.ldy + c0, c.ldy, d_y + r0 * c.kc, c.kc, cw, r1 - r0, cudaMemcpyDeviceToHost, p->down));
+            }
+        if (more && !y_alias) SPMV_TRY_CUDA(cudaEventRecord(p->y_free, p->down));
     }
     SPMV_TRY_CUDA(cudaStreamSynchronize(p->down));
     SPMV_TRY_CUDA(cudaStreamSynchronize(p->compute));
@@ -255,6 +321,9 @@ static void abort_pipeline(HostPipe *p) {  // after an error: nothing of this ca
     cudaStreamSynchronize(p->compute);
     cudaStreamSynchronize(p->down);
 }
+
+template <class V>
+static int no_tail(V *, long long, int) { return SPMV_B200_OK; }
 
 // ---- CSR --------------------------------------------------------------------------------------------------------
 static int csr_plan_windows(spmv_b200_csr *A, CsrPath path) {
@@ -340,6 +409,157 @@ static int time_products(long long M, long long N, const double *x, double *y, d
     return rc;
 }
 
+// ---- multi-vector products Y = A X on host buffers ------------------------------------------------------------------
+constexpr long long kSpmmPieceBytes = 256LL << 10;  // upload pieces end on 256 KB of the staged block, as for one vector
+
+// Y straight into the caller's pinned buffer (zero-copy) or staged and downloaded window by window.  Measured with
+// tools/spmm_host_bench.py --sweep-only on a build where this returns true, both ways in every cell (B200 at 1000 W,
+// profiles/r03j_spmm_host_y_sweep.json; DESIGN.md section 3, "Host buffers"), minima of 7 calls:
+//   * ldy > k: the 2-D downloads lose to the kernels' stores from 32 bytes a row (lap2d 4096^2 CSR k = 8, ldy = 11:
+//     39.2 against 55.9 ms) and are as fast or slower below; at 256 bytes zero-copy is 2-3 % slower on lap2d only;
+//   * ldy = k: zero-copy is faster at 8 bytes a row everywhere, at 16 on uniform and R-MAT (lap2d: 2.9 % slower), and
+//     from 32 bytes the 1-D downloads are faster on lap2d (k = 32: 91.1 against 102.6 ms) and uniform (3.5-5.5 %) while
+//     R-MAT gains 0.5-6 % from zero-copy.
+static bool spmm_zero_copy(int k, long long ldy, size_t elem) { return ldy != k || (size_t)k * elem <= 16; }
+
+// The window plan of the multi-vector products (rows for CSR, hacks for HLL), made once per handle and kept apart from
+// the single-vector plan, so that alternating the two entry points never plans again.  SPMV_B200_HOST_WINDOWS is read
+// here: a changed setting takes effect on a fresh handle.
+static int spmm_plan_csr(spmv_b200_csr *A) {
+    HostPipe *p = A->spmm_pipe;
+    const std::vector<long long> bounds = window_rows(A->M, A->N, A->M);
+    p->unit.clear();
+    p->row.clear();
+    std::vector<long long> elem;
+    for (size_t w = 0; w < bounds.size(); ++w) {
+        const int row = (int)bounds[w];
+        if (!p->unit.empty() && row <= p->unit.back() && w + 1 != bounds.size()) continue;  // an empty window
+        int off = 0;
+        SPMV_TRY_CUDA(cudaMemcpy(&off, A->row_ptr + row, sizeof off, cudaMemcpyDeviceToHost));
+        p->unit.push_back(row);
+        p->row.push_back(row);
+        elem.push_back(off);
+    }
+    const int W = (int)p->unit.size() - 1;
+    p->windows = W;
+    p->tail_window.clear();
+    if (A->num_long > 0) {  // the windows whose downloads wait for the long rows
+        std::vector<int> long_rows((size_t)A->num_long);
+        SPMV_TRY_CUDA(cudaMemcpy(long_rows.data(), A->long_rows, long_rows.size() * sizeof(int), cudaMemcpyDeviceToHost));
+        p->tail_window.assign((size_t)W, 0);
+        for (int r : long_rows)
+            p->tail_window[std::upper_bound(p->row.begin(), p->row.end(), (long long)r) - p->row.begin() - 1] = 1;
+    }
+    SPMV_TRY(plan_needs(p, A->col_idx, elem));
+    p->path = 0;
+    return SPMV_B200_OK;
+}
+
+static int spmm_plan_hll(spmv_b200_hll *H) {
+    HostPipe *p = H->spmm_pipe;
+    const std::vector<long long> bounds = window_rows(H->M, H->N, H->num_hacks);
+    p->unit.clear();
+    p->row.clear();
+    std::vector<long long> elem;
+    for (size_t w = 0; w < bounds.size(); ++w) {
+        const int hack = w + 1 == bounds.size() ? H->num_hacks : (int)(bounds[w] / HACK_SIZE);
+        if (!p->unit.empty() && hack <= p->unit.back() && w + 1 != bounds.size()) continue;
+        p->unit.push_back(hack);
+        p->row.push_back(std::min<long long>((long long)hack * HACK_SIZE, H->M));
+        elem.push_back(H->host_off[hack]);
+    }
+    p->windows = (int)p->unit.size() - 1;
+    SPMV_TRY(plan_needs(p, H->JA, elem));
+    p->path = 0;
+    return SPMV_B200_OK;
+}
+
+// The device staging of a k-column product: all k columns of X (and of Y when it is staged) when they fit half of the
+// free device memory, else blocks of kc columns that do (SPMV_B200_HOST_SPMM_COLS forces kc).  Kept on the handle, grown
+// as needed and freed with it.
+template <class V>
+static int spmm_stage(HostPipe *p, long long M, long long N, int k, bool stage_y, int *kc, V **d_x, V **d_y) {
+    size_t free_bytes = 0, total_bytes = 0;
+    SPMV_TRY_CUDA(cudaMemGetInfo(&free_bytes, &total_bytes));
+    const size_t budget = (free_bytes + p->stage_bytes) / 2;
+    const size_t per_col = (size_t)(N + (stage_y ? M : 0)) * sizeof(V);
+    int cols = k;
+    if (per_col > 0 && per_col * (size_t)k > budget) cols = (int)std::max<size_t>(1, budget / per_col);
+    const int forced = env_int("SPMV_B200_HOST_SPMM_COLS", 0);
+    if (forced > 0) cols = std::min(k, forced);
+    const size_t x_bytes = ((size_t)N * cols * sizeof(V) + 255) / 256 * 256;
+    const size_t bytes = std::max<size_t>(1, x_bytes + (stage_y ? (size_t)M * cols * sizeof(V) : 0));
+    if (bytes > p->stage_bytes) {
+        cudaFree(p->stage);
+        p->stage = nullptr;
+        p->stage_bytes = 0;
+        SPMV_TRY_CUDA(cudaMalloc(&p->stage, bytes));
+        p->stage_bytes = bytes;
+    }
+    *kc = cols;
+    *d_x = static_cast<V *>(p->stage);
+    *d_y = reinterpret_cast<V *>(static_cast<char *>(p->stage) + x_bytes);
+    return SPMV_B200_OK;
+}
+
+// The pass over the columns: staging, pieces aligned in bytes of the staged block, then run_pipeline.
+template <class V, class Launch, class Tail>
+static int spmm_host_pass(HostPipe *p, long long M, long long N, int k, const V *X, long long ldx, V *Y, long long ldy,
+                          bool accumulate, Launch launch, Tail tail) {
+    const bool zero_copy_ok = spmm_zero_copy(k, ldy, sizeof(V));
+    const bool stage_y = zero_copy_alias(zero_copy_ok, accumulate, M, Y) == nullptr;
+    int kc = 0;
+    V *d_x = nullptr, *d_y = nullptr;
+    SPMV_TRY(spmm_stage(p, M, N, k, stage_y, &kc, &d_x, &d_y));
+    const std::vector<long long> piece = pieces_of(p, N, std::max<long long>(1, kSpmmPieceBytes / ((long long)kc * (long long)sizeof(V))));
+    const HostCols c{k, kc, ldx, ldy};
+    const int rc = run_pipeline(p, M, N, X, Y, d_x, d_y, accumulate, zero_copy_ok, piece, c,
+                                [&](int w, V *y_base, long long ld, int cols) { return launch(w, d_x, (long long)kc, y_base, ld, cols); },
+                                [&](V *y_base, long long ld, int cols) { return tail(d_x, (long long)kc, y_base, ld, cols); });
+    if (rc != SPMV_B200_OK) abort_pipeline(p);
+    return rc;
+}
+
+template <class V>
+static int csr_spmm_host(const char *what, spmv_b200_csr *A, int k, const V *X, long long ldx, V *Y, long long ldy, int accumulate) {
+    SPMV_TRY(check_spmm_args(what, A, k, X, ldx, Y, ldy));
+    if (k == 0 || A->M == 0) return SPMV_B200_OK;
+    if (sizeof(V) == 4) {  // the float copy is made on the NULL stream; the non-blocking streams of the pass do not wait for it
+        SPMV_TRY(spmv_b200_csr_enable_f32(A, nullptr));
+        SPMV_TRY_CUDA(cudaStreamSynchronize(nullptr));
+    }
+    const V *values = sizeof(V) == 4 ? (const V *)A->values32 : (const V *)A->values;
+    if (!A->spmm_pipe) SPMV_TRY(pipe_create(&A->spmm_pipe));
+    HostPipe *p = A->spmm_pipe;
+    if (p->path < 0) SPMV_TRY(spmm_plan_csr(A));
+    return spmm_host_pass(p, A->M, A->N, k, X, ldx, Y, ldy, accumulate != 0,
+        [&](int w, const V *d_x, long long ld_x, V *y_base, long long ld_y, int cols) {
+            return csr_spmm_rows(A, values, p->unit[w], p->unit[w + 1], cols, d_x, ld_x, y_base, ld_y, accumulate, p->compute);
+        },
+        [&](const V *d_x, long long ld_x, V *y_base, long long ld_y, int cols) {
+            return csr_spmm_long(A, values, cols, d_x, ld_x, y_base, ld_y, accumulate, p->compute);
+        });
+}
+
+template <class V>
+static int hll_spmm_host(const char *what, spmv_b200_hll *H, int k, const V *X, long long ldx, V *Y, long long ldy) {
+    SPMV_TRY(check_spmm_args(what, H, k, X, ldx, Y, ldy));
+    if (k == 0 || H->M == 0 || H->num_hacks == 0) return SPMV_B200_OK;
+    if (sizeof(V) == 4) {  // the float copy is made on the NULL stream; the non-blocking streams of the pass do not wait for it
+        SPMV_TRY(spmv_b200_hll_enable_f32(H, nullptr));
+        SPMV_TRY_CUDA(cudaStreamSynchronize(nullptr));
+    }
+    const V *AS = sizeof(V) == 4 ? (const V *)H->AS32 : (const V *)H->AS;
+    if (!H->spmm_pipe) SPMV_TRY(pipe_create(&H->spmm_pipe));
+    HostPipe *p = H->spmm_pipe;
+    if (p->path < 0) SPMV_TRY(spmm_plan_hll(H));
+    return spmm_host_pass(p, H->M, H->N, k, X, ldx, Y, ldy, false,
+        [&](int w, const V *d_x, long long ld_x, V *y_base, long long ld_y, int cols) {
+            return hll_spmm_hacks(H, AS, p->unit[w], p->unit[w + 1], cols, d_x, ld_x, y_base, ld_y, p->compute);
+        },
+        [](const V *, long long, V *, long long, int) { return SPMV_B200_OK; });
+}
+
 }  // namespace spmv
 
 using namespace spmv;
@@ -360,9 +580,10 @@ int spmv_b200_csr_spmv_host(spmv_b200_csr *A, const double *x, double *y, int ac
     HostPipe *p = A->pipe;
     // the binned kernel's long rows are combined by a second kernel that may read y (accumulate); tiles with long rows too
     const bool zero_copy_ok = path != kPathBinned && A->num_long == 0;
-    const int rc = run_pipeline(p, A->M, x ? A->N : 0, x, y, A->stage_x, A->stage_y, accumulate != 0, zero_copy_ok, [&](int w, double *y_base) {
+    const int rc = run_pipeline(p, A->M, x ? A->N : 0, x, y, A->stage_x, A->stage_y, accumulate != 0, zero_copy_ok, p->piece, HostCols{},
+                                [&](int w, double *y_base, long long, int) {
         return csr_launch_window(A, path, p->unit[w], p->unit[w + 1], A->stage_x, y_base, accumulate, p->compute);
-    });
+    }, no_tail<double>);
     if (rc != SPMV_B200_OK) abort_pipeline(p);
     return rc;
 }
@@ -408,11 +629,28 @@ int spmv_b200_hll_spmv_host(spmv_b200_hll *H, const double *x, double *y) {
         plan_pieces(p, H->N);
         p->path = (int)path;
     }
-    const int rc = run_pipeline(p, H->M, x ? H->N : 0, x, y, H->stage_x, H->stage_y, false, true, [&](int w, double *y_base) {
+    const int rc = run_pipeline(p, H->M, x ? H->N : 0, x, y, H->stage_x, H->stage_y, false, true, p->piece, HostCols{},
+                                [&](int w, double *y_base, long long, int) {
         return hll_launch_window(H, path, p->unit[w], p->unit[w + 1], H->stage_x, y_base, p->compute);
-    });
+    }, no_tail<double>);
     if (rc != SPMV_B200_OK) abort_pipeline(p);
     return rc;
+}
+
+int spmv_b200_csr_spmm_host(spmv_b200_csr *A, int k, const double *X, long long ldx, double *Y, long long ldy, int accumulate) {
+    return csr_spmm_host("csr_spmm_host", A, k, X, ldx, Y, ldy, accumulate);
+}
+
+int spmv_b200_hll_spmm_host(spmv_b200_hll *H, int k, const double *X, long long ldx, double *Y, long long ldy) {
+    return hll_spmm_host("hll_spmm_host", H, k, X, ldx, Y, ldy);
+}
+
+int spmv_b200_csr_spmm_host_f32(spmv_b200_csr *A, int k, const float *X, long long ldx, float *Y, long long ldy, int accumulate) {
+    return csr_spmm_host("csr_spmm_host_f32", A, k, X, ldx, Y, ldy, accumulate);
+}
+
+int spmv_b200_hll_spmm_host_f32(spmv_b200_hll *H, int k, const float *X, long long ldx, float *Y, long long ldy) {
+    return hll_spmm_host("hll_spmm_host_f32", H, k, X, ldx, Y, ldy);
 }
 
 int spmv_b200_csr_time(spmv_b200_csr *A, const double *x, double *y, int algo, int warmup, int iters, double *mean_seconds,

@@ -251,7 +251,7 @@ struct HllSpmmLaunch {
     }
 };
 
-static int check_spmm_args(const char *what, const void *h, int k, const void *X, long long ldx, const void *Y,
+int check_spmm_args(const char *what, const void *h, int k, const void *X, long long ldx, const void *Y,
                            long long ldy) {
     if (k < 0) return fail(SPMV_B200_ERR_INVALID, "%s: negative k (%d)", what, k);
     if (ldx < k || ldy < k)
@@ -261,20 +261,29 @@ static int check_spmm_args(const char *what, const void *h, int k, const void *X
 }
 
 // The products behind the entry points (arguments checked, k > 0, M > 0): V = double on the fp64 values, V = float on
-// the copy of enable_f32; every sum is formed in double either way.
+// the copy of enable_f32; every sum is formed in double either way.  The host-buffer products (hostpath.cu) run the same
+// launches window by window: csr_spmm_rows on rows [r0, r1) (the long rows left out, as the kernel does everywhere) and
+// csr_spmm_long for the long rows, hll_spmm_hacks on hacks [h0, h1).  X and Y point at row 0 of the matrix.
 template <typename V>
-static int csr_spmm(const spmv_b200_csr *A, const V *values, int k, const V *d_X, long long ldx, V *d_Y, long long ldy,
-                    int accumulate, cudaStream_t stream) {
+int csr_spmm_rows(const spmv_b200_csr *A, const V *values, long long r0, long long r1, int k, const V *d_X, long long ldx,
+                  V *d_Y, long long ldy, int accumulate, cudaStream_t stream) {
     const int batch = spmm_batch(sizeof(V) == 4 ? kSpmmBatchCsr32 : kSpmmBatchCsr);
-    const int M = A->M;
+    const int M = (int)(r1 - r0);
     const int acc = accumulate ? 1 : 0;
-    SPMV_TRY(spmm_tiles(k, [&](int kt, int c0, int cols, int tiles) {
+    if (M <= 0) return SPMV_B200_OK;
+    return spmm_tiles(k, [&](int kt, int c0, int cols, int tiles) {
         const dim3 grid(blocks_for(M, kSpmmThreads / kt), (unsigned)tiles);
-        return spmm_dispatch<CsrSpmmLaunch>(kt, batch, grid, stream, M, (const int *)A->row_ptr, (const int *)A->col_idx,
-                                            values, A->long_threshold, c0, cols, d_X, ldx, d_Y, ldy, acc);
-    }));
+        return spmm_dispatch<CsrSpmmLaunch>(kt, batch, grid, stream, M, (const int *)(A->row_ptr + r0), (const int *)A->col_idx,
+                                            values, A->long_threshold, c0, cols, d_X, ldx, d_Y + r0 * ldy, ldy, acc);
+    });
+}
+
+template <typename V>
+int csr_spmm_long(const spmv_b200_csr *A, const V *values, int k, const V *d_X, long long ldx, V *d_Y, long long ldy,
+                  int accumulate, cudaStream_t stream) {
     if (A->num_long == 0) return SPMV_B200_OK;
-    // the long rows: one fragment + combine launch pair per column tile, through the handle's partials buffer
+    const int acc = accumulate ? 1 : 0;
+    // one fragment + combine launch pair per column tile, through the handle's partials buffer
     if (!A->spmm_partial) SPMV_TRY_CUDA(cudaMalloc(&A->spmm_partial, (size_t)A->num_frag * kSpmmTile * sizeof(double)));
     for (int c0 = 0; c0 < k; c0 += kSpmmTile) {
         const int cols = std::min(kSpmmTile, k - c0);
@@ -290,16 +299,43 @@ static int csr_spmm(const spmv_b200_csr *A, const V *values, int k, const V *d_X
 }
 
 template <typename V>
-static int hll_spmm(const spmv_b200_hll *H, const V *AS, int k, const V *d_X, long long ldx, V *d_Y, long long ldy,
-                    cudaStream_t stream) {
+static int csr_spmm(const spmv_b200_csr *A, const V *values, int k, const V *d_X, long long ldx, V *d_Y, long long ldy,
+                    int accumulate, cudaStream_t stream) {
+    SPMV_TRY(csr_spmm_rows(A, values, 0, A->M, k, d_X, ldx, d_Y, ldy, accumulate, stream));
+    return csr_spmm_long(A, values, k, d_X, ldx, d_Y, ldy, accumulate, stream);
+}
+
+template <typename V>
+int hll_spmm_hacks(const spmv_b200_hll *H, const V *AS, int h0, int h1, int k, const V *d_X, long long ldx, V *d_Y,
+                   long long ldy, cudaStream_t stream) {
     const int batch = spmm_batch(kSpmmBatchHll);
-    const long long rows = (long long)H->num_hacks * 32;
+    const int hacks = h1 - h0;
+    if (hacks <= 0) return SPMV_B200_OK;
+    const int M = (int)(std::min<long long>(H->M, 32LL * h1) - 32LL * h0);
+    const long long rows = (long long)hacks * 32;
     return spmm_tiles(k, [&](int kt, int c0, int cols, int tiles) {
         const dim3 grid(blocks_for(rows, kSpmmThreads / kt), (unsigned)tiles);
-        return spmm_dispatch<HllSpmmLaunch>(kt, batch, grid, stream, H->M, H->num_hacks, (const long long *)H->hack_off,
-                                            (const int *)H->JA, AS, c0, cols, d_X, ldx, d_Y, ldy);
+        return spmm_dispatch<HllSpmmLaunch>(kt, batch, grid, stream, M, hacks, (const long long *)(H->hack_off + h0),
+                                            (const int *)H->JA, AS, c0, cols, d_X, ldx, d_Y + 32LL * h0 * ldy, ldy);
     });
 }
+
+template <typename V>
+static int hll_spmm(const spmv_b200_hll *H, const V *AS, int k, const V *d_X, long long ldx, V *d_Y, long long ldy,
+                    cudaStream_t stream) {
+    return hll_spmm_hacks(H, AS, 0, H->num_hacks, k, d_X, ldx, d_Y, ldy, stream);
+}
+
+#define SPMV_SPMM_WINDOWS(V)                                                                                                \
+    template int csr_spmm_rows<V>(const spmv_b200_csr *, const V *, long long, long long, int, const V *, long long, V *,   \
+                                  long long, int, cudaStream_t);                                                            \
+    template int csr_spmm_long<V>(const spmv_b200_csr *, const V *, int, const V *, long long, V *, long long, int,         \
+                                  cudaStream_t);                                                                            \
+    template int hll_spmm_hacks<V>(const spmv_b200_hll *, const V *, int, int, int, const V *, long long, V *, long long,   \
+                                   cudaStream_t);
+SPMV_SPMM_WINDOWS(double)
+SPMV_SPMM_WINDOWS(float)
+#undef SPMV_SPMM_WINDOWS
 
 }  // namespace spmv
 

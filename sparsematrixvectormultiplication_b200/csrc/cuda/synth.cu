@@ -264,12 +264,13 @@ extern "C" {
 const char *spmv_b200_last_error(void) { return g_error; }
 void spmv_b200_clear_error(void) { g_error[0] = '\0'; }
 
-int spmv_b200_version(void) { return 107; }  // 101: spmv_b200_csr_spmm / spmv_b200_hll_spmm; 102: spmv_b200_csr_set_image;
+int spmv_b200_version(void) { return 108; }  // 101: spmv_b200_csr_spmm / spmv_b200_hll_spmm; 102: spmv_b200_csr_set_image;
                                               // 103: the narrow private image, spmv_b200_csr_info_t::image_index_bytes;
                                               // 104: the coded private image (set_image mode 2), image_value_bytes;
                                               // 105: spmv_b200_csr_spmm_f32 / spmv_b200_hll_spmm_f32;
                                               // 106: the pattern form of the private image (set_image mode 3), image_patterns;
-                                              // 107: image_windows (the tiled kernel of the pattern form)
+                                              // 107: image_windows (the tiled kernel of the pattern form);
+                                              // 108: spmv_b200_{csr,hll}_spmm_host[_f32]
 
 int spmv_b200_device_count(int *count) {
     if (!count) return fail(SPMV_B200_ERR_INVALID, "device_count: NULL argument");

@@ -78,11 +78,17 @@ def _dense_overlap(a, lda, b, ldb, k, size=8):
     """Do the row-major k-column blocks a (leading dimension lda) and b (ldb) of `size`-byte elements share an element?
     Exact when the leading dimensions are equal (interleaved column slices of one buffer do not overlap), conservative
     otherwise: then any intersection of the two address ranges counts."""
-    if k == 0 or a.numel() == 0 or b.numel() == 0:
+    if a.numel() == 0 or b.numel() == 0:
         return False
-    pa, pb = a.data_ptr(), b.data_ptr()
-    ea = pa + size * ((a.shape[0] - 1) * lda + k)
-    eb = pb + size * ((b.shape[0] - 1) * ldb + k)
+    return _block_overlap(a.data_ptr(), a.shape[0], lda, b.data_ptr(), b.shape[0], ldb, k, size)
+
+
+def _block_overlap(pa, rows_a, lda, pb, rows_b, ldb, k, size):
+    """_dense_overlap on addresses: blocks of rows_a and rows_b rows at pa and pb."""
+    if k == 0 or rows_a == 0 or rows_b == 0:
+        return False
+    ea = pa + size * ((rows_a - 1) * lda + k)
+    eb = pb + size * ((rows_b - 1) * ldb + k)
     if ea <= pb or eb <= pa:
         return False
     if lda != ldb or (pb - pa) % size:
@@ -99,6 +105,58 @@ def _spmm_operands(X, Y, M, N_, dtype="float64"):
     if _dense_overlap(X, ldx, Y, ldy, k, X.element_size()):
         raise ValueError("Y must not overlap X")
     return k, ldx, ldy
+
+
+def _check_host_dense(t, rows, what, dtype, writable=False):
+    """A row-major block of a host-buffer multi-vector product: a 2-D numpy array or CPU torch tensor of `dtype` with
+    `rows` rows, column stride 1 and a row stride (the leading dimension) of at least the column count, such as
+    big[:, :k].  Returns (columns, leading dimension, address)."""
+    import torch
+    if isinstance(t, np.ndarray):
+        if t.dtype != dtype or t.ndim != 2:
+            raise ValueError(f"{what} must be a 2-D {np.dtype(dtype).name} array")
+        n, k = t.shape
+        s0, s1 = t.strides
+        if t.size and ((k > 1 and s1 != t.itemsize) or (n > 1 and (s0 < 0 or s0 % t.itemsize))):
+            raise ValueError(f"{what} must have column stride 1 and a positive row stride (got strides {t.strides} in bytes)")
+        if writable and not t.flags.writeable:
+            raise ValueError(f"{what} must be writable")
+        ld, addr = (s0 // t.itemsize if n > 1 and t.size else k), t.ctypes.data
+    elif isinstance(t, torch.Tensor):
+        if t.device.type != "cpu" or t.dtype != getattr(torch, np.dtype(dtype).name) or t.dim() != 2:
+            raise ValueError(f"{what} must be a 2-D {np.dtype(dtype).name} CPU tensor")
+        n, k = t.shape
+        if t.numel() and k > 1 and t.stride(1) != 1:
+            raise ValueError(f"{what} must have column stride 1 (got strides {t.stride()})")
+        ld, addr = (t.stride(0) if n > 1 and t.numel() else k), t.data_ptr()
+    else:
+        raise ValueError(f"{what} must be a numpy array or a CPU torch tensor")
+    if n != rows:
+        raise ValueError(f"{what} must have {rows} rows (got shape {tuple(t.shape)})")
+    if ld < k:
+        raise ValueError(f"{what} must have a row stride of at least {k} elements (got {ld})")
+    return k, ld, addr or _NO_ROWS.ctypes.data  # an empty torch tensor has no address; its rows are never read
+
+
+_NO_ROWS = np.zeros(1)
+
+
+def _host_spmm_operands(X, Y, M, N_, dtype):
+    """Checks X (N_ x k) and Y (M x k, allocated like X when None: numpy, or a torch tensor pinned when X is) of a
+    host-buffer product.  Returns (Y, k, ldx, x address, ldy, y address)."""
+    import torch
+    k, ldx, px = _check_host_dense(X, N_, "X", dtype)
+    if Y is None:
+        if isinstance(X, np.ndarray):
+            Y = np.zeros((M, k), dtype)
+        else:
+            Y = torch.zeros((M, k), dtype=X.dtype, pin_memory=X.is_pinned())
+    ky, ldy, py = _check_host_dense(Y, M, "Y", dtype, writable=True)
+    if ky != k:
+        raise ValueError(f"X and Y must have the same number of columns (got {k} and {ky})")
+    if _block_overlap(px, N_, ldx, py, M, ldy, k, np.dtype(dtype).itemsize):
+        raise ValueError("Y must not overlap X")
+    return Y, k, ldx, px, ldy, py
 
 
 FORMAT_CSR, FORMAT_HLL = 0, 1
@@ -335,6 +393,18 @@ class DeviceCSR:
         """Same, on raw host addresses (e.g. pinned torch tensors' data_ptr())."""
         N.check(N.lib().spmv_b200_csr_spmv_host(self._h, C.c_void_p(x_ptr), C.c_void_p(y_ptr), int(bool(accumulate)), algo))
 
+    def spmm_host(self, X, Y=None, accumulate=False):
+        """Y = A X (or Y += A X) on host buffers, synchronous (spmv_b200_csr_spmm_host): X of shape (N, k) and Y of
+        shape (M, k), float64 numpy arrays or CPU torch tensors with column stride 1 and row stride >= k (views such as
+        big[:, :k] work).  Y is written in place, or allocated like X when None; pinned tensors give the overlap of the
+        uploads, products and downloads.  Every column has the bits of spmm on the same handle.  Raises ValueError
+        before any call on a bad or overlapping operand.  Returns Y."""
+        i = self.info()
+        Y, k, ldx, px, ldy, py = _host_spmm_operands(X, Y, i.M, i.N, np.float64)
+        if k and i.M:
+            N.check(N.lib().spmv_b200_csr_spmm_host(self._h, k, C.c_void_p(px), ldx, C.c_void_p(py), ldy, int(bool(accumulate))))
+        return Y
+
     # -- fp32 storage, fp64 arithmetic (SURVEY.md section 8(f).3) ----------------------------------------------
     def enable_f32(self, stream=None):
         N.check(N.lib().spmv_b200_csr_enable_f32(self._h, _stream(stream)))
@@ -367,6 +437,15 @@ class DeviceCSR:
         x, y = _host_vectors(x, y, i.N, i.M, np.float32)
         N.check(N.lib().spmv_b200_csr_spmv_host_f32(self._h, _ptr(x), _ptr(y)))
         return y
+
+    def spmm_host_f32(self, X, Y=None, accumulate=False):
+        """spmm_host on float32 buffers through the float copy of the values (enabled by the call itself): the bits of
+        spmm_f32 on the same handle (spmv_b200_csr_spmm_host_f32).  Returns Y."""
+        i = self.info()
+        Y, k, ldx, px, ldy, py = _host_spmm_operands(X, Y, i.M, i.N, np.float32)
+        if k and i.M:
+            N.check(N.lib().spmv_b200_csr_spmm_host_f32(self._h, k, C.c_void_p(px), ldx, C.c_void_p(py), ldy, int(bool(accumulate))))
+        return Y
 
     def algorithmic_bytes_f32(self) -> int:
         i = self.info()
@@ -480,6 +559,14 @@ class DeviceHLL:
         N.check(N.lib().spmv_b200_hll_spmv_host_f32(self._h, _ptr(x), _ptr(y)))
         return y
 
+    def spmm_host_f32(self, X, Y=None):
+        """spmm_host on float32 buffers (spmv_b200_hll_spmm_host_f32): the bits of spmm_f32 on the same handle."""
+        i = self.info()
+        Y, k, ldx, px, ldy, py = _host_spmm_operands(X, Y, i.M, i.N, np.float32)
+        if k and i.M:
+            N.check(N.lib().spmv_b200_hll_spmm_host_f32(self._h, k, C.c_void_p(px), ldx, C.c_void_p(py), ldy))
+        return Y
+
     def algorithmic_bytes_f32(self) -> int:
         i = self.info()
         return 8 * i.slots + 8 * (i.num_hacks + 1) + 4 * i.M + 4 * i.N
@@ -527,6 +614,15 @@ class DeviceHLL:
 
     def spmv_host_ptr(self, x_ptr: int, y_ptr: int):
         N.check(N.lib().spmv_b200_hll_spmv_host(self._h, C.c_void_p(x_ptr), C.c_void_p(y_ptr)))
+
+    def spmm_host(self, X, Y=None):
+        """Y = A X on host buffers, as DeviceCSR.spmm_host (spmv_b200_hll_spmm_host): the bits of spmm on the same
+        handle.  No accumulate flag.  Returns Y."""
+        i = self.info()
+        Y, k, ldx, px, ldy, py = _host_spmm_operands(X, Y, i.M, i.N, np.float64)
+        if k and i.M:
+            N.check(N.lib().spmv_b200_hll_spmm_host(self._h, k, C.c_void_p(px), ldx, C.c_void_p(py), ldy))
+        return Y
 
     def close(self):
         if self._h:
